@@ -4,6 +4,9 @@
     python bench.py --gpus N --steps K --warmup W            # this framework, N B200s
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm (oracle port of the reference)
     torchrun ... bench.py --gpus N ...                        # one rank per GPU (N > 1)
+    python bench.py ... --dump-outputs DIR                    # also save the last timed step's output
+
+The frames of the timed workload are seeded: the same arguments give the same frames on every run.
 
 A step = one pass of full-frame rectification over one batch of synthetic frames:
   workload c2 (default): 64 frames 1080x1920 single-channel fp32 (BASELINE configs[1])
@@ -158,6 +161,28 @@ def pinned_array(cc, shape, dtype):
     return np.frombuffer(buf, dtype=dtype).reshape(shape), p
 
 
+DUMP_MAX_ELEMS = 4 << 20        # 16 MB of float32 per dumped file
+
+
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: every array as <out_dir>/<name>.npy in float32, flattened.  One larger than
+    DUMP_MAX_ELEMS is reduced to a fixed sample (seed 0, sorted flat indices), the same for every run
+    of the same workload, so that the outputs of two builds can be compared element for element.
+    Every file holds finite numbers only: a NaN (the fill of a float frame's pixels that map outside
+    the source) is written as 0, and <name>_nonfinite.npy is 1.0 where the output was not finite."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        flat = t.reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), DUMP_MAX_ELEMS))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        vals = flat.float().cpu().numpy()
+        bad = ~np.isfinite(vals)
+        np.save(os.path.join(out_dir, name + ".npy"), np.where(bad, np.float32(0), vals))
+        np.save(os.path.join(out_dir, name + "_nonfinite.npy"), bad.astype(np.float32))
+
+
 def cpu_port(wl, nframes, nthreads, ratio, axs, steps=1, warmup=0):
     """The oracle restatement of the reference's warp on the host cores (checker code used
     only as the reported CPU baseline)."""
@@ -193,7 +218,15 @@ def main():
     ap.add_argument("--gather", default="auto", choices=["auto", "direct", "tma"])
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary workloads")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the output of the last timed step to DIR/rectified.npy (float32; a fixed "
+                         "sample of 4M elements of rank 0's frames, non-finite values as 0) and where it was "
+                         "not finite to DIR/rectified_nonfinite.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm sizes its sample from the host's speed)")
     args.warmup = max(args.warmup, 3)
     wl = WORKLOADS[args.workload]
     sz = wl["sz"]
@@ -293,6 +326,8 @@ def main():
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
     total_ms = float(tmax.item())
     value = world * npx * args.steps / (total_ms * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"rectified": dst})
 
     # in-bounds fraction of the output (what share of the counted source bytes is really read)
     if wl["u8"]:
