@@ -478,8 +478,10 @@ def test_rectify_bounds_checked_build(cc):
     if os.environ.get("CAMCAL_B200_LIB"):
         pytest.skip("already running against a variant library")
     env = dict(os.environ, CAMCAL_B200_LIB=lib)
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_parity.py"), "-x", "-q", "-m", "gpu",
-                        "-k", "bit_exact or tilted or horizon or views_is or views_one_launch or alternating or strided"],
+    # "batching" selects all of test_gpu_batching.py: frame groups, pair kernels, views with several groups per view
+    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(root, "tests", "test_gpu_parity.py"),
+                        os.path.join(root, "tests", "test_gpu_batching.py"), "-x", "-q", "-m", "gpu",
+                        "-k", "bit_exact or tilted or horizon or views_is or views_one_launch or alternating or strided or batching"],
                        env=env, capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
     assert " passed" in r.stdout
