@@ -60,6 +60,7 @@ class Calibration:
         self.files = list(files)
         self._intr = _lib.make_intr(frow, fcol, crow, ccol, self.k, 1.0 / self.scale)
         self._views = [_lib.make_view(r, t) for r, t in self.extrinsics]
+        self._view_rows = np.array([r + t for r, t in self.extrinsics], dtype=np.float64).reshape(-1, 6)
 
     # -- construction from fit results: obj2img, src/buildcalibrations.jl:1-6
     @classmethod
@@ -96,8 +97,42 @@ class Calibration:
         ins = (x, y) if z is None else (x, y, z)
         return _point_call("world2img", self, vi, ins, 2, z is not None)
 
+    # -- points of many views in one call: c.(pts_v, v) over views v ----------------
+    def img2world_views(self, row, col, extrinsics, counts, want_z: bool = True):
+        """Pixel -> world for consecutive segments of points with their own views: points
+        [sum(counts[:s]), sum(counts[:s+1])) use extrinsics[s] (view indices or file names, as
+        warp_views takes them).  One call (one launch for CUDA tensors); every point's result is
+        bit-identical to img2world with its segment's view."""
+        return _point_call("img2world", self, self._segments(extrinsics, counts), (row, col),
+                           3 if want_z else 2, want_z)
+
+    def world2img_views(self, x, y, z, extrinsics, counts):
+        """World -> pixel over segments of views, as img2world_views; z=None means z = 0."""
+        ins = (x, y) if z is None else (x, y, z)
+        return _point_call("world2img", self, self._segments(extrinsics, counts), ins, 2, z is not None)
+
+    def _segments(self, extrinsics, counts):
+        """(views, nviews, offsets) of cc_*_views as numpy arrays: cc_view rows [rvec | tvec] and size_t
+        offsets.  Built without a Python loop when the extrinsics are integers (10 000 views are common)."""
+        vis = np.asarray(extrinsics)
+        if vis.dtype.kind not in "iu":                    # file names or None: one at a time
+            vis = np.asarray([self._index(e) for e in extrinsics], dtype=np.int64)
+        elif vis.size and (vis.min() < 0 or vis.max() >= len(self._views)):
+            bad = int(vis[(vis < 0) | (vis >= len(self._views))][0])
+            raise IndexError(f"extrinsic index {bad} out of range 0:{len(self._views)}")  # BoundsError
+        counts = np.asarray(counts, dtype=np.int64).reshape(-1)
+        if vis.ndim != 1 or len(vis) != len(counts) or not len(vis):
+            raise ValueError("need one count per extrinsic, and at least one")
+        if counts.min() < 0:
+            raise ValueError("counts must be non-negative")
+        offsets = np.zeros(len(counts) + 1, dtype=np.uint64)
+        np.cumsum(counts, out=offsets[1:], dtype=np.uint64)
+        return np.ascontiguousarray(self._view_rows[vis]), len(vis), offsets
+
     # -- the reference's callable: dispatch on RowCol (.., 2) vs XYZ (.., 3) -------
     def __call__(self, pts, extrinsic=None):
+        if isinstance(extrinsic, (list, tuple)):
+            return self._call_views(pts, extrinsic)
         if _is_torch(pts):
             cols = [pts[..., i].contiguous().reshape(-1) for i in range(pts.shape[-1])]
             stack = lambda outs: torch.stack(outs, dim=-1).reshape(*pts.shape[:-1], len(outs))
@@ -112,6 +147,32 @@ class Calibration:
         if len(cols) == 3:
             return stack(list(self.world2img(cols[0], cols[1], cols[2], extrinsic)))
         raise TypeError("points must be RowCol (.., 2) or XYZ (.., 3)")
+
+    def _call_views(self, pts, extrinsics):
+        """c(list of (n_i, 2 | 3) arrays, list of extrinsics): one call over all of them, the list of
+        per-view results back."""
+        if len(pts) != len(extrinsics):
+            raise ValueError("need one point array per extrinsic")
+        is_t = bool(pts) and _is_torch(pts[0])
+        if is_t:
+            pts = [p.reshape(-1, p.shape[-1]) for p in pts]
+            cat = lambda cols: torch.cat(cols).contiguous()
+        else:
+            pts = [np.asarray(p) for p in pts]
+            dt = np.float32 if pts and all(p.dtype == np.float32 for p in pts) else np.float64
+            pts = [p.astype(dt, copy=False).reshape(-1, p.shape[-1]) for p in pts]
+            cat = lambda cols: np.ascontiguousarray(np.concatenate(cols))
+        dims = {p.shape[-1] for p in pts}
+        if len(dims) != 1 or not dims <= {2, 3}:
+            raise TypeError("points must all be RowCol (n, 2) or all XYZ (n, 3)")
+        d = dims.pop()
+        counts = [int(p.shape[0]) for p in pts]
+        cols = [cat([p[:, i] for p in pts]) for i in range(d)]
+        outs = (self.img2world_views(cols[0], cols[1], extrinsics, counts) if d == 2
+                else self.world2img_views(cols[0], cols[1], cols[2], extrinsics, counts))
+        stacked = torch.stack(outs, dim=-1) if is_t else np.stack(outs, axis=-1)
+        bounds = np.cumsum([0] + counts)
+        return [stacked[int(a):int(b)] for a, b in zip(bounds[:-1], bounds[1:])]
 
 
 def rectification(c: Calibration, extrinsic=None):
@@ -131,10 +192,13 @@ def rectification(c: Calibration, extrinsic=None):
     return f
 
 
-def _point_call(kind, c: Calibration, vi: int, ins, nout: int, flag: bool):
-    """kind: img2world (ins=row,col; outs x,y[,z]) or world2img (ins=x,y[,z]; outs row,col)."""
+def _point_call(kind, c: Calibration, vi, ins, nout: int, flag: bool):
+    """kind: img2world (ins=row,col; outs x,y[,z]) or world2img (ins=x,y[,z]; outs row,col).
+    vi: a view index, or the (views, nviews, offsets) of Calibration._segments for cc_*_views."""
     first = ins[0]
-    intr, view = C.byref(c._intr), C.byref(c._views[vi])
+    segs = isinstance(vi, tuple)     # the views form takes its point count from the offsets
+    head = (C.byref(c._intr),) + ((_np_ptr(vi[0]), vi[1], _np_ptr(vi[2])) if segs else (C.byref(c._views[vi]),))
+    sfx_v = "_views" if segs else ""
     if _is_torch(first):
         if not first.is_cuda:
             raise TypeError("torch inputs must be CUDA tensors (numpy arrays take the host path)")
@@ -150,14 +214,15 @@ def _point_call(kind, c: Calibration, vi: int, ins, nout: int, flag: bool):
         dev = first.device.index if first.device.index is not None else torch.cuda.current_device()
         ctx = _lib.context(dev)
         sfx = "f64" if dt == torch.float64 else "f32"
-        fn = getattr(lib, f"cc_{kind}_{sfx}")
+        fn = getattr(lib, f"cc_{kind}_{sfx}{sfx_v}")
         if kind == "img2world":
             args = [_t_ptr(ins[0]), _t_ptr(ins[1]), _t_ptr(outs[0]), _t_ptr(outs[1]),
                     _t_ptr(outs[2]) if flag else None]
         else:
             args = [_t_ptr(ins[0]), _t_ptr(ins[1]), _t_ptr(ins[2]) if flag else None,
                     _t_ptr(outs[0]), _t_ptr(outs[1])]
-        check(fn(ctx.handle, intr, view, *args, C.c_size_t(n), _stream_ptr(dev)))
+        _check_total(vi, n, segs)
+        check(fn(ctx.handle, *head, *args, *(() if segs else (C.c_size_t(n),)), _stream_ptr(dev)))
         return tuple(outs)
     # host path
     arrs = [np.asarray(a) for a in ins]
@@ -170,15 +235,22 @@ def _point_call(kind, c: Calibration, vi: int, ins, nout: int, flag: bool):
     outs = [np.empty(n, dtype=dt) for _ in range(nout)]
     ctx = _lib.context(_default_device())
     sfx = "f64" if dt == np.float64 else "f32"
-    fn = getattr(lib, f"cc_{kind}_{sfx}_host")
+    fn = getattr(lib, f"cc_{kind}_{sfx}{sfx_v}_host")
     if kind == "img2world":
         args = [_np_ptr(arrs[0]), _np_ptr(arrs[1]), _np_ptr(outs[0]), _np_ptr(outs[1]),
                 _np_ptr(outs[2]) if flag else None]
     else:
         args = [_np_ptr(arrs[0]), _np_ptr(arrs[1]), _np_ptr(arrs[2]) if flag else None,
                 _np_ptr(outs[0]), _np_ptr(outs[1])]
-    check(fn(ctx.handle, intr, view, *args, C.c_size_t(n)))
+    _check_total(vi, n, segs)
+    check(fn(ctx.handle, *head, *args, *(() if segs else (C.c_size_t(n),))))
     return tuple(outs)
+
+
+def _check_total(vi, n: int, segs: bool) -> None:
+    """The library takes the point count from the offsets: they must cover the arrays exactly."""
+    if segs and int(vi[2][-1]) != n:
+        raise ValueError(f"counts sum to {int(vi[2][-1])}, the point arrays hold {n}")
 
 
 def _default_device() -> int:

@@ -34,6 +34,15 @@ template <typename T>
 int launch_img2world(cc_ctx*, const ChainD&, const T*, const T*, T*, T*, T*, size_t, cudaStream_t);
 template <typename T>
 int launch_world2img(cc_ctx*, const ChainD&, const T*, const T*, const T*, T*, T*, size_t, cudaStream_t);
+template <typename T>
+int point_table_upload(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
+int point_table_release(cc_ctx*, cudaStream_t);
+template <typename T>
+int launch_img2world_views(cc_ctx*, const PointTable&, size_t, int, int, const T*, const T*, T*, T*, T*, size_t,
+                           cudaStream_t);
+template <typename T>
+int launch_world2img_views(cc_ctx*, const PointTable&, size_t, int, int, const T*, const T*, const T*, T*, T*,
+                           size_t, cudaStream_t);
 int check_rect_args(const int64_t axs_min[2], int sz1, int sz2, size_t pitch, size_t frame_stride,
                     int nframes, double ratio);
 int launch_rectify_f32c1(cc_ctx*, const ChainD&, double, const int64_t[2], const float*, float*, int,
@@ -186,6 +195,152 @@ static int world2img_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view,
     return drain(ctx);
 }
 
+// ---- points of many views in one call -----------------------------------------------------------
+// Points [offsets[s], offsets[s+1]) use views[s].  Checks everything before anything is written;
+// *n = offsets[nviews].
+static int check_views(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                       const size_t* offsets, size_t* n) {
+    CC_REQUIRE(ctx != nullptr, "ctx is NULL");
+    CC_REQUIRE(nviews >= 1, "nviews must be at least 1");
+    CC_REQUIRE(views != nullptr && offsets != nullptr, "views / offsets is NULL");
+    CC_REQUIRE(offsets[0] == 0, "offsets[0] must be 0");
+    for (int s = 0; s < nviews; ++s) CC_REQUIRE(offsets[s + 1] >= offsets[s], "offsets must not decrease");
+    *n = offsets[nviews];
+    return check_params(ctx, intr, views);
+}
+
+// The chains are expanded on the host, one per segment, exactly as the single-view entry points do:
+// every point's result is bit-identical to a single-view call with its own view.
+static std::vector<ChainD> view_chains(const cc_intr* intr, const cc_view* views, int nviews) {
+    std::vector<ChainD> chs((size_t)nviews);
+    for (int s = 0; s < nviews; ++s) build_chain(intr, views + s, &chs[s]);
+    return chs;
+}
+
+// Device form: one table upload and ONE launch on `st`, whatever nviews is.  IN / OUT: 2 + 3 arrays
+// (img2world) or 3 + 2 (world2img); LAUNCH runs the kernel over points base + [0, m) of segments [lo, hi).
+template <typename T, typename LAUNCH>
+static int views_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                        size_t n, bool to_img, cudaStream_t st, LAUNCH launch) {
+    int rc;
+    CC_GUARD;
+    if ((rc = enter(ctx))) return rc;
+    if (n == 0) return CC_OK;
+    const std::vector<ChainD> chs = view_chains(intr, views, nviews);
+    PointTable tb;
+    if ((rc = point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, st, &tb))) return rc;
+    rc = launch(tb, st);
+    const int rr = point_table_release(ctx, st);
+    return rc ? rc : rr;
+}
+
+// Host form: the table goes up once on slot 0's stream, every slot's stream waits for it, then the chunk
+// pipeline of the single-view *_host calls runs with one drain at the end.  A chunk's launch gets the
+// segments it covers and its first point's index in the call.  CHUNK(tb, k, off, m, lo, hi, cap) moves
+// and maps points [off, off + m) through slot k.
+template <typename T, typename CHUNK>
+static int views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                      size_t n, bool to_img, size_t in_arrays, size_t out_arrays, CHUNK chunk) {
+    int rc;
+    CC_GUARD;
+    if ((rc = enter(ctx))) return rc;
+    if (n == 0) return CC_OK;
+    const std::vector<ChainD> chs = view_chains(intr, views, nviews);
+    if ((rc = ensure_stream(ctx, 0))) return rc;
+    PointTable tb;
+    if ((rc = point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, ctx->pipe_stream[0], &tb))) return rc;
+    if ((rc = point_table_release(ctx, ctx->pipe_stream[0]))) return rc;
+    const size_t cap = n < kPointChunk ? round_up(n, 64) : kPointChunk;
+    const size_t nchunks = (n + cap - 1) / cap;
+    for (int k = 1; k < cc_ctx::NSLOT && (size_t)k < nchunks; ++k) {
+        if ((rc = ensure_stream(ctx, k))) return rc;
+        CC_CUDA(cudaStreamWaitEvent(ctx->pipe_stream[k], ctx->pt_event, 0));
+    }
+    size_t off = 0;
+    for (int it = 0; rc == CC_OK && off < n; ++it, off += cap) {
+        const int k = it % cc_ctx::NSLOT;
+        const size_t m = (n - off) < cap ? (n - off) : cap;
+        const int lo = (int)(std::upper_bound(offsets, offsets + nviews + 1, off) - offsets) - 1;
+        const int hi = (int)(std::upper_bound(offsets, offsets + nviews + 1, off + m - 1) - offsets);
+        if ((rc = ensure_slot(ctx, k, in_arrays * cap * sizeof(T), out_arrays * cap * sizeof(T)))) break;
+        rc = chunk(tb, k, off, m, lo, hi, cap);
+    }
+    const int rd = drain(ctx);                     // the table's readers are done before the call returns
+    return rc ? rc : rd;
+}
+
+template <typename T>
+static int img2world_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                           const size_t* offsets, const T* row, const T* col, T* x, T* y, T* z, cudaStream_t st) {
+    size_t n = 0;
+    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
+    if (rc) return rc;
+    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
+    return views_device<T>(ctx, intr, views, nviews, offsets, n, false, st, [&](const PointTable& tb, cudaStream_t s) {
+        return launch_img2world_views<T>(ctx, tb, 0, 0, nviews, row, col, x, y, z, n, s);
+    });
+}
+
+template <typename T>
+static int world2img_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                           const size_t* offsets, const T* x, const T* y, const T* z, T* row, T* col, cudaStream_t st) {
+    size_t n = 0;
+    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
+    if (rc) return rc;
+    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
+    return views_device<T>(ctx, intr, views, nviews, offsets, n, true, st, [&](const PointTable& tb, cudaStream_t s) {
+        return launch_world2img_views<T>(ctx, tb, 0, 0, nviews, x, y, z, row, col, n, s);
+    });
+}
+
+template <typename T>
+static int img2world_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const size_t* offsets, const T* row, const T* col, T* x, T* y, T* z) {
+    size_t n = 0;
+    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
+    if (rc) return rc;
+    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
+    return views_host<T>(ctx, intr, views, nviews, offsets, n, false, 2, 3,
+                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t cap) {
+        cudaStream_t st = ctx->pipe_stream[k];
+        T* din = static_cast<T*>(ctx->pipe_in[k]);
+        T* dout = static_cast<T*>(ctx->pipe_out[k]);
+        CC_CUDA(cudaMemcpyAsync(din, row + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
+        CC_CUDA(cudaMemcpyAsync(din + cap, col + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
+        int r = launch_img2world_views<T>(ctx, tb, off, lo, hi, din, din + cap, dout, dout + cap,
+                                          z ? dout + 2 * cap : nullptr, m, st);
+        if (r) return r;
+        CC_CUDA(cudaMemcpyAsync(x + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        CC_CUDA(cudaMemcpyAsync(y + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        if (z) CC_CUDA(cudaMemcpyAsync(z + off, dout + 2 * cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        return (int)CC_OK;
+    });
+}
+
+template <typename T>
+static int world2img_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const size_t* offsets, const T* x, const T* y, const T* z, T* row, T* col) {
+    size_t n = 0;
+    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
+    if (rc) return rc;
+    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
+    return views_host<T>(ctx, intr, views, nviews, offsets, n, true, 3, 2,
+                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t cap) {
+        cudaStream_t st = ctx->pipe_stream[k];
+        T* din = static_cast<T*>(ctx->pipe_in[k]);
+        T* dout = static_cast<T*>(ctx->pipe_out[k]);
+        CC_CUDA(cudaMemcpyAsync(din, x + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
+        CC_CUDA(cudaMemcpyAsync(din + cap, y + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
+        if (z) CC_CUDA(cudaMemcpyAsync(din + 2 * cap, z + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
+        int r = launch_world2img_views<T>(ctx, tb, off, lo, hi, din, din + cap, z ? din + 2 * cap : nullptr,
+                                          dout, dout + cap, m, st);
+        if (r) return r;
+        CC_CUDA(cudaMemcpyAsync(row + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        CC_CUDA(cudaMemcpyAsync(col + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        return (int)CC_OK;
+    });
+}
+
 // frames: chunk = a few whole frames (~32 MB per stage)
 template <typename PX, typename LAUNCH>
 static int rectify_host(cc_ctx* ctx, const PX* src, PX* dst, int sz1, int sz2, size_t pitch,
@@ -302,6 +457,7 @@ int cc_ctx_destroy(cc_ctx* ctx) {
     rectify_free_plans(ctx);
     rectify_free_sched(ctx);
     ingest_free(ctx);
+    point_table_free(ctx);
     delete ctx;
     return CC_OK;
 }
@@ -397,6 +553,43 @@ int cc_world2img_f64_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view,
 int cc_world2img_f32_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const float* x,
                           const float* y, const float* z, float* row, float* col, size_t n) {
     return world2img_host<float>(ctx, intr, view, x, y, z, row, col, n);
+}
+
+int cc_img2world_f64_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                           const double* row, const double* col, double* x, double* y, double* z, void* stream) {
+    return img2world_views<double>(ctx, intr, views, nviews, offsets, row, col, x, y, z, (cudaStream_t)stream);
+}
+int cc_img2world_f32_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                           const float* row, const float* col, float* x, float* y, float* z, void* stream) {
+    return img2world_views<float>(ctx, intr, views, nviews, offsets, row, col, x, y, z, (cudaStream_t)stream);
+}
+int cc_world2img_f64_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                           const double* x, const double* y, const double* z, double* row, double* col, void* stream) {
+    return world2img_views<double>(ctx, intr, views, nviews, offsets, x, y, z, row, col, (cudaStream_t)stream);
+}
+int cc_world2img_f32_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                           const float* x, const float* y, const float* z, float* row, float* col, void* stream) {
+    return world2img_views<float>(ctx, intr, views, nviews, offsets, x, y, z, row, col, (cudaStream_t)stream);
+}
+int cc_img2world_f64_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const size_t* offsets, const double* row, const double* col, double* x, double* y,
+                                double* z) {
+    return img2world_views_host<double>(ctx, intr, views, nviews, offsets, row, col, x, y, z);
+}
+int cc_img2world_f32_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const size_t* offsets, const float* row, const float* col, float* x, float* y,
+                                float* z) {
+    return img2world_views_host<float>(ctx, intr, views, nviews, offsets, row, col, x, y, z);
+}
+int cc_world2img_f64_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const size_t* offsets, const double* x, const double* y, const double* z,
+                                double* row, double* col) {
+    return world2img_views_host<double>(ctx, intr, views, nviews, offsets, x, y, z, row, col);
+}
+int cc_world2img_f32_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const size_t* offsets, const float* x, const float* y, const float* z,
+                                float* row, float* col) {
+    return world2img_views_host<float>(ctx, intr, views, nviews, offsets, x, y, z, row, col);
 }
 
 // ---- rectification ---------------------------------------------------------------

@@ -36,6 +36,12 @@ int jpeg_decode_u8c3(struct ::cc_ctx* ctx, const uint8_t* const* jpegs, const si
                      int sz1, int sz2, size_t pitch, size_t frame_stride, cudaStream_t st);
 void comm_free(struct ::cc_ctx* ctx);
 void lm_free_workspace(struct ::cc_ctx* ctx);
+void point_table_free(struct ::cc_ctx* ctx);
+// the device chain table of the multi-view point maps (pointmap.cu): rows, then segment offsets
+struct PointTable {
+    const void* rows;
+    const size_t* off;
+};
 
 // error plumbing (abi.cu)
 int set_error(int status, const char* fmt, ...);
@@ -88,6 +94,17 @@ struct cc_ctx {
     void* lm_ws;
     // nvJPEG handle / state / raster scratch of the image ingest (ingest.cu: Ingest), created on first use
     void* ingest;
+    // chain table of the multi-view point maps (pointmap.cu: point_table_upload), grown on demand; a call
+    // on a stream other than the previous user's waits for pt_event, recorded after that user's kernels
+    void* pt_table;
+    size_t pt_table_bytes;
+    cudaEvent_t pt_event;
+    cudaStream_t pt_stream;
+    int pt_used;
+    // pinned staging of the table upload; pt_stage_event: the last upload out of it has completed
+    void* pt_stage;
+    size_t pt_stage_bytes;
+    cudaEvent_t pt_stage_event;
 };
 
 #define CC_CUDA(call)                                                     \

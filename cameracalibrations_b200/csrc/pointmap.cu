@@ -9,6 +9,9 @@
 // independent vectors in flight per thread.  Algorithmic bytes per point:
 // img2world 40 B (f64) / 20 B (f32), 32 / 16 B without z; world2img 40 / 20 B
 // (32 / 16 B when z == NULL).
+#include <cstring>
+#include <type_traits>
+
 #include "chain_device.cuh"
 
 namespace cc {
@@ -26,23 +29,73 @@ template <> __device__ __forceinline__ float& lane<float>(float4& v, int i) {
 constexpr int kThreads = 256;
 constexpr int kUnroll = 2;
 
-template <typename T, bool HAS_Z>
-__global__ void __launch_bounds__(kThreads)
-img2world_kernel(const Chain<T> ch, const T* __restrict__ row, const T* __restrict__ col,
-                 T* __restrict__ x, T* __restrict__ y, T* __restrict__ z, size_t n, bool vec_ok) {
+// ---- view sources -------------------------------------------------------------------------------
+// SINGLE: one chain for every point, passed by value (constant bank) -- the source is a Chain<T>.
+// TABLE:  per-segment chains in a device table plus segment offsets -- the source is a ViewTable<Row>.
+//         Points [off[s], off[s+1]) use segment s; a launch covers points base + [0, n).
+//
+// The table stores only the fields of Chain<T> its direction reads (18 values instead of 35).
+template <typename T> struct RowW2I { T R[9], t[3], k, frow, fcol, crow, ccol, inv_cs; };
+template <typename T> struct RowI2W { T a_row, b_row, a_col, b_col, k, Rinv[9], tinv[3], cs_back; };
+
+template <typename T> __host__ __device__ __forceinline__ void pack(const Chain<T>& c, RowW2I<T>& r) {
+    for (int i = 0; i < 9; ++i) r.R[i] = c.R[i];
+    for (int i = 0; i < 3; ++i) r.t[i] = c.t[i];
+    r.k = c.k; r.frow = c.frow; r.fcol = c.fcol; r.crow = c.crow; r.ccol = c.ccol; r.inv_cs = c.inv_cs;
+}
+template <typename T> __host__ __device__ __forceinline__ void pack(const Chain<T>& c, RowI2W<T>& r) {
+    r.a_row = c.a_row; r.b_row = c.b_row; r.a_col = c.a_col; r.b_col = c.b_col; r.k = c.k;
+    for (int i = 0; i < 9; ++i) r.Rinv[i] = c.Rinv[i];
+    for (int i = 0; i < 3; ++i) r.tinv[i] = c.tinv[i];
+    r.cs_back = c.cs_back;
+}
+// the fields world2img / img2world do not read are left unset
+template <typename T> __device__ __forceinline__ void unpack(const RowW2I<T>& r, Chain<T>& c) {
+#pragma unroll
+    for (int i = 0; i < 9; ++i) c.R[i] = r.R[i];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) c.t[i] = r.t[i];
+    c.k = r.k; c.frow = r.frow; c.fcol = r.fcol; c.crow = r.crow; c.ccol = r.ccol; c.inv_cs = r.inv_cs;
+}
+template <typename T> __device__ __forceinline__ void unpack(const RowI2W<T>& r, Chain<T>& c) {
+    c.a_row = r.a_row; c.b_row = r.b_row; c.a_col = r.a_col; c.b_col = r.b_col; c.k = r.k;
+#pragma unroll
+    for (int i = 0; i < 9; ++i) c.Rinv[i] = r.Rinv[i];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) c.tinv[i] = r.tinv[i];
+    c.cs_back = r.cs_back;
+}
+
+template <typename Row> struct ViewTable {
+    const Row* rows;       // one per segment
+    const size_t* off;     // segment offsets, nseg + 1 entries
+    size_t base;           // index of this launch's point 0 among the call's points
+    int seg_lo, seg_hi;    // the launch's points lie in segments [seg_lo, seg_hi)
+};
+
+template <typename S> struct IsTable : std::false_type {};
+template <typename Row> struct IsTable<ViewTable<Row>> : std::true_type {};
+
+// ---- per-point loops ------------------------------------------------------------------------------
+// Points [p0, p1) (p0 a multiple of N): vectors of N points when vec_ok, thread `tid` of `nthreads`
+// taking vectors tid, tid + nthreads, ... two at a time, then the scalar tail; scalar throughout when
+// !vec_ok.  chain(p) gives the chain of point p, asked for in increasing p within a thread.
+template <typename T, bool HAS_Z, typename CH>
+__device__ __forceinline__ void img2world_range(CH&& chain, const T* __restrict__ row,
+                                                 const T* __restrict__ col, T* __restrict__ x,
+                                                 T* __restrict__ y, T* __restrict__ z, size_t p0,
+                                                 size_t p1, size_t tid, size_t nthreads, bool vec_ok) {
     using V = typename Vec<T>::type;
     constexpr int N = Vec<T>::N;
-    const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
-    const size_t nthreads = (size_t)gridDim.x * kThreads;
-    size_t done = 0;
+    size_t done = p0;
     if (vec_ok) {
-        const size_t nvec = n / N;
+        const size_t nvec = p1 / N;
         const V* rv = reinterpret_cast<const V*>(row);
         const V* cv = reinterpret_cast<const V*>(col);
         V* xv = reinterpret_cast<V*>(x);
         V* yv = reinterpret_cast<V*>(y);
         V* zv = reinterpret_cast<V*>(z);
-        for (size_t i = tid; i < nvec; i += nthreads * kUnroll) {
+        for (size_t i = p0 / N + tid; i < nvec; i += nthreads * kUnroll) {
             V r[kUnroll], c[kUnroll];
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
@@ -56,7 +109,7 @@ img2world_kernel(const Chain<T> ch, const T* __restrict__ row, const T* __restri
                     V ox, oy, oz;
 #pragma unroll
                     for (int e = 0; e < N; ++e)
-                        img2world(ch, lane<T>(r[u], e), lane<T>(c[u], e), lane<T>(ox, e),
+                        img2world(chain(j * N + e), lane<T>(r[u], e), lane<T>(c[u], e), lane<T>(ox, e),
                                   lane<T>(oy, e), lane<T>(oz, e));
                     stg_stream(xv + j, ox);
                     stg_stream(yv + j, oy);
@@ -66,32 +119,30 @@ img2world_kernel(const Chain<T> ch, const T* __restrict__ row, const T* __restri
         }
         done = nvec * N;
     }
-    for (size_t i = done + tid; i < n; i += nthreads) {   // tail / unaligned pointers
+    for (size_t i = done + tid; i < p1; i += nthreads) {   // tail / unaligned pointers
         T ox, oy, oz;
-        img2world(ch, row[i], col[i], ox, oy, oz);
+        img2world(chain(i), row[i], col[i], ox, oy, oz);
         x[i] = ox; y[i] = oy;
         if (HAS_Z) z[i] = oz;
     }
 }
 
-template <typename T, bool HAS_Z>
-__global__ void __launch_bounds__(kThreads)
-world2img_kernel(const Chain<T> ch, const T* __restrict__ x, const T* __restrict__ y,
-                 const T* __restrict__ z, T* __restrict__ row, T* __restrict__ col, size_t n,
-                 bool vec_ok) {
+template <typename T, bool HAS_Z, typename CH>
+__device__ __forceinline__ void world2img_range(CH&& chain, const T* __restrict__ x,
+                                                const T* __restrict__ y, const T* __restrict__ z,
+                                                T* __restrict__ row, T* __restrict__ col, size_t p0,
+                                                size_t p1, size_t tid, size_t nthreads, bool vec_ok) {
     using V = typename Vec<T>::type;
     constexpr int N = Vec<T>::N;
-    const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
-    const size_t nthreads = (size_t)gridDim.x * kThreads;
-    size_t done = 0;
+    size_t done = p0;
     if (vec_ok) {
-        const size_t nvec = n / N;
+        const size_t nvec = p1 / N;
         const V* xv = reinterpret_cast<const V*>(x);
         const V* yv = reinterpret_cast<const V*>(y);
         const V* zv = reinterpret_cast<const V*>(z);
         V* rv = reinterpret_cast<V*>(row);
         V* cv = reinterpret_cast<V*>(col);
-        for (size_t i = tid; i < nvec; i += nthreads * kUnroll) {
+        for (size_t i = p0 / N + tid; i < nvec; i += nthreads * kUnroll) {
             V a[kUnroll], b[kUnroll], c[kUnroll];
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
@@ -109,7 +160,7 @@ world2img_kernel(const Chain<T> ch, const T* __restrict__ x, const T* __restrict
                     V orow, ocol;
 #pragma unroll
                     for (int e = 0; e < N; ++e)
-                        world2img(ch, lane<T>(a[u], e), lane<T>(b[u], e),
+                        world2img(chain(j * N + e), lane<T>(a[u], e), lane<T>(b[u], e),
                                   HAS_Z ? lane<T>(c[u], e) : T(0), lane<T>(orow, e),
                                   lane<T>(ocol, e));
                     stg_stream(rv + j, orow);
@@ -119,10 +170,115 @@ world2img_kernel(const Chain<T> ch, const T* __restrict__ x, const T* __restrict
         }
         done = nvec * N;
     }
-    for (size_t i = done + tid; i < n; i += nthreads) {
+    for (size_t i = done + tid; i < p1; i += nthreads) {
         T orow, ocol;
-        world2img(ch, x[i], y[i], HAS_Z ? z[i] : T(0), orow, ocol);
+        world2img(chain(i), x[i], y[i], HAS_Z ? z[i] : T(0), orow, ocol);
         row[i] = orow; col[i] = ocol;
+    }
+}
+
+// ---- TABLE: tiles of segments ---------------------------------------------------------------------
+// Every CTA of the persistent grid takes a contiguous run of kTile-point tiles (kTile is a multiple
+// of both vector widths, so a tile's vectors stay 16-byte aligned whatever the segment boundaries).
+// Warp 0 finds the tile's first segment; a tile inside one segment (the common case for large
+// segments) runs the single-view loop on that chain, staged in shared memory; a tile that crosses
+// segment boundaries walks a per-thread segment cursor over the offsets and reads each point's chain
+// from the table (L1-resident).  The offsets are never expanded into a per-point index.
+constexpr size_t kTile = 4096;
+
+// First segment s in [lo, hi) with off[s + 1] > p; one exists.  The whole warp calls it.  The first
+// round looks at the 32 segments from lo on (the next tile usually starts in one of them); later
+// rounds split what is left 32 ways.
+__device__ __forceinline__ int find_segment(const size_t* __restrict__ off, int lo, int hi, size_t p) {
+    const int lane = threadIdx.x & 31;
+    for (bool near = true;; near = false) {
+        const int step = (near || hi - lo <= 32) ? 1 : (hi - lo + 31) / 32;
+        const int c = lo + lane * step;
+        const bool after = c >= hi || __ldg(off + c + 1) > p;       // monotone over the lanes
+        const unsigned b = __ballot_sync(0xffffffffu, after);
+        if (b == 0) { lo += 31 * step + 1; continue; }
+        const int L = __ffs(b) - 1;
+        if (step == 1) return lo + L;
+        if (L == 0) return lo;
+        const int nlo = lo + (L - 1) * step + 1;
+        hi = min(hi, lo + L * step + 1);
+        lo = nlo;
+    }
+}
+
+template <typename T, typename Row, typename BODY>
+__device__ __forceinline__ void for_each_tile(const ViewTable<Row>& tb, size_t n, BODY&& body) {
+    __shared__ Chain<T> s_chain[2];        // double-buffered: one barrier per tile
+    __shared__ int s_seg[2];
+    __shared__ int s_inside[2];
+    const size_t ntiles = (n + kTile - 1) / kTile;
+    const size_t per = ntiles / gridDim.x, extra = ntiles % gridDim.x;
+    const size_t t0 = blockIdx.x * per + min((size_t)blockIdx.x, extra);
+    const size_t t1 = t0 + per + (blockIdx.x < extra ? 1 : 0);
+    int lo = tb.seg_lo;
+    for (size_t t = t0; t < t1; ++t) {
+        const int b = (int)(t & 1);
+        const size_t p0 = t * kTile, p1 = min(n, p0 + kTile);
+        if (threadIdx.x < 32) {
+            lo = find_segment(tb.off, lo, tb.seg_hi, tb.base + p0);
+            if (threadIdx.x == 0) {
+                const int inside = __ldg(tb.off + lo + 1) >= tb.base + p1;
+                s_seg[b] = lo;
+                s_inside[b] = inside;
+                if (inside) unpack(tb.rows[lo], s_chain[b]);
+            }
+        }
+        __syncthreads();
+        if (s_inside[b]) {
+            body(p0, p1, [&](size_t) -> const Chain<T>& { return s_chain[b]; });
+        } else {
+            int s = s_seg[b];
+            body(p0, p1, [&](size_t p) {
+                while (__ldg(tb.off + s + 1) <= tb.base + p) ++s;
+                Chain<T> c;
+                unpack(tb.rows[s], c);
+                return c;
+            });
+        }
+    }
+}
+
+// Resident CTAs per SM asked of ptxas: none for SINGLE (its code is what it always was).  For TABLE, 3 where
+// that measured faster on a B200 (1000 W): FP64 pixel->world and FP32 world->pixel (0.72 -> 0.85x and
+// 0.95 -> 1.05x of the single-view rate at 1 segment); it made FP64 world->pixel slower (1.00 -> 0.90x) and
+// left FP32 pixel->world unchanged, so those two keep the compiler's choice.
+template <typename SRC, bool ASK> constexpr int kTableMinBlocks = IsTable<SRC>::value && ASK ? 3 : 0;
+
+template <typename T, bool HAS_Z, typename SRC = Chain<T>>
+__global__ void __launch_bounds__(kThreads, kTableMinBlocks<SRC, std::is_same<T, double>::value>)
+img2world_kernel(const SRC src, const T* __restrict__ row, const T* __restrict__ col,
+                 T* __restrict__ x, T* __restrict__ y, T* __restrict__ z, size_t n, bool vec_ok) {
+    if constexpr (IsTable<SRC>::value) {
+        for_each_tile<T>(src, n, [&](size_t p0, size_t p1, auto&& chain) {
+            img2world_range<T, HAS_Z>(chain, row, col, x, y, z, p0, p1, threadIdx.x, kThreads, vec_ok);
+        });
+    } else {
+        const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
+        const size_t nthreads = (size_t)gridDim.x * kThreads;
+        img2world_range<T, HAS_Z>([&](size_t) -> const Chain<T>& { return src; }, row, col, x, y, z,
+                                  0, n, tid, nthreads, vec_ok);
+    }
+}
+
+template <typename T, bool HAS_Z, typename SRC = Chain<T>>
+__global__ void __launch_bounds__(kThreads, kTableMinBlocks<SRC, std::is_same<T, float>::value>)
+world2img_kernel(const SRC src, const T* __restrict__ x, const T* __restrict__ y,
+                 const T* __restrict__ z, T* __restrict__ row, T* __restrict__ col, size_t n,
+                 bool vec_ok) {
+    if constexpr (IsTable<SRC>::value) {
+        for_each_tile<T>(src, n, [&](size_t p0, size_t p1, auto&& chain) {
+            world2img_range<T, HAS_Z>(chain, x, y, z, row, col, p0, p1, threadIdx.x, kThreads, vec_ok);
+        });
+    } else {
+        const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
+        const size_t nthreads = (size_t)gridDim.x * kThreads;
+        world2img_range<T, HAS_Z>([&](size_t) -> const Chain<T>& { return src; }, x, y, z, row, col,
+                                  0, n, tid, nthreads, vec_ok);
     }
 }
 
@@ -190,6 +346,128 @@ int launch_world2img(cc_ctx* ctx, const ChainD& chd, const T* x, const T* y, con
     CC_CUDA(cudaGetLastError());
     return CC_OK;
 }
+
+// ---- multi-view calls: the device chain table ----------------------------------------------------
+// One table per context: the rows of the call's segments, then its nseg + 1 offsets.  It is
+// uploaded on the caller's stream from pinned staging, grows on demand and is freed with the
+// context.  Calls on different streams of one context may overlap: a call on a stream other than
+// the previous user's waits for the event that user recorded after its last kernel, so the table is
+// never overwritten under a kernel still reading it.  The staging buffer is rewritten only after
+// the previous upload out of it has completed.
+template <typename T>
+int point_table_upload(cc_ctx* ctx, bool to_img, const ChainD* chains, int nseg, const size_t* offsets,
+                       cudaStream_t st, PointTable* out) {
+    const size_t row_bytes = to_img ? sizeof(RowW2I<T>) : sizeof(RowI2W<T>);
+    const size_t rows_bytes = ((size_t)nseg * row_bytes + 15) / 16 * 16;
+    const size_t bytes = rows_bytes + ((size_t)nseg + 1) * sizeof(size_t);
+    if (ctx->pt_stage_event) CC_CUDA(cudaEventSynchronize(ctx->pt_stage_event));
+    else CC_CUDA(cudaEventCreateWithFlags(&ctx->pt_stage_event, cudaEventDisableTiming));
+    if (ctx->pt_stage_bytes < bytes) {
+        if (ctx->pt_stage) CC_CUDA(cudaFreeHost(ctx->pt_stage));
+        ctx->pt_stage = nullptr; ctx->pt_stage_bytes = 0;
+        CC_CUDA(cudaHostAlloc(&ctx->pt_stage, bytes, cudaHostAllocPortable));
+        ctx->pt_stage_bytes = bytes;
+    }
+    uint8_t* h = static_cast<uint8_t*>(ctx->pt_stage);
+    for (int s = 0; s < nseg; ++s) {
+        const Chain<T> c = pick_chain<T>(chains[s]);
+        if (to_img) pack(c, reinterpret_cast<RowW2I<T>*>(h)[s]);
+        else pack(c, reinterpret_cast<RowI2W<T>*>(h)[s]);
+    }
+    memcpy(h + rows_bytes, offsets, ((size_t)nseg + 1) * sizeof(size_t));
+    if (ctx->pt_used && ctx->pt_stream != st) CC_CUDA(cudaStreamWaitEvent(st, ctx->pt_event, 0));
+    if (ctx->pt_table_bytes < bytes) {
+        if (ctx->pt_table) {
+            if (ctx->pt_used) CC_CUDA(cudaEventSynchronize(ctx->pt_event));
+            CC_CUDA(cudaFree(ctx->pt_table));
+        }
+        ctx->pt_table = nullptr; ctx->pt_table_bytes = 0;
+        CC_CUDA(cudaMalloc(&ctx->pt_table, bytes));
+        ctx->pt_table_bytes = bytes;
+    }
+    uint8_t* d = static_cast<uint8_t*>(ctx->pt_table);
+    CC_CUDA(cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, st));
+    CC_CUDA(cudaEventRecord(ctx->pt_stage_event, st));
+    out->rows = d;
+    out->off = reinterpret_cast<const size_t*>(d + rows_bytes);
+    return CC_OK;
+}
+
+// after the call's last kernel that reads the table, on that kernel's stream
+int point_table_release(cc_ctx* ctx, cudaStream_t st) {
+    if (!ctx->pt_event) CC_CUDA(cudaEventCreateWithFlags(&ctx->pt_event, cudaEventDisableTiming));
+    CC_CUDA(cudaEventRecord(ctx->pt_event, st));
+    ctx->pt_stream = st;
+    ctx->pt_used = 1;
+    return CC_OK;
+}
+
+void point_table_free(cc_ctx* ctx) {
+    if (ctx->pt_event) cudaEventSynchronize(ctx->pt_event);
+    if (ctx->pt_stage_event) cudaEventSynchronize(ctx->pt_stage_event);
+    if (ctx->pt_table) cudaFree(ctx->pt_table);
+    if (ctx->pt_stage) cudaFreeHost(ctx->pt_stage);
+    if (ctx->pt_event) cudaEventDestroy(ctx->pt_event);
+    if (ctx->pt_stage_event) cudaEventDestroy(ctx->pt_stage_event);
+}
+
+template <typename K>
+static int grid_tiles(cc_ctx* ctx, K kernel, size_t n) {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0) != cudaSuccess ||
+        per_sm < 1)
+        per_sm = 1;
+    const size_t tiles = (n + kTile - 1) / kTile;
+    const size_t cap = (size_t)ctx->sm_count * per_sm;
+    return (int)(tiles < cap ? tiles : cap);
+}
+
+template <typename T>
+int launch_img2world_views(cc_ctx* ctx, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
+                           const T* row, const T* col, T* x, T* y, T* z, size_t n, cudaStream_t st) {
+    if (n == 0) return CC_OK;
+    using Src = ViewTable<RowI2W<T>>;
+    const Src src{static_cast<const RowI2W<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
+    const bool vec = aligned16(row) && aligned16(col) && aligned16(x) && aligned16(y) &&
+                     (z == nullptr || aligned16(z));
+    if (z) {
+        auto k = img2world_kernel<T, true, Src>;
+        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, row, col, x, y, z, n, vec);
+    } else {
+        auto k = img2world_kernel<T, false, Src>;
+        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, row, col, x, y, z, n, vec);
+    }
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+template <typename T>
+int launch_world2img_views(cc_ctx* ctx, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
+                           const T* x, const T* y, const T* z, T* row, T* col, size_t n, cudaStream_t st) {
+    if (n == 0) return CC_OK;
+    using Src = ViewTable<RowW2I<T>>;
+    const Src src{static_cast<const RowW2I<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
+    const bool vec = aligned16(x) && aligned16(y) && aligned16(row) && aligned16(col) &&
+                     (z == nullptr || aligned16(z));
+    if (z) {
+        auto k = world2img_kernel<T, true, Src>;
+        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, x, y, z, row, col, n, vec);
+    } else {
+        auto k = world2img_kernel<T, false, Src>;
+        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, x, y, z, row, col, n, vec);
+    }
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+template int point_table_upload<double>(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
+template int point_table_upload<float>(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
+template int launch_img2world_views<double>(cc_ctx*, const PointTable&, size_t, int, int, const double*, const double*, double*, double*, double*, size_t, cudaStream_t);
+template int launch_img2world_views<float>(cc_ctx*, const PointTable&, size_t, int, int, const float*, const float*, float*, float*, float*, size_t, cudaStream_t);
+template int launch_world2img_views<double>(cc_ctx*, const PointTable&, size_t, int, int, const double*, const double*, const double*, double*, double*, size_t, cudaStream_t);
+template int launch_world2img_views<float>(cc_ctx*, const PointTable&, size_t, int, int, const float*, const float*, const float*, float*, float*, size_t, cudaStream_t);
 
 template int launch_img2world<double>(cc_ctx*, const ChainD&, const double*, const double*, double*, double*, double*, size_t, cudaStream_t);
 template int launch_img2world<float>(cc_ctx*, const ChainD&, const float*, const float*, float*, float*, float*, size_t, cudaStream_t);

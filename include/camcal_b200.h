@@ -128,6 +128,40 @@ int cc_world2img_f32_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *view,
                           const float *x, const float *y, const float *z, float *row,
                           float *col, size_t n);
 
+/* ---- points of MANY views in one call: the broadcasts c.(pts_v, v) over the views of a calibration
+ *      (src/buildcalibrations.jl:29,46; src/plot_calibration.jl:36-42).  Points
+ *      [offsets[s], offsets[s+1]) use views[s].  offsets: HOST array of nviews + 1 entries,
+ *      offsets[0] == 0, non-decreasing, n = offsets[nviews].  views: HOST array (a view may appear in
+ *      several segments; empty segments are allowed).  Same arithmetic as the single-view entry
+ *      points: every point's result is bit-identical to calling cc_img2world_* / cc_world2img_* with
+ *      its own view.  z == NULL as there.  The device forms upload a per-segment table to the
+ *      context (on `stream`) and make ONE launch whatever nviews is; the *_host forms upload it
+ *      once and run the chunked pipeline.  n == 0: CC_OK, nothing launched. */
+int cc_img2world_f64_views(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                           const size_t *offsets, const double *row, const double *col, double *x,
+                           double *y, double *z, void *stream);
+int cc_img2world_f32_views(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                           const size_t *offsets, const float *row, const float *col, float *x,
+                           float *y, float *z, void *stream);
+int cc_world2img_f64_views(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                           const size_t *offsets, const double *x, const double *y, const double *z,
+                           double *row, double *col, void *stream);
+int cc_world2img_f32_views(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                           const size_t *offsets, const float *x, const float *y, const float *z,
+                           float *row, float *col, void *stream);
+int cc_img2world_f64_views_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                                const size_t *offsets, const double *row, const double *col,
+                                double *x, double *y, double *z);
+int cc_img2world_f32_views_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                                const size_t *offsets, const float *row, const float *col, float *x,
+                                float *y, float *z);
+int cc_world2img_f64_views_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                                const size_t *offsets, const double *x, const double *y,
+                                const double *z, double *row, double *col);
+int cc_world2img_f32_views_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                                const size_t *offsets, const float *x, const float *y, const float *z,
+                                float *row, float *col);
+
 /* ---- full-frame rectification:  warp(img, tform, axs)  src/plot_calibration.jl:40
  *      with tform = real2image[i] o push(.,0) o inv(LinearMap(ratio*I)) (:17-18) and
  *      axs from get_axes (:1-6): output index (I1, I2) = axs_min + (a, b), same size

@@ -125,6 +125,47 @@ function (c::Calibration)(x::Vector{Float64}, y::Vector{Float64}, z::Vector{Floa
     rows, cols
 end
 
+# ---- many views in one call: the broadcasts c.(pts_v, v) over the views, src/buildcalibrations.jl:29,46 ----
+# Points [sum(counts[1:s-1]) + 1, sum(counts[1:s])] use view idxs[s]; one library call (one table upload, one
+# pipeline, one wait) for all of them.  Every point's result equals the single-view method's bit for bit.
+function _offsets(c::Calibration, n::Integer, idxs::AbstractVector{Int}, counts::AbstractVector{<:Integer})
+    @assert length(idxs) == length(counts) >= 1 && all(>=(0), counts) && sum(counts) == n
+    foreach(i -> checkbounds(c.extrinsics, i), idxs)        # BoundsError like the reference
+    Csize_t[0; cumsum(counts)]
+end
+
+"""
+    c(rows, cols, idxs::AbstractVector{Int}, counts) -> (x, y, z)
+
+Pixel -> world for consecutive segments of points, segment s with view `idxs[s]` (host arrays).
+"""
+function (c::Calibration)(rows::Vector{Float64}, cols::Vector{Float64}, idxs::AbstractVector{Int},
+                          counts::AbstractVector{<:Integer})
+    n = length(rows); @assert length(cols) == n
+    offsets = _offsets(c, n, idxs, counts)
+    views = [CcView(c, i) for i in idxs]
+    x, y, z = similar(rows), similar(rows), similar(rows)
+    check(ccall((:cc_img2world_f64_views_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Csize_t}, Ptr{Cdouble}, Ptr{Cdouble},
+                 Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}),
+                context().handle, Ref(CcIntr(c)), views, length(views), offsets, rows, cols, x, y, z))
+    x, y, z
+end
+
+"World -> pixel for consecutive segments of points, segment s with view `idxs[s]` (host arrays)."
+function (c::Calibration)(x::Vector{Float64}, y::Vector{Float64}, z::Vector{Float64}, idxs::AbstractVector{Int},
+                          counts::AbstractVector{<:Integer})
+    n = length(x); @assert length(y) == n && length(z) == n
+    offsets = _offsets(c, n, idxs, counts)
+    views = [CcView(c, i) for i in idxs]
+    rows, cols = similar(x), similar(x)
+    check(ccall((:cc_world2img_f64_views_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Csize_t}, Ptr{Cdouble}, Ptr{Cdouble},
+                 Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}),
+                context().handle, Ref(CcIntr(c)), views, length(views), offsets, x, y, z, rows, cols))
+    rows, cols
+end
+
 # ---- full-frame rectification: warp(img, tform, axs), src/plot_calibration.jl:40 -------------
 # `imgs` is a stack of frames of size (sz1, sz2, nframes): the memory is passed as is (first
 # RowCol axis contiguous).  `ratio` from get_ratio (:8-13), `axs` from get_axes (:1-6).
