@@ -352,17 +352,23 @@ def warp_views(c: Calibration, extrinsics, frames, ratios, axs_mins, fill=None, 
     """Rectify frames that belong to DIFFERENT views in one call -- the loop of the reference's plot
     (src/plot_calibration.jl:36-42: every calibration image with its own extrinsic, ratio, axes).
 
-    extrinsics: view indices / file names, one per group; frames: CUDA tensor (nviews * k, sz2, sz1)
-    float32 or (nviews * k, sz2, sz1, 3) uint8 -- frames [v*k, (v+1)*k) belong to extrinsics[v];
-    ratios[v], axs_mins[v] as returned by image_transformations for that view."""
+    extrinsics: view indices / file names, one per group; frames: (nviews * k, sz2, sz1) float32 or
+    (nviews * k, sz2, sz1, 3) uint8 -- frames [v*k, (v+1)*k) belong to extrinsics[v]; ratios[v], axs_mins[v]
+    as returned by image_transformations for that view.  A CUDA tensor is rectified on its stream; a numpy
+    array takes the host pipeline over all views in one call (cc_rectify_views_*_host) and returns numpy."""
     vis = [c._index(e) for e in extrinsics]
     nv = len(vis)
     flags = {"f64": _lib.COORD_F64, "f32": _lib.COORD_F32}[coord] | {
         "auto": _lib.GATHER_AUTO, "direct": _lib.GATHER_DIRECT, "tma": _lib.GATHER_TMA}[gather]
-    if not _is_torch(frames) or not frames.is_cuda:
-        raise TypeError("warp_views takes CUDA tensors")
-    u8 = frames.dtype == torch.uint8
-    frames = frames.contiguous()
+    is_t = _is_torch(frames)
+    if is_t and not frames.is_cuda:
+        raise TypeError("warp_views takes CUDA tensors or numpy arrays")
+    if is_t:
+        u8 = frames.dtype == torch.uint8
+        frames = frames.contiguous()
+    else:
+        u8 = np.asarray(frames).dtype == np.uint8
+        frames = np.ascontiguousarray(frames, dtype=np.uint8 if u8 else np.float32)
     if frames.ndim != (4 if u8 else 3) or (u8 and frames.shape[-1] != 3) or nv == 0 or frames.shape[0] % nv:
         raise ValueError("frames must be (nviews * k, sz2, sz1) float32 or (nviews * k, sz2, sz1, 3) uint8")
     k, sz2, sz1 = int(frames.shape[0]) // nv, int(frames.shape[1]), int(frames.shape[2])
@@ -370,16 +376,21 @@ def warp_views(c: Calibration, extrinsics, frames, ratios, axs_mins, fill=None, 
     rat = (C.c_double * nv)(*[float(r) for r in ratios])
     axs = (C.c_int64 * (2 * nv))(*[int(a) for am in axs_mins for a in am])
     if out is None:
-        out = torch.empty_like(frames)
-    dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
+        out = torch.empty_like(frames) if is_t else np.empty_like(frames)
     if u8:
         fv = (C.c_uint8 * 3)(*([0, 0, 0] if fill is None else [int(v) for v in fill]))
-        fn = lib.cc_rectify_u8c3_views
     else:
         fv = C.c_float(float("nan") if fill is None else float(fill))
-        fn = lib.cc_rectify_f32c1_views
-    check(fn(_lib.context(dev).handle, C.byref(c._intr), views, nv, rat, axs, _t_ptr(frames), _t_ptr(out), sz1, sz2,
-             C.c_size_t(sz1), C.c_size_t(sz1 * sz2), k, fv, flags, _stream_ptr(dev)))
+    geom = (sz1, sz2, C.c_size_t(sz1), C.c_size_t(sz1 * sz2), k, fv, flags)
+    if is_t:
+        dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
+        fn = lib.cc_rectify_u8c3_views if u8 else lib.cc_rectify_f32c1_views
+        check(fn(_lib.context(dev).handle, C.byref(c._intr), views, nv, rat, axs, _t_ptr(frames), _t_ptr(out), *geom,
+                 _stream_ptr(dev)))
+    else:
+        fn = lib.cc_rectify_views_u8c3_host if u8 else lib.cc_rectify_views_f32c1_host
+        check(fn(_lib.context(_default_device()).handle, C.byref(c._intr), views, nv, rat, axs, _np_ptr(frames),
+                 _np_ptr(out), *geom))
     return out
 
 

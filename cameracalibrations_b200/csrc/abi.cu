@@ -54,6 +54,15 @@ int launch_rectify_f32c1_views(cc_ctx*, const ChainD*, const double*, const int6
 int launch_rectify_u8c3_views(cc_ctx*, const ChainD*, const double*, const int64_t*, int, const uint8_t*, uint8_t*, int,
                               int, size_t, size_t, int, const uint8_t[3], unsigned, cudaStream_t, bool*);
 int rectify_views_per_launch();
+struct RectViewsHost;
+int rect_vh_begin(cc_ctx*, const ChainD*, const double*, const int64_t*, int, int, int, size_t, int, int, bool,
+                  RectViewsHost**);
+int rect_vh_prepare(RectViewsHost*, int);
+int rect_vh_launch_f32c1(RectViewsHost*, int, int, int, const float*, float*, float, unsigned, cudaStream_t, bool*);
+int rect_vh_launch_u8c3(RectViewsHost*, int, int, int, const uint8_t*, uint8_t*, const uint8_t[3], unsigned, cudaStream_t,
+                        bool*);
+void rect_vh_retire(RectViewsHost*, int);
+int rect_vh_end(RectViewsHost*);
 int launch_rectify_map(cc_ctx*, const ChainD&, double, const int64_t[2], double*, double*, int, int,
                        size_t, cudaStream_t);
 int launch_rectify_map_f32(cc_ctx*, const ChainD&, double, const int64_t[2], float*, float*, int, int,
@@ -128,6 +137,8 @@ static int drain(cc_ctx* ctx) {
         if (ctx->pipe_stream[k]) CC_CUDA(cudaStreamSynchronize(ctx->pipe_stream[k]));
     return CC_OK;
 }
+
+static int cuda_check(cudaError_t e, const char* what) { return e == cudaSuccess ? (int)CC_OK : cuda_fail(e, what); }
 
 static size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
@@ -341,6 +352,35 @@ static int world2img_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view*
     });
 }
 
+// Frames per chunk of the frame pipelines: a few whole frames, ~32 MB per chunk (measured on B200 / PCIe Gen5:
+// 8 MB chunks 9.7, 16 MB 10.7, 32 MB 11.0, 64 MB 10.8 Gpix/s end to end on 64 x 1080p fp32 frames), at most
+// max_per.  The first chunk's upload and the last chunk's download overlap with nothing: the batch starts with
+// chunks of 1, 2, 4 ... frames and ends with ... 4, 2, 1 (CAMCAL_CHUNK_RAMP=0: uniform chunks), so the exposed
+// head and tail are one frame each instead of one 32 MB chunk each.  *per_out: the body's chunk.
+static std::vector<int> chunk_schedule(int nframes, size_t frame_bytes, int max_per, int* per_out) {
+    size_t chunk_mb = 32;
+    if (const char* e = getenv("CAMCAL_CHUNK_MB")) chunk_mb = (size_t)std::max(1, atoi(e));   // tuning knob
+    int per = (int)((chunk_mb << 20) / frame_bytes);
+    if (per < 1) per = 1;
+    if (per > max_per) per = max_per;
+    if (per > nframes) per = nframes;
+    bool ramp = true;
+    if (const char* e = getenv("CAMCAL_CHUNK_RAMP")) ramp = atoi(e) != 0;   // tuning knob
+    int ramp_frames = 0, ramp_steps = 0;                     // frames / chunks of one ramp: 1 + 2 + ... (< per)
+    for (int c = 1; ramp && c < per; c *= 2) { ramp_frames += c; ++ramp_steps; }
+    if (2 * ramp_frames + per > nframes) ramp_frames = ramp_steps = 0;
+    std::vector<int> sizes;
+    for (int f0 = 0, it = 0, m = 0; f0 < nframes; f0 += m, ++it) {
+        const int left = nframes - f0;
+        if (it < ramp_steps) m = 1 << it;                                    // head: 1, 2, 4 ...
+        else if (left > ramp_frames) m = std::min(per, left - ramp_frames);  // body
+        else { m = 1; while (2 * m - 1 < left) m *= 2; }                     // tail: left = 2m - 1 -> m, ... 2, 1
+        sizes.push_back(m);
+    }
+    *per_out = per;
+    return sizes;
+}
+
 // frames: chunk = a few whole frames (~32 MB per stage)
 template <typename PX, typename LAUNCH>
 static int rectify_host(cc_ctx* ctx, const PX* src, PX* dst, int sz1, int sz2, size_t pitch,
@@ -350,28 +390,12 @@ static int rectify_host(cc_ctx* ctx, const PX* src, PX* dst, int sz1, int sz2, s
     if ((rc = enter(ctx))) return rc;
     const size_t frame_elems = pitch * (size_t)sz2;          // device frames are stored pitch*sz2
     const size_t frame_bytes = frame_elems * px_bytes;
-    // chunk = a few whole frames, ~32 MB per stage (measured on B200 / PCIe Gen5: 8 MB chunks
-    // 9.7, 16 MB 10.7, 32 MB 11.0, 64 MB 10.8 Gpix/s end to end on 64 x 1080p fp32 frames)
-    size_t chunk_mb = 32;
-    if (const char* e = getenv("CAMCAL_CHUNK_MB")) chunk_mb = (size_t)std::max(1, atoi(e));   // tuning knob
-    int per = (int)((chunk_mb << 20) / frame_bytes);
-    if (per < 1) per = 1;
-    if (per > nframes) per = nframes;
+    int per = 0;
+    const std::vector<int> chunks = chunk_schedule(nframes, frame_bytes, nframes, &per);
     const bool dense = frame_stride == frame_elems && pitch == (size_t)sz1;
-    // The first chunk's upload and the last chunk's download overlap with nothing: the batch starts with
-    // chunks of 1, 2, 4 ... frames and ends with ... 4, 2, 1 (CAMCAL_CHUNK_RAMP=0: uniform chunks), so the
-    // exposed head and tail are one frame each instead of one 32 MB chunk each.
-    bool ramp = true;
-    if (const char* e = getenv("CAMCAL_CHUNK_RAMP")) ramp = atoi(e) != 0;   // tuning knob
-    int ramp_frames = 0, ramp_steps = 0;                     // frames / chunks of one ramp: 1 + 2 + ... (< per)
-    for (int c = 1; ramp && c < per; c *= 2) { ramp_frames += c; ++ramp_steps; }
-    if (2 * ramp_frames + per > nframes) ramp_frames = ramp_steps = 0;
     for (int f0 = 0, it = 0, m = 0; f0 < nframes; f0 += m, ++it) {
         const int k = it % cc_ctx::NSLOT;
-        const int left = nframes - f0;
-        if (it < ramp_steps) m = 1 << it;                                    // head: 1, 2, 4 ...
-        else if (left > ramp_frames) m = std::min(per, left - ramp_frames);  // body
-        else { m = 1; while (2 * m - 1 < left) m *= 2; }                     // tail: left = 2m - 1 -> m, ... 2, 1
+        m = chunks[it];
         // +64 bytes: vector gathers may touch the aligned word holding the last texel
         if ((rc = ensure_slot(ctx, k, per * frame_bytes + 64, per * frame_bytes + 64))) return rc;
         cudaStream_t st = ctx->pipe_stream[k];
@@ -630,15 +654,10 @@ int cc_rectify_u8c3(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, doubl
 
 }  // extern "C"
 
-// Frames with DIFFERENT views in one call: the reference's plot loop rectifies every calibration
-// image with its own extrinsic (src/plot_calibration.jl:36-42).  frames [v * frames_per_view,
-// (v + 1) * frames_per_view) use views[v], ratios[v], axs_mins[2v .. 2v+1].  Every view is one
-// launch with its own cached tile plan.
-template <typename P, typename F, typename G>
-static int rectify_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
-                         const int64_t* axs_mins, const P* src, P* dst, int sz1, int sz2, size_t pitch,
-                         size_t frame_stride, int frames_per_view, int channels, cudaStream_t stream, F launch,
-                         G launch_group) {
+// the argument rules of the many-view rectification calls (device and host forms alike)
+static int check_rect_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                            const int64_t* axs_mins, const void* src, const void* dst, int sz1, int sz2, size_t pitch,
+                            size_t frame_stride, int frames_per_view) {
     CC_REQUIRE(ctx && intr && (nviews == 0 || (views && ratios && axs_mins)), "NULL argument");
     CC_REQUIRE(nviews >= 0 && frames_per_view >= 0, "bad counts");
     CC_REQUIRE((long long)nviews * frames_per_view <= 65535, "at most 65535 frames per call");
@@ -648,8 +667,23 @@ static int rectify_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views,
         if ((rc = check_rect_args(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, frames_per_view, ratios[v]))) return rc;
     }
     CC_REQUIRE(nviews * frames_per_view == 0 || (src && dst), "NULL frame pointer");
-    CC_REQUIRE(nviews * frames_per_view == 0 || (const void*)src != (const void*)dst, "rectification is not in place: src == dst");
+    CC_REQUIRE(nviews * frames_per_view == 0 || src != dst, "rectification is not in place: src == dst");
     CC_REQUIRE(nviews * frames_per_view <= 1 || frame_stride >= pitch * (size_t)(sz2 - 1) + sz1, "frames overlap");
+    return CC_OK;
+}
+
+// Frames with DIFFERENT views in one call: the reference's plot loop rectifies every calibration
+// image with its own extrinsic (src/plot_calibration.jl:36-42).  frames [v * frames_per_view,
+// (v + 1) * frames_per_view) use views[v], ratios[v], axs_mins[2v .. 2v+1].  Every view is one
+// launch with its own cached tile plan.
+template <typename P, typename F, typename G>
+static int rectify_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                         const int64_t* axs_mins, const P* src, P* dst, int sz1, int sz2, size_t pitch,
+                         size_t frame_stride, int frames_per_view, int channels, cudaStream_t stream, F launch,
+                         G launch_group) {
+    int rc = check_rect_views(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
+                              frames_per_view);
+    if (rc) return rc;
     CC_GUARD;
     if ((rc = enter(ctx))) return rc;
     if (nviews == 0 || frames_per_view == 0) return CC_OK;
@@ -701,6 +735,104 @@ static int rectify_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views,
         cudaEventDestroy(fork);
     }
     return rc;
+}
+
+
+// Frames of many views from host memory in one call (cc_rectify_views_*_host): the chunk pipeline of rectify_host
+// over the frame axis of the whole call.  Chunks ignore view boundaries and span at most two 64-view groups (a
+// chunk holds at most 64 views' frames).  A chunk makes one staged launch per group it touches, over the window of
+// that group's frames it holds (rectify.cu: RectViewsHost); a group without a staged plan runs the window's views
+// through the single-view kernels on the chunk's own slot stream.  The next group's plan is built on host threads
+// while the device streams the current one: before waiting for it, the uploads of the next NSLOT chunks are
+// enqueued.  LAUNCH_GROUP(vh, g, w0, wn, src, dst, st, ok) / LAUNCH_ONE(v, src, dst, nframes, st).
+template <typename PX, typename LAUNCH_GROUP, typename LAUNCH_ONE>
+static int rectify_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                              const int64_t* axs_mins, const PX* src, PX* dst, int sz1, int sz2, size_t pitch,
+                              size_t frame_stride, int fpv, int pxb, unsigned flags, std::vector<ChainD>* chs,
+                              LAUNCH_GROUP launch_group, LAUNCH_ONE launch_one) {
+    int rc = check_rect_views(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride, fpv);
+    if (rc) return rc;
+    CC_GUARD;
+    if ((rc = enter(ctx))) return rc;
+    if (nviews == 0 || fpv == 0) return CC_OK;
+    chs->resize((size_t)nviews);
+    for (int v = 0; v < nviews; ++v) build_chain(intr, views + v, &(*chs)[v]);
+    const int nframes = nviews * fpv, gframes = rectify_views_per_launch() * fpv;
+    const size_t frame_elems = pitch * (size_t)sz2;          // device frames are stored pitch*sz2
+    const size_t frame_bytes = frame_elems * pxb;
+    int per = 0;
+    const std::vector<int> chunks = chunk_schedule(nframes, frame_bytes, gframes, &per);
+    const int nchunks = (int)chunks.size();
+    std::vector<int> first((size_t)nchunks + 1, 0);
+    for (int c = 0; c < nchunks; ++c) first[c + 1] = first[c] + chunks[c];
+    const bool dense = frame_stride == frame_elems && pitch == (size_t)sz1;
+    const uint8_t* hsrc = reinterpret_cast<const uint8_t*>(src);
+    uint8_t* hdst = reinterpret_cast<uint8_t*>(dst);
+    RectViewsHost* vh = nullptr;
+    if ((rc = rect_vh_begin(ctx, chs->data(), ratios, axs_mins, nviews, sz1, sz2, pitch, fpv, pxb,
+                            !(flags & CC_GATHER_DIRECT), &vh)))
+        return rc;
+    std::vector<char> uploaded((size_t)nchunks, 0), prepared((size_t)((nframes + gframes - 1) / gframes), 0);
+    // chunk c's frames to its slot (the slot's previous chunk, c - NSLOT, is enqueued in full by then)
+    auto upload = [&](int c) -> int {
+        if (c >= nchunks || uploaded[c]) return CC_OK;
+        const int k = c % cc_ctx::NSLOT, m = chunks[c];
+        int r = ensure_slot(ctx, k, per * frame_bytes + 64, per * frame_bytes + 64);   // +64: see rectify_host
+        if (r) return r;
+        uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[k]);
+        const uint8_t* hs = hsrc + (size_t)first[c] * frame_stride * pxb;
+        if (dense) {
+            CC_CUDA(cudaMemcpyAsync(din, hs, (size_t)m * frame_bytes, cudaMemcpyHostToDevice, ctx->pipe_stream[k]));
+        } else {
+            for (int f = 0; f < m; ++f)
+                CC_CUDA(cudaMemcpy2DAsync(din + (size_t)f * frame_bytes, pitch * pxb, hs + (size_t)f * frame_stride * pxb,
+                                          pitch * pxb, (size_t)sz1 * pxb, sz2, cudaMemcpyHostToDevice, ctx->pipe_stream[k]));
+        }
+        uploaded[c] = 1;
+        return CC_OK;
+    };
+    int retired = 0;                                        // groups whose chunks are all enqueued
+    for (int c = 0; rc == CC_OK && c < nchunks; ++c) {
+        const int f0 = first[c], m = chunks[c], g_lo = f0 / gframes, g_hi = (f0 + m - 1) / gframes;
+        for (int gi = g_lo; rc == CC_OK && gi <= g_hi; ++gi) {
+            if (prepared[gi]) continue;
+            for (int j = 0; rc == CC_OK && j < cc_ctx::NSLOT; ++j) rc = upload(c + j);
+            if (rc == CC_OK) rc = rect_vh_prepare(vh, gi);
+            prepared[gi] = 1;
+        }
+        if (rc == CC_OK) rc = upload(c);
+        if (rc) break;
+        const int k = c % cc_ctx::NSLOT;
+        cudaStream_t st = ctx->pipe_stream[k];
+        uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[k]);
+        uint8_t* dout = static_cast<uint8_t*>(ctx->pipe_out[k]);
+        for (int gi = g_lo; rc == CC_OK && gi <= g_hi; ++gi) {
+            const int a = std::max(f0, gi * gframes), b = std::min(f0 + m, (gi + 1) * gframes);
+            const size_t off = (size_t)(a - f0) * frame_bytes;
+            bool ok = false;
+            rc = launch_group(vh, gi, a - gi * gframes, b - a, reinterpret_cast<const PX*>(din + off),
+                              reinterpret_cast<PX*>(dout + off), st, &ok);
+            for (int v = a / fpv; rc == CC_OK && !ok && v <= (b - 1) / fpv; ++v) {
+                const int fa = std::max(a, v * fpv), fb = std::min(b, (v + 1) * fpv);
+                const size_t o = (size_t)(fa - f0) * frame_bytes;
+                rc = launch_one(v, reinterpret_cast<const PX*>(din + o), reinterpret_cast<PX*>(dout + o), fb - fa, st);
+            }
+        }
+        if (rc) break;
+        uint8_t* hd = hdst + (size_t)f0 * frame_stride * pxb;
+        if (dense) {
+            rc = cuda_check(cudaMemcpyAsync(hd, dout, (size_t)m * frame_bytes, cudaMemcpyDeviceToHost, st), "copy");
+        } else {
+            for (int f = 0; rc == CC_OK && f < m; ++f)
+                rc = cuda_check(cudaMemcpy2DAsync(hd + (size_t)f * frame_stride * pxb, pitch * pxb, dout + (size_t)f * frame_bytes,
+                                                  pitch * pxb, (size_t)sz1 * pxb, sz2, cudaMemcpyDeviceToHost, st), "copy");
+        }
+        for (; retired < g_hi || (retired == g_hi && f0 + m == std::min(nframes, (g_hi + 1) * gframes)); ++retired)
+            rect_vh_retire(vh, retired);
+    }
+    const int re = rect_vh_end(vh);                         // every plan fenced, uploads complete
+    const int rd = drain(ctx);
+    return rc ? rc : re ? re : rd;
 }
 
 extern "C" {
@@ -800,6 +932,40 @@ int cc_rectify_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, 
             return launch_rectify_u8c3(ctx, ch, ratio, axs_min, s, d, sz1, sz2, pitch, fs, m, fill,
                                        flags, st);
         });
+}
+
+// ---- many views from host memory ----------------------------------------------------
+int cc_rectify_views_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const double* ratios, const int64_t* axs_mins, const float* src, float* dst,
+                                int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
+                                float fill, unsigned flags) {
+    std::vector<ChainD> chs;
+    return rectify_views_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
+                              frames_per_view, (int)sizeof(float), flags, &chs,
+                              [&](RectViewsHost* vh, int gi, int w0, int wn, const float* s, float* d, cudaStream_t st, bool* ok) {
+                                  return rect_vh_launch_f32c1(vh, gi, w0, wn, s, d, fill, flags, st, ok);
+                              },
+                              [&](int v, const float* s, float* d, int m, cudaStream_t st) {
+                                  return launch_rectify_f32c1(ctx, chs[v], ratios[v], axs_mins + 2 * v, s, d, sz1, sz2,
+                                                              pitch, pitch * (size_t)sz2, m, fill, flags, st);
+                              });
+}
+
+int cc_rectify_views_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                               const double* ratios, const int64_t* axs_mins, const uint8_t* src, uint8_t* dst,
+                               int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
+                               const uint8_t fill[3], unsigned flags) {
+    CC_REQUIRE(fill != nullptr, "fill is NULL");
+    std::vector<ChainD> chs;
+    return rectify_views_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
+                              frames_per_view, 3, flags, &chs,
+                              [&](RectViewsHost* vh, int gi, int w0, int wn, const uint8_t* s, uint8_t* d, cudaStream_t st, bool* ok) {
+                                  return rect_vh_launch_u8c3(vh, gi, w0, wn, s, d, fill, flags, st, ok);
+                              },
+                              [&](int v, const uint8_t* s, uint8_t* d, int m, cudaStream_t st) {
+                                  return launch_rectify_u8c3(ctx, chs[v], ratios[v], axs_mins + 2 * v, s, d, sz1, sz2,
+                                                             pitch, pitch * (size_t)sz2, m, fill, flags, st);
+                              });
 }
 
 int cc_rectify_map_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,

@@ -79,6 +79,11 @@ struct cc_ctx {
     static const int NMULTI = 4;
     void* multi_plans[NMULTI];
     int multi_plan_next;
+    // cc_rectify_views_*_host: group plans go up on rect_upload; a plan's fence joins the slot streams on
+    // rect_join (rect_join_event: one per slot); multi_retired: evicted plans whose buffers did not fit a new one
+    cudaStream_t rect_upload, rect_join;
+    cudaEvent_t rect_join_event[NSLOT];
+    void* multi_retired;
     // ticket counters of the persistent rectification kernels (rectify.cu: RectSched)
     static const int NSCHED = 16;
     void* sched_pool;

@@ -119,6 +119,11 @@ struct TileCfg {
     int fpv;               // frames per view
     int gpv;               // frame groups per view
     int tiles;             // strips * ntiles2
+    // *_views_kernel frame window: the launch covers frames [w0, w0 + g.nframes) of the group (the tensor map and
+    // dst start at frame w0).  Units cover the frame groups g0, g0 + 1 ... that meet the window; frame groups
+    // stay inside a view, and those at the window's edges are cut to it.  w0 = g0 = 0: the whole group.
+    int w0;
+    uint32_t g0;
 };
 
 // Frames with different views in one launch (cc_rectify_*_views): what the single-view kernels take as
@@ -300,6 +305,7 @@ static void plan_free(RectPlan* p) {
 }
 
 static void multi_free(void* mp);
+static void multi_free_retired(cc_ctx* ctx);
 
 void rectify_free_plans(cc_ctx* ctx) {
     for (int i = 0; i < cc_ctx::NPLAN; ++i) {
@@ -310,6 +316,11 @@ void rectify_free_plans(cc_ctx* ctx) {
         multi_free(ctx->multi_plans[i]);
         ctx->multi_plans[i] = nullptr;
     }
+    multi_free_retired(ctx);
+    if (ctx->rect_upload) { cudaStreamSynchronize(ctx->rect_upload); cudaStreamDestroy(ctx->rect_upload); ctx->rect_upload = nullptr; }
+    if (ctx->rect_join) { cudaStreamSynchronize(ctx->rect_join); cudaStreamDestroy(ctx->rect_join); ctx->rect_join = nullptr; }
+    for (int k = 0; k < cc_ctx::NSLOT; ++k)
+        if (ctx->rect_join_event[k]) { cudaEventDestroy(ctx->rect_join_event[k]); ctx->rect_join_event[k] = nullptr; }
 }
 
 static void plan_footprints(RectPlan* p, bool threads) {
@@ -850,8 +861,20 @@ struct MultiPlan {
     int n1, n2;
     TileHdr* d_hdr;                // [view][tile]
     double* d_q2;                  // [view][sz2]
+    size_t hdr_cap, q2_cap;        // bytes allocated at d_hdr / d_q2
     int per_sm[2];
     size_t per_sm_smem[2];
+    std::vector<TileHdr> h_hdr;    // the tables on the host, until their upload has completed
+    std::vector<double> h_q2;
+    // The host form (cc_rectify_views_*_host) uploads on its own stream: `ready` follows the upload, and the slot
+    // streams wait for it.  `fence` follows the last launches that read the tables, on `fence_stream` (a device
+    // call on another stream waits for it first, so it covers every reader): the host form reuses or frees the
+    // buffers of an evicted plan after it, without synchronising the device.
+    cudaEvent_t ready;
+    cudaEvent_t fence;
+    cudaStream_t fence_stream;
+    bool fenced;
+    MultiPlan* next_retired;       // cc_ctx::multi_retired: evicted, freed once its fence has passed
 };
 
 static void multi_free(void* p) {
@@ -859,31 +882,35 @@ static void multi_free(void* p) {
     if (!mp) return;
     if (mp->d_hdr) cudaFree(mp->d_hdr);
     if (mp->d_q2) cudaFree(mp->d_q2);
+    if (mp->ready) cudaEventDestroy(mp->ready);
+    if (mp->fence) cudaEventDestroy(mp->fence);
     delete mp;
 }
 
-// find or build the plan of a group of views; nullptr: not stageable (or out of memory) -- the caller falls
-// back to one launch per view
-static MultiPlan* multi_get(cc_ctx* ctx, const ChainD* chs, const double* ratios, const RectGeom* gs, int nviews,
-                            int tw, int tl, int pxb, cudaStream_t st) {
-    std::vector<PlanKey> keys((size_t)nviews);
-    for (int v = 0; v < nviews; ++v) keys[v] = plan_key(chs[v], ratios[v], gs[v], tw, tl, pxb);
+// plans retired by the host form: their readers are fenced, so this waits for those only
+static void multi_free_retired(cc_ctx* ctx) {
+    MultiPlan* mp = static_cast<MultiPlan*>(ctx->multi_retired);
+    ctx->multi_retired = nullptr;
+    while (mp) {
+        MultiPlan* next = mp->next_retired;
+        if (mp->fenced) cudaEventSynchronize(mp->fence);
+        multi_free(mp);
+        mp = next;
+    }
+}
+
+static MultiPlan* multi_find(cc_ctx* ctx, const std::vector<PlanKey>& keys) {
     for (int i = 0; i < cc_ctx::NMULTI; ++i) {
         MultiPlan* mp = static_cast<MultiPlan*>(ctx->multi_plans[i]);
         if (mp && mp->keys.size() == keys.size() && memcmp(mp->keys.data(), keys.data(), keys.size() * sizeof(PlanKey)) == 0)
             return mp;
     }
-    // footprints per view: the cached RectPlans, the missing ones built on up to 16 host threads (the plot loop
-    // is a one-shot call: 64 cold views cost 64 x ~0.5 ms of host arithmetic on one thread) and cached without
-    // their device tables (the group uploads its own).  Copied at once: inserting may evict an earlier plan.
-    std::vector<RectPlan*> pl((size_t)nviews, nullptr);
-    std::vector<int> missing;
-    for (int v = 0; v < nviews; ++v) {
-        pl[v] = plan_find(ctx, keys[v]);
-        bool dup = false;                                  // the same view twice: build it once
-        for (int w = 0; w < v && !pl[v] && !dup; ++w) dup = memcmp(&keys[w], &keys[v], sizeof(PlanKey)) == 0;
-        if (!pl[v] && !dup) missing.push_back(v);
-    }
+    return nullptr;
+}
+
+// the views [missing] of a group on up to 16 host threads (the plot loop is a one-shot call: 64 cold views cost
+// 64 x ~0.5 ms of host arithmetic on one thread); then every duplicate of an earlier view gets that view's plan
+static void plans_build(const std::vector<PlanKey>& keys, std::vector<RectPlan*>& pl, const std::vector<int>& missing) {
     if (!missing.empty()) {
         const int nt = (int)std::min<size_t>(missing.size(), std::min(16u, std::max(1u, std::thread::hardware_concurrency())));
         std::vector<std::thread> th;
@@ -895,49 +922,81 @@ static MultiPlan* multi_get(cc_ctx* ctx, const ChainD* chs, const double* ratios
         work(0);
         for (auto& x : th) x.join();
     }
-    std::vector<RectPlan> fp;
-    fp.reserve((size_t)nviews);
+    for (size_t v = 0; v < pl.size(); ++v)
+        if (!pl[v])                                        // a duplicate of an earlier view (or out of memory)
+            for (size_t w = 0; w < v && !pl[v]; ++w)
+                if (memcmp(&keys[w], &keys[v], sizeof(PlanKey)) == 0) pl[v] = pl[w];
+}
+
+// views of a group without a plan, each distinct view once
+static std::vector<int> plans_missing(const std::vector<PlanKey>& keys, const std::vector<RectPlan*>& pl) {
+    std::vector<int> missing;
+    for (size_t v = 0; v < keys.size(); ++v) {
+        bool dup = false;                                  // the same view twice: build it once
+        for (size_t w = 0; w < v && !pl[v] && !dup; ++w) dup = memcmp(&keys[w], &keys[v], sizeof(PlanKey)) == 0;
+        if (!pl[v] && !dup) missing.push_back((int)v);
+    }
+    return missing;
+}
+
+// the common box and the host tables of a group from its views' footprints (host arithmetic only);
+// nullptr: a view has no plan (out of memory) or the group cannot be staged
+static MultiPlan* multi_assemble(const std::vector<PlanKey>& keys, const std::vector<RectPlan*>& pl, int pxb) {
+    const int nviews = (int)keys.size();
     int need1 = 0, need2 = 0;
     long long tilt = 0;
-    bool oom = false;
     for (int v = 0; v < nviews; ++v) {
-        if (!pl[v])                                        // a duplicate of an earlier view (or out of memory)
-            for (int w = 0; w < v && !pl[v]; ++w)
-                if (memcmp(&keys[w], &keys[v], sizeof(PlanKey)) == 0) pl[v] = pl[w];
-        if (!pl[v]) { oom = true; continue; }
-        fp.push_back(*pl[v]);
+        if (!pl[v]) return nullptr;
         need1 = std::max(need1, pl[v]->need1); need2 = std::max(need2, pl[v]->need2);
         tilt += pl[v]->tilt;
     }
-    for (int v : missing) if (pl[v]) plan_insert(ctx, pl[v]);
-    if (oom) return nullptr;
     MultiPlan* mp = new (std::nothrow) MultiPlan();
     if (!mp) return nullptr;
     mp->keys = keys;
     mp->d = box_dims(need1, need2, tilt >= 0 ? 1 : -1, pxb);
-    mp->n1 = fp[0].n1; mp->n2 = fp[0].n2;
-    mp->d_hdr = nullptr; mp->d_q2 = nullptr;
-    mp->per_sm[0] = mp->per_sm[1] = 0; mp->per_sm_smem[0] = mp->per_sm_smem[1] = 0;
+    mp->n1 = pl[0]->n1; mp->n2 = pl[0]->n2;
     if (getenv("CAMCAL_DEBUG"))
         fprintf(stderr, "[camcal] views: common footprint %d x %d -> box %d x %d pitch %d (%d B)\n", need1, need2, mp->d.box1,
                 mp->d.box2, mp->d.pitch_b, mp->d.box_bytes);
     if (!mp->d.box_bytes) { delete mp; return nullptr; }
-    const size_t ntiles = (size_t)mp->n1 * mp->n2, sz2 = (size_t)gs[0].sz2;
-    std::vector<TileHdr> hdr(ntiles * nviews);
-    std::vector<double> q2(sz2 * nviews);
+    const size_t ntiles = (size_t)mp->n1 * mp->n2, sz2 = (size_t)keys[0].g.sz2;
+    mp->h_hdr.resize(ntiles * nviews);
+    mp->h_q2.resize(sz2 * nviews);
     for (int v = 0; v < nviews; ++v) {
-        fill_headers(&fp[v], mp->d, hdr.data() + (size_t)v * ntiles);
-        memcpy(q2.data() + (size_t)v * sz2, fp[v].q2.data(), sz2 * sizeof(double));
+        fill_headers(pl[v], mp->d, mp->h_hdr.data() + (size_t)v * ntiles);
+        memcpy(mp->h_q2.data() + (size_t)v * sz2, pl[v]->q2.data(), sz2 * sizeof(double));
     }
-    const size_t hb = hdr.size() * sizeof(TileHdr), qb = q2.size() * sizeof(double);
+    return mp;
+}
+
+// find or build the plan of a group of views; nullptr: not stageable (or out of memory) -- the caller falls
+// back to one launch per view
+static MultiPlan* multi_get(cc_ctx* ctx, const ChainD* chs, const double* ratios, const RectGeom* gs, int nviews,
+                            int tw, int tl, int pxb, cudaStream_t st) {
+    std::vector<PlanKey> keys((size_t)nviews);
+    for (int v = 0; v < nviews; ++v) keys[v] = plan_key(chs[v], ratios[v], gs[v], tw, tl, pxb);
+    if (MultiPlan* mp = multi_find(ctx, keys)) return mp;
+    // footprints per view: the cached RectPlans, the missing ones built on host threads and cached without their
+    // device tables (the group uploads its own).  Assembled before inserting: inserting may evict an earlier plan.
+    std::vector<RectPlan*> pl((size_t)nviews, nullptr);
+    for (int v = 0; v < nviews; ++v) pl[v] = plan_find(ctx, keys[v]);
+    const std::vector<int> missing = plans_missing(keys, pl);
+    plans_build(keys, pl, missing);
+    MultiPlan* mp = multi_assemble(keys, pl, pxb);
+    for (int v : missing) if (pl[v]) plan_insert(ctx, pl[v]);
+    if (!mp) return nullptr;
+    const size_t hb = mp->h_hdr.size() * sizeof(TileHdr), qb = mp->h_q2.size() * sizeof(double);
     if (cudaMalloc(&mp->d_hdr, hb) != cudaSuccess || cudaMalloc(&mp->d_q2, qb) != cudaSuccess ||
-        cudaMemcpyAsync(mp->d_hdr, hdr.data(), hb, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(mp->d_q2, q2.data(), qb, cudaMemcpyHostToDevice, st) != cudaSuccess) {
+        cudaMemcpyAsync(mp->d_hdr, mp->h_hdr.data(), hb, cudaMemcpyHostToDevice, st) != cudaSuccess ||
+        cudaMemcpyAsync(mp->d_q2, mp->h_q2.data(), qb, cudaMemcpyHostToDevice, st) != cudaSuccess) {
         cudaGetLastError();
         multi_free(mp);
         return nullptr;
     }
+    mp->hdr_cap = hb; mp->q2_cap = qb;
     cudaStreamSynchronize(st);         // the host vectors go away; later calls may come on other streams
+    std::vector<TileHdr>().swap(mp->h_hdr);
+    std::vector<double>().swap(mp->h_q2);
     const int slot = ctx->multi_plan_next++ % cc_ctx::NMULTI;
     if (ctx->multi_plans[slot]) {
         cudaDeviceSynchronize();       // an evicted plan may still be read by a running kernel
@@ -945,6 +1004,18 @@ static MultiPlan* multi_get(cc_ctx* ctx, const ChainD* chs, const double* ratios
     }
     ctx->multi_plans[slot] = mp;
     return mp;
+}
+
+// a launch on `st` reads mp's tables: readers on another stream come first (the fence then covers them all)
+static void multi_read_begin(MultiPlan* mp, cudaStream_t st) {
+    if (mp->ready) cudaStreamWaitEvent(st, mp->ready, 0);
+    if (mp->fenced && mp->fence_stream != st) cudaStreamWaitEvent(st, mp->fence, 0);
+}
+static void multi_read_end(MultiPlan* mp, cudaStream_t st) {
+    if (!mp->fence && cudaEventCreateWithFlags(&mp->fence, cudaEventDisableTiming) != cudaSuccess) { mp->fence = nullptr; return; }
+    cudaEventRecord(mp->fence, st);
+    mp->fenced = true;
+    mp->fence_stream = st;
 }
 
 struct ViewsLaunch {
@@ -955,31 +1026,32 @@ struct ViewsLaunch {
     MultiPlan* mp;
 };
 
-// tensor map, unit configuration and view table of one group; *ok = false: the single launch does not apply
-static int views_prepare(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews,
-                         const void* src, int pxb, int tl, int sz1, int sz2, size_t pitch, size_t frame_stride, int fpv,
-                         int fg_max, cudaStream_t st, ViewsLaunch* L, bool* ok) {
+// frame groups of fg frames (inside views of fpv frames) that meet frames [w0, w0 + wn) of a group; *g0: the first
+static long long window_groups(int fpv, int fg, int w0, int wn, uint32_t* g0) {
+    const int gpv = (fpv + fg - 1) / fg;
+    const int v_lo = w0 / fpv, v_hi = (w0 + wn - 1) / fpv;
+    const long long lo = (long long)v_lo * gpv + (w0 - v_lo * fpv) / fg;
+    const long long hi = (long long)v_hi * gpv + (w0 + wn - 1 - v_hi * fpv) / fg;
+    *g0 = (uint32_t)lo;
+    return hi - lo + 1;
+}
+
+// tensor map, unit configuration and view table of one launch of a group's plan over frames [w0, w0 + wn) of the
+// group; src: the window's first frame; frames frame_stride elements apart.  *ok = false: the launch does not apply
+static int views_window(cc_ctx* ctx, MultiPlan* mp, const ChainD* chs, const double* ratios, const int64_t* axs_mins,
+                        int nviews, const void* src, int pxb, int tl, int sz1, int sz2, size_t pitch, size_t frame_stride,
+                        int fpv, int w0, int wn, int fg_max, ViewsLaunch* L, bool* ok) {
     *ok = false;
-    if (nviews < 1 || nviews > kMaxViews || fpv < 1) return CC_OK;
-    const int nframes = nviews * fpv;
-    const size_t pitch_b = pitch * pxb, frame_b = frame_stride * pxb;
-    if ((reinterpret_cast<uintptr_t>(src) & 15u) || (pitch_b & 15u) || (nframes > 1 && (frame_b & 15u))) return CC_OK;
     EncodeTiledFn enc = encoder(ctx);
     if (!enc) return CC_OK;
-    std::vector<RectGeom> gs((size_t)nviews);
-    for (int v = 0; v < nviews; ++v) gs[v] = make_geom(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, nframes);
-    MultiPlan* mp = multi_get(ctx, chs, ratios, gs.data(), nviews, kT, tl, pxb, st);
-    if (!mp) {
-        if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %d not stageable (pxb %d)\n", nviews, pxb);
-        return CC_OK;
-    }
+    const size_t pitch_b = pitch * pxb, frame_b = frame_stride * pxb;
     int stages = std::min(kMaxStages, std::max(2, CAMCAL_RING_BYTES / mp->d.box_bytes));
     if (const char* e = getenv("CAMCAL_STAGES")) stages = std::min(kMaxStages, std::max(1, atoi(e)));   // tuning knob
     while (stages > 2 && stages * mp->d.box_bytes > 56 * 1024) --stages;
     memset(&L->tmap, 0, sizeof(L->tmap));
     const int box1_elems = (pxb == 4) ? mp->d.pitch_b / 4 : mp->d.pitch_b;
-    cuuint64_t dims[3] = {(cuuint64_t)sz1 * (pxb == 4 ? 1 : 3), (cuuint64_t)sz2, (cuuint64_t)nframes};
-    cuuint64_t strides[2] = {(cuuint64_t)pitch_b, (cuuint64_t)(nframes > 1 ? frame_b : pitch_b * sz2)};
+    cuuint64_t dims[3] = {(cuuint64_t)sz1 * (pxb == 4 ? 1 : 3), (cuuint64_t)sz2, (cuuint64_t)wn};
+    cuuint64_t strides[2] = {(cuuint64_t)pitch_b, (cuuint64_t)(wn > 1 ? frame_b : pitch_b * sz2)};
     cuuint32_t box[3] = {(cuuint32_t)box1_elems, (cuuint32_t)mp->d.box2, 1};
     cuuint32_t estr[3] = {1, 1, 1};
     if (enc(&L->tmap, pxb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3,
@@ -996,23 +1068,91 @@ static int views_prepare(cc_ctx* ctx, const ChainD* chs, const double* ratios, c
     // frames per group: as unit_cfg (keep ~8 units per resident CTA slot), within a view
     const long long want = (long long)ctx->sm_count * 6 * 8;
     int fg = std::min(fg_max, fpv);
-    while (fg > 1 && (long long)cfg.tiles * nviews * ((fpv + fg - 1) / fg) < want) fg = (fg + 1) / 2;
+    uint32_t g0 = 0;
+    while (fg > 1 && (long long)cfg.tiles * window_groups(fpv, fg, w0, wn, &g0) < want) fg = (fg + 1) / 2;
+    const long long units = (long long)cfg.tiles * window_groups(fpv, fg, w0, wn, &g0);
     cfg.fg = fg;
     cfg.fpv = fpv;
     cfg.gpv = (fpv + fg - 1) / fg;
-    const long long units = (long long)cfg.tiles * nviews * cfg.gpv;
+    cfg.w0 = w0;
+    cfg.g0 = g0;
     CC_REQUIRE(units < (1ll << 31), "too many tiles in one call: split the batch");
     cfg.units = (uint32_t)units;
     cfg.widen_mul = 0x20000000u;
     for (int v = 0; v < nviews; ++v) {
+        const RectGeom gv = make_geom(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, wn);
         L->vt.v[v].pe = make_exact(chs[v], ratios[v]);
-        L->vt.v[v].pf = make_fast(chs[v], ratios[v], gs[v]);
-        L->vt.v[v].g = gs[v];
+        L->vt.v[v].pf = make_fast(chs[v], ratios[v], gv);
+        L->vt.v[v].g = gv;
     }
     for (int v = nviews; v < kMaxViews; ++v) L->vt.v[v] = L->vt.v[0];
-    L->g = gs[0];
+    L->g = L->vt.v[0].g;
     L->mp = mp;
     *ok = true;
+    return CC_OK;
+}
+
+// tensor map, unit configuration and view table of one group's launch over all its frames; *ok = false: the
+// single launch does not apply
+static int views_prepare(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews,
+                         const void* src, int pxb, int tl, int sz1, int sz2, size_t pitch, size_t frame_stride, int fpv,
+                         int fg_max, cudaStream_t st, ViewsLaunch* L, bool* ok) {
+    *ok = false;
+    if (nviews < 1 || nviews > kMaxViews || fpv < 1) return CC_OK;
+    const int nframes = nviews * fpv;
+    const size_t pitch_b = pitch * pxb, frame_b = frame_stride * pxb;
+    if ((reinterpret_cast<uintptr_t>(src) & 15u) || (pitch_b & 15u) || (nframes > 1 && (frame_b & 15u))) return CC_OK;
+    if (!encoder(ctx)) return CC_OK;
+    std::vector<RectGeom> gs((size_t)nviews);
+    for (int v = 0; v < nviews; ++v) gs[v] = make_geom(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, nframes);
+    MultiPlan* mp = multi_get(ctx, chs, ratios, gs.data(), nviews, kT, tl, pxb, st);
+    if (!mp) {
+        if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %d not stageable (pxb %d)\n", nviews, pxb);
+        return CC_OK;
+    }
+    return views_window(ctx, mp, chs, ratios, axs_mins, nviews, src, pxb, tl, sz1, sz2, pitch, frame_stride, fpv, 0,
+                        nframes, fg_max, L, ok);
+}
+
+// the staged views kernels on a prepared launch
+static int views_run_f32c1(cc_ctx* ctx, ViewsLaunch* Lp, bool exact, const float* src, float* dst, float fill,
+                           cudaStream_t st) {
+    const size_t smem = (size_t)Lp->cfg.stages * Lp->cfg.box_bytes;
+    uint32_t gsz = 0;
+    int rc = exact ? persistent_grid(ctx, 6, rectify_f32c1_views_kernel<true>, smem, Lp->cfg, Lp->mp, true, &gsz)
+                   : persistent_grid(ctx, 7, rectify_f32c1_views_kernel<false>, smem, Lp->cfg, Lp->mp, false, &gsz);
+    RectSched* sched = nullptr;
+    if (!rc) rc = sched_acquire(ctx, st, &sched);
+    if (rc) return rc;
+    multi_read_begin(Lp->mp, st);
+    if (exact) rectify_f32c1_views_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, fill);
+    else       rectify_f32c1_views_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, fill);
+    multi_read_end(Lp->mp, st);
+    sched_release(ctx, st);
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+static int views_run_u8c3(cc_ctx* ctx, ViewsLaunch* Lp, bool exact, const uint8_t* src, uint8_t* dst, const uint8_t fill[3],
+                          int sz1, int sz2, size_t pitch, cudaStream_t st) {
+    const uchar3 f = make_uchar3(fill[0], fill[1], fill[2]);
+    const unsigned frame_bytes = (unsigned)((pitch * (size_t)(sz2 - 1) + (size_t)sz1) * 3);
+    Lp->cfg.stages = std::max(2, Lp->cfg.stages / kU8FramesPerStage);
+    const size_t smem = (size_t)Lp->cfg.stages * kU8FramesPerStage * Lp->cfg.box_bytes + 16;
+    uint32_t gsz = 0;
+    int rc = exact ? persistent_grid(ctx, 8, rectify_u8c3_views_kernel<true>, smem, Lp->cfg, Lp->mp, true, &gsz)
+                   : persistent_grid(ctx, 9, rectify_u8c3_views_kernel<false>, smem, Lp->cfg, Lp->mp, false, &gsz);
+    RectSched* sched = nullptr;
+    if (!rc) rc = sched_acquire(ctx, st, &sched);
+    if (rc) return rc;
+    multi_read_begin(Lp->mp, st);
+    if (exact) rectify_u8c3_views_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, f, frame_bytes);
+    else       rectify_u8c3_views_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, f, frame_bytes);
+    multi_read_end(Lp->mp, st);
+    sched_release(ctx, st);
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
     return CC_OK;
 }
 
@@ -1022,23 +1162,10 @@ int launch_rectify_f32c1_views(cc_ctx* ctx, const ChainD* chs, const double* rat
     const bool exact = !(flags & CC_COORD_F32);
     *ok = false;
     ViewsLaunch L;                     // 15 KB: the view table goes to the kernel by value
-    ViewsLaunch* Lp = &L;
     int rc = views_prepare(ctx, chs, ratios, axs_mins, nviews, src, 4, kTLf, sz1, sz2, pitch, frame_stride, fpv,
-                           exact ? kFGf32Exact : kFGf32Fast, st, Lp, ok);
+                           exact ? kFGf32Exact : kFGf32Fast, st, &L, ok);
     if (rc || !*ok) return rc;
-    const size_t smem = (size_t)Lp->cfg.stages * Lp->cfg.box_bytes;
-    uint32_t gsz = 0;
-    rc = exact ? persistent_grid(ctx, 6, rectify_f32c1_views_kernel<true>, smem, Lp->cfg, Lp->mp, true, &gsz)
-               : persistent_grid(ctx, 7, rectify_f32c1_views_kernel<false>, smem, Lp->cfg, Lp->mp, false, &gsz);
-    RectSched* sched = nullptr;
-    if (!rc) rc = sched_acquire(ctx, st, &sched);
-    if (rc) return rc;
-    if (exact) rectify_f32c1_views_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, fill);
-    else       rectify_f32c1_views_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, fill);
-    sched_release(ctx, st);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
+    return views_run_f32c1(ctx, &L, exact, src, dst, fill, st);
 }
 
 int launch_rectify_u8c3_views(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews,
@@ -1052,26 +1179,234 @@ int launch_rectify_u8c3_views(cc_ctx* ctx, const ChainD* chs, const double* rati
                         (nframes <= 1 || ((frame_stride * 3) & 3u) == 0);
     if (!dst_ok) return CC_OK;
     ViewsLaunch L;
-    ViewsLaunch* Lp = &L;
     int rc = views_prepare(ctx, chs, ratios, axs_mins, nviews, src, 3, kTLu, sz1, sz2, pitch, frame_stride, fpv,
-                           exact ? kFGu8Exact : kFGu8Fast, st, Lp, ok);
+                           exact ? kFGu8Exact : kFGu8Fast, st, &L, ok);
     if (rc || !*ok) return rc;
-    const uchar3 f = make_uchar3(fill[0], fill[1], fill[2]);
-    const unsigned frame_bytes = (unsigned)((pitch * (size_t)(sz2 - 1) + (size_t)sz1) * 3);
-    Lp->cfg.stages = std::max(2, Lp->cfg.stages / kU8FramesPerStage);
-    const size_t smem = (size_t)Lp->cfg.stages * kU8FramesPerStage * Lp->cfg.box_bytes + 16;
-    uint32_t gsz = 0;
-    rc = exact ? persistent_grid(ctx, 8, rectify_u8c3_views_kernel<true>, smem, Lp->cfg, Lp->mp, true, &gsz)
-               : persistent_grid(ctx, 9, rectify_u8c3_views_kernel<false>, smem, Lp->cfg, Lp->mp, false, &gsz);
-    RectSched* sched = nullptr;
-    if (!rc) rc = sched_acquire(ctx, st, &sched);
-    if (rc) return rc;
-    if (exact) rectify_u8c3_views_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, f, frame_bytes);
-    else       rectify_u8c3_views_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, f, frame_bytes);
-    sched_release(ctx, st);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
+    return views_run_u8c3(ctx, &L, exact, src, dst, fill, sz1, sz2, pitch, st);
+}
+
+// --------------------------------------------------------------------------------------
+// Frames of many views from host memory (cc_rectify_views_*_host): the chunk pipeline of abi.cu moves the
+// frames; this session owns the group plans of the call.  Each group of up to 64 views gets its plan once per
+// call.  A missing plan is built on host threads while the device streams the previous group's chunks, goes up
+// on the context's upload stream, and the slot streams wait for its `ready` event.  Nothing here synchronises
+// the device: an evicted plan's buffers are reused (or retired) after its fence.
+// --------------------------------------------------------------------------------------
+struct RectViewsHost {
+    cc_ctx* ctx;
+    const ChainD* chs;
+    const double* ratios;
+    const int64_t* axs_mins;
+    int nviews, ngroups, sz1, sz2, fpv, pxb, tl;
+    size_t pitch;
+    bool stage;                            // the layout can be staged at all
+    std::vector<MultiPlan*> mp;            // per group: its plan (nullptr: per-view launches)
+    std::vector<char> state;               // per group: 0 nothing yet, 1 being built, 2 ready
+    std::vector<char> used;                // per group: a launch read its plan since the last fence
+    // the group being built off this thread: keys, copies of the cached footprints, result
+    int job_group;
+    std::thread job;
+    std::vector<PlanKey> job_keys;
+    std::vector<RectPlan> job_found;
+    MultiPlan* job_out;
+    std::vector<MultiPlan*> installed;     // plans this call uploaded (their host tables go at the end)
+    std::vector<std::vector<TileHdr>> held_hdr;   // host tables of plans evicted during the call (uploads in flight)
+    std::vector<std::vector<double>> held_q2;
+};
+
+static std::vector<PlanKey> group_keys(const RectViewsHost* h, int gi) {
+    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->nviews - v0);
+    std::vector<PlanKey> keys((size_t)nv);
+    for (int v = 0; v < nv; ++v) {
+        const RectGeom g = make_geom(h->axs_mins + 2 * (v0 + v), h->sz1, h->sz2, h->pitch, 0, 0);
+        keys[v] = plan_key(h->chs[v0 + v], h->ratios[v0 + v], g, kT, h->tl, h->pxb);
+    }
+    return keys;
+}
+
+// the host half of group gi's plan (footprints, box, tables) on its own thread; a cached group plan is taken as is
+static void vh_start(RectViewsHost* h, int gi) {
+    if (gi >= h->ngroups || h->state[gi] || !h->stage) return;
+    std::vector<PlanKey> keys = group_keys(h, gi);
+    if (MultiPlan* mp = multi_find(h->ctx, keys)) { h->mp[gi] = mp; h->state[gi] = 2; return; }
+    // copies of the cached footprints: the context's plan cache may change while the job runs
+    h->job_found.clear();
+    h->job_found.reserve(keys.size());
+    std::vector<int> found_at(keys.size(), -1);
+    for (size_t v = 0; v < keys.size(); ++v)
+        if (RectPlan* p = plan_find(h->ctx, keys[v])) { found_at[v] = (int)h->job_found.size(); h->job_found.push_back(*p); }
+    h->job_keys.swap(keys);
+    h->job_out = nullptr;
+    h->job_group = gi;
+    h->state[gi] = 1;
+    auto work = [h, found_at]() {
+        const std::vector<PlanKey>& keys = h->job_keys;
+        std::vector<RectPlan*> pl(keys.size(), nullptr);
+        for (size_t v = 0; v < keys.size(); ++v) if (found_at[v] >= 0) pl[v] = &h->job_found[found_at[v]];
+        const std::vector<int> missing = plans_missing(keys, pl);
+        plans_build(keys, pl, missing);
+        h->job_out = multi_assemble(keys, pl, h->pxb);
+        for (int v : missing) plan_free(pl[v]);        // the footprints live on in the group plan only
+    };
+    try { h->job = std::thread(work); }
+    catch (...) { work(); }                             // no thread to be had: built here
+}
+
+// wait for the job of group gi; the tables go up on the upload stream into a free or evicted slot (never the
+// plan of group gi - 1, whose chunks may still be enqueued)
+static int vh_install(RectViewsHost* h, int gi) {
+    cc_ctx* ctx = h->ctx;
+    if (h->job.joinable()) h->job.join();
+    h->job_found.clear();
+    MultiPlan* mp = h->job_out;
+    h->job_out = nullptr;
+    h->state[gi] = 2;
+    if (!mp) {
+        if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %zu not stageable (pxb %d)\n", h->job_keys.size(), h->pxb);
+        return CC_OK;
+    }
+    const MultiPlan* keep = gi > 0 ? h->mp[gi - 1] : nullptr;
+    int slot = -1;
+    for (int i = 0; i < cc_ctx::NMULTI && slot < 0; ++i) {
+        const int s = (ctx->multi_plan_next + i) % cc_ctx::NMULTI;
+        if (!ctx->multi_plans[s] || ctx->multi_plans[s] != keep) slot = s;
+    }
+    ctx->multi_plan_next = slot + 1;
+    const size_t hb = mp->h_hdr.size() * sizeof(TileHdr), qb = mp->h_q2.size() * sizeof(double);
+    if (MultiPlan* old = static_cast<MultiPlan*>(ctx->multi_plans[slot])) {
+        ctx->multi_plans[slot] = nullptr;
+        h->installed.erase(std::remove(h->installed.begin(), h->installed.end(), old), h->installed.end());
+        h->held_hdr.emplace_back(); h->held_hdr.back().swap(old->h_hdr);
+        h->held_q2.emplace_back(); h->held_q2.back().swap(old->h_q2);
+        if (old->fenced) CC_CUDA(cudaStreamWaitEvent(ctx->rect_upload, old->fence, 0));
+        if (old->hdr_cap >= hb && old->q2_cap >= qb) {  // same frame size: the upload overwrites it after its readers
+            mp->d_hdr = old->d_hdr; mp->d_q2 = old->d_q2; mp->hdr_cap = old->hdr_cap; mp->q2_cap = old->q2_cap;
+            old->d_hdr = nullptr; old->d_q2 = nullptr;
+            multi_free(old);
+        } else {                                        // freed at the start of the next host call
+            old->next_retired = static_cast<MultiPlan*>(ctx->multi_retired);
+            ctx->multi_retired = old;
+        }
+    }
+    if (!mp->d_hdr) {                                   // room for a full group: later groups of this size reuse it
+        const size_t hcap = std::max(hb, (size_t)mp->n1 * mp->n2 * kMaxViews * sizeof(TileHdr));
+        const size_t qcap = std::max(qb, (size_t)h->sz2 * kMaxViews * sizeof(double));
+        if (cudaMalloc(&mp->d_hdr, hcap) != cudaSuccess || cudaMalloc(&mp->d_q2, qcap) != cudaSuccess) {
+            cudaGetLastError();
+            multi_free(mp);
+            return set_error(CC_ERR_CUDA, "out of device memory for the tile plans of a group of views");
+        }
+        mp->hdr_cap = hcap; mp->q2_cap = qcap;
+    }
+    if (cudaEventCreateWithFlags(&mp->ready, cudaEventDisableTiming) != cudaSuccess) {
+        mp->ready = nullptr;
+        multi_free(mp);
+        cudaGetLastError();
+        return set_error(CC_ERR_CUDA, "cannot create the upload event of a group plan");
+    }
+    ctx->multi_plans[slot] = mp;
+    h->installed.push_back(mp);
+    h->mp[gi] = mp;
+    CC_CUDA(cudaMemcpyAsync(mp->d_hdr, mp->h_hdr.data(), hb, cudaMemcpyHostToDevice, ctx->rect_upload));
+    CC_CUDA(cudaMemcpyAsync(mp->d_q2, mp->h_q2.data(), qb, cudaMemcpyHostToDevice, ctx->rect_upload));
+    CC_CUDA(cudaEventRecord(mp->ready, ctx->rect_upload));
     return CC_OK;
+}
+
+int rect_vh_begin(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews, int sz1,
+                  int sz2, size_t pitch, int fpv, int pxb, bool stage, RectViewsHost** out) {
+    *out = nullptr;
+    multi_free_retired(ctx);
+    if (!ctx->rect_upload) CC_CUDA(cudaStreamCreateWithFlags(&ctx->rect_upload, cudaStreamNonBlocking));
+    if (!ctx->rect_join) CC_CUDA(cudaStreamCreateWithFlags(&ctx->rect_join, cudaStreamNonBlocking));
+    for (int k = 0; k < cc_ctx::NSLOT; ++k)
+        if (!ctx->rect_join_event[k]) CC_CUDA(cudaEventCreateWithFlags(&ctx->rect_join_event[k], cudaEventDisableTiming));
+    RectViewsHost* h = new (std::nothrow) RectViewsHost();
+    if (!h) return set_error(CC_ERR_NOMEM, "out of host memory");
+    h->ctx = ctx; h->chs = chs; h->ratios = ratios; h->axs_mins = axs_mins;
+    h->nviews = nviews; h->ngroups = (nviews + kMaxViews - 1) / kMaxViews;
+    h->sz1 = sz1; h->sz2 = sz2; h->pitch = pitch; h->fpv = fpv; h->pxb = pxb; h->tl = pxb == 4 ? kTLf : kTLu;
+    // staged iff the device frames (pitch * sz2 elements, buffers 256-byte aligned) can be TMA-addressed
+    h->stage = stage && ((pitch * pxb) & 15u) == 0 && encoder(ctx) != nullptr;
+    h->mp.assign((size_t)h->ngroups, nullptr);
+    h->state.assign((size_t)h->ngroups, 0);
+    h->used.assign((size_t)h->ngroups, 0);
+    h->job_group = -1;
+    h->job_out = nullptr;
+    *out = h;
+    vh_start(h, 0);
+    return CC_OK;
+}
+
+int rect_vh_prepare(RectViewsHost* h, int gi) {
+    int rc = CC_OK;
+    if (h->stage && h->state[gi] != 2) {
+        if (h->state[gi] == 0) vh_start(h, gi);
+        if (h->state[gi] == 1 && (rc = vh_install(h, gi))) return rc;
+    }
+    vh_start(h, gi + 1);                               // the next group's plan is built while this one streams
+    return CC_OK;
+}
+
+// frames [w0, w0 + wn) of group gi, src / dst: the window's first frame, frames pitch * sz2 apart, on st;
+// *ok = false: the group has no plan (the caller runs its single-view launches)
+int rect_vh_launch_f32c1(RectViewsHost* h, int gi, int w0, int wn, const float* src, float* dst, float fill,
+                         unsigned flags, cudaStream_t st, bool* ok) {
+    *ok = false;
+    if (!h->mp[gi]) return CC_OK;
+    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->nviews - v0);
+    const bool exact = !(flags & CC_COORD_F32);
+    ViewsLaunch L;
+    int rc = views_window(h->ctx, h->mp[gi], h->chs + v0, h->ratios + v0, h->axs_mins + 2 * v0, nv, src, 4, kTLf, h->sz1,
+                          h->sz2, h->pitch, h->pitch * (size_t)h->sz2, h->fpv, w0, wn, exact ? kFGf32Exact : kFGf32Fast, &L, ok);
+    if (rc || !*ok) return rc;
+    h->used[gi] = 1;
+    return views_run_f32c1(h->ctx, &L, exact, src, dst, fill, st);
+}
+
+int rect_vh_launch_u8c3(RectViewsHost* h, int gi, int w0, int wn, const uint8_t* src, uint8_t* dst, const uint8_t fill[3],
+                        unsigned flags, cudaStream_t st, bool* ok) {
+    *ok = false;
+    if (!h->mp[gi]) return CC_OK;
+    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->nviews - v0);
+    const bool exact = !(flags & CC_COORD_F32);
+    ViewsLaunch L;
+    int rc = views_window(h->ctx, h->mp[gi], h->chs + v0, h->ratios + v0, h->axs_mins + 2 * v0, nv, src, 3, kTLu, h->sz1,
+                          h->sz2, h->pitch, h->pitch * (size_t)h->sz2, h->fpv, w0, wn, exact ? kFGu8Exact : kFGu8Fast, &L, ok);
+    if (rc || !*ok) return rc;
+    h->used[gi] = 1;
+    return views_run_u8c3(h->ctx, &L, exact, src, dst, fill, h->sz1, h->sz2, h->pitch, st);
+}
+
+// no chunk of this call reads group gi's plan after the ones enqueued so far: its fence joins the slot streams
+void rect_vh_retire(RectViewsHost* h, int gi) {
+    cc_ctx* ctx = h->ctx;
+    MultiPlan* mp = gi < h->ngroups ? h->mp[gi] : nullptr;
+    if (!mp || !h->used[gi]) return;
+    h->used[gi] = 0;
+    for (int k = 0; k < cc_ctx::NSLOT; ++k) {
+        if (!ctx->pipe_stream[k]) continue;
+        cudaEventRecord(ctx->rect_join_event[k], ctx->pipe_stream[k]);
+        cudaStreamWaitEvent(ctx->rect_join, ctx->rect_join_event[k], 0);
+    }
+    multi_read_end(mp, ctx->rect_join);
+}
+
+// after the last chunk (or an error): every plan fenced, the uploads complete, the host tables released
+int rect_vh_end(RectViewsHost* h) {
+    if (!h) return CC_OK;
+    cc_ctx* ctx = h->ctx;
+    if (h->job.joinable()) h->job.join();
+    if (h->job_out) multi_free(h->job_out);
+    for (int gi = 0; gi < h->ngroups; ++gi) rect_vh_retire(h, gi);
+    const cudaError_t e = cudaStreamSynchronize(ctx->rect_upload);
+    for (MultiPlan* mp : h->installed) {
+        std::vector<TileHdr>().swap(mp->h_hdr);
+        std::vector<double>().swap(mp->h_q2);
+        if (mp->ready) { cudaEventDestroy(mp->ready); mp->ready = nullptr; }
+    }
+    delete h;
+    return e == cudaSuccess ? CC_OK : cuda_fail(e, "plan upload");
 }
 
 int rectify_views_per_launch() { return kMaxViews; }

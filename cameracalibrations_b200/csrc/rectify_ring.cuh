@@ -66,6 +66,8 @@ __device__ __forceinline__ uint32_t take_ticket(RectSched* sched, int lane_id) {
 // the odd end of a unit -- so the consumers pay one hand-over per pair)
 // VIEWS: frames with different views in one launch -- the third unit coordinate counts (view, frame group of
 // the view), the view's tables start at view * tiles / view * sz2, and the view index travels in the header.
+// The launch may cover a window of the group's frames (TileCfg.w0 / g0, g.nframes = its length): the frame
+// index published to the consumers and given to TMA is relative to the window, the view stays the group's.
 template <bool EXACT, int TL, int PXB, int NF = 1, bool VIEWS = false>
 __device__ __forceinline__ void producer_loop(const CUtensorMap* tmap, const RectGeom& g, const TileCfg& cfg,
                                               const TileHdr* __restrict__ plan,
@@ -89,10 +91,13 @@ __device__ __forceinline__ void producer_loop(const CUtensorMap* tmap, const Rec
         const double* q2_v = q2tab;
         [[maybe_unused]] uint32_t view = 0;
         if (VIEWS) {
-            const uint32_t grp = r / (uint32_t)cfg.ntiles2;
+            const uint32_t grp = cfg.g0 + r / (uint32_t)cfg.ntiles2;
             view = grp / (uint32_t)cfg.gpv;
             f0 = (int)view * cfg.fpv + (int)(grp - view * (uint32_t)cfg.gpv) * cfg.fg;
             f1 = min(f0 + cfg.fg, ((int)view + 1) * cfg.fpv);
+            // the frame window (TileCfg.w0): frames of the group -> frames of the launch
+            f0 = max(f0, cfg.w0) - cfg.w0;
+            f1 = min(f1, cfg.w0 + g.nframes) - cfg.w0;
             hdr_v = plan + (size_t)view * cfg.tiles;
             q2_v = q2tab + (size_t)view * g.sz2;
         }

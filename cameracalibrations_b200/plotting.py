@@ -68,9 +68,9 @@ def plot(c: Calibration, imgpointss, n_corners, checker_size, sz, dir="debug", c
     for i in range(len(files)):
         _draw_crosses(frames[i], ips[i], n1, RED)
     tf = [image_transformations(c, i, ips, checker_size, n_corners, sz) for i in range(len(files))]
-    d_frames = torch.from_numpy(frames).cuda()
-    warped = warp_views(c, list(range(len(files))), d_frames, [t[0] for t in tf], [t[1] for t in tf],
-                        fill=(0, 0, 0), coord=coord).cpu().numpy()
+    # host frames: one pipelined call over all views (cc_rectify_views_u8c3_host)
+    warped = warp_views(c, list(range(len(files))), frames, [t[0] for t in tf], [t[1] for t in tf],
+                        fill=(0, 0, 0), coord=coord)
     written = []
     for i, f in enumerate(files):
         ratio, axs = tf[i]

@@ -207,6 +207,23 @@ int cc_rectify_u8c3_views(cc_ctx *ctx, const cc_intr *intr, const cc_view *views
                           uint8_t *dst, int sz1, int sz2, size_t pitch, size_t frame_stride,
                           int frames_per_view, const uint8_t fill[3], unsigned flags,
                           void *stream);
+/* The same from HOST memory (pinned or pageable): arguments as cc_rectify_*_views, any number
+ * of views; returns when dst holds the result.  The frames stream through the chunk pipeline of
+ * cc_rectify_*_host (4 slot streams, ~32 MB chunks, CAMCAL_CHUNK_MB / CAMCAL_CHUNK_RAMP); a chunk
+ * may start or end inside a view and span two 64-view groups, and makes one staged launch per
+ * group it touches.  Each group's plan is obtained once per call; a missing one is built on host
+ * threads while the previous group streams.  A group the staged kernels cannot take (1080p u8c3
+ * lines of 3240 bytes, CC_GATHER_DIRECT, footprints too large to stage) runs one launch per view
+ * on the chunk's stream.  Every frame is bit-identical to cc_rectify_*_views; host padding
+ * between lines and frames is never written. */
+int cc_rectify_views_f32c1_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                                const double *ratios, const int64_t *axs_mins, const float *src,
+                                float *dst, int sz1, int sz2, size_t pitch, size_t frame_stride,
+                                int frames_per_view, float fill, unsigned flags);
+int cc_rectify_views_u8c3_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                               const double *ratios, const int64_t *axs_mins, const uint8_t *src,
+                               uint8_t *dst, int sz1, int sz2, size_t pitch, size_t frame_stride,
+                               int frames_per_view, const uint8_t fill[3], unsigned flags);
 /* the map alone (source row/col sampled by each output pixel), FP64, frame layout */
 int cc_rectify_map_f64(cc_ctx *ctx, const cc_intr *intr, const cc_view *view, double ratio,
                        const int64_t axs_min[2], double *map_row, double *map_col, int sz1,

@@ -198,23 +198,41 @@ function warp_batch(c::Calibration, i::Int, imgs::Array{UInt8,4}, ratio::Float64
     out
 end
 
-# The reference's plot loop (src/plot_calibration.jl:36-42) in ONE call: frame v of `imgs` is
-# rectified with view v, ratios[v] and axs[v].  Device-resident arrays are what cc_rectify_*_views
-# takes; this host convenience copies in and out around it.
+# The reference's plot loop (src/plot_calibration.jl:36-42) in ONE call: frames of `imgs` belong to the
+# views in order, nframes ÷ length(views) each (frames [(v-1)k+1, vk] use view v, ratios[v] and axs[v]).
+# Host arrays go through cc_rectify_views_*_host: one chunk pipeline over all views, with the views' tile
+# plans built while the frames stream.
 function warp_views(d::DeviceCalibration, imgs::Array{Float32,3}, ratios::Vector{Float64},
                     axss::Vector{<:NTuple{2,<:AbstractUnitRange}}; fill::Float32 = NaN32, fast::Bool = false)
     sz1, sz2, nf = size(imgs)
-    @assert nf == length(d.views) == length(ratios) == length(axss)
+    nv = length(d.views)
+    @assert nv > 0 && nf % nv == 0 && nv == length(ratios) == length(axss)
     out = similar(imgs)
-    for v in 1:nf                                    # host arrays: one pipelined call per view
-        axs_min = Int64[first(axss[v][1]), first(axss[v][2])]
-        check(ccall((:cc_rectify_f32c1_host, libcamcal), Cint,
-                    (Ptr{Cvoid}, Ref{CcIntr}, Ref{CcView}, Cdouble, Ptr{Int64}, Ptr{Cfloat}, Ptr{Cfloat},
-                     Cint, Cint, Csize_t, Csize_t, Cint, Cfloat, Cuint),
-                    context().handle, Ref(d.intr), Ref(d.views[v]), ratios[v], axs_min,
-                    pointer(imgs, (v - 1) * sz1 * sz2 + 1), pointer(out, (v - 1) * sz1 * sz2 + 1),
-                    sz1, sz2, sz1, sz1 * sz2, 1, fill, fast ? 1 : 0))
-    end
+    axs_mins = Int64[first(a[j]) for a in axss for j in 1:2]
+    check(ccall((:cc_rectify_views_f32c1_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Cdouble}, Ptr{Int64}, Ptr{Cfloat}, Ptr{Cfloat},
+                 Cint, Cint, Csize_t, Csize_t, Cint, Cfloat, Cuint),
+                context().handle, Ref(d.intr), d.views, nv, ratios, axs_mins, imgs, out,
+                sz1, sz2, sz1, sz1 * sz2, nf ÷ nv, fill, fast ? 1 : 0))
+    out
+end
+
+# RGB{N0f8} frames -- what the reference's plot warps (RGB.(load(file))): reinterpret(UInt8, imgs) has
+# size (3, sz1, sz2, nframes) = u8c3 layout
+function warp_views(d::DeviceCalibration, imgs::Array{UInt8,4}, ratios::Vector{Float64},
+                    axss::Vector{<:NTuple{2,<:AbstractUnitRange}}; fill::NTuple{3,UInt8} = (0x00, 0x00, 0x00),
+                    fast::Bool = false)
+    @assert size(imgs, 1) == 3
+    _, sz1, sz2, nf = size(imgs)
+    nv = length(d.views)
+    @assert nv > 0 && nf % nv == 0 && nv == length(ratios) == length(axss)
+    out = similar(imgs)
+    axs_mins = Int64[first(a[j]) for a in axss for j in 1:2]
+    check(ccall((:cc_rectify_views_u8c3_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Cdouble}, Ptr{Int64}, Ptr{UInt8}, Ptr{UInt8},
+                 Cint, Cint, Csize_t, Csize_t, Cint, Ptr{UInt8}, Cuint),
+                context().handle, Ref(d.intr), d.views, nv, ratios, axs_mins, imgs, out,
+                sz1, sz2, sz1, sz1 * sz2, nf ÷ nv, UInt8[fill...], fast ? 1 : 0))
     out
 end
 
