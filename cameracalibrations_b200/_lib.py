@@ -90,6 +90,14 @@ _SIGS = {
     "cc_img2world_f32_views_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "cc_world2img_f64_views_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "cc_world2img_f32_views_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "cc_img2world_f64_aos": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _i, _sz, _vp]),
+    "cc_img2world_f32_aos": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _i, _sz, _vp]),
+    "cc_world2img_f64_aos": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _vp, _sz, _vp]),
+    "cc_world2img_f32_aos": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _vp, _sz, _vp]),
+    "cc_img2world_f64_aos_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _i, _sz]),
+    "cc_img2world_f32_aos_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _i, _sz]),
+    "cc_world2img_f64_aos_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _vp, _sz]),
+    "cc_world2img_f32_aos_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _vp, _sz]),
     "cc_rectify_f32c1": (_i, [_vp, _pI, _pV, _d, _i64p, _vp, _vp, _i, _i, _sz, _sz, _i, _f, _u, _vp]),
     "cc_rectify_u8c3": (_i, [_vp, _pI, _pV, _d, _i64p, _vp, _vp, _i, _i, _sz, _sz, _i, _u8p, _u, _vp]),
     "cc_rectify_f32c1_host": (_i, [_vp, _pI, _pV, _d, _i64p, _vp, _vp, _i, _i, _sz, _sz, _i, _f, _u]),

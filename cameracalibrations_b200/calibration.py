@@ -6,7 +6,8 @@ language are listed in INTEGRATION.md:
   * view indices are 0-based here (Julia: 1-based);
   * `c(points, idx)` takes a BATCH: an (n, 2) array is RowCol -> returns (n, 3) XYZ, an
     (n, 3) array is XYZ -> returns (n, 2) RowCol (Julia dispatches on SVector{2}/{3} and
-    is applied by broadcast, src/buildcalibrations.jl:29,46);
+    is applied by broadcast, src/buildcalibrations.jl:29,46).  The points stay interleaved, as
+    the reference keeps them: the cc_*_aos entry points read and write that layout directly;
   * numpy arrays take the `*_host` entry points (chunked H2D -> kernel -> D2H), CUDA
     torch tensors take the device entry points on torch's current stream.
 Every numeric result comes from the CUDA kernels; there is no Python/numpy fallback.
@@ -133,46 +134,38 @@ class Calibration:
     def __call__(self, pts, extrinsic=None):
         if isinstance(extrinsic, (list, tuple)):
             return self._call_views(pts, extrinsic)
-        if _is_torch(pts):
-            cols = [pts[..., i].contiguous().reshape(-1) for i in range(pts.shape[-1])]
-            stack = lambda outs: torch.stack(outs, dim=-1).reshape(*pts.shape[:-1], len(outs))
-        else:
+        if not _is_torch(pts):
             pts = np.asarray(pts)
             if pts.dtype not in (np.float32, np.float64):
                 pts = pts.astype(np.float64)
-            cols = [np.ascontiguousarray(pts[..., i]).reshape(-1) for i in range(pts.shape[-1])]
-            stack = lambda outs: np.stack(outs, axis=-1).reshape(*pts.shape[:-1], len(outs))
-        if len(cols) == 2:
-            return stack(list(self.img2world(cols[0], cols[1], extrinsic)))
-        if len(cols) == 3:
-            return stack(list(self.world2img(cols[0], cols[1], cols[2], extrinsic)))
+        if pts.shape[-1] == 2:
+            return _aos_call("img2world", self, self._index(extrinsic), pts, 3)
+        if pts.shape[-1] == 3:
+            return _aos_call("world2img", self, self._index(extrinsic), pts, 2)
         raise TypeError("points must be RowCol (.., 2) or XYZ (.., 3)")
 
     def _call_views(self, pts, extrinsics):
         """c(list of (n_i, 2 | 3) arrays, list of extrinsics): one call over all of them, the list of
-        per-view results back."""
+        per-view results back (slices of one output)."""
         if len(pts) != len(extrinsics):
             raise ValueError("need one point array per extrinsic")
         is_t = bool(pts) and _is_torch(pts[0])
         if is_t:
             pts = [p.reshape(-1, p.shape[-1]) for p in pts]
-            cat = lambda cols: torch.cat(cols).contiguous()
         else:
             pts = [np.asarray(p) for p in pts]
             dt = np.float32 if pts and all(p.dtype == np.float32 for p in pts) else np.float64
             pts = [p.astype(dt, copy=False).reshape(-1, p.shape[-1]) for p in pts]
-            cat = lambda cols: np.ascontiguousarray(np.concatenate(cols))
         dims = {p.shape[-1] for p in pts}
         if len(dims) != 1 or not dims <= {2, 3}:
             raise TypeError("points must all be RowCol (n, 2) or all XYZ (n, 3)")
         d = dims.pop()
         counts = [int(p.shape[0]) for p in pts]
-        cols = [cat([p[:, i] for p in pts]) for i in range(d)]
-        outs = (self.img2world_views(cols[0], cols[1], extrinsics, counts) if d == 2
-                else self.world2img_views(cols[0], cols[1], cols[2], extrinsics, counts))
-        stacked = torch.stack(outs, dim=-1) if is_t else np.stack(outs, axis=-1)
+        segs = self._segments(extrinsics, counts)
+        cat = torch.cat(pts) if is_t else np.concatenate(pts)
+        out = _aos_call("img2world" if d == 2 else "world2img", self, segs, cat, 5 - d)
         bounds = np.cumsum([0] + counts)
-        return [stacked[int(a):int(b)] for a, b in zip(bounds[:-1], bounds[1:])]
+        return [out[int(a):int(b)] for a, b in zip(bounds[:-1], bounds[1:])]
 
 
 def rectification(c: Calibration, extrinsic=None):
@@ -180,16 +173,47 @@ def rectification(c: Calibration, extrinsic=None):
     vi = c._index(extrinsic)
 
     def f(rc):
-        if _is_torch(rc):
-            x, y = c.img2world(rc[..., 0].contiguous().reshape(-1), rc[..., 1].contiguous().reshape(-1),
-                               vi, want_z=False)
-            return torch.stack([x, y], dim=-1).reshape(*rc.shape[:-1], 2)
-        rc = np.asarray(rc, dtype=np.float64) if np.asarray(rc).dtype != np.float32 else np.asarray(rc)
-        x, y = c.img2world(np.ascontiguousarray(rc[..., 0]).reshape(-1),
-                           np.ascontiguousarray(rc[..., 1]).reshape(-1), vi, want_z=False)
-        return np.stack([x, y], axis=-1).reshape(*rc.shape[:-1], 2)
+        if not _is_torch(rc):
+            rc = np.asarray(rc)
+            if rc.dtype != np.float32:
+                rc = rc.astype(np.float64, copy=False)
+        if rc.shape[-1] != 2:                  # (row, col) are the first two coordinates
+            rc = rc[..., :2]
+            if rc.shape[-1] != 2:
+                raise IndexError("points need a row and a column coordinate")
+        return _aos_call("img2world", c, vi, rc, 2)
 
     return f
+
+
+def _aos_call(kind, c: Calibration, vi, pts, out_dim: int):
+    """One cc_{kind}_{f64|f32}_aos[_host] call on interleaved points pts (..., 2 | 3); returns (..., out_dim)
+    in pts' dtype.  vi: a view index, or the (views, nviews, offsets) of Calibration._segments.  A
+    C-contiguous input is passed as is; any other is copied once."""
+    segs = isinstance(vi, tuple)
+    views = (_np_ptr(vi[0]), vi[1], _np_ptr(vi[2])) if segs else (C.byref(c._views[vi]), 1, None)
+    lead, in_dim = tuple(pts.shape[:-1]), int(pts.shape[-1])
+    if _is_torch(pts):
+        if not pts.is_cuda:
+            raise TypeError("torch inputs must be CUDA tensors (numpy arrays take the host path)")
+        if pts.dtype not in (torch.float32, torch.float64):
+            raise TypeError("float32 or float64 points only")
+        pts = pts.contiguous()
+        out = torch.empty(lead + (out_dim,), dtype=pts.dtype, device=pts.device)
+        dev = pts.device.index if pts.device.index is not None else torch.cuda.current_device()
+        ctx, ptr, host, tail = _lib.context(dev), _t_ptr, "", (_stream_ptr(dev),)
+        sfx = "f64" if pts.dtype == torch.float64 else "f32"
+    else:
+        pts = np.ascontiguousarray(pts, dtype=np.float32 if pts.dtype == np.float32 else np.float64)
+        out = np.empty(lead + (out_dim,), dtype=pts.dtype)
+        ctx, ptr, host, tail = _lib.context(_default_device()), _np_ptr, "_host", ()
+        sfx = "f64" if pts.dtype == np.float64 else "f32"
+    n = math.prod(lead)
+    _check_total(vi, n, segs)
+    fn = getattr(lib, f"cc_{kind}_{sfx}_aos{host}")
+    io = (ptr(pts), ptr(out), out_dim) if kind == "img2world" else (ptr(pts), in_dim, ptr(out))
+    check(fn(ctx.handle, C.byref(c._intr), *views, *io, C.c_size_t(n), *tail))
+    return out
 
 
 def _point_call(kind, c: Calibration, vi, ins, nout: int, flag: bool):

@@ -43,6 +43,12 @@ int launch_img2world_views(cc_ctx*, const PointTable&, size_t, int, int, const T
 template <typename T>
 int launch_world2img_views(cc_ctx*, const PointTable&, size_t, int, int, const T*, const T*, const T*, T*, T*,
                            size_t, cudaStream_t);
+template <typename T>
+int launch_img2world_aos(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const T*, T*, bool, size_t,
+                         cudaStream_t);
+template <typename T>
+int launch_world2img_aos(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const T*, bool, T*, size_t,
+                         cudaStream_t);
 int check_rect_args(const int64_t axs_min[2], int sz1, int sz2, size_t pitch, size_t frame_stride,
                     int nframes, double ratio);
 int launch_rectify_f32c1(cc_ctx*, const ChainD&, double, const int64_t[2], const float*, float*, int,
@@ -248,31 +254,37 @@ static int views_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, 
 // Host form: the table goes up once on slot 0's stream, every slot's stream waits for it, then the chunk
 // pipeline of the single-view *_host calls runs with one drain at the end.  A chunk's launch gets the
 // segments it covers and its first point's index in the call.  CHUNK(tb, k, off, m, lo, hi, cap) moves
-// and maps points [off, off + m) through slot k.
+// and maps points [off, off + m) through slot k.  !table: a call whose launches take one chain by value;
+// nothing is uploaded and offsets are not read (lo = hi = 0).
 template <typename T, typename CHUNK>
 static int views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
-                      size_t n, bool to_img, size_t in_arrays, size_t out_arrays, CHUNK chunk) {
+                      size_t n, bool to_img, bool table, size_t in_arrays, size_t out_arrays, CHUNK chunk) {
     int rc;
     CC_GUARD;
     if ((rc = enter(ctx))) return rc;
     if (n == 0) return CC_OK;
-    const std::vector<ChainD> chs = view_chains(intr, views, nviews);
-    if ((rc = ensure_stream(ctx, 0))) return rc;
-    PointTable tb;
-    if ((rc = point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, ctx->pipe_stream[0], &tb))) return rc;
-    if ((rc = point_table_release(ctx, ctx->pipe_stream[0]))) return rc;
     const size_t cap = n < kPointChunk ? round_up(n, 64) : kPointChunk;
     const size_t nchunks = (n + cap - 1) / cap;
-    for (int k = 1; k < cc_ctx::NSLOT && (size_t)k < nchunks; ++k) {
-        if ((rc = ensure_stream(ctx, k))) return rc;
-        CC_CUDA(cudaStreamWaitEvent(ctx->pipe_stream[k], ctx->pt_event, 0));
+    PointTable tb{};
+    if (table) {
+        const std::vector<ChainD> chs = view_chains(intr, views, nviews);
+        if ((rc = ensure_stream(ctx, 0))) return rc;
+        if ((rc = point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, ctx->pipe_stream[0], &tb))) return rc;
+        if ((rc = point_table_release(ctx, ctx->pipe_stream[0]))) return rc;
+        for (int k = 1; k < cc_ctx::NSLOT && (size_t)k < nchunks; ++k) {
+            if ((rc = ensure_stream(ctx, k))) return rc;
+            CC_CUDA(cudaStreamWaitEvent(ctx->pipe_stream[k], ctx->pt_event, 0));
+        }
     }
     size_t off = 0;
     for (int it = 0; rc == CC_OK && off < n; ++it, off += cap) {
         const int k = it % cc_ctx::NSLOT;
         const size_t m = (n - off) < cap ? (n - off) : cap;
-        const int lo = (int)(std::upper_bound(offsets, offsets + nviews + 1, off) - offsets) - 1;
-        const int hi = (int)(std::upper_bound(offsets, offsets + nviews + 1, off + m - 1) - offsets);
+        int lo = 0, hi = 0;
+        if (table) {
+            lo = (int)(std::upper_bound(offsets, offsets + nviews + 1, off) - offsets) - 1;
+            hi = (int)(std::upper_bound(offsets, offsets + nviews + 1, off + m - 1) - offsets);
+        }
         if ((rc = ensure_slot(ctx, k, in_arrays * cap * sizeof(T), out_arrays * cap * sizeof(T)))) break;
         rc = chunk(tb, k, off, m, lo, hi, cap);
     }
@@ -311,7 +323,7 @@ static int img2world_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view*
     int rc = check_views(ctx, intr, views, nviews, offsets, &n);
     if (rc) return rc;
     CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return views_host<T>(ctx, intr, views, nviews, offsets, n, false, 2, 3,
+    return views_host<T>(ctx, intr, views, nviews, offsets, n, false, true, 2, 3,
                          [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t cap) {
         cudaStream_t st = ctx->pipe_stream[k];
         T* din = static_cast<T*>(ctx->pipe_in[k]);
@@ -335,7 +347,7 @@ static int world2img_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view*
     int rc = check_views(ctx, intr, views, nviews, offsets, &n);
     if (rc) return rc;
     CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return views_host<T>(ctx, intr, views, nviews, offsets, n, true, 3, 2,
+    return views_host<T>(ctx, intr, views, nviews, offsets, n, true, true, 3, 2,
                          [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t cap) {
         cudaStream_t st = ctx->pipe_stream[k];
         T* din = static_cast<T*>(ctx->pipe_in[k]);
@@ -348,6 +360,110 @@ static int world2img_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view*
         if (r) return r;
         CC_CUDA(cudaMemcpyAsync(row + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
         CC_CUDA(cudaMemcpyAsync(col + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        return (int)CC_OK;
+    });
+}
+
+// ---- interleaved points: cc_*_aos[_host] --------------------------------------------------------
+// rc: n (row, col) pairs; pts: n points of `dim` coordinates ((x, y, z), or (x, y) with z not computed / z = 0).
+// offsets == NULL: views[0] for every point (nviews must be 1).  Otherwise the segments of cc_*_views, and
+// offsets[nviews] must be n.  Checks everything before anything is written.  *single: the view whose segment
+// holds every point (the call then takes the SINGLE kernel, chain by value, no table), or -1.
+static int check_aos(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                     const void* rc, const void* pts, int dim, size_t n, int* single) {
+    CC_REQUIRE(dim == 2 || dim == 3, "out_dim / in_dim must be 2 or 3");
+    CC_REQUIRE(n == 0 || (rc && pts), "NULL point array");
+    *single = 0;
+    if (offsets == nullptr) {
+        CC_REQUIRE(nviews == 1, "offsets == NULL needs nviews == 1");
+        return check_params(ctx, intr, views);
+    }
+    size_t total = 0;
+    const int rv = check_views(ctx, intr, views, nviews, offsets, &total);
+    if (rv) return rv;
+    CC_REQUIRE(total == n, "offsets[nviews] must equal n");
+    *single = -1;
+    for (int s = 0; s < nviews && *single < 0; ++s)
+        if (offsets[s + 1] - offsets[s] == n) *single = s;
+    return CC_OK;
+}
+
+template <typename T>
+static int img2world_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         const T* rc, T* out, int out_dim, size_t n, cudaStream_t st) {
+    int single;
+    int r = check_aos(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, &single);
+    if (r) return r;
+    if (single < 0)
+        return views_device<T>(ctx, intr, views, nviews, offsets, n, false, st, [&](const PointTable& tb, cudaStream_t s) {
+            return launch_img2world_aos<T>(ctx, nullptr, tb, 0, 0, nviews, rc, out, out_dim == 3, n, s);
+        });
+    CC_GUARD;
+    if ((r = enter(ctx))) return r;
+    ChainD ch;
+    build_chain(intr, views + single, &ch);
+    return launch_img2world_aos<T>(ctx, &ch, PointTable{}, 0, 0, 0, rc, out, out_dim == 3, n, st);
+}
+
+template <typename T>
+static int world2img_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         const T* pts, int in_dim, T* rc, size_t n, cudaStream_t st) {
+    int single;
+    int r = check_aos(ctx, intr, views, nviews, offsets, rc, pts, in_dim, n, &single);
+    if (r) return r;
+    if (single < 0)
+        return views_device<T>(ctx, intr, views, nviews, offsets, n, true, st, [&](const PointTable& tb, cudaStream_t s) {
+            return launch_world2img_aos<T>(ctx, nullptr, tb, 0, 0, nviews, pts, in_dim == 3, rc, n, s);
+        });
+    CC_GUARD;
+    if ((r = enter(ctx))) return r;
+    ChainD ch;
+    build_chain(intr, views + single, &ch);
+    return launch_world2img_aos<T>(ctx, &ch, PointTable{}, 0, 0, 0, pts, in_dim == 3, rc, n, st);
+}
+
+// One contiguous byte range per direction and chunk: one H2D and one D2H copy.  The slot buffers are
+// aligned, so every chunk takes the vector path.
+template <typename T>
+static int img2world_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const size_t* offsets, const T* rc, T* out, int out_dim, size_t n) {
+    int single;
+    int r = check_aos(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, &single);
+    if (r) return r;
+    ChainD ch;
+    if (single >= 0) build_chain(intr, views + single, &ch);
+    const size_t D = (size_t)out_dim;
+    return views_host<T>(ctx, intr, views, nviews, offsets, n, false, single < 0, 2, D,
+                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t) {
+        cudaStream_t st = ctx->pipe_stream[k];
+        T* din = static_cast<T*>(ctx->pipe_in[k]);
+        T* dout = static_cast<T*>(ctx->pipe_out[k]);
+        CC_CUDA(cudaMemcpyAsync(din, rc + 2 * off, 2 * m * sizeof(T), cudaMemcpyHostToDevice, st));
+        int e = launch_img2world_aos<T>(ctx, single >= 0 ? &ch : nullptr, tb, off, lo, hi, din, dout, D == 3, m, st);
+        if (e) return e;
+        CC_CUDA(cudaMemcpyAsync(out + D * off, dout, D * m * sizeof(T), cudaMemcpyDeviceToHost, st));
+        return (int)CC_OK;
+    });
+}
+
+template <typename T>
+static int world2img_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const size_t* offsets, const T* pts, int in_dim, T* rc, size_t n) {
+    int single;
+    int r = check_aos(ctx, intr, views, nviews, offsets, rc, pts, in_dim, n, &single);
+    if (r) return r;
+    ChainD ch;
+    if (single >= 0) build_chain(intr, views + single, &ch);
+    const size_t D = (size_t)in_dim;
+    return views_host<T>(ctx, intr, views, nviews, offsets, n, true, single < 0, D, 2,
+                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t) {
+        cudaStream_t st = ctx->pipe_stream[k];
+        T* din = static_cast<T*>(ctx->pipe_in[k]);
+        T* dout = static_cast<T*>(ctx->pipe_out[k]);
+        CC_CUDA(cudaMemcpyAsync(din, pts + D * off, D * m * sizeof(T), cudaMemcpyHostToDevice, st));
+        int e = launch_world2img_aos<T>(ctx, single >= 0 ? &ch : nullptr, tb, off, lo, hi, din, D == 3, dout, m, st);
+        if (e) return e;
+        CC_CUDA(cudaMemcpyAsync(rc + 2 * off, dout, 2 * m * sizeof(T), cudaMemcpyDeviceToHost, st));
         return (int)CC_OK;
     });
 }
@@ -614,6 +730,39 @@ int cc_world2img_f32_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view*
                                 const size_t* offsets, const float* x, const float* y, const float* z,
                                 float* row, float* col) {
     return world2img_views_host<float>(ctx, intr, views, nviews, offsets, x, y, z, row, col);
+}
+
+int cc_img2world_f64_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         const double* rc, double* out, int out_dim, size_t n, void* stream) {
+    return img2world_aos<double>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, (cudaStream_t)stream);
+}
+int cc_img2world_f32_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         const float* rc, float* out, int out_dim, size_t n, void* stream) {
+    return img2world_aos<float>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, (cudaStream_t)stream);
+}
+int cc_world2img_f64_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         const double* pts, int in_dim, double* rc, size_t n, void* stream) {
+    return world2img_aos<double>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n, (cudaStream_t)stream);
+}
+int cc_world2img_f32_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         const float* pts, int in_dim, float* rc, size_t n, void* stream) {
+    return world2img_aos<float>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n, (cudaStream_t)stream);
+}
+int cc_img2world_f64_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const size_t* offsets, const double* rc, double* out, int out_dim, size_t n) {
+    return img2world_aos_host<double>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n);
+}
+int cc_img2world_f32_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const size_t* offsets, const float* rc, float* out, int out_dim, size_t n) {
+    return img2world_aos_host<float>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n);
+}
+int cc_world2img_f64_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const size_t* offsets, const double* pts, int in_dim, double* rc, size_t n) {
+    return world2img_aos_host<double>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n);
+}
+int cc_world2img_f32_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const size_t* offsets, const float* pts, int in_dim, float* rc, size_t n) {
+    return world2img_aos_host<float>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n);
 }
 
 // ---- rectification ---------------------------------------------------------------

@@ -1,4 +1,4 @@
-// pointmap.cu -- batched pixel<->world maps over SoA point sets.
+// pointmap.cu -- batched pixel<->world maps over SoA point sets and interleaved (AoS) points.
 //
 // Replaces the Julia broadcasts c.(imgpoints, i) / c.(objpoints, i)
 // (src/buildcalibrations.jl:29,46) over the callables of src/meta.jl:82,88.
@@ -76,17 +76,33 @@ template <typename Row> struct ViewTable {
 template <typename S> struct IsTable : std::false_type {};
 template <typename Row> struct IsTable<ViewTable<Row>> : std::true_type {};
 
+// ---- layouts ---------------------------------------------------------------------------------------
+// SoA: one array per coordinate.  AoS: one array of packed points, D coordinates each ((row, col) pairs,
+// (x, y, z) or (x, y) points).  A group of N consecutive points (N = Vec<T>::N) is D 16-byte vectors in
+// either layout: vector g of each coordinate array (SoA), or vectors D*g .. D*g + D-1 of the packed array
+// (AoS).  Coordinate d of the group's point e is lane e of vector d (SoA), or scalar k = D*e + d of the
+// group: lane k % N of vector k / N (AoS).  The indices are compile-time constants after unrolling, so the
+// AoS permutation is register moves only.
+template <typename T, int D, bool AOS>
+__device__ __forceinline__ T& coord(typename Vec<T>::type* g, int d, int e) {
+    constexpr int N = Vec<T>::N;
+    if constexpr (AOS) return lane<T>(g[(D * e + d) / N], (D * e + d) % N);
+    else return lane<T>(g[d], e);
+}
+
 // ---- per-point loops ------------------------------------------------------------------------------
-// Points [p0, p1) (p0 a multiple of N): vectors of N points when vec_ok, thread `tid` of `nthreads`
-// taking vectors tid, tid + nthreads, ... two at a time, then the scalar tail; scalar throughout when
-// !vec_ok.  chain(p) gives the chain of point p, asked for in increasing p within a thread.
-template <typename T, bool HAS_Z, typename CH>
+// Points [p0, p1) (p0 a multiple of N): groups of N points through 16-byte vectors when vec_ok, thread
+// `tid` of `nthreads` taking groups tid, tid + nthreads, ... two at a time, then the scalar tail; scalar
+// throughout when !vec_ok.  chain(p) gives the chain of point p, asked for in increasing p within a thread.
+// AOS: `row` holds the (row, col) pairs and `x` the (x, y[, z]) points; col, y and z are not used.
+template <typename T, bool HAS_Z, bool AOS, typename CH>
 __device__ __forceinline__ void img2world_range(CH&& chain, const T* __restrict__ row,
                                                  const T* __restrict__ col, T* __restrict__ x,
                                                  T* __restrict__ y, T* __restrict__ z, size_t p0,
                                                  size_t p1, size_t tid, size_t nthreads, bool vec_ok) {
     using V = typename Vec<T>::type;
     constexpr int N = Vec<T>::N;
+    constexpr int DO = HAS_Z ? 3 : 2;
     size_t done = p0;
     if (vec_ok) {
         const size_t nvec = p1 / N;
@@ -96,24 +112,33 @@ __device__ __forceinline__ void img2world_range(CH&& chain, const T* __restrict_
         V* yv = reinterpret_cast<V*>(y);
         V* zv = reinterpret_cast<V*>(z);
         for (size_t i = p0 / N + tid; i < nvec; i += nthreads * kUnroll) {
-            V r[kUnroll], c[kUnroll];
+            V in[kUnroll][2];
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
                 const size_t j = i + u * nthreads;
-                if (j < nvec) { r[u] = ldg_stream(rv + j); c[u] = ldg_stream(cv + j); }
+                if (j < nvec) {
+                    if constexpr (AOS) { in[u][0] = ldg_stream(rv + 2 * j); in[u][1] = ldg_stream(rv + 2 * j + 1); }
+                    else { in[u][0] = ldg_stream(rv + j); in[u][1] = ldg_stream(cv + j); }
+                }
             }
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
                 const size_t j = i + u * nthreads;
                 if (j < nvec) {
-                    V ox, oy, oz;
+                    V o[3];            // o[2]: z lanes that are computed but not stored when !HAS_Z
 #pragma unroll
                     for (int e = 0; e < N; ++e)
-                        img2world(chain(j * N + e), lane<T>(r[u], e), lane<T>(c[u], e), lane<T>(ox, e),
-                                  lane<T>(oy, e), lane<T>(oz, e));
-                    stg_stream(xv + j, ox);
-                    stg_stream(yv + j, oy);
-                    if (HAS_Z) stg_stream(zv + j, oz);
+                        img2world(chain(j * N + e), coord<T, 2, AOS>(in[u], 0, e), coord<T, 2, AOS>(in[u], 1, e),
+                                  coord<T, DO, AOS>(o, 0, e), coord<T, DO, AOS>(o, 1, e),
+                                  HAS_Z ? coord<T, DO, AOS>(o, 2, e) : lane<T>(o[2], e));
+                    if constexpr (AOS) {
+#pragma unroll
+                        for (int d = 0; d < DO; ++d) stg_stream(xv + DO * j + d, o[d]);
+                    } else {
+                        stg_stream(xv + j, o[0]);
+                        stg_stream(yv + j, o[1]);
+                        if (HAS_Z) stg_stream(zv + j, o[2]);
+                    }
                 }
             }
         }
@@ -121,19 +146,27 @@ __device__ __forceinline__ void img2world_range(CH&& chain, const T* __restrict_
     }
     for (size_t i = done + tid; i < p1; i += nthreads) {   // tail / unaligned pointers
         T ox, oy, oz;
-        img2world(chain(i), row[i], col[i], ox, oy, oz);
-        x[i] = ox; y[i] = oy;
-        if (HAS_Z) z[i] = oz;
+        if constexpr (AOS) {
+            img2world(chain(i), row[2 * i], row[2 * i + 1], ox, oy, oz);
+            x[DO * i] = ox; x[DO * i + 1] = oy;
+            if (HAS_Z) x[DO * i + 2] = oz;
+        } else {
+            img2world(chain(i), row[i], col[i], ox, oy, oz);
+            x[i] = ox; y[i] = oy;
+            if (HAS_Z) z[i] = oz;
+        }
     }
 }
 
-template <typename T, bool HAS_Z, typename CH>
+// AOS: `x` holds the (x, y[, z]) points and `row` the (row, col) pairs; y, z and col are not used.
+template <typename T, bool HAS_Z, bool AOS, typename CH>
 __device__ __forceinline__ void world2img_range(CH&& chain, const T* __restrict__ x,
                                                 const T* __restrict__ y, const T* __restrict__ z,
                                                 T* __restrict__ row, T* __restrict__ col, size_t p0,
                                                 size_t p1, size_t tid, size_t nthreads, bool vec_ok) {
     using V = typename Vec<T>::type;
     constexpr int N = Vec<T>::N;
+    constexpr int DI = HAS_Z ? 3 : 2;
     size_t done = p0;
     if (vec_ok) {
         const size_t nvec = p1 / N;
@@ -143,28 +176,38 @@ __device__ __forceinline__ void world2img_range(CH&& chain, const T* __restrict_
         V* rv = reinterpret_cast<V*>(row);
         V* cv = reinterpret_cast<V*>(col);
         for (size_t i = p0 / N + tid; i < nvec; i += nthreads * kUnroll) {
-            V a[kUnroll], b[kUnroll], c[kUnroll];
+            V in[kUnroll][3];
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
                 const size_t j = i + u * nthreads;
                 if (j < nvec) {
-                    a[u] = ldg_stream(xv + j);
-                    b[u] = ldg_stream(yv + j);
-                    if (HAS_Z) c[u] = ldg_stream(zv + j);
+                    if constexpr (AOS) {
+#pragma unroll
+                        for (int d = 0; d < DI; ++d) in[u][d] = ldg_stream(xv + DI * j + d);
+                    } else {
+                        in[u][0] = ldg_stream(xv + j);
+                        in[u][1] = ldg_stream(yv + j);
+                        if (HAS_Z) in[u][2] = ldg_stream(zv + j);
+                    }
                 }
             }
 #pragma unroll
             for (int u = 0; u < kUnroll; ++u) {
                 const size_t j = i + u * nthreads;
                 if (j < nvec) {
-                    V orow, ocol;
+                    V o[2];
 #pragma unroll
                     for (int e = 0; e < N; ++e)
-                        world2img(chain(j * N + e), lane<T>(a[u], e), lane<T>(b[u], e),
-                                  HAS_Z ? lane<T>(c[u], e) : T(0), lane<T>(orow, e),
-                                  lane<T>(ocol, e));
-                    stg_stream(rv + j, orow);
-                    stg_stream(cv + j, ocol);
+                        world2img(chain(j * N + e), coord<T, DI, AOS>(in[u], 0, e), coord<T, DI, AOS>(in[u], 1, e),
+                                  HAS_Z ? coord<T, DI, AOS>(in[u], 2, e) : T(0), coord<T, 2, AOS>(o, 0, e),
+                                  coord<T, 2, AOS>(o, 1, e));
+                    if constexpr (AOS) {
+                        stg_stream(rv + 2 * j, o[0]);
+                        stg_stream(rv + 2 * j + 1, o[1]);
+                    } else {
+                        stg_stream(rv + j, o[0]);
+                        stg_stream(cv + j, o[1]);
+                    }
                 }
             }
         }
@@ -172,8 +215,13 @@ __device__ __forceinline__ void world2img_range(CH&& chain, const T* __restrict_
     }
     for (size_t i = done + tid; i < p1; i += nthreads) {
         T orow, ocol;
-        world2img(chain(i), x[i], y[i], HAS_Z ? z[i] : T(0), orow, ocol);
-        row[i] = orow; col[i] = ocol;
+        if constexpr (AOS) {
+            world2img(chain(i), x[DI * i], x[DI * i + 1], HAS_Z ? x[DI * i + 2] : T(0), orow, ocol);
+            row[2 * i] = orow; row[2 * i + 1] = ocol;
+        } else {
+            world2img(chain(i), x[i], y[i], HAS_Z ? z[i] : T(0), orow, ocol);
+            row[i] = orow; col[i] = ocol;
+        }
     }
 }
 
@@ -255,13 +303,13 @@ img2world_kernel(const SRC src, const T* __restrict__ row, const T* __restrict__
                  T* __restrict__ x, T* __restrict__ y, T* __restrict__ z, size_t n, bool vec_ok) {
     if constexpr (IsTable<SRC>::value) {
         for_each_tile<T>(src, n, [&](size_t p0, size_t p1, auto&& chain) {
-            img2world_range<T, HAS_Z>(chain, row, col, x, y, z, p0, p1, threadIdx.x, kThreads, vec_ok);
+            img2world_range<T, HAS_Z, false>(chain, row, col, x, y, z, p0, p1, threadIdx.x, kThreads, vec_ok);
         });
     } else {
         const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
         const size_t nthreads = (size_t)gridDim.x * kThreads;
-        img2world_range<T, HAS_Z>([&](size_t) -> const Chain<T>& { return src; }, row, col, x, y, z,
-                                  0, n, tid, nthreads, vec_ok);
+        img2world_range<T, HAS_Z, false>([&](size_t) -> const Chain<T>& { return src; }, row, col, x, y, z,
+                                         0, n, tid, nthreads, vec_ok);
     }
 }
 
@@ -272,13 +320,47 @@ world2img_kernel(const SRC src, const T* __restrict__ x, const T* __restrict__ y
                  bool vec_ok) {
     if constexpr (IsTable<SRC>::value) {
         for_each_tile<T>(src, n, [&](size_t p0, size_t p1, auto&& chain) {
-            world2img_range<T, HAS_Z>(chain, x, y, z, row, col, p0, p1, threadIdx.x, kThreads, vec_ok);
+            world2img_range<T, HAS_Z, false>(chain, x, y, z, row, col, p0, p1, threadIdx.x, kThreads, vec_ok);
         });
     } else {
         const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
         const size_t nthreads = (size_t)gridDim.x * kThreads;
-        world2img_range<T, HAS_Z>([&](size_t) -> const Chain<T>& { return src; }, x, y, z, row, col,
-                                  0, n, tid, nthreads, vec_ok);
+        world2img_range<T, HAS_Z, false>([&](size_t) -> const Chain<T>& { return src; }, x, y, z, row, col,
+                                         0, n, tid, nthreads, vec_ok);
+    }
+}
+
+// AoS kernels: rc = n (row, col) pairs; xyz = n points of 3 (HAS_Z) or 2 coordinates.  Their bodies repeat
+// the SoA kernels' instead of sharing a device function: with one, the SoA kernels' code changed.
+template <typename T, bool HAS_Z, typename SRC = Chain<T>>
+__global__ void __launch_bounds__(kThreads, kTableMinBlocks<SRC, std::is_same<T, double>::value>)
+img2world_aos_kernel(const SRC src, const T* __restrict__ rc, T* __restrict__ xyz, size_t n, bool vec_ok) {
+    if constexpr (IsTable<SRC>::value) {
+        for_each_tile<T>(src, n, [&](size_t p0, size_t p1, auto&& chain) {
+            img2world_range<T, HAS_Z, true>(chain, rc, nullptr, xyz, nullptr, nullptr, p0, p1, threadIdx.x, kThreads,
+                                            vec_ok);
+        });
+    } else {
+        const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
+        const size_t nthreads = (size_t)gridDim.x * kThreads;
+        img2world_range<T, HAS_Z, true>([&](size_t) -> const Chain<T>& { return src; }, rc, nullptr, xyz, nullptr,
+                                        nullptr, 0, n, tid, nthreads, vec_ok);
+    }
+}
+
+template <typename T, bool HAS_Z, typename SRC = Chain<T>>
+__global__ void __launch_bounds__(kThreads, kTableMinBlocks<SRC, std::is_same<T, float>::value>)
+world2img_aos_kernel(const SRC src, const T* __restrict__ xyz, T* __restrict__ rc, size_t n, bool vec_ok) {
+    if constexpr (IsTable<SRC>::value) {
+        for_each_tile<T>(src, n, [&](size_t p0, size_t p1, auto&& chain) {
+            world2img_range<T, HAS_Z, true>(chain, xyz, nullptr, nullptr, rc, nullptr, p0, p1, threadIdx.x, kThreads,
+                                            vec_ok);
+        });
+    } else {
+        const size_t tid = (size_t)blockIdx.x * kThreads + threadIdx.x;
+        const size_t nthreads = (size_t)gridDim.x * kThreads;
+        world2img_range<T, HAS_Z, true>([&](size_t) -> const Chain<T>& { return src; }, xyz, nullptr, nullptr, rc,
+                                        nullptr, 0, n, tid, nthreads, vec_ok);
     }
 }
 
@@ -461,6 +543,67 @@ int launch_world2img_views(cc_ctx* ctx, const PointTable& tb, size_t base, int s
     CC_CUDA(cudaGetLastError());
     return CC_OK;
 }
+
+// ---- interleaved points (cc_*_aos[_host]) ------------------------------------------------------
+// chd != nullptr: the SINGLE kernel with that chain.  Otherwise the TABLE kernel over tb, points base + [0, n)
+// of segments [seg_lo, seg_hi), as launch_*_views.  The vector path needs only the two base pointers aligned.
+template <typename T, bool HAS_Z>
+static void img2world_aos_grid(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo,
+                               int seg_hi, const T* rc, T* xyz, size_t n, bool vec, cudaStream_t st) {
+    if (chd) {
+        auto k = img2world_aos_kernel<T, HAS_Z>;
+        k<<<grid_for(ctx, k, vec ? n / Vec<T>::N + 1 : n), kThreads, 0, st>>>(pick_chain<T>(*chd), rc, xyz, n, vec);
+    } else {
+        using Src = ViewTable<RowI2W<T>>;
+        const Src src{static_cast<const RowI2W<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
+        auto k = img2world_aos_kernel<T, HAS_Z, Src>;
+        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, rc, xyz, n, vec);
+    }
+}
+
+template <typename T, bool HAS_Z>
+static void world2img_aos_grid(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo,
+                               int seg_hi, const T* xyz, T* rc, size_t n, bool vec, cudaStream_t st) {
+    if (chd) {
+        auto k = world2img_aos_kernel<T, HAS_Z>;
+        k<<<grid_for(ctx, k, vec ? n / Vec<T>::N + 1 : n), kThreads, 0, st>>>(pick_chain<T>(*chd), xyz, rc, n, vec);
+    } else {
+        using Src = ViewTable<RowW2I<T>>;
+        const Src src{static_cast<const RowW2I<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
+        auto k = world2img_aos_kernel<T, HAS_Z, Src>;
+        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, xyz, rc, n, vec);
+    }
+}
+
+// xyz: points of 3 coordinates (has_z) or 2 (z not computed / z = 0)
+template <typename T>
+int launch_img2world_aos(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
+                         const T* rc, T* xyz, bool has_z, size_t n, cudaStream_t st) {
+    if (n == 0) return CC_OK;
+    const bool vec = aligned16(rc) && aligned16(xyz);
+    if (has_z) img2world_aos_grid<T, true>(ctx, chd, tb, base, seg_lo, seg_hi, rc, xyz, n, vec, st);
+    else img2world_aos_grid<T, false>(ctx, chd, tb, base, seg_lo, seg_hi, rc, xyz, n, vec, st);
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+template <typename T>
+int launch_world2img_aos(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
+                         const T* xyz, bool has_z, T* rc, size_t n, cudaStream_t st) {
+    if (n == 0) return CC_OK;
+    const bool vec = aligned16(xyz) && aligned16(rc);
+    if (has_z) world2img_aos_grid<T, true>(ctx, chd, tb, base, seg_lo, seg_hi, xyz, rc, n, vec, st);
+    else world2img_aos_grid<T, false>(ctx, chd, tb, base, seg_lo, seg_hi, xyz, rc, n, vec, st);
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+template int launch_img2world_aos<double>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const double*, double*, bool, size_t, cudaStream_t);
+template int launch_img2world_aos<float>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const float*, float*, bool, size_t, cudaStream_t);
+template int launch_world2img_aos<double>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const double*, bool, double*, size_t, cudaStream_t);
+template int launch_world2img_aos<float>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const float*, bool, float*, size_t, cudaStream_t);
 
 template int point_table_upload<double>(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
 template int point_table_upload<float>(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);

@@ -162,6 +162,44 @@ int cc_world2img_f32_views_host(cc_ctx *ctx, const cc_intr *intr, const cc_view 
                                 const size_t *offsets, const float *x, const float *y, const float *z,
                                 float *row, float *col);
 
+/* ---- interleaved points, the reference's own layout: Vector{RowCol} / Matrix{RowCol} (src/detect_fit.jl:19)
+ *      and arrays of XYZ are (row, col) pairs and (x, y, z) triples in memory.
+ *      rc: n x 2 interleaved (row, col).  img2world: out = n x out_dim interleaved, out_dim 3 gives
+ *      (x, y, z) = c(::RowCol, i), out_dim 2 gives (x, y) = rectification(c, i) with z not computed.
+ *      world2img: pts = n x in_dim interleaved, in_dim 3 is (x, y, z), in_dim 2 is (x, y) with z = 0.
+ *      offsets == NULL: every point uses views[0] (nviews must be 1).  offsets != NULL: the segments of
+ *      cc_*_views, and offsets[nviews] must equal n.  Every point's result is bit-identical to the SoA
+ *      entry point with the same view.  16-byte aligned rc / out / pts take 128-bit accesses; any other
+ *      base takes a scalar path with the same results.  Bad arguments (out_dim / in_dim not 2 or 3, a NULL
+ *      point array with n > 0, offsets == NULL with nviews != 1, n != offsets[nviews], and what cc_*_views
+ *      rejects) return CC_ERR_INVALID_ARG and write nothing.  n == 0: CC_OK, nothing launched.  The device
+ *      forms make ONE launch on `stream`; the *_host forms run the chunked pipeline with one contiguous
+ *      copy per direction and chunk. */
+int cc_img2world_f64_aos(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                         const size_t *offsets, const double *rc, double *out, int out_dim,
+                         size_t n, void *stream);
+int cc_img2world_f32_aos(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                         const size_t *offsets, const float *rc, float *out, int out_dim,
+                         size_t n, void *stream);
+int cc_world2img_f64_aos(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                         const size_t *offsets, const double *pts, int in_dim, double *rc,
+                         size_t n, void *stream);
+int cc_world2img_f32_aos(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                         const size_t *offsets, const float *pts, int in_dim, float *rc,
+                         size_t n, void *stream);
+int cc_img2world_f64_aos_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                              const size_t *offsets, const double *rc, double *out, int out_dim,
+                              size_t n);
+int cc_img2world_f32_aos_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                              const size_t *offsets, const float *rc, float *out, int out_dim,
+                              size_t n);
+int cc_world2img_f64_aos_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                              const size_t *offsets, const double *pts, int in_dim, double *rc,
+                              size_t n);
+int cc_world2img_f32_aos_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                              const size_t *offsets, const float *pts, int in_dim, float *rc,
+                              size_t n);
+
 /* ---- full-frame rectification:  warp(img, tform, axs)  src/plot_calibration.jl:40
  *      with tform = real2image[i] o push(.,0) o inv(LinearMap(ratio*I)) (:17-18) and
  *      axs from get_axes (:1-6): output index (I1, I2) = axs_min + (a, b), same size

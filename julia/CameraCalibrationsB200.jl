@@ -166,6 +166,63 @@ function (c::Calibration)(x::Vector{Float64}, y::Vector{Float64}, z::Vector{Floa
     rows, cols
 end
 
+# ---- the reference's own point types: c(pts, i) on Array{RowCol} / Array{XYZ}, src/meta.jl:82,88 --------
+# A RowCol is an SVector{2,Float64} and an XYZ an SVector{3,Float64}, so an Array of them is the packed
+# n × 2 / n × 3 layout of cc_*_aos: its memory goes to the library as is, and the result comes back in the
+# caller's shape.  These are methods on whole arrays; the scalar callables and `c.(pts, i)` are untouched.
+function _map_aos(sym::Symbol, c::Calibration, i::Int, pts::Array, out::Array, dim::Integer)
+    checkbounds(c.extrinsics, i)             # BoundsError like the reference
+    if sym === :img2world
+        check(ccall((:cc_img2world_f64_aos_host, libcamcal), Cint,
+                    (Ptr{Cvoid}, Ref{CcIntr}, Ref{CcView}, Cint, Ptr{Csize_t}, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Csize_t),
+                    context().handle, Ref(CcIntr(c)), Ref(CcView(c, i)), 1, C_NULL, pts, out, dim, length(pts)))
+    else
+        check(ccall((:cc_world2img_f64_aos_host, libcamcal), Cint,
+                    (Ptr{Cvoid}, Ref{CcIntr}, Ref{CcView}, Cint, Ptr{Csize_t}, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Csize_t),
+                    context().handle, Ref(CcIntr(c)), Ref(CcView(c, i)), 1, C_NULL, pts, dim, out, length(pts)))
+    end
+    out
+end
+
+"`c(pts::Array{RowCol}, i)`: `c.(pts, i)` in one call, an Array{XYZ} of the same shape."
+(c::Calibration)(pts::Array{RowCol,N}, i::Int) where {N} =
+    _map_aos(:img2world, c, i, pts, Array{XYZ,N}(undef, size(pts)), 3)
+
+"`c(pts::Array{XYZ}, i)`: `c.(pts, i)` in one call, an Array{RowCol} of the same shape."
+(c::Calibration)(pts::Array{XYZ,N}, i::Int) where {N} =
+    _map_aos(:world2img, c, i, pts, Array{RowCol,N}(undef, size(pts)), 3)
+
+"`rectification(c, i).(pts)` in one call (src/meta.jl:99): z is not computed."
+rectification_batch(c::Calibration, i::Int, pts::Array{RowCol,N}) where {N} =
+    _map_aos(:img2world, c, i, pts, Array{SVector{2,Float64},N}(undef, size(pts)), 2)
+
+# Many views: the loop `c.(pts_v, v)` over views as one concatenation, one call and one array back per view.
+function _map_aos_views(sym::Symbol, c::Calibration, ptss::AbstractVector, idxs::AbstractVector{Int}, ::Type{O},
+                        dim::Integer) where {O}
+    @assert length(ptss) == length(idxs) >= 1
+    counts = length.(ptss)
+    offsets = _offsets(c, sum(counts), idxs, counts)
+    views = [CcView(c, i) for i in idxs]
+    pts = reduce(vcat, vec.(ptss))
+    out = Vector{O}(undef, length(pts))
+    if sym === :img2world
+        check(ccall((:cc_img2world_f64_aos_host, libcamcal), Cint,
+                    (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Csize_t}, Ptr{Cdouble}, Ptr{Cdouble}, Cint, Csize_t),
+                    context().handle, Ref(CcIntr(c)), views, length(views), offsets, pts, out, dim, length(pts)))
+    else
+        check(ccall((:cc_world2img_f64_aos_host, libcamcal), Cint,
+                    (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Csize_t}, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Csize_t),
+                    context().handle, Ref(CcIntr(c)), views, length(views), offsets, pts, dim, out, length(pts)))
+    end
+    [reshape(out[offsets[s]+1:offsets[s+1]], size(ptss[s])) for s in eachindex(ptss)]
+end
+
+"`c(ptss, idxs)`: `[c.(ptss[s], idxs[s]) for s in eachindex(ptss)]` in one call."
+(c::Calibration)(ptss::AbstractVector{<:Array{RowCol}}, idxs::AbstractVector{Int}) =
+    _map_aos_views(:img2world, c, ptss, idxs, XYZ, 3)
+(c::Calibration)(ptss::AbstractVector{<:Array{XYZ}}, idxs::AbstractVector{Int}) =
+    _map_aos_views(:world2img, c, ptss, idxs, RowCol, 3)
+
 # ---- full-frame rectification: warp(img, tform, axs), src/plot_calibration.jl:40 -------------
 # `imgs` is a stack of frames of size (sz1, sz2, nframes): the memory is passed as is (first
 # RowCol axis contiguous).  `ratio` from get_ratio (:8-13), `axs` from get_axes (:1-6).
