@@ -8,6 +8,7 @@
 #include <cstring>
 #include <cmath>
 #include <new>
+#include <optional>
 
 #include "common.cuh"
 
@@ -31,24 +32,10 @@ int cuda_fail(cudaError_t e, const char* what) {
 
 // launchers implemented in the kernel translation units
 template <typename T>
-int launch_img2world(cc_ctx*, const ChainD&, const T*, const T*, T*, T*, T*, size_t, cudaStream_t);
-template <typename T>
-int launch_world2img(cc_ctx*, const ChainD&, const T*, const T*, const T*, T*, T*, size_t, cudaStream_t);
-template <typename T>
 int point_table_upload(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
 int point_table_release(cc_ctx*, cudaStream_t);
 template <typename T>
-int launch_img2world_views(cc_ctx*, const PointTable&, size_t, int, int, const T*, const T*, T*, T*, T*, size_t,
-                           cudaStream_t);
-template <typename T>
-int launch_world2img_views(cc_ctx*, const PointTable&, size_t, int, int, const T*, const T*, const T*, T*, T*,
-                           size_t, cudaStream_t);
-template <typename T>
-int launch_img2world_aos(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const T*, T*, bool, size_t,
-                         cudaStream_t);
-template <typename T>
-int launch_world2img_aos(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const T*, bool, T*, size_t,
-                         cudaStream_t);
+int launch_points(cc_ctx*, const PointSrc&, const PointIO<T>&, size_t, cudaStream_t);
 int check_rect_args(const int64_t axs_min[2], int sz1, int sz2, size_t pitch, size_t frame_stride,
                     int nframes, double ratio);
 int launch_rectify_f32c1(cc_ctx*, const ChainD&, double, const int64_t[2], const float*, float*, int,
@@ -150,126 +137,133 @@ static size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
 constexpr size_t kPointChunk = (size_t)1 << 22;   // points per pipeline stage
 
+// ---- point-map pipelines ----------------------------------------------------------
+// Every point-map entry point fills a PointIO and calls points_device or points_host.  offsets == NULL: views[0]
+// maps all `count` points (nviews must be 1).  Otherwise points [offsets[s], offsets[s+1]) use views[s], and
+// offsets[nviews] must equal count; the SoA `_views` calls pass no count, so their offsets are required and give it.
+template <typename T> static PointIO<T> soa_img2world(const T* row, const T* col, T* x, T* y, T* z) {
+    return {false, false, 2, z ? 3 : 2, {row, col}, {x, y, z}};
+}
+template <typename T> static PointIO<T> soa_world2img(const T* x, const T* y, const T* z, T* row, T* col) {
+    return {true, false, z ? 3 : 2, 2, {x, y, z}, {row, col}};
+}
+template <typename T> static PointIO<T> aos_img2world(const T* rc, T* out, int out_dim) {
+    return {false, true, 2, out_dim, {rc}, {out}};
+}
+template <typename T> static PointIO<T> aos_world2img(const T* pts, int in_dim, T* rc) {
+    return {true, true, in_dim, 2, {pts}, {rc}};
+}
+
+// Checks everything before anything is written or enqueued.  *n: the call's points.  *single: the view whose chain
+// maps every point, passed by value with no table (the SINGLE kernel), or -1 (TABLE).
 template <typename T>
-static int img2world_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const T* row,
-                          const T* col, T* x, T* y, T* z, size_t n) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    const size_t cap = n < kPointChunk ? round_up(n ? n : 1, 64) : kPointChunk;
-    size_t off = 0;
-    for (int it = 0; off < n; ++it, off += cap) {
-        const int k = it % cc_ctx::NSLOT;
-        const size_t m = (n - off) < cap ? (n - off) : cap;
-        if ((rc = ensure_slot(ctx, k, 2 * cap * sizeof(T), 3 * cap * sizeof(T)))) return rc;
-        cudaStream_t st = ctx->pipe_stream[k];
-        T* din = static_cast<T*>(ctx->pipe_in[k]);
-        T* dout = static_cast<T*>(ctx->pipe_out[k]);
-        CC_CUDA(cudaMemcpyAsync(din, row + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(din + cap, col + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        if ((rc = launch_img2world<T>(ctx, ch, din, din + cap, dout, dout + cap,
-                                      z ? dout + 2 * cap : nullptr, m, st)))
-            return rc;
-        CC_CUDA(cudaMemcpyAsync(x + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        CC_CUDA(cudaMemcpyAsync(y + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        if (z) CC_CUDA(cudaMemcpyAsync(z + off, dout + 2 * cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+static int check_points(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                        const size_t* offsets, std::optional<size_t> count, const PointIO<T>& io, size_t* n,
+                        int* single) {
+    CC_REQUIRE(io.in_dim >= 2 && io.in_dim <= 3 && io.out_dim >= 2 && io.out_dim <= 3,
+               "out_dim / in_dim must be 2 or 3");
+    if (count && offsets == nullptr) {
+        CC_REQUIRE(nviews == 1, "offsets == NULL needs nviews == 1");
+    } else {
+        CC_REQUIRE(ctx != nullptr, "ctx is NULL");
+        CC_REQUIRE(nviews >= 1, "nviews must be at least 1");
+        CC_REQUIRE(views != nullptr && offsets != nullptr, "views / offsets is NULL");
+        CC_REQUIRE(offsets[0] == 0, "offsets[0] must be 0");
+        for (int s = 0; s < nviews; ++s) CC_REQUIRE(offsets[s + 1] >= offsets[s], "offsets must not decrease");
     }
-    return drain(ctx);
+    const int rc = check_params(ctx, intr, views);
+    if (rc) return rc;
+    *n = count ? *count : offsets[nviews];
+    CC_REQUIRE(offsets == nullptr || offsets[nviews] == *n, "offsets[nviews] must equal n");
+    bool arrays = true;
+    for (int d = 0; d < io.in_arrays(); ++d) arrays = arrays && io.in[d];
+    for (int d = 0; d < io.out_arrays(); ++d) arrays = arrays && io.out[d];
+    CC_REQUIRE(*n == 0 || arrays, "NULL point array");
+    // An AoS call whose points all lie in one segment takes that view's SINGLE kernel.  The SoA `_views` calls
+    // keep the table even then: at one segment it is faster than SINGLE for some maps and slower for others
+    // (DESIGN.md §4.1).
+    *single = offsets == nullptr ? 0 : -1;
+    for (int s = 0; io.aos && offsets && s < nviews && *single < 0; ++s)
+        if (offsets[s + 1] - offsets[s] == *n) *single = s;
+    return CC_OK;
 }
 
+// SINGLE: views[single]'s chain in *ch.  TABLE: the chains of all segments, uploaded on st.  The chains are built
+// on the host, one per segment, exactly as for one view: every point's result is bit-identical to a single-view
+// call with its own view.
 template <typename T>
-static int world2img_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const T* x,
-                          const T* y, const T* z, T* row, T* col, size_t n) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    const size_t cap = n < kPointChunk ? round_up(n ? n : 1, 64) : kPointChunk;
-    size_t off = 0;
-    for (int it = 0; off < n; ++it, off += cap) {
-        const int k = it % cc_ctx::NSLOT;
-        const size_t m = (n - off) < cap ? (n - off) : cap;
-        if ((rc = ensure_slot(ctx, k, 3 * cap * sizeof(T), 2 * cap * sizeof(T)))) return rc;
-        cudaStream_t st = ctx->pipe_stream[k];
-        T* din = static_cast<T*>(ctx->pipe_in[k]);
-        T* dout = static_cast<T*>(ctx->pipe_out[k]);
-        CC_CUDA(cudaMemcpyAsync(din, x + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(din + cap, y + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        if (z) CC_CUDA(cudaMemcpyAsync(din + 2 * cap, z + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        if ((rc = launch_world2img<T>(ctx, ch, din, din + cap, z ? din + 2 * cap : nullptr, dout,
-                                      dout + cap, m, st)))
-            return rc;
-        CC_CUDA(cudaMemcpyAsync(row + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        CC_CUDA(cudaMemcpyAsync(col + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
+static int point_src(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                     int single, bool to_img, cudaStream_t st, ChainD* ch, PointSrc* src) {
+    *src = PointSrc{nullptr, {}, 0, 0, nviews};
+    if (single >= 0) {
+        build_chain(intr, views + single, ch);
+        src->chain = ch;
+        return CC_OK;
     }
-    return drain(ctx);
-}
-
-// ---- points of many views in one call -----------------------------------------------------------
-// Points [offsets[s], offsets[s+1]) use views[s].  Checks everything before anything is written;
-// *n = offsets[nviews].
-static int check_views(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                       const size_t* offsets, size_t* n) {
-    CC_REQUIRE(ctx != nullptr, "ctx is NULL");
-    CC_REQUIRE(nviews >= 1, "nviews must be at least 1");
-    CC_REQUIRE(views != nullptr && offsets != nullptr, "views / offsets is NULL");
-    CC_REQUIRE(offsets[0] == 0, "offsets[0] must be 0");
-    for (int s = 0; s < nviews; ++s) CC_REQUIRE(offsets[s + 1] >= offsets[s], "offsets must not decrease");
-    *n = offsets[nviews];
-    return check_params(ctx, intr, views);
-}
-
-// The chains are expanded on the host, one per segment, exactly as the single-view entry points do:
-// every point's result is bit-identical to a single-view call with its own view.
-static std::vector<ChainD> view_chains(const cc_intr* intr, const cc_view* views, int nviews) {
     std::vector<ChainD> chs((size_t)nviews);
     for (int s = 0; s < nviews; ++s) build_chain(intr, views + s, &chs[s]);
-    return chs;
+    return point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, st, &src->tb);
 }
 
-// Device form: one table upload and ONE launch on `st`, whatever nviews is.  IN / OUT: 2 + 3 arrays
-// (img2world) or 3 + 2 (world2img); LAUNCH runs the kernel over points base + [0, m) of segments [lo, hi).
-template <typename T, typename LAUNCH>
-static int views_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
-                        size_t n, bool to_img, cudaStream_t st, LAUNCH launch) {
-    int rc;
+// Device form: at most one table upload and ONE launch on the caller's stream, whatever nviews is.
+template <typename T>
+static int points_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                         std::optional<size_t> count, const PointIO<T>& io, void* stream) {
+    size_t n = 0;
+    int single = -1, rc = check_points(ctx, intr, views, nviews, offsets, count, io, &n, &single);
+    if (rc) return rc;
     CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    if (n == 0) return CC_OK;
-    const std::vector<ChainD> chs = view_chains(intr, views, nviews);
-    PointTable tb;
-    if ((rc = point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, st, &tb))) return rc;
-    rc = launch(tb, st);
-    const int rr = point_table_release(ctx, st);
+    if ((rc = enter(ctx)) || n == 0) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    ChainD ch;
+    PointSrc src;
+    if ((rc = point_src<T>(ctx, intr, views, nviews, offsets, single, io.to_img, st, &ch, &src))) return rc;
+    rc = launch_points<T>(ctx, src, io, n, st);
+    const int rr = src.chain ? (int)CC_OK : point_table_release(ctx, st);
     return rc ? rc : rr;
 }
 
-// Host form: the table goes up once on slot 0's stream, every slot's stream waits for it, then the chunk
-// pipeline of the single-view *_host calls runs with one drain at the end.  A chunk's launch gets the
-// segments it covers and its first point's index in the call.  CHUNK(tb, k, off, m, lo, hi, cap) moves
-// and maps points [off, off + m) through slot k.  !table: a call whose launches take one chain by value;
-// nothing is uploaded and offsets are not read (lo = hi = 0).
-template <typename T, typename CHUNK>
-static int views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
-                      size_t n, bool to_img, bool table, size_t in_arrays, size_t out_arrays, CHUNK chunk) {
-    int rc;
+// Moves points [off, off + m) of a host call through slot k: up, one launch, down.  A side of `dim` coordinates
+// takes dim arrays of m points at stride cap in the slot (SoA), or one range of dim * m elements (AoS).  cap is a
+// multiple of 64, so every chunk takes the vector path.
+template <typename T>
+static int stage_chunk(cc_ctx* ctx, int k, const PointSrc& src, const PointIO<T>& io, size_t off, size_t m,
+                       size_t cap) {
+    cudaStream_t st = ctx->pipe_stream[k];
+    const size_t ein = io.aos ? io.in_dim : 1, eout = io.aos ? io.out_dim : 1;   // elements per point and array
+    PointIO<T> dev = io;
+    for (int d = 0; d < io.in_arrays(); ++d) {
+        T* slot = static_cast<T*>(ctx->pipe_in[k]) + d * cap;
+        dev.in[d] = slot;
+        CC_CUDA(cudaMemcpyAsync(slot, io.in[d] + ein * off, ein * m * sizeof(T), cudaMemcpyHostToDevice, st));
+    }
+    for (int d = 0; d < io.out_arrays(); ++d) dev.out[d] = static_cast<T*>(ctx->pipe_out[k]) + d * cap;
+    const int rc = launch_points<T>(ctx, src, dev, m, st);
+    if (rc) return rc;
+    for (int d = 0; d < io.out_arrays(); ++d)
+        CC_CUDA(cudaMemcpyAsync(io.out[d] + eout * off, dev.out[d], eout * m * sizeof(T), cudaMemcpyDeviceToHost, st));
+    return CC_OK;
+}
+
+// Host form: chunks of kPointChunk points go round-robin through the NSLOT slots, with one drain at the end.  A
+// table goes up once on slot 0's stream and every other slot's stream waits for it; each chunk's launch gets the
+// segments it covers and its first point's index in the call.
+template <typename T>
+static int points_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
+                       std::optional<size_t> count, const PointIO<T>& io) {
+    size_t n = 0;
+    int single = -1, rc = check_points(ctx, intr, views, nviews, offsets, count, io, &n, &single);
+    if (rc) return rc;
     CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    if (n == 0) return CC_OK;
+    if ((rc = enter(ctx)) || n == 0) return rc;
     const size_t cap = n < kPointChunk ? round_up(n, 64) : kPointChunk;
     const size_t nchunks = (n + cap - 1) / cap;
-    PointTable tb{};
-    if (table) {
-        const std::vector<ChainD> chs = view_chains(intr, views, nviews);
-        if ((rc = ensure_stream(ctx, 0))) return rc;
-        if ((rc = point_table_upload<T>(ctx, to_img, chs.data(), nviews, offsets, ctx->pipe_stream[0], &tb))) return rc;
+    ChainD ch;
+    PointSrc src;
+    if ((rc = ensure_stream(ctx, 0))) return rc;
+    if ((rc = point_src<T>(ctx, intr, views, nviews, offsets, single, io.to_img, ctx->pipe_stream[0], &ch, &src)))
+        return rc;
+    if (!src.chain) {
         if ((rc = point_table_release(ctx, ctx->pipe_stream[0]))) return rc;
         for (int k = 1; k < cc_ctx::NSLOT && (size_t)k < nchunks; ++k) {
             if ((rc = ensure_stream(ctx, k))) return rc;
@@ -280,192 +274,16 @@ static int views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, in
     for (int it = 0; rc == CC_OK && off < n; ++it, off += cap) {
         const int k = it % cc_ctx::NSLOT;
         const size_t m = (n - off) < cap ? (n - off) : cap;
-        int lo = 0, hi = 0;
-        if (table) {
-            lo = (int)(std::upper_bound(offsets, offsets + nviews + 1, off) - offsets) - 1;
-            hi = (int)(std::upper_bound(offsets, offsets + nviews + 1, off + m - 1) - offsets);
+        if (!src.chain) {
+            src.base = off;
+            src.seg_lo = (int)(std::upper_bound(offsets, offsets + nviews + 1, off) - offsets) - 1;
+            src.seg_hi = (int)(std::upper_bound(offsets, offsets + nviews + 1, off + m - 1) - offsets);
         }
-        if ((rc = ensure_slot(ctx, k, in_arrays * cap * sizeof(T), out_arrays * cap * sizeof(T)))) break;
-        rc = chunk(tb, k, off, m, lo, hi, cap);
+        if ((rc = ensure_slot(ctx, k, io.in_dim * cap * sizeof(T), io.out_dim * cap * sizeof(T)))) break;
+        rc = stage_chunk<T>(ctx, k, src, io, off, m, cap);
     }
     const int rd = drain(ctx);                     // the table's readers are done before the call returns
     return rc ? rc : rd;
-}
-
-template <typename T>
-static int img2world_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                           const size_t* offsets, const T* row, const T* col, T* x, T* y, T* z, cudaStream_t st) {
-    size_t n = 0;
-    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
-    if (rc) return rc;
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return views_device<T>(ctx, intr, views, nviews, offsets, n, false, st, [&](const PointTable& tb, cudaStream_t s) {
-        return launch_img2world_views<T>(ctx, tb, 0, 0, nviews, row, col, x, y, z, n, s);
-    });
-}
-
-template <typename T>
-static int world2img_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                           const size_t* offsets, const T* x, const T* y, const T* z, T* row, T* col, cudaStream_t st) {
-    size_t n = 0;
-    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
-    if (rc) return rc;
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return views_device<T>(ctx, intr, views, nviews, offsets, n, true, st, [&](const PointTable& tb, cudaStream_t s) {
-        return launch_world2img_views<T>(ctx, tb, 0, 0, nviews, x, y, z, row, col, n, s);
-    });
-}
-
-template <typename T>
-static int img2world_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                                const size_t* offsets, const T* row, const T* col, T* x, T* y, T* z) {
-    size_t n = 0;
-    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
-    if (rc) return rc;
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return views_host<T>(ctx, intr, views, nviews, offsets, n, false, true, 2, 3,
-                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t cap) {
-        cudaStream_t st = ctx->pipe_stream[k];
-        T* din = static_cast<T*>(ctx->pipe_in[k]);
-        T* dout = static_cast<T*>(ctx->pipe_out[k]);
-        CC_CUDA(cudaMemcpyAsync(din, row + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(din + cap, col + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        int r = launch_img2world_views<T>(ctx, tb, off, lo, hi, din, din + cap, dout, dout + cap,
-                                          z ? dout + 2 * cap : nullptr, m, st);
-        if (r) return r;
-        CC_CUDA(cudaMemcpyAsync(x + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        CC_CUDA(cudaMemcpyAsync(y + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        if (z) CC_CUDA(cudaMemcpyAsync(z + off, dout + 2 * cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        return (int)CC_OK;
-    });
-}
-
-template <typename T>
-static int world2img_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                                const size_t* offsets, const T* x, const T* y, const T* z, T* row, T* col) {
-    size_t n = 0;
-    int rc = check_views(ctx, intr, views, nviews, offsets, &n);
-    if (rc) return rc;
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return views_host<T>(ctx, intr, views, nviews, offsets, n, true, true, 3, 2,
-                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t cap) {
-        cudaStream_t st = ctx->pipe_stream[k];
-        T* din = static_cast<T*>(ctx->pipe_in[k]);
-        T* dout = static_cast<T*>(ctx->pipe_out[k]);
-        CC_CUDA(cudaMemcpyAsync(din, x + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(din + cap, y + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        if (z) CC_CUDA(cudaMemcpyAsync(din + 2 * cap, z + off, m * sizeof(T), cudaMemcpyHostToDevice, st));
-        int r = launch_world2img_views<T>(ctx, tb, off, lo, hi, din, din + cap, z ? din + 2 * cap : nullptr,
-                                          dout, dout + cap, m, st);
-        if (r) return r;
-        CC_CUDA(cudaMemcpyAsync(row + off, dout, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        CC_CUDA(cudaMemcpyAsync(col + off, dout + cap, m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        return (int)CC_OK;
-    });
-}
-
-// ---- interleaved points: cc_*_aos[_host] --------------------------------------------------------
-// rc: n (row, col) pairs; pts: n points of `dim` coordinates ((x, y, z), or (x, y) with z not computed / z = 0).
-// offsets == NULL: views[0] for every point (nviews must be 1).  Otherwise the segments of cc_*_views, and
-// offsets[nviews] must be n.  Checks everything before anything is written.  *single: the view whose segment
-// holds every point (the call then takes the SINGLE kernel, chain by value, no table), or -1.
-static int check_aos(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
-                     const void* rc, const void* pts, int dim, size_t n, int* single) {
-    CC_REQUIRE(dim == 2 || dim == 3, "out_dim / in_dim must be 2 or 3");
-    CC_REQUIRE(n == 0 || (rc && pts), "NULL point array");
-    *single = 0;
-    if (offsets == nullptr) {
-        CC_REQUIRE(nviews == 1, "offsets == NULL needs nviews == 1");
-        return check_params(ctx, intr, views);
-    }
-    size_t total = 0;
-    const int rv = check_views(ctx, intr, views, nviews, offsets, &total);
-    if (rv) return rv;
-    CC_REQUIRE(total == n, "offsets[nviews] must equal n");
-    *single = -1;
-    for (int s = 0; s < nviews && *single < 0; ++s)
-        if (offsets[s + 1] - offsets[s] == n) *single = s;
-    return CC_OK;
-}
-
-template <typename T>
-static int img2world_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
-                         const T* rc, T* out, int out_dim, size_t n, cudaStream_t st) {
-    int single;
-    int r = check_aos(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, &single);
-    if (r) return r;
-    if (single < 0)
-        return views_device<T>(ctx, intr, views, nviews, offsets, n, false, st, [&](const PointTable& tb, cudaStream_t s) {
-            return launch_img2world_aos<T>(ctx, nullptr, tb, 0, 0, nviews, rc, out, out_dim == 3, n, s);
-        });
-    CC_GUARD;
-    if ((r = enter(ctx))) return r;
-    ChainD ch;
-    build_chain(intr, views + single, &ch);
-    return launch_img2world_aos<T>(ctx, &ch, PointTable{}, 0, 0, 0, rc, out, out_dim == 3, n, st);
-}
-
-template <typename T>
-static int world2img_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
-                         const T* pts, int in_dim, T* rc, size_t n, cudaStream_t st) {
-    int single;
-    int r = check_aos(ctx, intr, views, nviews, offsets, rc, pts, in_dim, n, &single);
-    if (r) return r;
-    if (single < 0)
-        return views_device<T>(ctx, intr, views, nviews, offsets, n, true, st, [&](const PointTable& tb, cudaStream_t s) {
-            return launch_world2img_aos<T>(ctx, nullptr, tb, 0, 0, nviews, pts, in_dim == 3, rc, n, s);
-        });
-    CC_GUARD;
-    if ((r = enter(ctx))) return r;
-    ChainD ch;
-    build_chain(intr, views + single, &ch);
-    return launch_world2img_aos<T>(ctx, &ch, PointTable{}, 0, 0, 0, pts, in_dim == 3, rc, n, st);
-}
-
-// One contiguous byte range per direction and chunk: one H2D and one D2H copy.  The slot buffers are
-// aligned, so every chunk takes the vector path.
-template <typename T>
-static int img2world_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                              const size_t* offsets, const T* rc, T* out, int out_dim, size_t n) {
-    int single;
-    int r = check_aos(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, &single);
-    if (r) return r;
-    ChainD ch;
-    if (single >= 0) build_chain(intr, views + single, &ch);
-    const size_t D = (size_t)out_dim;
-    return views_host<T>(ctx, intr, views, nviews, offsets, n, false, single < 0, 2, D,
-                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t) {
-        cudaStream_t st = ctx->pipe_stream[k];
-        T* din = static_cast<T*>(ctx->pipe_in[k]);
-        T* dout = static_cast<T*>(ctx->pipe_out[k]);
-        CC_CUDA(cudaMemcpyAsync(din, rc + 2 * off, 2 * m * sizeof(T), cudaMemcpyHostToDevice, st));
-        int e = launch_img2world_aos<T>(ctx, single >= 0 ? &ch : nullptr, tb, off, lo, hi, din, dout, D == 3, m, st);
-        if (e) return e;
-        CC_CUDA(cudaMemcpyAsync(out + D * off, dout, D * m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        return (int)CC_OK;
-    });
-}
-
-template <typename T>
-static int world2img_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                              const size_t* offsets, const T* pts, int in_dim, T* rc, size_t n) {
-    int single;
-    int r = check_aos(ctx, intr, views, nviews, offsets, rc, pts, in_dim, n, &single);
-    if (r) return r;
-    ChainD ch;
-    if (single >= 0) build_chain(intr, views + single, &ch);
-    const size_t D = (size_t)in_dim;
-    return views_host<T>(ctx, intr, views, nviews, offsets, n, true, single < 0, D, 2,
-                         [&](const PointTable& tb, int k, size_t off, size_t m, int lo, int hi, size_t) {
-        cudaStream_t st = ctx->pipe_stream[k];
-        T* din = static_cast<T*>(ctx->pipe_in[k]);
-        T* dout = static_cast<T*>(ctx->pipe_out[k]);
-        CC_CUDA(cudaMemcpyAsync(din, pts + D * off, D * m * sizeof(T), cudaMemcpyHostToDevice, st));
-        int e = launch_world2img_aos<T>(ctx, single >= 0 ? &ch : nullptr, tb, off, lo, hi, din, D == 3, dout, m, st);
-        if (e) return e;
-        CC_CUDA(cudaMemcpyAsync(rc + 2 * off, dout, 2 * m * sizeof(T), cudaMemcpyDeviceToHost, st));
-        return (int)CC_OK;
-    });
 }
 
 // Frames per chunk of the frame pipelines: a few whole frames, ~32 MB per chunk (measured on B200 / PCIe Gen5:
@@ -643,126 +461,110 @@ int cc_host_unregister(void* ptr) {
 }
 
 // ---- point maps ------------------------------------------------------------------
-#define CC_POINT_ENTRY(NAME, T, DIR)                                                              \
-    int rc = check_params(ctx, intr, view);                                                       \
-    if (rc) return rc;                                                                            \
-    CC_GUARD;                                                            \
-    if ((rc = enter(ctx))) return rc;                                                             \
-    ChainD ch;                                                                                    \
-    build_chain(intr, view, &ch);
-
 int cc_img2world_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const double* row,
                      const double* col, double* x, double* y, double* z, size_t n, void* stream) {
-    CC_POINT_ENTRY(img2world, double, 0)
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return launch_img2world<double>(ctx, ch, row, col, x, y, z, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, view, 1, nullptr, n, soa_img2world(row, col, x, y, z), stream);
 }
 int cc_img2world_f32(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const float* row,
                      const float* col, float* x, float* y, float* z, size_t n, void* stream) {
-    CC_POINT_ENTRY(img2world, float, 0)
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return launch_img2world<float>(ctx, ch, row, col, x, y, z, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, view, 1, nullptr, n, soa_img2world(row, col, x, y, z), stream);
 }
 int cc_world2img_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const double* x,
                      const double* y, const double* z, double* row, double* col, size_t n,
                      void* stream) {
-    CC_POINT_ENTRY(world2img, double, 1)
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return launch_world2img<double>(ctx, ch, x, y, z, row, col, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, view, 1, nullptr, n, soa_world2img(x, y, z, row, col), stream);
 }
 int cc_world2img_f32(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const float* x,
                      const float* y, const float* z, float* row, float* col, size_t n,
                      void* stream) {
-    CC_POINT_ENTRY(world2img, float, 1)
-    CC_REQUIRE(n == 0 || (row && col && x && y), "NULL point array");
-    return launch_world2img<float>(ctx, ch, x, y, z, row, col, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, view, 1, nullptr, n, soa_world2img(x, y, z, row, col), stream);
 }
 
 int cc_img2world_f64_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const double* row,
                           const double* col, double* x, double* y, double* z, size_t n) {
-    return img2world_host<double>(ctx, intr, view, row, col, x, y, z, n);
+    return points_host(ctx, intr, view, 1, nullptr, n, soa_img2world(row, col, x, y, z));
 }
 int cc_img2world_f32_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const float* row,
                           const float* col, float* x, float* y, float* z, size_t n) {
-    return img2world_host<float>(ctx, intr, view, row, col, x, y, z, n);
+    return points_host(ctx, intr, view, 1, nullptr, n, soa_img2world(row, col, x, y, z));
 }
 int cc_world2img_f64_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const double* x,
                           const double* y, const double* z, double* row, double* col, size_t n) {
-    return world2img_host<double>(ctx, intr, view, x, y, z, row, col, n);
+    return points_host(ctx, intr, view, 1, nullptr, n, soa_world2img(x, y, z, row, col));
 }
 int cc_world2img_f32_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, const float* x,
                           const float* y, const float* z, float* row, float* col, size_t n) {
-    return world2img_host<float>(ctx, intr, view, x, y, z, row, col, n);
+    return points_host(ctx, intr, view, 1, nullptr, n, soa_world2img(x, y, z, row, col));
 }
 
 int cc_img2world_f64_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                            const double* row, const double* col, double* x, double* y, double* z, void* stream) {
-    return img2world_views<double>(ctx, intr, views, nviews, offsets, row, col, x, y, z, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, std::nullopt, soa_img2world(row, col, x, y, z), stream);
 }
 int cc_img2world_f32_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                            const float* row, const float* col, float* x, float* y, float* z, void* stream) {
-    return img2world_views<float>(ctx, intr, views, nviews, offsets, row, col, x, y, z, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, std::nullopt, soa_img2world(row, col, x, y, z), stream);
 }
 int cc_world2img_f64_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                            const double* x, const double* y, const double* z, double* row, double* col, void* stream) {
-    return world2img_views<double>(ctx, intr, views, nviews, offsets, x, y, z, row, col, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, std::nullopt, soa_world2img(x, y, z, row, col), stream);
 }
 int cc_world2img_f32_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                            const float* x, const float* y, const float* z, float* row, float* col, void* stream) {
-    return world2img_views<float>(ctx, intr, views, nviews, offsets, x, y, z, row, col, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, std::nullopt, soa_world2img(x, y, z, row, col), stream);
 }
 int cc_img2world_f64_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                                 const size_t* offsets, const double* row, const double* col, double* x, double* y,
                                 double* z) {
-    return img2world_views_host<double>(ctx, intr, views, nviews, offsets, row, col, x, y, z);
+    return points_host(ctx, intr, views, nviews, offsets, std::nullopt, soa_img2world(row, col, x, y, z));
 }
 int cc_img2world_f32_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                                 const size_t* offsets, const float* row, const float* col, float* x, float* y,
                                 float* z) {
-    return img2world_views_host<float>(ctx, intr, views, nviews, offsets, row, col, x, y, z);
+    return points_host(ctx, intr, views, nviews, offsets, std::nullopt, soa_img2world(row, col, x, y, z));
 }
 int cc_world2img_f64_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                                 const size_t* offsets, const double* x, const double* y, const double* z,
                                 double* row, double* col) {
-    return world2img_views_host<double>(ctx, intr, views, nviews, offsets, x, y, z, row, col);
+    return points_host(ctx, intr, views, nviews, offsets, std::nullopt, soa_world2img(x, y, z, row, col));
 }
 int cc_world2img_f32_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                                 const size_t* offsets, const float* x, const float* y, const float* z,
                                 float* row, float* col) {
-    return world2img_views_host<float>(ctx, intr, views, nviews, offsets, x, y, z, row, col);
+    return points_host(ctx, intr, views, nviews, offsets, std::nullopt, soa_world2img(x, y, z, row, col));
 }
 
 int cc_img2world_f64_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                          const double* rc, double* out, int out_dim, size_t n, void* stream) {
-    return img2world_aos<double>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, n, aos_img2world(rc, out, out_dim), stream);
 }
 int cc_img2world_f32_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                          const float* rc, float* out, int out_dim, size_t n, void* stream) {
-    return img2world_aos<float>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, n, aos_img2world(rc, out, out_dim), stream);
 }
 int cc_world2img_f64_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                          const double* pts, int in_dim, double* rc, size_t n, void* stream) {
-    return world2img_aos<double>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, n, aos_world2img(pts, in_dim, rc), stream);
 }
 int cc_world2img_f32_aos(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const size_t* offsets,
                          const float* pts, int in_dim, float* rc, size_t n, void* stream) {
-    return world2img_aos<float>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n, (cudaStream_t)stream);
+    return points_device(ctx, intr, views, nviews, offsets, n, aos_world2img(pts, in_dim, rc), stream);
 }
 int cc_img2world_f64_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                               const size_t* offsets, const double* rc, double* out, int out_dim, size_t n) {
-    return img2world_aos_host<double>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n);
+    return points_host(ctx, intr, views, nviews, offsets, n, aos_img2world(rc, out, out_dim));
 }
 int cc_img2world_f32_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                               const size_t* offsets, const float* rc, float* out, int out_dim, size_t n) {
-    return img2world_aos_host<float>(ctx, intr, views, nviews, offsets, rc, out, out_dim, n);
+    return points_host(ctx, intr, views, nviews, offsets, n, aos_img2world(rc, out, out_dim));
 }
 int cc_world2img_f64_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                               const size_t* offsets, const double* pts, int in_dim, double* rc, size_t n) {
-    return world2img_aos_host<double>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n);
+    return points_host(ctx, intr, views, nviews, offsets, n, aos_world2img(pts, in_dim, rc));
 }
 int cc_world2img_f32_aos_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                               const size_t* offsets, const float* pts, int in_dim, float* rc, size_t n) {
-    return world2img_aos_host<float>(ctx, intr, views, nviews, offsets, pts, in_dim, rc, n);
+    return points_host(ctx, intr, views, nviews, offsets, n, aos_world2img(pts, in_dim, rc));
 }
 
 // ---- rectification ---------------------------------------------------------------

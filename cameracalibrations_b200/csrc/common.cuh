@@ -42,6 +42,25 @@ struct PointTable {
     const void* rows;
     const size_t* off;
 };
+// The arrays of a point map.  SoA: one array per coordinate.  AoS: in[0] / out[0] hold packed points of in_dim /
+// out_dim coordinates.  img2world out_dim 2: z is not computed; world2img in_dim 2: z = 0.  Unused entries are NULL.
+template <typename T> struct PointIO {
+    bool to_img;           // world -> pixel
+    bool aos;
+    int in_dim, out_dim;   // 2 or 3
+    const T* in[3];
+    T* out[3];
+    int in_arrays() const { return aos ? 1 : in_dim; }
+    int out_arrays() const { return aos ? 1 : out_dim; }
+};
+// The views of one launch.  SINGLE (chain != NULL): every point uses *chain, passed by value.  TABLE: the launch's
+// points are points base + [0, n) of the call, in segments [seg_lo, seg_hi) of the uploaded table tb.
+struct PointSrc {
+    const ChainD* chain;
+    PointTable tb;
+    size_t base;
+    int seg_lo, seg_hi;
+};
 
 // error plumbing (abi.cu)
 int set_error(int status, const char* fmt, ...);

@@ -378,56 +378,9 @@ static int grid_for(cc_ctx* ctx, K kernel, size_t work_items) {
     return (int)(want < cap ? want : cap);
 }
 
-template <typename T>
-int launch_img2world(cc_ctx* ctx, const ChainD& chd, const T* row, const T* col, T* x, T* y, T* z,
-                     size_t n, cudaStream_t st);
-template <typename T>
-int launch_world2img(cc_ctx* ctx, const ChainD& chd, const T* x, const T* y, const T* z, T* row,
-                     T* col, size_t n, cudaStream_t st);
-
 template <typename T> static Chain<T> pick_chain(const ChainD& d);
 template <> Chain<double> pick_chain<double>(const ChainD& d) { return d; }
 template <> Chain<float> pick_chain<float>(const ChainD& d) { ChainF f; narrow_chain(d, &f); return f; }
-
-template <typename T>
-int launch_img2world(cc_ctx* ctx, const ChainD& chd, const T* row, const T* col, T* x, T* y, T* z,
-                     size_t n, cudaStream_t st) {
-    if (n == 0) return CC_OK;
-    const Chain<T> ch = pick_chain<T>(chd);
-    const bool vec = aligned16(row) && aligned16(col) && aligned16(x) && aligned16(y) &&
-                     (z == nullptr || aligned16(z));
-    const size_t items = vec ? n / Vec<T>::N + 1 : n;
-    if (z) {
-        auto k = img2world_kernel<T, true>;
-        k<<<grid_for(ctx, k, items), kThreads, 0, st>>>(ch, row, col, x, y, z, n, vec);
-    } else {
-        auto k = img2world_kernel<T, false>;
-        k<<<grid_for(ctx, k, items), kThreads, 0, st>>>(ch, row, col, x, y, z, n, vec);
-    }
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
-template <typename T>
-int launch_world2img(cc_ctx* ctx, const ChainD& chd, const T* x, const T* y, const T* z, T* row,
-                     T* col, size_t n, cudaStream_t st) {
-    if (n == 0) return CC_OK;
-    const Chain<T> ch = pick_chain<T>(chd);
-    const bool vec = aligned16(x) && aligned16(y) && aligned16(row) && aligned16(col) &&
-                     (z == nullptr || aligned16(z));
-    const size_t items = vec ? n / Vec<T>::N + 1 : n;
-    if (z) {
-        auto k = world2img_kernel<T, true>;
-        k<<<grid_for(ctx, k, items), kThreads, 0, st>>>(ch, x, y, z, row, col, n, vec);
-    } else {
-        auto k = world2img_kernel<T, false>;
-        k<<<grid_for(ctx, k, items), kThreads, 0, st>>>(ch, x, y, z, row, col, n, vec);
-    }
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
 
 // ---- multi-view calls: the device chain table ----------------------------------------------------
 // One table per context: the rows of the call's segments, then its nseg + 1 offsets.  It is
@@ -504,117 +457,55 @@ static int grid_tiles(cc_ctx* ctx, K kernel, size_t n) {
     return (int)(tiles < cap ? tiles : cap);
 }
 
+// ---- the launcher ------------------------------------------------------------------------------
+// The kernel of one direction, layout, z and view source: SINGLE on a grid-stride grid over the vectors (the points
+// when !vec), TABLE on one CTA per tile up to the resident limit.
+template <typename T, bool TO_IMG, bool AOS, bool HAS_Z, typename SRC>
+static void launch_kernel(cc_ctx* ctx, const SRC& src, const PointIO<T>& io, size_t n, bool vec, cudaStream_t st) {
+    auto go = [&](auto k, auto... arrays) {
+        const int grid = IsTable<SRC>::value ? grid_tiles(ctx, k, n) : grid_for(ctx, k, vec ? n / Vec<T>::N + 1 : n);
+        k<<<grid, kThreads, 0, st>>>(src, arrays..., n, vec);
+    };
+    if constexpr (AOS && TO_IMG) go(world2img_aos_kernel<T, HAS_Z, SRC>, io.in[0], io.out[0]);
+    else if constexpr (AOS) go(img2world_aos_kernel<T, HAS_Z, SRC>, io.in[0], io.out[0]);
+    else if constexpr (TO_IMG) go(world2img_kernel<T, HAS_Z, SRC>, io.in[0], io.in[1], io.in[2], io.out[0], io.out[1]);
+    else go(img2world_kernel<T, HAS_Z, SRC>, io.in[0], io.in[1], io.out[0], io.out[1], io.out[2]);
+}
+
+// f(std::true_type) or f(std::false_type): a run-time flag as a template argument
+template <typename F> static void with_bool(bool b, F&& f) {
+    if (b) f(std::true_type{});
+    else f(std::false_type{});
+}
+
+// One launch over points [0, n) of io on st; none when n == 0.  The vector path needs every array the kernel
+// dereferences 16-byte aligned.
 template <typename T>
-int launch_img2world_views(cc_ctx* ctx, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
-                           const T* row, const T* col, T* x, T* y, T* z, size_t n, cudaStream_t st) {
+int launch_points(cc_ctx* ctx, const PointSrc& src, const PointIO<T>& io, size_t n, cudaStream_t st) {
     if (n == 0) return CC_OK;
-    using Src = ViewTable<RowI2W<T>>;
-    const Src src{static_cast<const RowI2W<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
-    const bool vec = aligned16(row) && aligned16(col) && aligned16(x) && aligned16(y) &&
-                     (z == nullptr || aligned16(z));
-    if (z) {
-        auto k = img2world_kernel<T, true, Src>;
-        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, row, col, x, y, z, n, vec);
-    } else {
-        auto k = img2world_kernel<T, false, Src>;
-        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, row, col, x, y, z, n, vec);
-    }
+    bool vec = true;
+    for (int d = 0; d < io.in_arrays(); ++d) vec = vec && aligned16(io.in[d]);
+    for (int d = 0; d < io.out_arrays(); ++d) vec = vec && aligned16(io.out[d]);
+    const bool has_z = (io.to_img ? io.in_dim : io.out_dim) == 3;
+    with_bool(io.to_img, [&](auto to_img) { with_bool(io.aos, [&](auto aos) { with_bool(has_z, [&](auto z) {
+        constexpr bool TO_IMG = decltype(to_img)::value, AOS = decltype(aos)::value, HAS_Z = decltype(z)::value;
+        using Row = std::conditional_t<TO_IMG, RowW2I<T>, RowI2W<T>>;
+        if (src.chain)
+            launch_kernel<T, TO_IMG, AOS, HAS_Z>(ctx, pick_chain<T>(*src.chain), io, n, vec, st);
+        else
+            launch_kernel<T, TO_IMG, AOS, HAS_Z>(
+                ctx, ViewTable<Row>{static_cast<const Row*>(src.tb.rows), src.tb.off, src.base, src.seg_lo, src.seg_hi},
+                io, n, vec, st);
+    }); }); });
     ctx->launches++;
     CC_CUDA(cudaGetLastError());
     return CC_OK;
 }
-
-template <typename T>
-int launch_world2img_views(cc_ctx* ctx, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
-                           const T* x, const T* y, const T* z, T* row, T* col, size_t n, cudaStream_t st) {
-    if (n == 0) return CC_OK;
-    using Src = ViewTable<RowW2I<T>>;
-    const Src src{static_cast<const RowW2I<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
-    const bool vec = aligned16(x) && aligned16(y) && aligned16(row) && aligned16(col) &&
-                     (z == nullptr || aligned16(z));
-    if (z) {
-        auto k = world2img_kernel<T, true, Src>;
-        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, x, y, z, row, col, n, vec);
-    } else {
-        auto k = world2img_kernel<T, false, Src>;
-        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, x, y, z, row, col, n, vec);
-    }
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
-// ---- interleaved points (cc_*_aos[_host]) ------------------------------------------------------
-// chd != nullptr: the SINGLE kernel with that chain.  Otherwise the TABLE kernel over tb, points base + [0, n)
-// of segments [seg_lo, seg_hi), as launch_*_views.  The vector path needs only the two base pointers aligned.
-template <typename T, bool HAS_Z>
-static void img2world_aos_grid(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo,
-                               int seg_hi, const T* rc, T* xyz, size_t n, bool vec, cudaStream_t st) {
-    if (chd) {
-        auto k = img2world_aos_kernel<T, HAS_Z>;
-        k<<<grid_for(ctx, k, vec ? n / Vec<T>::N + 1 : n), kThreads, 0, st>>>(pick_chain<T>(*chd), rc, xyz, n, vec);
-    } else {
-        using Src = ViewTable<RowI2W<T>>;
-        const Src src{static_cast<const RowI2W<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
-        auto k = img2world_aos_kernel<T, HAS_Z, Src>;
-        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, rc, xyz, n, vec);
-    }
-}
-
-template <typename T, bool HAS_Z>
-static void world2img_aos_grid(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo,
-                               int seg_hi, const T* xyz, T* rc, size_t n, bool vec, cudaStream_t st) {
-    if (chd) {
-        auto k = world2img_aos_kernel<T, HAS_Z>;
-        k<<<grid_for(ctx, k, vec ? n / Vec<T>::N + 1 : n), kThreads, 0, st>>>(pick_chain<T>(*chd), xyz, rc, n, vec);
-    } else {
-        using Src = ViewTable<RowW2I<T>>;
-        const Src src{static_cast<const RowW2I<T>*>(tb.rows), tb.off, base, seg_lo, seg_hi};
-        auto k = world2img_aos_kernel<T, HAS_Z, Src>;
-        k<<<grid_tiles(ctx, k, n), kThreads, 0, st>>>(src, xyz, rc, n, vec);
-    }
-}
-
-// xyz: points of 3 coordinates (has_z) or 2 (z not computed / z = 0)
-template <typename T>
-int launch_img2world_aos(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
-                         const T* rc, T* xyz, bool has_z, size_t n, cudaStream_t st) {
-    if (n == 0) return CC_OK;
-    const bool vec = aligned16(rc) && aligned16(xyz);
-    if (has_z) img2world_aos_grid<T, true>(ctx, chd, tb, base, seg_lo, seg_hi, rc, xyz, n, vec, st);
-    else img2world_aos_grid<T, false>(ctx, chd, tb, base, seg_lo, seg_hi, rc, xyz, n, vec, st);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
-template <typename T>
-int launch_world2img_aos(cc_ctx* ctx, const ChainD* chd, const PointTable& tb, size_t base, int seg_lo, int seg_hi,
-                         const T* xyz, bool has_z, T* rc, size_t n, cudaStream_t st) {
-    if (n == 0) return CC_OK;
-    const bool vec = aligned16(xyz) && aligned16(rc);
-    if (has_z) world2img_aos_grid<T, true>(ctx, chd, tb, base, seg_lo, seg_hi, xyz, rc, n, vec, st);
-    else world2img_aos_grid<T, false>(ctx, chd, tb, base, seg_lo, seg_hi, xyz, rc, n, vec, st);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
-template int launch_img2world_aos<double>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const double*, double*, bool, size_t, cudaStream_t);
-template int launch_img2world_aos<float>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const float*, float*, bool, size_t, cudaStream_t);
-template int launch_world2img_aos<double>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const double*, bool, double*, size_t, cudaStream_t);
-template int launch_world2img_aos<float>(cc_ctx*, const ChainD*, const PointTable&, size_t, int, int, const float*, bool, float*, size_t, cudaStream_t);
 
 template int point_table_upload<double>(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
 template int point_table_upload<float>(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
-template int launch_img2world_views<double>(cc_ctx*, const PointTable&, size_t, int, int, const double*, const double*, double*, double*, double*, size_t, cudaStream_t);
-template int launch_img2world_views<float>(cc_ctx*, const PointTable&, size_t, int, int, const float*, const float*, float*, float*, float*, size_t, cudaStream_t);
-template int launch_world2img_views<double>(cc_ctx*, const PointTable&, size_t, int, int, const double*, const double*, const double*, double*, double*, size_t, cudaStream_t);
-template int launch_world2img_views<float>(cc_ctx*, const PointTable&, size_t, int, int, const float*, const float*, const float*, float*, float*, size_t, cudaStream_t);
-
-template int launch_img2world<double>(cc_ctx*, const ChainD&, const double*, const double*, double*, double*, double*, size_t, cudaStream_t);
-template int launch_img2world<float>(cc_ctx*, const ChainD&, const float*, const float*, float*, float*, float*, size_t, cudaStream_t);
-template int launch_world2img<double>(cc_ctx*, const ChainD&, const double*, const double*, const double*, double*, double*, size_t, cudaStream_t);
-template int launch_world2img<float>(cc_ctx*, const ChainD&, const float*, const float*, const float*, float*, float*, size_t, cudaStream_t);
+template int launch_points<double>(cc_ctx*, const PointSrc&, const PointIO<double>&, size_t, cudaStream_t);
+template int launch_points<float>(cc_ctx*, const PointSrc&, const PointIO<float>&, size_t, cudaStream_t);
 
 }  // namespace cc
+
