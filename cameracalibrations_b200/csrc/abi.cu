@@ -36,30 +36,21 @@ int point_table_upload(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStr
 int point_table_release(cc_ctx*, cudaStream_t);
 template <typename T>
 int launch_points(cc_ctx*, const PointSrc&, const PointIO<T>&, size_t, cudaStream_t);
-int check_rect_args(const int64_t axs_min[2], int sz1, int sz2, size_t pitch, size_t frame_stride,
-                    int nframes, double ratio);
-int launch_rectify_f32c1(cc_ctx*, const ChainD&, double, const int64_t[2], const float*, float*, int,
-                         int, size_t, size_t, int, float, unsigned, cudaStream_t);
-int launch_rectify_u8c3(cc_ctx*, const ChainD&, double, const int64_t[2], const uint8_t*, uint8_t*,
-                        int, int, size_t, size_t, int, const uint8_t[3], unsigned, cudaStream_t);
-int launch_rectify_f32c1_views(cc_ctx*, const ChainD*, const double*, const int64_t*, int, const float*, float*, int, int,
-                               size_t, size_t, int, float, unsigned, cudaStream_t, bool*);
-int launch_rectify_u8c3_views(cc_ctx*, const ChainD*, const double*, const int64_t*, int, const uint8_t*, uint8_t*, int,
-                              int, size_t, size_t, int, const uint8_t[3], unsigned, cudaStream_t, bool*);
+template <typename PX>
+int launch_rectify(cc_ctx*, const RectCall<PX>&, int, int, const PX*, PX*, cudaStream_t);
+template <typename PX>
+int launch_rectify_group(cc_ctx*, const RectCall<PX>&, int, int, const PX*, PX*, cudaStream_t, bool*);
 int rectify_views_per_launch();
 struct RectViewsHost;
-int rect_vh_begin(cc_ctx*, const ChainD*, const double*, const int64_t*, int, int, int, size_t, int, int, bool,
-                  RectViewsHost**);
+template <typename PX>
+int rect_vh_begin(cc_ctx*, const RectCall<PX>&, RectViewsHost**);
 int rect_vh_prepare(RectViewsHost*, int);
-int rect_vh_launch_f32c1(RectViewsHost*, int, int, int, const float*, float*, float, unsigned, cudaStream_t, bool*);
-int rect_vh_launch_u8c3(RectViewsHost*, int, int, int, const uint8_t*, uint8_t*, const uint8_t[3], unsigned, cudaStream_t,
-                        bool*);
+template <typename PX>
+int rect_vh_launch(RectViewsHost*, const RectCall<PX>&, int, int, int, const PX*, PX*, cudaStream_t, bool*);
 void rect_vh_retire(RectViewsHost*, int);
 int rect_vh_end(RectViewsHost*);
-int launch_rectify_map(cc_ctx*, const ChainD&, double, const int64_t[2], double*, double*, int, int,
-                       size_t, cudaStream_t);
-int launch_rectify_map_f32(cc_ctx*, const ChainD&, double, const int64_t[2], float*, float*, int, int,
-                           size_t, cudaStream_t);
+template <typename T>
+int launch_rectify_map(cc_ctx*, const ChainD&, double, const int64_t[2], T*, T*, int, int, size_t, cudaStream_t);
 int launch_reproj_jtj(cc_ctx*, const cc_intr*, double, const cc_view*, int, const double*,
                       const double*, int, double*, double*, cudaStream_t);
 int launch_calc_errors(cc_ctx*, const cc_intr*, const cc_view*, int, const double*, const double*,
@@ -130,8 +121,6 @@ static int drain(cc_ctx* ctx) {
         if (ctx->pipe_stream[k]) CC_CUDA(cudaStreamSynchronize(ctx->pipe_stream[k]));
     return CC_OK;
 }
-
-static int cuda_check(cudaError_t e, const char* what) { return e == cudaSuccess ? (int)CC_OK : cuda_fail(e, what); }
 
 static size_t round_up(size_t v, size_t m) { return (v + m - 1) / m * m; }
 
@@ -315,48 +304,227 @@ static std::vector<int> chunk_schedule(int nframes, size_t frame_bytes, int max_
     return sizes;
 }
 
-// frames: chunk = a few whole frames (~32 MB per stage)
-template <typename PX, typename LAUNCH>
-static int rectify_host(cc_ctx* ctx, const PX* src, PX* dst, int sz1, int sz2, size_t pitch,
-                        size_t frame_stride, int nframes, size_t px_bytes, LAUNCH launch) {
-    int rc;
+// ---- rectification ---------------------------------------------------------------
+// Every rectification entry point calls rectify_device or rectify_host with its views and its frame layout: a
+// single-view call is one view whose frames per view are the call's nframes; `many` marks the `_views` calls.
+
+// Every rule of a rectification call, checked before anything is written, enqueued or the device is touched.  The
+// map entry points pass fr.fpv = 0: no frames.
+static int check_rect(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                      const int64_t* axs_mins, const RectFrames& fr, const void* src, const void* dst, bool fill_ok) {
+    CC_REQUIRE(ctx != nullptr, "ctx is NULL");
+    CC_REQUIRE(intr != nullptr, "intr is NULL");
+    CC_REQUIRE(nviews >= 0 && fr.fpv >= 0, "bad counts: nviews and frame counts must not be negative");
+    const long long nframes = (long long)nviews * fr.fpv;
+    CC_REQUIRE(nframes <= 65535, "at most 65535 frames per call");
+    if (nviews > 0) {
+        CC_REQUIRE(views != nullptr, "view is NULL");
+        CC_REQUIRE(ratios != nullptr, "ratios is NULL");
+        CC_REQUIRE(axs_mins != nullptr, "axs_min is NULL");
+        CC_REQUIRE(fr.sz1 > 0 && fr.sz2 > 0, "frame size must be positive");
+        CC_REQUIRE(fr.sz1 < (1 << 22) && fr.sz2 < (1 << 22), "frame extent must be < 2^22");
+        CC_REQUIRE(fr.pitch >= (size_t)fr.sz1, "pitch smaller than sz1");
+        CC_REQUIRE(nframes <= 1 || fr.frame_stride >= fr.pitch * (size_t)(fr.sz2 - 1) + fr.sz1, "frames overlap");
+        CC_REQUIRE(fr.pitch * (size_t)fr.sz2 < (size_t)1 << 30, "frame too large (pitch*sz2 must be < 2^30)");
+    }
+    const int64_t lim = (int64_t)1 << 30;
+    for (int v = 0; v < nviews; ++v) {
+        const int rc = check_params(ctx, intr, views + v);
+        if (rc) return rc;
+        CC_REQUIRE(ratios[v] > 0.0 && ratios[v] == ratios[v], "ratio must be positive");
+        const int64_t* axs = axs_mins + 2 * v;
+        CC_REQUIRE(axs[0] > -lim && axs[0] < lim && axs[1] > -lim && axs[1] < lim, "axs_min out of range");
+    }
+    CC_REQUIRE(nframes == 0 || (src && dst), "NULL frame pointer");
+    CC_REQUIRE(nframes == 0 || src != dst, "rectification is not in place: src == dst");
+    CC_REQUIRE(fill_ok, "fill is NULL");
+    return CC_OK;
+}
+
+// the fill of a call as the kernels take it; false: a NULL u8c3 fill
+static bool make_fill(float f, float* out) {
+    *out = f;
+    return true;
+}
+static bool make_fill(const uint8_t* f, uchar3* out) {
+    if (f) *out = make_uchar3(f[0], f[1], f[2]);
+    return f != nullptr;
+}
+
+// Device form.  A single-view call is one launch on the caller's stream.  A `_views` call launches groups of up to 64
+// views in one staged launch each (CAMCAL_VIEWS_SINGLE=0, a tuning knob, turns that off); the views of a group that
+// cannot be staged get one launch each.
+template <typename PX, typename FILL>
+static int rectify_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                          const int64_t* axs_mins, const PX* src, PX* dst, const RectFrames& fr, FILL fill,
+                          unsigned flags, void* stream, bool many) {
+    RectCall<PX> c{fr, {nullptr, ratios, axs_mins, nviews}, {}, flags};
+    int rc = check_rect(ctx, intr, views, nviews, ratios, axs_mins, fr, src, dst, make_fill(fill, &c.fill));
+    if (rc) return rc;
     CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    const size_t frame_elems = pitch * (size_t)sz2;          // device frames are stored pitch*sz2
-    const size_t frame_bytes = frame_elems * px_bytes;
-    int per = 0;
-    const std::vector<int> chunks = chunk_schedule(nframes, frame_bytes, nframes, &per);
-    const bool dense = frame_stride == frame_elems && pitch == (size_t)sz1;
-    for (int f0 = 0, it = 0, m = 0; f0 < nframes; f0 += m, ++it) {
-        const int k = it % cc_ctx::NSLOT;
-        m = chunks[it];
-        // +64 bytes: vector gathers may touch the aligned word holding the last texel
-        if ((rc = ensure_slot(ctx, k, per * frame_bytes + 64, per * frame_bytes + 64))) return rc;
-        cudaStream_t st = ctx->pipe_stream[k];
-        uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[k]);
-        uint8_t* dout = static_cast<uint8_t*>(ctx->pipe_out[k]);
-        const uint8_t* hs = reinterpret_cast<const uint8_t*>(src) + (size_t)f0 * frame_stride * px_bytes;
-        uint8_t* hd = reinterpret_cast<uint8_t*>(dst) + (size_t)f0 * frame_stride * px_bytes;
-        if (dense) {
-            CC_CUDA(cudaMemcpyAsync(din, hs, (size_t)m * frame_bytes, cudaMemcpyHostToDevice, st));
-        } else {
-            for (int f = 0; f < m; ++f)
-                CC_CUDA(cudaMemcpy2DAsync(din + (size_t)f * frame_bytes, pitch * px_bytes,
-                                          hs + (size_t)f * frame_stride * px_bytes, pitch * px_bytes,
-                                          (size_t)sz1 * px_bytes, sz2, cudaMemcpyHostToDevice, st));
-        }
-        if ((rc = launch(reinterpret_cast<const PX*>(din), reinterpret_cast<PX*>(dout), frame_elems, m, st)))
+    if ((rc = enter(ctx)) || nviews == 0 || fr.fpv == 0) return rc;
+    std::vector<ChainD> chs((size_t)nviews);
+    for (int v = 0; v < nviews; ++v) build_chain(intr, views + v, &chs[v]);
+    c.views.chs = chs.data();
+    cudaStream_t stream_ = (cudaStream_t)stream;
+    if (!many) return launch_rectify(ctx, c, 0, fr.fpv, src, dst, stream_);
+    const size_t view_elems = (size_t)fr.fpv * fr.frame_stride * RectPx<PX>::channels;
+    std::vector<char> done((size_t)nviews, 0);
+    bool single = true;
+    if (const char* e = getenv("CAMCAL_VIEWS_SINGLE")) single = atoi(e) != 0;
+    int ndone = 0;
+    const int per = rectify_views_per_launch();
+    for (int v0 = 0; single && v0 < nviews; v0 += per) {
+        const int nv = std::min(per, nviews - v0);
+        bool ok = false;
+        if ((rc = launch_rectify_group(ctx, c, v0, nv, src + v0 * view_elems, dst + v0 * view_elems, stream_, &ok)))
             return rc;
-        if (dense) {
-            CC_CUDA(cudaMemcpyAsync(hd, dout, (size_t)m * frame_bytes, cudaMemcpyDeviceToHost, st));
-        } else {
-            for (int f = 0; f < m; ++f)
-                CC_CUDA(cudaMemcpy2DAsync(hd + (size_t)f * frame_stride * px_bytes, pitch * px_bytes,
-                                          dout + (size_t)f * frame_bytes, pitch * px_bytes,
-                                          (size_t)sz1 * px_bytes, sz2, cudaMemcpyDeviceToHost, st));
+        if (ok) { for (int v = v0; v < v0 + nv; ++v) done[v] = 1; ndone += nv; }
+    }
+    if (ndone == nviews) return CC_OK;
+    // One launch per view.  On a single stream the launches serialise: every persistent kernel ramps up
+    // and drains alone (a 1080p frame is ~15 us of launch + tail for ~5 us of work).  The views are
+    // therefore spread round-robin over the context's side streams, forked from and joined to `stream`
+    // with events, so consecutive views overlap.
+    const int lanes = std::min<int>(cc_ctx::NSLOT, nviews);
+    cudaEvent_t fork = nullptr, join[cc_ctx::NSLOT] = {};
+    if (lanes > 1) {
+        CC_CUDA(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
+        CC_CUDA(cudaEventRecord(fork, stream_));
+        for (int k = 0; k < lanes; ++k) {
+            if ((rc = ensure_stream(ctx, k))) return rc;
+            CC_CUDA(cudaStreamWaitEvent(ctx->pipe_stream[k], fork, 0));
         }
     }
-    return drain(ctx);
+    for (int v = 0; v < nviews; ++v) {
+        if (done[v]) continue;
+        cudaStream_t st = lanes > 1 ? ctx->pipe_stream[v % lanes] : stream_;
+        if ((rc = launch_rectify(ctx, c, v, fr.fpv, src + v * view_elems, dst + v * view_elems, st))) break;
+    }
+    if (lanes > 1) {                                  // join even after an error: nothing stays forked
+        for (int k = 0; k < lanes; ++k) {
+            if (cudaEventCreateWithFlags(&join[k], cudaEventDisableTiming) == cudaSuccess) {
+                cudaEventRecord(join[k], ctx->pipe_stream[k]);
+                cudaStreamWaitEvent(stream_, join[k], 0);
+                cudaEventDestroy(join[k]);            // released once the wait has consumed it
+            }
+        }
+        cudaEventDestroy(fork);
+    }
+    return rc;
+}
+
+// m frames from `from` to `to` (kind: which way): one side is a slot, frames pitch * sz2 apart, the other the caller's
+// host frames, frame_stride apart.  One copy when the host frames are dense, else one 2-D copy per frame.
+static int copy_frames(const RectFrames& fr, size_t pxb, int m, const void* from, void* to, cudaMemcpyKind kind,
+                       cudaStream_t st) {
+    const size_t line = fr.pitch * pxb, slot_frame = line * fr.sz2, host_frame = fr.frame_stride * pxb;
+    const bool up = kind == cudaMemcpyHostToDevice, dense = host_frame == slot_frame && fr.pitch == (size_t)fr.sz1;
+    const size_t from_frame = up ? host_frame : slot_frame, to_frame = up ? slot_frame : host_frame;
+    for (int f = 0; f < (dense ? 1 : m); ++f) {
+        const uint8_t* s = static_cast<const uint8_t*>(from) + (size_t)f * from_frame;
+        uint8_t* d = static_cast<uint8_t*>(to) + (size_t)f * to_frame;
+        const cudaError_t e = dense ? cudaMemcpyAsync(d, s, (size_t)m * slot_frame, kind, st)
+                                    : cudaMemcpy2DAsync(d, line, s, line, (size_t)fr.sz1 * pxb, fr.sz2, kind, st);
+        if (e != cudaSuccess) return cuda_fail(e, "copy");
+    }
+    return CC_OK;
+}
+
+// Host form: the chunk pipeline over the frame axis of the whole call.  Chunks of whole frames (chunk_schedule) go
+// round-robin through the NSLOT slots: up, launches, down.  A single-view call launches the single-view kernels over
+// each chunk.  The chunks of a `_views` call ignore view boundaries and span at most two 64-view groups (a chunk holds
+// at most 64 views' frames).  Such a chunk makes one staged launch per group it touches, over the window of that
+// group's frames it holds (rectify.cu: RectViewsHost); a group without a staged plan runs the window's views through
+// the single-view kernels on the chunk's own slot stream.  The next group's plan is built on host threads while the
+// device streams the current one: before waiting for it, the uploads of the next NSLOT chunks are enqueued.  Every
+// call drains the slot streams before it returns, after an error too, so no copy into `dst` is left in flight.
+template <typename PX, typename FILL>
+static int rectify_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                        const int64_t* axs_mins, const PX* src, PX* dst, const RectFrames& fr, FILL fill,
+                        unsigned flags, bool many) {
+    RectCall<PX> c{fr, {nullptr, ratios, axs_mins, nviews}, {}, flags};
+    int rc = check_rect(ctx, intr, views, nviews, ratios, axs_mins, fr, src, dst, make_fill(fill, &c.fill));
+    if (rc) return rc;
+    CC_GUARD;
+    if ((rc = enter(ctx)) || nviews == 0 || fr.fpv == 0) return rc;
+    std::vector<ChainD> chs((size_t)nviews);
+    for (int v = 0; v < nviews; ++v) build_chain(intr, views + v, &chs[v]);
+    c.views.chs = chs.data();
+    const size_t pxb = RectPx<PX>::bytes, frame_bytes = fr.pitch * (size_t)fr.sz2 * pxb;
+    c.fr.frame_stride = fr.pitch * (size_t)fr.sz2;           // device frames are stored pitch*sz2
+    const int nframes = nviews * fr.fpv, gframes = many ? rectify_views_per_launch() * fr.fpv : nframes;
+    int per = 0;
+    const std::vector<int> chunks = chunk_schedule(nframes, frame_bytes, gframes, &per);
+    const int nchunks = (int)chunks.size();
+    std::vector<int> first((size_t)nchunks + 1, 0);
+    for (int i = 0; i < nchunks; ++i) first[i + 1] = first[i] + chunks[i];
+    const uint8_t* hsrc = reinterpret_cast<const uint8_t*>(src);
+    uint8_t* hdst = reinterpret_cast<uint8_t*>(dst);
+    // frame f of a chunk in slot buffer p
+    auto at = [&](void* p, int f) { return reinterpret_cast<PX*>(static_cast<uint8_t*>(p) + (size_t)f * frame_bytes); };
+    RectViewsHost* vh = nullptr;
+    if (many && (rc = rect_vh_begin(ctx, c, &vh))) return rc;
+    std::vector<char> uploaded((size_t)nchunks, 0), prepared((size_t)((nframes + gframes - 1) / gframes), 0);
+    // chunk i's frames to its slot (the slot's previous chunk, i - NSLOT, is enqueued in full by then); +64 bytes:
+    // vector gathers may touch the aligned word holding the last texel
+    auto upload = [&](int i) -> int {
+        if (i >= nchunks || uploaded[i]) return CC_OK;
+        const int k = i % cc_ctx::NSLOT;
+        int r = ensure_slot(ctx, k, per * frame_bytes + 64, per * frame_bytes + 64);
+        if (!r) r = copy_frames(fr, pxb, chunks[i], hsrc + (size_t)first[i] * fr.frame_stride * pxb, ctx->pipe_in[k],
+                                cudaMemcpyHostToDevice, ctx->pipe_stream[k]);
+        uploaded[i] = r == CC_OK;
+        return r;
+    };
+    int retired = 0;                                        // groups whose chunks are all enqueued
+    for (int i = 0; rc == CC_OK && i < nchunks; ++i) {
+        const int f0 = first[i], m = chunks[i], g_lo = f0 / gframes, g_hi = (f0 + m - 1) / gframes;
+        for (int gi = g_lo; vh && rc == CC_OK && gi <= g_hi; ++gi) {
+            if (prepared[gi]) continue;
+            for (int j = 0; rc == CC_OK && j < cc_ctx::NSLOT; ++j) rc = upload(i + j);
+            if (rc == CC_OK) rc = rect_vh_prepare(vh, gi);
+            prepared[gi] = 1;
+        }
+        if (rc == CC_OK) rc = upload(i);
+        if (rc) break;
+        const int k = i % cc_ctx::NSLOT;
+        cudaStream_t st = ctx->pipe_stream[k];
+        if (!vh) rc = launch_rectify(ctx, c, 0, m, at(ctx->pipe_in[k], 0), at(ctx->pipe_out[k], 0), st);
+        for (int gi = g_lo; vh && rc == CC_OK && gi <= g_hi; ++gi) {
+            const int a = std::max(f0, gi * gframes), b = std::min(f0 + m, (gi + 1) * gframes);
+            bool ok = false;
+            rc = rect_vh_launch(vh, c, gi, a - gi * gframes, b - a, at(ctx->pipe_in[k], a - f0),
+                                at(ctx->pipe_out[k], a - f0), st, &ok);
+            for (int v = a / fr.fpv; rc == CC_OK && !ok && v <= (b - 1) / fr.fpv; ++v) {
+                const int fa = std::max(a, v * fr.fpv), fb = std::min(b, (v + 1) * fr.fpv);
+                rc = launch_rectify(ctx, c, v, fb - fa, at(ctx->pipe_in[k], fa - f0), at(ctx->pipe_out[k], fa - f0), st);
+            }
+        }
+        if (rc) break;
+        rc = copy_frames(fr, pxb, m, ctx->pipe_out[k], hdst + (size_t)f0 * fr.frame_stride * pxb, cudaMemcpyDeviceToHost,
+                         st);
+        for (; vh && (retired < g_hi || (retired == g_hi && f0 + m == std::min(nframes, (g_hi + 1) * gframes))); ++retired)
+            rect_vh_retire(vh, retired);
+    }
+    const int re = rect_vh_end(vh);                         // every plan fenced, uploads complete
+    const int rd = drain(ctx);
+    return rc ? rc : re ? re : rd;
+}
+
+// the map alone: FP64 (the exact coordinates) or FP32 (the fast ones)
+template <typename T>
+static int rectify_map(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio, const int64_t* axs_min,
+                       T* map_row, T* map_col, int sz1, int sz2, size_t pitch, void* stream) {
+    int rc = check_rect(ctx, intr, view, 1, &ratio, axs_min, {sz1, sz2, pitch, pitch * (size_t)sz2, 0}, nullptr,
+                        nullptr, true);
+    if (rc) return rc;
+    CC_REQUIRE(map_row && map_col, "NULL map pointer");
+    CC_GUARD;
+    if ((rc = enter(ctx))) return rc;
+    ChainD ch;
+    build_chain(intr, view, &ch);
+    return launch_rectify_map<T>(ctx, ch, ratio, axs_min, map_row, map_col, sz1, sz2, pitch, (cudaStream_t)stream);
 }
 
 }  // namespace cc
@@ -572,258 +740,76 @@ int cc_rectify_f32c1(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, doub
                      const int64_t axs_min[2], const float* src, float* dst, int sz1, int sz2,
                      size_t pitch, size_t frame_stride, int nframes, float fill, unsigned flags,
                      void* stream) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    if ((rc = check_rect_args(axs_min, sz1, sz2, pitch, frame_stride, nframes, ratio))) return rc;
-    CC_REQUIRE(nframes == 0 || (src && dst), "NULL frame pointer");
-    CC_REQUIRE(nframes == 0 || (const void*)src != (const void*)dst, "rectification is not in place: src == dst");
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    return launch_rectify_f32c1(ctx, ch, ratio, axs_min, src, dst, sz1, sz2, pitch, frame_stride,
-                                nframes, fill, flags, (cudaStream_t)stream);
+    return rectify_device(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+                          flags, stream, false);
 }
 
 int cc_rectify_u8c3(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
                     const int64_t axs_min[2], const uint8_t* src, uint8_t* dst, int sz1, int sz2,
                     size_t pitch, size_t frame_stride, int nframes, const uint8_t fill[3],
                     unsigned flags, void* stream) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    if ((rc = check_rect_args(axs_min, sz1, sz2, pitch, frame_stride, nframes, ratio))) return rc;
-    CC_REQUIRE(nframes == 0 || (src && dst), "NULL frame pointer");
-    CC_REQUIRE(nframes == 0 || (const void*)src != (const void*)dst, "rectification is not in place: src == dst");
-    CC_REQUIRE(fill != nullptr, "fill is NULL");
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    return launch_rectify_u8c3(ctx, ch, ratio, axs_min, src, dst, sz1, sz2, pitch, frame_stride,
-                               nframes, fill, flags, (cudaStream_t)stream);
+    return rectify_device(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+                          flags, stream, false);
 }
-
-}  // extern "C"
-
-// the argument rules of the many-view rectification calls (device and host forms alike)
-static int check_rect_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
-                            const int64_t* axs_mins, const void* src, const void* dst, int sz1, int sz2, size_t pitch,
-                            size_t frame_stride, int frames_per_view) {
-    CC_REQUIRE(ctx && intr && (nviews == 0 || (views && ratios && axs_mins)), "NULL argument");
-    CC_REQUIRE(nviews >= 0 && frames_per_view >= 0, "bad counts");
-    CC_REQUIRE((long long)nviews * frames_per_view <= 65535, "at most 65535 frames per call");
-    int rc = CC_OK;
-    for (int v = 0; v < nviews; ++v) {
-        if ((rc = check_params(ctx, intr, views + v))) return rc;
-        if ((rc = check_rect_args(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, frames_per_view, ratios[v]))) return rc;
-    }
-    CC_REQUIRE(nviews * frames_per_view == 0 || (src && dst), "NULL frame pointer");
-    CC_REQUIRE(nviews * frames_per_view == 0 || src != dst, "rectification is not in place: src == dst");
-    CC_REQUIRE(nviews * frames_per_view <= 1 || frame_stride >= pitch * (size_t)(sz2 - 1) + sz1, "frames overlap");
-    return CC_OK;
-}
-
-// Frames with DIFFERENT views in one call: the reference's plot loop rectifies every calibration
-// image with its own extrinsic (src/plot_calibration.jl:36-42).  frames [v * frames_per_view,
-// (v + 1) * frames_per_view) use views[v], ratios[v], axs_mins[2v .. 2v+1].  Every view is one
-// launch with its own cached tile plan.
-template <typename P, typename F, typename G>
-static int rectify_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
-                         const int64_t* axs_mins, const P* src, P* dst, int sz1, int sz2, size_t pitch,
-                         size_t frame_stride, int frames_per_view, int channels, cudaStream_t stream, F launch,
-                         G launch_group) {
-    int rc = check_rect_views(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
-                              frames_per_view);
-    if (rc) return rc;
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    if (nviews == 0 || frames_per_view == 0) return CC_OK;
-    // Groups of up to 64 views in ONE launch each (rectify.cu: launch_rectify_*_views) when the layout can be
-    // staged; CAMCAL_VIEWS_SINGLE=0 (tuning knob) or a group that cannot be staged: one launch per view, below.
-    std::vector<ChainD> chs((size_t)nviews);
-    for (int v = 0; v < nviews; ++v) build_chain(intr, views + v, &chs[v]);
-    std::vector<char> done((size_t)nviews, 0);
-    bool single = true;
-    if (const char* e = getenv("CAMCAL_VIEWS_SINGLE")) single = atoi(e) != 0;
-    int ndone = 0;
-    const int per = rectify_views_per_launch();
-    for (int v0 = 0; single && v0 < nviews; v0 += per) {
-        const int nv = std::min(per, nviews - v0);
-        const size_t off = (size_t)v0 * frames_per_view * frame_stride * channels;
-        bool ok = false;
-        if ((rc = launch_group(chs.data() + v0, ratios + v0, axs_mins + 2 * v0, nv, src + off, dst + off, stream, &ok))) return rc;
-        if (ok) { for (int v = v0; v < v0 + nv; ++v) done[v] = 1; ndone += nv; }
-    }
-    if (ndone == nviews) return CC_OK;
-    // One launch per view.  On a single stream the launches serialise: every persistent kernel ramps up
-    // and drains alone (a 1080p frame is ~15 us of launch + tail for ~5 us of work).  The views are
-    // therefore spread round-robin over the context's side streams, forked from and joined to `stream`
-    // with events, so consecutive views overlap.
-    const int lanes = std::min<int>(cc_ctx::NSLOT, nviews);
-    cudaEvent_t fork = nullptr, join[cc_ctx::NSLOT] = {};
-    if (lanes > 1) {
-        CC_CUDA(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-        CC_CUDA(cudaEventRecord(fork, stream));
-        for (int k = 0; k < lanes; ++k) {
-            if ((rc = ensure_stream(ctx, k))) return rc;
-            CC_CUDA(cudaStreamWaitEvent(ctx->pipe_stream[k], fork, 0));
-        }
-    }
-    for (int v = 0; v < nviews; ++v) {
-        if (done[v]) continue;
-        const size_t off = (size_t)v * frames_per_view * frame_stride * channels;
-        cudaStream_t st = lanes > 1 ? ctx->pipe_stream[v % lanes] : stream;
-        if ((rc = launch(chs[v], ratios[v], axs_mins + 2 * v, src + off, dst + off, st))) break;
-    }
-    if (lanes > 1) {                                  // join even after an error: nothing stays forked
-        for (int k = 0; k < lanes; ++k) {
-            if (cudaEventCreateWithFlags(&join[k], cudaEventDisableTiming) == cudaSuccess) {
-                cudaEventRecord(join[k], ctx->pipe_stream[k]);
-                cudaStreamWaitEvent(stream, join[k], 0);
-                cudaEventDestroy(join[k]);            // released once the wait has consumed it
-            }
-        }
-        cudaEventDestroy(fork);
-    }
-    return rc;
-}
-
-
-// Frames of many views from host memory in one call (cc_rectify_views_*_host): the chunk pipeline of rectify_host
-// over the frame axis of the whole call.  Chunks ignore view boundaries and span at most two 64-view groups (a
-// chunk holds at most 64 views' frames).  A chunk makes one staged launch per group it touches, over the window of
-// that group's frames it holds (rectify.cu: RectViewsHost); a group without a staged plan runs the window's views
-// through the single-view kernels on the chunk's own slot stream.  The next group's plan is built on host threads
-// while the device streams the current one: before waiting for it, the uploads of the next NSLOT chunks are
-// enqueued.  LAUNCH_GROUP(vh, g, w0, wn, src, dst, st, ok) / LAUNCH_ONE(v, src, dst, nframes, st).
-template <typename PX, typename LAUNCH_GROUP, typename LAUNCH_ONE>
-static int rectify_views_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
-                              const int64_t* axs_mins, const PX* src, PX* dst, int sz1, int sz2, size_t pitch,
-                              size_t frame_stride, int fpv, int pxb, unsigned flags, std::vector<ChainD>* chs,
-                              LAUNCH_GROUP launch_group, LAUNCH_ONE launch_one) {
-    int rc = check_rect_views(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride, fpv);
-    if (rc) return rc;
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    if (nviews == 0 || fpv == 0) return CC_OK;
-    chs->resize((size_t)nviews);
-    for (int v = 0; v < nviews; ++v) build_chain(intr, views + v, &(*chs)[v]);
-    const int nframes = nviews * fpv, gframes = rectify_views_per_launch() * fpv;
-    const size_t frame_elems = pitch * (size_t)sz2;          // device frames are stored pitch*sz2
-    const size_t frame_bytes = frame_elems * pxb;
-    int per = 0;
-    const std::vector<int> chunks = chunk_schedule(nframes, frame_bytes, gframes, &per);
-    const int nchunks = (int)chunks.size();
-    std::vector<int> first((size_t)nchunks + 1, 0);
-    for (int c = 0; c < nchunks; ++c) first[c + 1] = first[c] + chunks[c];
-    const bool dense = frame_stride == frame_elems && pitch == (size_t)sz1;
-    const uint8_t* hsrc = reinterpret_cast<const uint8_t*>(src);
-    uint8_t* hdst = reinterpret_cast<uint8_t*>(dst);
-    RectViewsHost* vh = nullptr;
-    if ((rc = rect_vh_begin(ctx, chs->data(), ratios, axs_mins, nviews, sz1, sz2, pitch, fpv, pxb,
-                            !(flags & CC_GATHER_DIRECT), &vh)))
-        return rc;
-    std::vector<char> uploaded((size_t)nchunks, 0), prepared((size_t)((nframes + gframes - 1) / gframes), 0);
-    // chunk c's frames to its slot (the slot's previous chunk, c - NSLOT, is enqueued in full by then)
-    auto upload = [&](int c) -> int {
-        if (c >= nchunks || uploaded[c]) return CC_OK;
-        const int k = c % cc_ctx::NSLOT, m = chunks[c];
-        int r = ensure_slot(ctx, k, per * frame_bytes + 64, per * frame_bytes + 64);   // +64: see rectify_host
-        if (r) return r;
-        uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[k]);
-        const uint8_t* hs = hsrc + (size_t)first[c] * frame_stride * pxb;
-        if (dense) {
-            CC_CUDA(cudaMemcpyAsync(din, hs, (size_t)m * frame_bytes, cudaMemcpyHostToDevice, ctx->pipe_stream[k]));
-        } else {
-            for (int f = 0; f < m; ++f)
-                CC_CUDA(cudaMemcpy2DAsync(din + (size_t)f * frame_bytes, pitch * pxb, hs + (size_t)f * frame_stride * pxb,
-                                          pitch * pxb, (size_t)sz1 * pxb, sz2, cudaMemcpyHostToDevice, ctx->pipe_stream[k]));
-        }
-        uploaded[c] = 1;
-        return CC_OK;
-    };
-    int retired = 0;                                        // groups whose chunks are all enqueued
-    for (int c = 0; rc == CC_OK && c < nchunks; ++c) {
-        const int f0 = first[c], m = chunks[c], g_lo = f0 / gframes, g_hi = (f0 + m - 1) / gframes;
-        for (int gi = g_lo; rc == CC_OK && gi <= g_hi; ++gi) {
-            if (prepared[gi]) continue;
-            for (int j = 0; rc == CC_OK && j < cc_ctx::NSLOT; ++j) rc = upload(c + j);
-            if (rc == CC_OK) rc = rect_vh_prepare(vh, gi);
-            prepared[gi] = 1;
-        }
-        if (rc == CC_OK) rc = upload(c);
-        if (rc) break;
-        const int k = c % cc_ctx::NSLOT;
-        cudaStream_t st = ctx->pipe_stream[k];
-        uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[k]);
-        uint8_t* dout = static_cast<uint8_t*>(ctx->pipe_out[k]);
-        for (int gi = g_lo; rc == CC_OK && gi <= g_hi; ++gi) {
-            const int a = std::max(f0, gi * gframes), b = std::min(f0 + m, (gi + 1) * gframes);
-            const size_t off = (size_t)(a - f0) * frame_bytes;
-            bool ok = false;
-            rc = launch_group(vh, gi, a - gi * gframes, b - a, reinterpret_cast<const PX*>(din + off),
-                              reinterpret_cast<PX*>(dout + off), st, &ok);
-            for (int v = a / fpv; rc == CC_OK && !ok && v <= (b - 1) / fpv; ++v) {
-                const int fa = std::max(a, v * fpv), fb = std::min(b, (v + 1) * fpv);
-                const size_t o = (size_t)(fa - f0) * frame_bytes;
-                rc = launch_one(v, reinterpret_cast<const PX*>(din + o), reinterpret_cast<PX*>(dout + o), fb - fa, st);
-            }
-        }
-        if (rc) break;
-        uint8_t* hd = hdst + (size_t)f0 * frame_stride * pxb;
-        if (dense) {
-            rc = cuda_check(cudaMemcpyAsync(hd, dout, (size_t)m * frame_bytes, cudaMemcpyDeviceToHost, st), "copy");
-        } else {
-            for (int f = 0; rc == CC_OK && f < m; ++f)
-                rc = cuda_check(cudaMemcpy2DAsync(hd + (size_t)f * frame_stride * pxb, pitch * pxb, dout + (size_t)f * frame_bytes,
-                                                  pitch * pxb, (size_t)sz1 * pxb, sz2, cudaMemcpyDeviceToHost, st), "copy");
-        }
-        for (; retired < g_hi || (retired == g_hi && f0 + m == std::min(nframes, (g_hi + 1) * gframes)); ++retired)
-            rect_vh_retire(vh, retired);
-    }
-    const int re = rect_vh_end(vh);                         // every plan fenced, uploads complete
-    const int rd = drain(ctx);
-    return rc ? rc : re ? re : rd;
-}
-
-extern "C" {
 
 int cc_rectify_f32c1_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
                            const int64_t* axs_mins, const float* src, float* dst, int sz1, int sz2, size_t pitch,
                            size_t frame_stride, int frames_per_view, float fill, unsigned flags, void* stream) {
-    return rectify_views(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
-                         frames_per_view, 1, (cudaStream_t)stream,
-                         [&](const ChainD& ch, double ratio, const int64_t* axs, const float* s, float* d, cudaStream_t st) {
-                             return launch_rectify_f32c1(ctx, ch, ratio, axs, s, d, sz1, sz2, pitch, frame_stride,
-                                                         frames_per_view, fill, flags, st);
-                         },
-                         [&](const ChainD* chs, const double* rs, const int64_t* axs, int nv, const float* s, float* d,
-                             cudaStream_t st, bool* ok) {
-                             *ok = false;
-                             if (flags & CC_GATHER_DIRECT) return (int)CC_OK;
-                             return launch_rectify_f32c1_views(ctx, chs, rs, axs, nv, s, d, sz1, sz2, pitch, frame_stride,
-                                                               frames_per_view, fill, flags, st, ok);
-                         });
+    return rectify_device(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                          {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, stream, true);
 }
 
 int cc_rectify_u8c3_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
                           const int64_t* axs_mins, const uint8_t* src, uint8_t* dst, int sz1, int sz2, size_t pitch,
                           size_t frame_stride, int frames_per_view, const uint8_t fill[3], unsigned flags,
                           void* stream) {
-    CC_REQUIRE(fill != nullptr, "fill is NULL");
-    return rectify_views(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
-                         frames_per_view, 3, (cudaStream_t)stream,
-                         [&](const ChainD& ch, double ratio, const int64_t* axs, const uint8_t* s, uint8_t* d, cudaStream_t st) {
-                             return launch_rectify_u8c3(ctx, ch, ratio, axs, s, d, sz1, sz2, pitch, frame_stride,
-                                                        frames_per_view, fill, flags, st);
-                         },
-                         [&](const ChainD* chs, const double* rs, const int64_t* axs, int nv, const uint8_t* s, uint8_t* d,
-                             cudaStream_t st, bool* ok) {
-                             *ok = false;
-                             if (flags & CC_GATHER_DIRECT) return (int)CC_OK;
-                             return launch_rectify_u8c3_views(ctx, chs, rs, axs, nv, s, d, sz1, sz2, pitch, frame_stride,
-                                                              frames_per_view, fill, flags, st, ok);
-                         });
+    return rectify_device(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                          {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, stream, true);
+}
+
+int cc_rectify_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
+                          const int64_t axs_min[2], const float* src, float* dst, int sz1, int sz2,
+                          size_t pitch, size_t frame_stride, int nframes, float fill,
+                          unsigned flags) {
+    return rectify_host(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+                        flags, false);
+}
+
+int cc_rectify_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
+                         const int64_t axs_min[2], const uint8_t* src, uint8_t* dst, int sz1,
+                         int sz2, size_t pitch, size_t frame_stride, int nframes,
+                         const uint8_t fill[3], unsigned flags) {
+    return rectify_host(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+                        flags, false);
+}
+
+// many views from host memory
+int cc_rectify_views_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                const double* ratios, const int64_t* axs_mins, const float* src, float* dst,
+                                int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
+                                float fill, unsigned flags) {
+    return rectify_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                        {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, true);
+}
+
+int cc_rectify_views_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                               const double* ratios, const int64_t* axs_mins, const uint8_t* src, uint8_t* dst,
+                               int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
+                               const uint8_t fill[3], unsigned flags) {
+    return rectify_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                        {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, true);
+}
+
+int cc_rectify_map_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
+                       const int64_t axs_min[2], double* map_row, double* map_col, int sz1, int sz2,
+                       size_t pitch, void* stream) {
+    return rectify_map(ctx, intr, view, ratio, axs_min, map_row, map_col, sz1, sz2, pitch, stream);
+}
+
+int cc_rectify_map_f32(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
+                       const int64_t axs_min[2], float* map_row, float* map_col, int sz1, int sz2,
+                       size_t pitch, void* stream) {
+    return rectify_map(ctx, intr, view, ratio, axs_min, map_row, map_col, sz1, sz2, pitch, stream);
 }
 
 int cc_jpeg_info(const uint8_t* jpeg, size_t length, int* sz1, int* sz2, int* channels) {
@@ -844,109 +830,6 @@ int cc_jpeg_decode_u8c3(cc_ctx* ctx, const uint8_t* const* jpegs, const size_t* 
     CC_GUARD;
     if ((rc = enter(ctx))) return rc;
     return jpeg_decode_u8c3(ctx, jpegs, lengths, n, dst, sz1, sz2, pitch, frame_stride, (cudaStream_t)stream);
-}
-
-int cc_rectify_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
-                          const int64_t axs_min[2], const float* src, float* dst, int sz1, int sz2,
-                          size_t pitch, size_t frame_stride, int nframes, float fill,
-                          unsigned flags) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    if ((rc = check_rect_args(axs_min, sz1, sz2, pitch, frame_stride, nframes, ratio))) return rc;
-    CC_REQUIRE(nframes == 0 || (src && dst), "NULL frame pointer");
-    CC_REQUIRE(nframes == 0 || (const void*)src != (const void*)dst, "rectification is not in place: src == dst");
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    return rectify_host<float>(
-        ctx, src, dst, sz1, sz2, pitch, frame_stride, nframes, sizeof(float),
-        [&](const float* s, float* d, size_t fs, int m, cudaStream_t st) {
-            return launch_rectify_f32c1(ctx, ch, ratio, axs_min, s, d, sz1, sz2, pitch, fs, m, fill,
-                                        flags, st);
-        });
-}
-
-int cc_rectify_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
-                         const int64_t axs_min[2], const uint8_t* src, uint8_t* dst, int sz1,
-                         int sz2, size_t pitch, size_t frame_stride, int nframes,
-                         const uint8_t fill[3], unsigned flags) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    if ((rc = check_rect_args(axs_min, sz1, sz2, pitch, frame_stride, nframes, ratio))) return rc;
-    CC_REQUIRE(nframes == 0 || (src && dst), "NULL frame pointer");
-    CC_REQUIRE(nframes == 0 || (const void*)src != (const void*)dst, "rectification is not in place: src == dst");
-    CC_REQUIRE(fill != nullptr, "fill is NULL");
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    return rectify_host<uint8_t>(
-        ctx, src, dst, sz1, sz2, pitch, frame_stride, nframes, 3,
-        [&](const uint8_t* s, uint8_t* d, size_t fs, int m, cudaStream_t st) {
-            return launch_rectify_u8c3(ctx, ch, ratio, axs_min, s, d, sz1, sz2, pitch, fs, m, fill,
-                                       flags, st);
-        });
-}
-
-// ---- many views from host memory ----------------------------------------------------
-int cc_rectify_views_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                                const double* ratios, const int64_t* axs_mins, const float* src, float* dst,
-                                int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
-                                float fill, unsigned flags) {
-    std::vector<ChainD> chs;
-    return rectify_views_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
-                              frames_per_view, (int)sizeof(float), flags, &chs,
-                              [&](RectViewsHost* vh, int gi, int w0, int wn, const float* s, float* d, cudaStream_t st, bool* ok) {
-                                  return rect_vh_launch_f32c1(vh, gi, w0, wn, s, d, fill, flags, st, ok);
-                              },
-                              [&](int v, const float* s, float* d, int m, cudaStream_t st) {
-                                  return launch_rectify_f32c1(ctx, chs[v], ratios[v], axs_mins + 2 * v, s, d, sz1, sz2,
-                                                              pitch, pitch * (size_t)sz2, m, fill, flags, st);
-                              });
-}
-
-int cc_rectify_views_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
-                               const double* ratios, const int64_t* axs_mins, const uint8_t* src, uint8_t* dst,
-                               int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
-                               const uint8_t fill[3], unsigned flags) {
-    CC_REQUIRE(fill != nullptr, "fill is NULL");
-    std::vector<ChainD> chs;
-    return rectify_views_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst, sz1, sz2, pitch, frame_stride,
-                              frames_per_view, 3, flags, &chs,
-                              [&](RectViewsHost* vh, int gi, int w0, int wn, const uint8_t* s, uint8_t* d, cudaStream_t st, bool* ok) {
-                                  return rect_vh_launch_u8c3(vh, gi, w0, wn, s, d, fill, flags, st, ok);
-                              },
-                              [&](int v, const uint8_t* s, uint8_t* d, int m, cudaStream_t st) {
-                                  return launch_rectify_u8c3(ctx, chs[v], ratios[v], axs_mins + 2 * v, s, d, sz1, sz2,
-                                                             pitch, pitch * (size_t)sz2, m, fill, flags, st);
-                              });
-}
-
-int cc_rectify_map_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
-                       const int64_t axs_min[2], double* map_row, double* map_col, int sz1, int sz2,
-                       size_t pitch, void* stream) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    if ((rc = check_rect_args(axs_min, sz1, sz2, pitch, pitch * (size_t)sz2, 1, ratio))) return rc;
-    CC_REQUIRE(map_row && map_col, "NULL map pointer");
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    return launch_rectify_map(ctx, ch, ratio, axs_min, map_row, map_col, sz1, sz2, pitch,
-                              (cudaStream_t)stream);
-}
-
-int cc_rectify_map_f32(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
-                       const int64_t axs_min[2], float* map_row, float* map_col, int sz1, int sz2,
-                       size_t pitch, void* stream) {
-    int rc = check_params(ctx, intr, view);
-    if (rc) return rc;
-    if ((rc = check_rect_args(axs_min, sz1, sz2, pitch, pitch * (size_t)sz2, 1, ratio))) return rc;
-    CC_REQUIRE(map_row && map_col, "NULL map pointer");
-    CC_GUARD;
-    if ((rc = enter(ctx))) return rc;
-    ChainD ch;
-    build_chain(intr, view, &ch);
-    return launch_rectify_map_f32(ctx, ch, ratio, axs_min, map_row, map_col, sz1, sz2, pitch,
-                                  (cudaStream_t)stream);
 }
 
 // get_ratio, src/plot_calibration.jl:8-13

@@ -61,6 +61,31 @@ struct PointSrc {
     size_t base;
     int seg_lo, seg_hi;
 };
+// The pixel of a rectified frame: PX elements (channels) and bytes per pixel, and the fill as the kernels take it
+// (f32c1: one float; u8c3: three bytes)
+template <typename PX> struct RectPx;
+template <> struct RectPx<float> { static constexpr int channels = 1, bytes = 4; using Fill = float; };
+template <> struct RectPx<uint8_t> { static constexpr int channels = 3, bytes = 3; using Fill = uchar3; };
+// A rectification call.  Frames are sz1 x sz2 pixels, lines `pitch` pixels and frames `frame_stride` pixels apart.
+// View v (chs[v], ratios[v], axs_mins[2v .. 2v+1]) rectifies frames [v * fpv, (v + 1) * fpv); a single-view call is
+// one view with all the frames.
+struct RectFrames {
+    int sz1, sz2;
+    size_t pitch, frame_stride;
+    int fpv;
+};
+struct RectViews {
+    const ChainD* chs;
+    const double* ratios;
+    const int64_t* axs_mins;
+    int n;
+};
+template <typename PX> struct RectCall {
+    RectFrames fr;
+    RectViews views;
+    typename RectPx<PX>::Fill fill;
+    unsigned flags;
+};
 
 // error plumbing (abi.cu)
 int set_error(int status, const char* fmt, ...);

@@ -244,22 +244,6 @@ static RectFast make_fast(const ChainD& ch, double ratio, const RectGeom& g) {
     return p;
 }
 
-int check_rect_args(const int64_t axs_min[2], int sz1, int sz2, size_t pitch, size_t frame_stride,
-                    int nframes, double ratio) {
-    CC_REQUIRE(axs_min != nullptr, "axs_min is NULL");
-    CC_REQUIRE(sz1 > 0 && sz2 > 0 && nframes >= 0, "frame size must be positive");
-    CC_REQUIRE(sz1 < (1 << 22) && sz2 < (1 << 22), "frame extent must be < 2^22");
-    CC_REQUIRE(pitch >= (size_t)sz1, "pitch smaller than sz1");
-    CC_REQUIRE(nframes <= 1 || frame_stride >= pitch * (size_t)(sz2 - 1) + sz1, "frames overlap");
-    CC_REQUIRE(pitch * (size_t)sz2 < (size_t)1 << 30, "frame too large (pitch*sz2 must be < 2^30)");
-    CC_REQUIRE(nframes <= 65535, "at most 65535 frames per call");
-    CC_REQUIRE(ratio > 0.0 && ratio == ratio, "ratio must be positive");
-    const int64_t lim = (int64_t)1 << 30;
-    CC_REQUIRE(axs_min[0] > -lim && axs_min[0] < lim && axs_min[1] > -lim && axs_min[1] < lim,
-               "axs_min out of range");
-    return CC_OK;
-}
-
 // host evaluation of the map (double) for the box-size estimate only
 static void host_coord(const ChainD& ch, double inv_ratio, long long I1, long long I2, double* row,
                        double* col) {
@@ -604,30 +588,31 @@ static EncodeTiledFn encoder(cc_ctx* ctx) {
     return reinterpret_cast<EncodeTiledFn>(ctx->encode_tiled);
 }
 
-// Decide whether the TMA-staged variant applies and build its tensor map + tile config.
-// pxb: bytes per pixel (4: one float element; 3: three u8 elements).
-static bool plan_tma(cc_ctx* ctx, const ChainD& ch, double ratio, const RectGeom& g, const void* src,
-                     int pxb, int tw, int tl, cudaStream_t st, CUtensorMap* tmap, TileCfg* cfg,
-                     RectPlan** plan_out) {
-    const size_t pitch_b = (size_t)g.pitch * pxb, frame_b = (size_t)g.frame_stride * pxb;
-    if ((reinterpret_cast<uintptr_t>(src) & 15u) || (pitch_b & 15u) || (g.nframes > 1 && (frame_b & 15u)))
-        return false;
+// ring stages of a staged box: measured (profiles/r1_rectify.md), occupancy beats ring depth; small boxes afford more
+// stages.  The ring hides the TMA round trip: per SM, (stages - 1) x resident CTAs x the USEFUL bytes of a box must
+// cover bandwidth x latency (~30 KB of reads at the HBM roofline, profiles/r2_rectify.md)
+static int ring_stages(int box_bytes) {
+    int stages = std::min(kMaxStages, std::max(2, CAMCAL_RING_BYTES / box_bytes));
+    if (const char* e = getenv("CAMCAL_STAGES")) stages = std::min(kMaxStages, std::max(1, atoi(e)));   // tuning knob
+    while (stages > 2 && stages * box_bytes > 56 * 1024) --stages;
+    return stages;
+}
+
+// TMA can address the frames: 16-byte aligned base, lines and (more than one frame) frames
+static bool tma_aligned(const void* src, int pxb, size_t pitch, size_t frame_stride, int nframes) {
+    return !((reinterpret_cast<uintptr_t>(src) & 15u) || ((pitch * pxb) & 15u) || (nframes > 1 && ((frame_stride * pxb) & 15u)));
+}
+
+// the tensor map of `nframes` frames at src (pxb bytes per pixel) in boxes d, and the box and ring of *cfg; false: the
+// map cannot be encoded
+static bool stage_box(cc_ctx* ctx, const void* src, int pxb, int sz1, int sz2, size_t pitch, size_t frame_stride,
+                      int nframes, const BoxDims& d, CUtensorMap* tmap, TileCfg* cfg) {
     EncodeTiledFn enc = encoder(ctx);
     if (!enc) return false;
-    RectPlan* plan = plan_get(ctx, ch, ratio, g, tw, tl, pxb, st);
-    if (!plan || !plan->box_bytes) return false;
-    // measured (profiles/r1_rectify.md): occupancy beats ring depth; small boxes afford more stages
-    // the ring hides the TMA round trip: per SM, (stages - 1) x resident CTAs x the USEFUL bytes of a box
-    // must cover bandwidth x latency (~30 KB of reads at the HBM roofline, profiles/r2_rectify.md)
-    int stages = std::min(kMaxStages, std::max(2, CAMCAL_RING_BYTES / plan->box_bytes));
-    if (const char* e = getenv("CAMCAL_STAGES")) stages = std::min(kMaxStages, std::max(1, atoi(e)));   // tuning knob
-    while (stages > 2 && stages * plan->box_bytes > 56 * 1024) --stages;
-
-    const int box1_elems = (pxb == 4) ? plan->pitch_b / 4 : plan->pitch_b;
-    cuuint64_t dims[3] = {(cuuint64_t)g.sz1 * (pxb == 4 ? 1 : 3), (cuuint64_t)g.sz2,
-                          (cuuint64_t)std::max(g.nframes, 1)};
-    cuuint64_t strides[2] = {(cuuint64_t)pitch_b, (cuuint64_t)(g.nframes > 1 ? frame_b : pitch_b * g.sz2)};
-    cuuint32_t box[3] = {(cuuint32_t)box1_elems, (cuuint32_t)plan->box2, 1};
+    const size_t pitch_b = pitch * pxb;
+    cuuint64_t dims[3] = {(cuuint64_t)sz1 * (pxb == 4 ? 1 : 3), (cuuint64_t)sz2, (cuuint64_t)std::max(nframes, 1)};
+    cuuint64_t strides[2] = {(cuuint64_t)pitch_b, (cuuint64_t)(nframes > 1 ? frame_stride * pxb : pitch_b * sz2)};
+    cuuint32_t box[3] = {(cuuint32_t)(pxb == 4 ? d.pitch_b / 4 : d.pitch_b), (cuuint32_t)d.box2, 1};
     cuuint32_t estr[3] = {1, 1, 1};
     CUtensorMapL2promotion l2promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
     if (const char* e = getenv("CAMCAL_L2PROMO")) {     // tuning knob: 0 none, 64, 128, 256
@@ -635,13 +620,24 @@ static bool plan_tma(cc_ctx* ctx, const ChainD& ch, double ratio, const RectGeom
         l2promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
                 : v == 256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
     }
-    const CUresult r = enc(tmap, pxb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3,
-                           const_cast<void*>(src), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                           CU_TENSOR_MAP_SWIZZLE_NONE, l2promo,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return false;
-    cfg->box1 = plan->box1; cfg->box2 = plan->box2; cfg->stages = stages; cfg->box_bytes = plan->box_bytes;
-    cfg->pitch_b = plan->pitch_b;
+    memset(tmap, 0, sizeof(*tmap));
+    if (enc(tmap, pxb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(src),
+            dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, l2promo,
+            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+        return false;
+    cfg->box1 = d.box1; cfg->box2 = d.box2; cfg->pitch_b = d.pitch_b; cfg->box_bytes = d.box_bytes;
+    cfg->stages = ring_stages(d.box_bytes);
+    return true;
+}
+
+// Decide whether the TMA-staged variant applies and build its tensor map + tile config.
+static bool plan_tma(cc_ctx* ctx, const ChainD& ch, double ratio, const RectGeom& g, const void* src, int pxb, int tl,
+                     cudaStream_t st, CUtensorMap* tmap, TileCfg* cfg, RectPlan** plan_out) {
+    if (!tma_aligned(src, pxb, g.pitch, g.frame_stride, g.nframes) || !encoder(ctx)) return false;
+    RectPlan* plan = plan_get(ctx, ch, ratio, g, kT, tl, pxb, st);
+    if (!plan || !plan->box_bytes) return false;
+    const BoxDims d = {plan->box1, plan->box2, plan->pitch_b, plan->box_bytes};
+    if (!stage_box(ctx, src, pxb, g.sz1, g.sz2, g.pitch, g.frame_stride, g.nframes, d, tmap, cfg)) return false;
     *plan_out = plan;
     return true;
 }
@@ -744,104 +740,101 @@ static dim3 direct_grid(cc_ctx* ctx, int sz1, int sz2, int nframes, int* lines) 
     return dim3(strips, (sz2 + *lines - 1) / *lines, nframes);
 }
 
-int launch_rectify_f32c1(cc_ctx* ctx, const ChainD& chd, double ratio, const int64_t axs_min[2],
-                         const float* src, float* dst, int sz1, int sz2, size_t pitch,
-                         size_t frame_stride, int nframes, float fill, unsigned flags,
-                         cudaStream_t st) {
-    if (nframes == 0) return CC_OK;
-    const RectGeom g = make_geom(axs_min, sz1, sz2, pitch, frame_stride, nframes);
-    const RectExact pe = make_exact(chd, ratio);
-    const RectFast pf = make_fast(chd, ratio, g);
-    const bool exact = !(flags & CC_COORD_F32);
-    CUtensorMap tmap;
-    memset(&tmap, 0, sizeof(tmap));
-    TileCfg cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    RectPlan* plan = nullptr;
-    const bool tma = !(flags & CC_GATHER_DIRECT) && plan_tma(ctx, chd, ratio, g, src, 4, kT, kTLf, st, &tmap, &cfg, &plan);
-    if ((flags & CC_GATHER_TMA) && !tma)
-        return set_error(CC_ERR_INVALID_ARG, "TMA gather not available for this layout / footprint");
-    int rc = CC_OK;
-    if (tma) {
-        if ((rc = unit_cfg(ctx, &cfg, sz1, sz2, nframes, kT, kTLf, exact ? kFGf32Exact : kFGf32Fast))) return rc;
-        cfg.widen_mul = 0x20000000u;
-        // two frames per ring stage when the ring holds at least four boxes (large boxes keep one) and the
-        // units have at least two frames (single frames, e.g. the per-view launches of cc_rectify_*_views, keep one)
-        const int nf = (kF32FramesPerStage == 2 && cfg.stages >= 4 && cfg.fg >= 2) ? 2 : 1;
-        cfg.stages /= nf;
-        const size_t smem = (size_t)cfg.stages * nf * cfg.box_bytes;
-        uint32_t gsz = 0;
-        if (nf == 2) rc = exact ? persistent_grid(ctx, 0, rectify_f32c1_kernel<true>, smem, cfg, plan, true, &gsz)
-                                : persistent_grid(ctx, 1, rectify_f32c1_kernel<false>, smem, cfg, plan, false, &gsz);
-        else         rc = exact ? persistent_grid(ctx, 4, rectify_f32c1_single_kernel<true>, smem, cfg, plan, true, &gsz)
-                                : persistent_grid(ctx, 5, rectify_f32c1_single_kernel<false>, smem, cfg, plan, false, &gsz);
-        if (rc) return rc;
-        RectSched* sched = nullptr;
-        if ((rc = sched_acquire(ctx, st, &sched))) return rc;
-        if (nf == 2) {
-            if (exact) rectify_f32c1_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst, fill);
-            else       rectify_f32c1_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst, fill);
-        } else {
-            if (exact) rectify_f32c1_single_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst, fill);
-            else       rectify_f32c1_single_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst, fill);
-        }
-        sched_release(ctx, st);
-    } else {
-        int lines = 0;
-        const dim3 grid = direct_grid(ctx, sz1, sz2, nframes, &lines);
-        if (exact) rectify_f32c1_direct_kernel<true><<<grid, kConsumerThreads, 0, st>>>(pe, pf, g, lines, src, dst, fill);
-        else       rectify_f32c1_direct_kernel<false><<<grid, kConsumerThreads, 0, st>>>(pe, pf, g, lines, src, dst, fill);
-    }
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
+// --------------------------------------------------------------------------------------
+// The pixel formats: every fact the launchers below need that differs between fp32 gray and 8-bit RGB.  staged /
+// views / direct: the kernel of each family; *_slot: its g_smem_attr slot (exact; + 1: fast); ring: the ring of a
+// staged launch (nf: frames per stage), returns its dynamic shared memory; launch: the one <<<>>> of every kernel of
+// the format, with the format's arguments after `dst`.
+// --------------------------------------------------------------------------------------
+template <typename PX> struct RectFmt;
 
-int launch_rectify_u8c3(cc_ctx* ctx, const ChainD& chd, double ratio, const int64_t axs_min[2],
-                        const uint8_t* src, uint8_t* dst, int sz1, int sz2, size_t pitch,
-                        size_t frame_stride, int nframes, const uint8_t fill[3], unsigned flags,
-                        cudaStream_t st) {
+template <> struct RectFmt<float> {
+    static constexpr int pxb = RectPx<float>::bytes, tl = kTLf, fg_exact = kFGf32Exact, fg_fast = kFGf32Fast, views_slot = 6;
+    static auto staged(bool e, int nf) {
+        return nf == 2 ? (e ? rectify_f32c1_kernel<true> : rectify_f32c1_kernel<false>)
+                       : (e ? rectify_f32c1_single_kernel<true> : rectify_f32c1_single_kernel<false>);
+    }
+    static int staged_slot(int nf) { return nf == 2 ? 0 : 4; }
+    static auto views(bool e) { return e ? rectify_f32c1_views_kernel<true> : rectify_f32c1_views_kernel<false>; }
+    static auto direct(bool e) { return e ? rectify_f32c1_direct_kernel<true> : rectify_f32c1_direct_kernel<false>; }
+    // two frames per ring stage when the ring holds at least four boxes (large boxes keep one) and the units have at
+    // least two frames (single frames, e.g. the per-view launches of cc_rectify_*_views, keep one); the views kernel
+    // holds one frame per stage
+    static size_t ring(TileCfg& cfg, bool views, int* nf) {
+        *nf = (!views && kF32FramesPerStage == 2 && cfg.stages >= 4 && cfg.fg >= 2) ? 2 : 1;
+        cfg.stages /= *nf;
+        return (size_t)cfg.stages * *nf * cfg.box_bytes;
+    }
+    static bool dst_ok(const float*, const RectFrames&, int) { return true; }
+    template <typename K, typename... A>
+    static void launch(K k, dim3 grid, int threads, size_t smem, cudaStream_t st, const RectCall<float>& c, const A&... a) {
+        k<<<grid, threads, smem, st>>>(a..., c.fill);
+    }
+};
+
+template <> struct RectFmt<uint8_t> {
+    static constexpr int pxb = RectPx<uint8_t>::bytes, tl = kTLu, fg_exact = kFGu8Exact, fg_fast = kFGu8Fast, views_slot = 8;
+    static auto staged(bool e, int) { return e ? rectify_u8c3_kernel<true> : rectify_u8c3_kernel<false>; }
+    static int staged_slot(int) { return 2; }
+    static auto views(bool e) { return e ? rectify_u8c3_views_kernel<true> : rectify_u8c3_views_kernel<false>; }
+    static auto direct(bool e) { return e ? rectify_u8c3_direct_kernel<true> : rectify_u8c3_direct_kernel<false>; }
+    // a stage holds kU8FramesPerStage boxes; + 16: the word-granular gather may read the aligned words that hold the
+    // last tap bytes
+    static size_t ring(TileCfg& cfg, bool, int* nf) {
+        *nf = kU8FramesPerStage;
+        cfg.stages = std::max(2, cfg.stages / kU8FramesPerStage);
+        return (size_t)cfg.stages * kU8FramesPerStage * cfg.box_bytes + 16;
+    }
+    // the staged kernel writes whole 32-bit words: 4-byte aligned output lines
+    static bool dst_ok(const uint8_t* dst, const RectFrames& fr, int nframes) {
+        return (reinterpret_cast<uintptr_t>(dst) & 3u) == 0 && ((fr.pitch * 3) & 3u) == 0 &&
+               (nframes <= 1 || ((fr.frame_stride * 3) & 3u) == 0);
+    }
+    // frame_bytes: the bytes of one frame that belong to the caller (the last line is only sz1 pixels long)
+    template <typename K, typename... A>
+    static void launch(K k, dim3 grid, int threads, size_t smem, cudaStream_t st, const RectCall<uint8_t>& c,
+                       const A&... a) {
+        const unsigned frame_bytes = (unsigned)((c.fr.pitch * (size_t)(c.fr.sz2 - 1) + (size_t)c.fr.sz1) * 3);
+        k<<<grid, threads, smem, st>>>(a..., c.fill, frame_bytes);
+    }
+};
+
+// One launch of the single-view kernels: frames [0, nframes) of view v at src / dst (the call's layout), on st.
+template <typename PX>
+int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const PX* src, PX* dst, cudaStream_t st) {
+    using F = RectFmt<PX>;
     if (nframes == 0) return CC_OK;
-    const RectGeom g = make_geom(axs_min, sz1, sz2, pitch, frame_stride, nframes);
-    const RectExact pe = make_exact(chd, ratio);
-    const RectFast pf = make_fast(chd, ratio, g);
-    const bool exact = !(flags & CC_COORD_F32);
-    const uchar3 f = make_uchar3(fill[0], fill[1], fill[2]);
-    // bytes of one frame that belong to the caller: the last line is only sz1 pixels long
-    const unsigned frame_bytes = (unsigned)((pitch * (size_t)(sz2 - 1) + (size_t)sz1) * 3);
+    const ChainD& ch = c.views.chs[v];
+    const double ratio = c.views.ratios[v];
+    const RectGeom g = make_geom(c.views.axs_mins + 2 * v, c.fr.sz1, c.fr.sz2, c.fr.pitch, c.fr.frame_stride, nframes);
+    const RectExact pe = make_exact(ch, ratio);
+    const RectFast pf = make_fast(ch, ratio, g);
+    const bool exact = !(c.flags & CC_COORD_F32);
     CUtensorMap tmap;
-    memset(&tmap, 0, sizeof(tmap));
     TileCfg cfg;
     memset(&cfg, 0, sizeof(cfg));
     RectPlan* plan = nullptr;
-    // the staged kernel writes whole 32-bit words: 4-byte aligned output lines
-    const bool dst_ok = (reinterpret_cast<uintptr_t>(dst) & 3u) == 0 && ((pitch * 3) & 3u) == 0 &&
-                        (nframes <= 1 || ((frame_stride * 3) & 3u) == 0);
-    const bool tma = !(flags & CC_GATHER_DIRECT) && dst_ok &&
-                     plan_tma(ctx, chd, ratio, g, src, 3, kT, kTLu, st, &tmap, &cfg, &plan);
-    if ((flags & CC_GATHER_TMA) && !tma)
+    const bool tma = !(c.flags & CC_GATHER_DIRECT) && F::dst_ok(dst, c.fr, nframes) &&
+                     plan_tma(ctx, ch, ratio, g, src, F::pxb, F::tl, st, &tmap, &cfg, &plan);
+    if ((c.flags & CC_GATHER_TMA) && !tma)
         return set_error(CC_ERR_INVALID_ARG, "TMA gather not available for this layout / footprint");
     int rc = CC_OK;
     if (tma) {
-        if ((rc = unit_cfg(ctx, &cfg, sz1, sz2, nframes, kT, kTLu, exact ? kFGu8Exact : kFGu8Fast))) return rc;
-        // + 16: the word-granular gather may read the aligned words that hold the last tap bytes
-        cfg.stages = std::max(2, cfg.stages / kU8FramesPerStage);        // a stage holds kU8FramesPerStage boxes
-        const size_t smem = (size_t)cfg.stages * kU8FramesPerStage * cfg.box_bytes + 16;
+        if ((rc = unit_cfg(ctx, &cfg, c.fr.sz1, c.fr.sz2, nframes, kT, F::tl, exact ? F::fg_exact : F::fg_fast))) return rc;
+        cfg.widen_mul = 0x20000000u;
+        int nf = 1;
+        const size_t smem = F::ring(cfg, false, &nf);
+        const auto k = F::staged(exact, nf);
         uint32_t gsz = 0;
-        if ((rc = exact ? persistent_grid(ctx, 2, rectify_u8c3_kernel<true>, smem, cfg, plan, true, &gsz)
-                        : persistent_grid(ctx, 3, rectify_u8c3_kernel<false>, smem, cfg, plan, false, &gsz))) return rc;
+        if ((rc = persistent_grid(ctx, F::staged_slot(nf) + !exact, k, smem, cfg, plan, exact, &gsz))) return rc;
         RectSched* sched = nullptr;
         if ((rc = sched_acquire(ctx, st, &sched))) return rc;
-        if (exact)
-            rectify_u8c3_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst, f, frame_bytes);
-        else
-            rectify_u8c3_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst, f, frame_bytes);
+        F::launch(k, gsz, kConsumerThreads + 32, smem, st, c, tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst);
         sched_release(ctx, st);
     } else {
         int lines = 0;
-        const dim3 grid = direct_grid(ctx, sz1, sz2, nframes, &lines);
-        if (exact) rectify_u8c3_direct_kernel<true><<<grid, kConsumerThreads, 0, st>>>(pe, pf, g, lines, src, dst, f, frame_bytes);
-        else       rectify_u8c3_direct_kernel<false><<<grid, kConsumerThreads, 0, st>>>(pe, pf, g, lines, src, dst, f, frame_bytes);
+        const dim3 grid = direct_grid(ctx, c.fr.sz1, c.fr.sz2, nframes, &lines);
+        F::launch(F::direct(exact), grid, kConsumerThreads, 0, st, c, pe, pf, g, lines, src, dst);
     }
     ctx->launches++;
     CC_CUDA(cudaGetLastError());
@@ -1036,153 +1029,94 @@ static long long window_groups(int fpv, int fg, int w0, int wn, uint32_t* g0) {
     return hi - lo + 1;
 }
 
-// tensor map, unit configuration and view table of one launch of a group's plan over frames [w0, w0 + wn) of the
-// group; src: the window's first frame; frames frame_stride elements apart.  *ok = false: the launch does not apply
-static int views_window(cc_ctx* ctx, MultiPlan* mp, const ChainD* chs, const double* ratios, const int64_t* axs_mins,
-                        int nviews, const void* src, int pxb, int tl, int sz1, int sz2, size_t pitch, size_t frame_stride,
-                        int fpv, int w0, int wn, int fg_max, ViewsLaunch* L, bool* ok) {
+// tensor map, unit configuration and view table of one launch of a group's plan (views [v0, v0 + nv) of the call)
+// over frames [w0, w0 + wn) of the group; src: the window's first frame.  *ok = false: the launch does not apply
+template <typename PX>
+static int views_window(cc_ctx* ctx, MultiPlan* mp, const RectCall<PX>& c, int v0, int nv, const PX* src, int w0,
+                        int wn, ViewsLaunch* L, bool* ok) {
+    using F = RectFmt<PX>;
+    const RectFrames& fr = c.fr;
     *ok = false;
-    EncodeTiledFn enc = encoder(ctx);
-    if (!enc) return CC_OK;
-    const size_t pitch_b = pitch * pxb, frame_b = frame_stride * pxb;
-    int stages = std::min(kMaxStages, std::max(2, CAMCAL_RING_BYTES / mp->d.box_bytes));
-    if (const char* e = getenv("CAMCAL_STAGES")) stages = std::min(kMaxStages, std::max(1, atoi(e)));   // tuning knob
-    while (stages > 2 && stages * mp->d.box_bytes > 56 * 1024) --stages;
-    memset(&L->tmap, 0, sizeof(L->tmap));
-    const int box1_elems = (pxb == 4) ? mp->d.pitch_b / 4 : mp->d.pitch_b;
-    cuuint64_t dims[3] = {(cuuint64_t)sz1 * (pxb == 4 ? 1 : 3), (cuuint64_t)sz2, (cuuint64_t)wn};
-    cuuint64_t strides[2] = {(cuuint64_t)pitch_b, (cuuint64_t)(wn > 1 ? frame_b : pitch_b * sz2)};
-    cuuint32_t box[3] = {(cuuint32_t)box1_elems, (cuuint32_t)mp->d.box2, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    if (enc(&L->tmap, pxb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3,
-            const_cast<void*>(src), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
-        return CC_OK;
     TileCfg& cfg = L->cfg;
     memset(&cfg, 0, sizeof(cfg));
-    cfg.box1 = mp->d.box1; cfg.box2 = mp->d.box2; cfg.pitch_b = mp->d.pitch_b; cfg.box_bytes = mp->d.box_bytes;
-    cfg.stages = stages;
-    cfg.strips = (sz1 + kT - 1) / kT;
-    cfg.ntiles2 = (sz2 + tl - 1) / tl;
+    if (!stage_box(ctx, src, F::pxb, fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, wn, mp->d, &L->tmap, &cfg)) return CC_OK;
+    cfg.strips = (fr.sz1 + kT - 1) / kT;
+    cfg.ntiles2 = (fr.sz2 + F::tl - 1) / F::tl;
     cfg.tiles = cfg.strips * cfg.ntiles2;
     // frames per group: as unit_cfg (keep ~8 units per resident CTA slot), within a view
     const long long want = (long long)ctx->sm_count * 6 * 8;
-    int fg = std::min(fg_max, fpv);
+    int fg = std::min(!(c.flags & CC_COORD_F32) ? F::fg_exact : F::fg_fast, fr.fpv);
     uint32_t g0 = 0;
-    while (fg > 1 && (long long)cfg.tiles * window_groups(fpv, fg, w0, wn, &g0) < want) fg = (fg + 1) / 2;
-    const long long units = (long long)cfg.tiles * window_groups(fpv, fg, w0, wn, &g0);
+    while (fg > 1 && (long long)cfg.tiles * window_groups(fr.fpv, fg, w0, wn, &g0) < want) fg = (fg + 1) / 2;
+    const long long units = (long long)cfg.tiles * window_groups(fr.fpv, fg, w0, wn, &g0);
     cfg.fg = fg;
-    cfg.fpv = fpv;
-    cfg.gpv = (fpv + fg - 1) / fg;
+    cfg.fpv = fr.fpv;
+    cfg.gpv = (fr.fpv + fg - 1) / fg;
     cfg.w0 = w0;
     cfg.g0 = g0;
     CC_REQUIRE(units < (1ll << 31), "too many tiles in one call: split the batch");
     cfg.units = (uint32_t)units;
     cfg.widen_mul = 0x20000000u;
-    for (int v = 0; v < nviews; ++v) {
-        const RectGeom gv = make_geom(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, wn);
-        L->vt.v[v].pe = make_exact(chs[v], ratios[v]);
-        L->vt.v[v].pf = make_fast(chs[v], ratios[v], gv);
+    for (int v = 0; v < nv; ++v) {
+        const RectGeom gv = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, wn);
+        L->vt.v[v].pe = make_exact(c.views.chs[v0 + v], c.views.ratios[v0 + v]);
+        L->vt.v[v].pf = make_fast(c.views.chs[v0 + v], c.views.ratios[v0 + v], gv);
         L->vt.v[v].g = gv;
     }
-    for (int v = nviews; v < kMaxViews; ++v) L->vt.v[v] = L->vt.v[0];
+    for (int v = nv; v < kMaxViews; ++v) L->vt.v[v] = L->vt.v[0];
     L->g = L->vt.v[0].g;
     L->mp = mp;
     *ok = true;
     return CC_OK;
 }
 
-// tensor map, unit configuration and view table of one group's launch over all its frames; *ok = false: the
-// single launch does not apply
-static int views_prepare(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews,
-                         const void* src, int pxb, int tl, int sz1, int sz2, size_t pitch, size_t frame_stride, int fpv,
-                         int fg_max, cudaStream_t st, ViewsLaunch* L, bool* ok) {
+// the staged views kernel on a prepared launch
+template <typename PX>
+static int views_run(cc_ctx* ctx, ViewsLaunch* L, const RectCall<PX>& c, const PX* src, PX* dst, cudaStream_t st) {
+    using F = RectFmt<PX>;
+    const bool exact = !(c.flags & CC_COORD_F32);
+    int nf = 1;
+    const size_t smem = F::ring(L->cfg, true, &nf);
+    const auto k = F::views(exact);
+    uint32_t gsz = 0;
+    int rc = persistent_grid(ctx, F::views_slot + !exact, k, smem, L->cfg, L->mp, exact, &gsz);
+    RectSched* sched = nullptr;
+    if (!rc) rc = sched_acquire(ctx, st, &sched);
+    if (rc) return rc;
+    multi_read_begin(L->mp, st);
+    F::launch(k, gsz, kConsumerThreads + 32, smem, st, c, L->tmap, L->vt, L->g, L->cfg, L->mp->d_hdr, L->mp->d_q2, sched,
+              src, dst);
+    multi_read_end(L->mp, st);
+    sched_release(ctx, st);
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+// Views [v0, v0 + nv) of a device call in one staged launch; src / dst: the group's first frame.  *ok = false: the
+// group cannot be staged (the caller runs one launch per view).
+template <typename PX>
+int launch_rectify_group(cc_ctx* ctx, const RectCall<PX>& c, int v0, int nv, const PX* src, PX* dst, cudaStream_t st,
+                         bool* ok) {
+    using F = RectFmt<PX>;
+    const RectFrames& fr = c.fr;
+    const int nframes = nv * fr.fpv;
     *ok = false;
-    if (nviews < 1 || nviews > kMaxViews || fpv < 1) return CC_OK;
-    const int nframes = nviews * fpv;
-    const size_t pitch_b = pitch * pxb, frame_b = frame_stride * pxb;
-    if ((reinterpret_cast<uintptr_t>(src) & 15u) || (pitch_b & 15u) || (nframes > 1 && (frame_b & 15u))) return CC_OK;
-    if (!encoder(ctx)) return CC_OK;
-    std::vector<RectGeom> gs((size_t)nviews);
-    for (int v = 0; v < nviews; ++v) gs[v] = make_geom(axs_mins + 2 * v, sz1, sz2, pitch, frame_stride, nframes);
-    MultiPlan* mp = multi_get(ctx, chs, ratios, gs.data(), nviews, kT, tl, pxb, st);
+    if ((c.flags & CC_GATHER_DIRECT) || !F::dst_ok(dst, fr, nframes) || nv < 1 || nv > kMaxViews || fr.fpv < 1 ||
+        !tma_aligned(src, F::pxb, fr.pitch, fr.frame_stride, nframes) || !encoder(ctx))
+        return CC_OK;
+    std::vector<RectGeom> gs((size_t)nv);
+    for (int v = 0; v < nv; ++v)
+        gs[v] = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, nframes);
+    MultiPlan* mp = multi_get(ctx, c.views.chs + v0, c.views.ratios + v0, gs.data(), nv, kT, F::tl, F::pxb, st);
     if (!mp) {
-        if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %d not stageable (pxb %d)\n", nviews, pxb);
+        if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %d not stageable (pxb %d)\n", nv, F::pxb);
         return CC_OK;
     }
-    return views_window(ctx, mp, chs, ratios, axs_mins, nviews, src, pxb, tl, sz1, sz2, pitch, frame_stride, fpv, 0,
-                        nframes, fg_max, L, ok);
-}
-
-// the staged views kernels on a prepared launch
-static int views_run_f32c1(cc_ctx* ctx, ViewsLaunch* Lp, bool exact, const float* src, float* dst, float fill,
-                           cudaStream_t st) {
-    const size_t smem = (size_t)Lp->cfg.stages * Lp->cfg.box_bytes;
-    uint32_t gsz = 0;
-    int rc = exact ? persistent_grid(ctx, 6, rectify_f32c1_views_kernel<true>, smem, Lp->cfg, Lp->mp, true, &gsz)
-                   : persistent_grid(ctx, 7, rectify_f32c1_views_kernel<false>, smem, Lp->cfg, Lp->mp, false, &gsz);
-    RectSched* sched = nullptr;
-    if (!rc) rc = sched_acquire(ctx, st, &sched);
-    if (rc) return rc;
-    multi_read_begin(Lp->mp, st);
-    if (exact) rectify_f32c1_views_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, fill);
-    else       rectify_f32c1_views_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, fill);
-    multi_read_end(Lp->mp, st);
-    sched_release(ctx, st);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
-static int views_run_u8c3(cc_ctx* ctx, ViewsLaunch* Lp, bool exact, const uint8_t* src, uint8_t* dst, const uint8_t fill[3],
-                          int sz1, int sz2, size_t pitch, cudaStream_t st) {
-    const uchar3 f = make_uchar3(fill[0], fill[1], fill[2]);
-    const unsigned frame_bytes = (unsigned)((pitch * (size_t)(sz2 - 1) + (size_t)sz1) * 3);
-    Lp->cfg.stages = std::max(2, Lp->cfg.stages / kU8FramesPerStage);
-    const size_t smem = (size_t)Lp->cfg.stages * kU8FramesPerStage * Lp->cfg.box_bytes + 16;
-    uint32_t gsz = 0;
-    int rc = exact ? persistent_grid(ctx, 8, rectify_u8c3_views_kernel<true>, smem, Lp->cfg, Lp->mp, true, &gsz)
-                   : persistent_grid(ctx, 9, rectify_u8c3_views_kernel<false>, smem, Lp->cfg, Lp->mp, false, &gsz);
-    RectSched* sched = nullptr;
-    if (!rc) rc = sched_acquire(ctx, st, &sched);
-    if (rc) return rc;
-    multi_read_begin(Lp->mp, st);
-    if (exact) rectify_u8c3_views_kernel<true><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, f, frame_bytes);
-    else       rectify_u8c3_views_kernel<false><<<gsz, kConsumerThreads + 32, smem, st>>>(Lp->tmap, Lp->vt, Lp->g, Lp->cfg, Lp->mp->d_hdr, Lp->mp->d_q2, sched, src, dst, f, frame_bytes);
-    multi_read_end(Lp->mp, st);
-    sched_release(ctx, st);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
-int launch_rectify_f32c1_views(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews,
-                               const float* src, float* dst, int sz1, int sz2, size_t pitch, size_t frame_stride,
-                               int fpv, float fill, unsigned flags, cudaStream_t st, bool* ok) {
-    const bool exact = !(flags & CC_COORD_F32);
-    *ok = false;
     ViewsLaunch L;                     // 15 KB: the view table goes to the kernel by value
-    int rc = views_prepare(ctx, chs, ratios, axs_mins, nviews, src, 4, kTLf, sz1, sz2, pitch, frame_stride, fpv,
-                           exact ? kFGf32Exact : kFGf32Fast, st, &L, ok);
+    int rc = views_window(ctx, mp, c, v0, nv, src, 0, nframes, &L, ok);
     if (rc || !*ok) return rc;
-    return views_run_f32c1(ctx, &L, exact, src, dst, fill, st);
-}
-
-int launch_rectify_u8c3_views(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews,
-                              const uint8_t* src, uint8_t* dst, int sz1, int sz2, size_t pitch, size_t frame_stride,
-                              int fpv, const uint8_t fill[3], unsigned flags, cudaStream_t st, bool* ok) {
-    const bool exact = !(flags & CC_COORD_F32);
-    *ok = false;
-    const int nframes = nviews * fpv;
-    // the staged kernel writes whole 32-bit words: 4-byte aligned output lines
-    const bool dst_ok = (reinterpret_cast<uintptr_t>(dst) & 3u) == 0 && ((pitch * 3) & 3u) == 0 &&
-                        (nframes <= 1 || ((frame_stride * 3) & 3u) == 0);
-    if (!dst_ok) return CC_OK;
-    ViewsLaunch L;
-    int rc = views_prepare(ctx, chs, ratios, axs_mins, nviews, src, 3, kTLu, sz1, sz2, pitch, frame_stride, fpv,
-                           exact ? kFGu8Exact : kFGu8Fast, st, &L, ok);
-    if (rc || !*ok) return rc;
-    return views_run_u8c3(ctx, &L, exact, src, dst, fill, sz1, sz2, pitch, st);
+    return views_run(ctx, &L, c, src, dst, st);
 }
 
 // --------------------------------------------------------------------------------------
@@ -1194,11 +1128,9 @@ int launch_rectify_u8c3_views(cc_ctx* ctx, const ChainD* chs, const double* rati
 // --------------------------------------------------------------------------------------
 struct RectViewsHost {
     cc_ctx* ctx;
-    const ChainD* chs;
-    const double* ratios;
-    const int64_t* axs_mins;
-    int nviews, ngroups, sz1, sz2, fpv, pxb, tl;
-    size_t pitch;
+    RectViews views;
+    RectFrames fr;                         // the layout of the slot buffers: frames pitch * sz2 apart
+    int ngroups, pxb, tl;
     bool stage;                            // the layout can be staged at all
     std::vector<MultiPlan*> mp;            // per group: its plan (nullptr: per-view launches)
     std::vector<char> state;               // per group: 0 nothing yet, 1 being built, 2 ready
@@ -1215,11 +1147,11 @@ struct RectViewsHost {
 };
 
 static std::vector<PlanKey> group_keys(const RectViewsHost* h, int gi) {
-    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->nviews - v0);
+    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->views.n - v0);
     std::vector<PlanKey> keys((size_t)nv);
     for (int v = 0; v < nv; ++v) {
-        const RectGeom g = make_geom(h->axs_mins + 2 * (v0 + v), h->sz1, h->sz2, h->pitch, 0, 0);
-        keys[v] = plan_key(h->chs[v0 + v], h->ratios[v0 + v], g, kT, h->tl, h->pxb);
+        const RectGeom g = make_geom(h->views.axs_mins + 2 * (v0 + v), h->fr.sz1, h->fr.sz2, h->fr.pitch, 0, 0);
+        keys[v] = plan_key(h->views.chs[v0 + v], h->views.ratios[v0 + v], g, kT, h->tl, h->pxb);
     }
     return keys;
 }
@@ -1290,7 +1222,7 @@ static int vh_install(RectViewsHost* h, int gi) {
     }
     if (!mp->d_hdr) {                                   // room for a full group: later groups of this size reuse it
         const size_t hcap = std::max(hb, (size_t)mp->n1 * mp->n2 * kMaxViews * sizeof(TileHdr));
-        const size_t qcap = std::max(qb, (size_t)h->sz2 * kMaxViews * sizeof(double));
+        const size_t qcap = std::max(qb, (size_t)h->fr.sz2 * kMaxViews * sizeof(double));
         if (cudaMalloc(&mp->d_hdr, hcap) != cudaSuccess || cudaMalloc(&mp->d_q2, qcap) != cudaSuccess) {
             cudaGetLastError();
             multi_free(mp);
@@ -1313,8 +1245,10 @@ static int vh_install(RectViewsHost* h, int gi) {
     return CC_OK;
 }
 
-int rect_vh_begin(cc_ctx* ctx, const ChainD* chs, const double* ratios, const int64_t* axs_mins, int nviews, int sz1,
-                  int sz2, size_t pitch, int fpv, int pxb, bool stage, RectViewsHost** out) {
+// dc: the call in the layout of the slot buffers (frames pitch * sz2 apart)
+template <typename PX>
+int rect_vh_begin(cc_ctx* ctx, const RectCall<PX>& dc, RectViewsHost** out) {
+    using F = RectFmt<PX>;
     *out = nullptr;
     multi_free_retired(ctx);
     if (!ctx->rect_upload) CC_CUDA(cudaStreamCreateWithFlags(&ctx->rect_upload, cudaStreamNonBlocking));
@@ -1323,11 +1257,11 @@ int rect_vh_begin(cc_ctx* ctx, const ChainD* chs, const double* ratios, const in
         if (!ctx->rect_join_event[k]) CC_CUDA(cudaEventCreateWithFlags(&ctx->rect_join_event[k], cudaEventDisableTiming));
     RectViewsHost* h = new (std::nothrow) RectViewsHost();
     if (!h) return set_error(CC_ERR_NOMEM, "out of host memory");
-    h->ctx = ctx; h->chs = chs; h->ratios = ratios; h->axs_mins = axs_mins;
-    h->nviews = nviews; h->ngroups = (nviews + kMaxViews - 1) / kMaxViews;
-    h->sz1 = sz1; h->sz2 = sz2; h->pitch = pitch; h->fpv = fpv; h->pxb = pxb; h->tl = pxb == 4 ? kTLf : kTLu;
+    h->ctx = ctx; h->views = dc.views; h->fr = dc.fr;
+    h->ngroups = (dc.views.n + kMaxViews - 1) / kMaxViews;
+    h->pxb = F::pxb; h->tl = F::tl;
     // staged iff the device frames (pitch * sz2 elements, buffers 256-byte aligned) can be TMA-addressed
-    h->stage = stage && ((pitch * pxb) & 15u) == 0 && encoder(ctx) != nullptr;
+    h->stage = !(dc.flags & CC_GATHER_DIRECT) && ((dc.fr.pitch * F::pxb) & 15u) == 0 && encoder(ctx) != nullptr;
     h->mp.assign((size_t)h->ngroups, nullptr);
     h->state.assign((size_t)h->ngroups, 0);
     h->used.assign((size_t)h->ngroups, 0);
@@ -1348,34 +1282,19 @@ int rect_vh_prepare(RectViewsHost* h, int gi) {
     return CC_OK;
 }
 
-// frames [w0, w0 + wn) of group gi, src / dst: the window's first frame, frames pitch * sz2 apart, on st;
-// *ok = false: the group has no plan (the caller runs its single-view launches)
-int rect_vh_launch_f32c1(RectViewsHost* h, int gi, int w0, int wn, const float* src, float* dst, float fill,
-                         unsigned flags, cudaStream_t st, bool* ok) {
+// frames [w0, w0 + wn) of group gi, src / dst: the window's first frame in a slot, on st; *ok = false: the group has
+// no plan (the caller runs its single-view launches)
+template <typename PX>
+int rect_vh_launch(RectViewsHost* h, const RectCall<PX>& dc, int gi, int w0, int wn, const PX* src, PX* dst,
+                   cudaStream_t st, bool* ok) {
     *ok = false;
     if (!h->mp[gi]) return CC_OK;
-    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->nviews - v0);
-    const bool exact = !(flags & CC_COORD_F32);
+    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->views.n - v0);
     ViewsLaunch L;
-    int rc = views_window(h->ctx, h->mp[gi], h->chs + v0, h->ratios + v0, h->axs_mins + 2 * v0, nv, src, 4, kTLf, h->sz1,
-                          h->sz2, h->pitch, h->pitch * (size_t)h->sz2, h->fpv, w0, wn, exact ? kFGf32Exact : kFGf32Fast, &L, ok);
+    int rc = views_window(h->ctx, h->mp[gi], dc, v0, nv, src, w0, wn, &L, ok);
     if (rc || !*ok) return rc;
     h->used[gi] = 1;
-    return views_run_f32c1(h->ctx, &L, exact, src, dst, fill, st);
-}
-
-int rect_vh_launch_u8c3(RectViewsHost* h, int gi, int w0, int wn, const uint8_t* src, uint8_t* dst, const uint8_t fill[3],
-                        unsigned flags, cudaStream_t st, bool* ok) {
-    *ok = false;
-    if (!h->mp[gi]) return CC_OK;
-    const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->nviews - v0);
-    const bool exact = !(flags & CC_COORD_F32);
-    ViewsLaunch L;
-    int rc = views_window(h->ctx, h->mp[gi], h->chs + v0, h->ratios + v0, h->axs_mins + 2 * v0, nv, src, 3, kTLu, h->sz1,
-                          h->sz2, h->pitch, h->pitch * (size_t)h->sz2, h->fpv, w0, wn, exact ? kFGu8Exact : kFGu8Fast, &L, ok);
-    if (rc || !*ok) return rc;
-    h->used[gi] = 1;
-    return views_run_u8c3(h->ctx, &L, exact, src, dst, fill, h->sz1, h->sz2, h->pitch, st);
+    return views_run(h->ctx, &L, dc, src, dst, st);
 }
 
 // no chunk of this call reads group gi's plan after the ones enqueued so far: its fence joins the slot streams
@@ -1411,25 +1330,36 @@ int rect_vh_end(RectViewsHost* h) {
 
 int rectify_views_per_launch() { return kMaxViews; }
 
-int launch_rectify_map(cc_ctx* ctx, const ChainD& chd, double ratio, const int64_t axs_min[2],
-                       double* map_row, double* map_col, int sz1, int sz2, size_t pitch,
-                       cudaStream_t st) {
+// the map alone of one view: FP64 with the exact kernels' arithmetic, FP32 with the fast ones'
+template <typename T>
+int launch_rectify_map(cc_ctx* ctx, const ChainD& chd, double ratio, const int64_t axs_min[2], T* map_row, T* map_col,
+                       int sz1, int sz2, size_t pitch, cudaStream_t st) {
     const RectGeom g = make_geom(axs_min, sz1, sz2, pitch, pitch * (size_t)sz2, 1);
     const dim3 grid((sz1 + kT - 1) / kT, (sz2 + kT - 1) / kT);
-    rectify_map_kernel<<<grid, kConsumerThreads, 0, st>>>(make_exact(chd, ratio), g, map_row, map_col);
+    if constexpr (std::is_same_v<T, double>)
+        rectify_map_kernel<<<grid, kConsumerThreads, 0, st>>>(make_exact(chd, ratio), g, map_row, map_col);
+    else
+        rectify_map_f32_kernel<<<grid, kConsumerThreads, 0, st>>>(make_fast(chd, ratio, g), g, map_row, map_col);
     ctx->launches++;
     CC_CUDA(cudaGetLastError());
     return CC_OK;
 }
 
-int launch_rectify_map_f32(cc_ctx* ctx, const ChainD& chd, double ratio, const int64_t axs_min[2],
-                           float* map_row, float* map_col, int sz1, int sz2, size_t pitch, cudaStream_t st) {
-    const RectGeom g = make_geom(axs_min, sz1, sz2, pitch, pitch * (size_t)sz2, 1);
-    const dim3 grid((sz1 + kT - 1) / kT, (sz2 + kT - 1) / kT);
-    rectify_map_f32_kernel<<<grid, kConsumerThreads, 0, st>>>(make_fast(chd, ratio, g), g, map_row, map_col);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
+template int launch_rectify<float>(cc_ctx*, const RectCall<float>&, int, int, const float*, float*, cudaStream_t);
+template int launch_rectify<uint8_t>(cc_ctx*, const RectCall<uint8_t>&, int, int, const uint8_t*, uint8_t*, cudaStream_t);
+template int launch_rectify_group<float>(cc_ctx*, const RectCall<float>&, int, int, const float*, float*, cudaStream_t,
+                                         bool*);
+template int launch_rectify_group<uint8_t>(cc_ctx*, const RectCall<uint8_t>&, int, int, const uint8_t*, uint8_t*,
+                                           cudaStream_t, bool*);
+template int rect_vh_begin<float>(cc_ctx*, const RectCall<float>&, RectViewsHost**);
+template int rect_vh_begin<uint8_t>(cc_ctx*, const RectCall<uint8_t>&, RectViewsHost**);
+template int rect_vh_launch<float>(RectViewsHost*, const RectCall<float>&, int, int, int, const float*, float*,
+                                   cudaStream_t, bool*);
+template int rect_vh_launch<uint8_t>(RectViewsHost*, const RectCall<uint8_t>&, int, int, int, const uint8_t*, uint8_t*,
+                                     cudaStream_t, bool*);
+template int launch_rectify_map<double>(cc_ctx*, const ChainD&, double, const int64_t[2], double*, double*, int, int,
+                                        size_t, cudaStream_t);
+template int launch_rectify_map<float>(cc_ctx*, const ChainD&, double, const int64_t[2], float*, float*, int, int,
+                                       size_t, cudaStream_t);
 
 }  // namespace cc

@@ -77,7 +77,7 @@ def _tiles(sz):
 
 
 def _mirror_fg(units_per_group, fg_max, n):
-    """unit_cfg / views_prepare (rectify.cu): halve the group until there are ~8 units per resident CTA slot
+    """unit_cfg / views_window (rectify.cu): halve the group until there are ~8 units per resident CTA slot
     (sm_count * 48 units); units_per_group = tiles (x views) of one frame group."""
     want = torch.cuda.get_device_properties(0).multi_processor_count * 48
     fg = min(fg_max, n)

@@ -351,35 +351,6 @@ def test_host_call_between_device_calls(cc, fmt, coord):
         _assert_equal(host, vs.oracle(fmt, frames, 2), "oracle")
 
 
-# ------------------------------------------------------------------ arguments
-@pytest.mark.gpu
-@pytest.mark.parametrize("fmt", ["f32", "u8"])
-def test_argument_errors(cc, fmt):
-    """Every rule of cc_rectify_*_views: CC_ERR_INVALID_ARG and nothing written."""
-    sz = (64, 48)
-    vs = _Views(cc, 3, sz, scale=0.016)
-    frames = vs.frames(fmt, 6, 1700)
-    bad_axs = (C.c_int64 * 6)(0, 0, 1 << 31, 0, 0, 0)
-    bad_ratio = (C.c_double * 3)(vs.ratios[0], -1.0, vs.ratios[2])
-    cases = {"ctx": dict(ctx=None), "intr": dict(intr=None), "views": dict(views=None), "ratios": dict(ratios=None),
-             "axs": dict(axs=None), "nviews<0": dict(nviews=-1), "fpv<0": dict(fpv=-1),
-             "65536 frames": dict(fpv=65536 // 3 + 1), "ratio": dict(ratios=bad_ratio), "axs range": dict(axs=bad_axs),
-             "sz1": dict(sz1=0), "sz2": dict(sz2=-4), "pitch": dict(pitch=sz[0] - 1),
-             "overlap": dict(stride=sz[0] * sz[1] - 1), "src": dict(src=None), "dst": dict(dst=None)}
-    if fmt == "u8":
-        cases["fill"] = dict(fill=None)
-    for what, over in cases.items():
-        out = _out_like(frames, fmt)
-        assert vs.host(fmt, frames, out, **over) == -1, what
-        assert np.array_equal(out, _out_like(frames, fmt)), what
-    out = _out_like(frames, fmt)
-    assert vs.host(fmt, frames, out, src=C.c_void_p(out.ctypes.data)) == -1          # in place
-    for over in (dict(nviews=0), dict(fpv=0)):
-        out = _out_like(frames, fmt)
-        assert vs.host(fmt, frames, out, **over) == 0
-        assert np.array_equal(out, _out_like(frames, fmt))
-
-
 # ------------------------------------------------------------------ Python
 @pytest.mark.gpu
 @pytest.mark.parametrize("coord", ["f64", "f32"])
