@@ -1,6 +1,6 @@
 // abi.cu -- the extern "C" surface of libcamcal_b200.so (include/camcal_b200.h):
-// argument checking, per-device context, and the chunked host pipeline behind the
-// *_host entry points.  No compute lives here and nothing here can fall back to the CPU.
+// argument checking, per-device context, and the host pipelines behind the *_host entry points.
+// No compute lives here and nothing here can fall back to the CPU.
 #include <algorithm>
 #include <vector>
 #include <cstdarg>
@@ -10,7 +10,7 @@
 #include <new>
 #include <optional>
 
-#include "common.cuh"
+#include "lm_state.cuh"
 
 namespace cc {
 
@@ -30,7 +30,7 @@ int cuda_fail(cudaError_t e, const char* what) {
     return set_error(st, "%s: %s (%s)", what, cudaGetErrorString(e), cudaGetErrorName(e));
 }
 
-// launchers implemented in the kernel translation units
+// launchers implemented in the kernel translation units (the fit's: lm_state.cuh)
 template <typename T>
 int point_table_upload(cc_ctx*, bool, const ChainD*, int, const size_t*, cudaStream_t, PointTable*);
 int point_table_release(cc_ctx*, cudaStream_t);
@@ -51,19 +51,6 @@ void rect_vh_retire(RectViewsHost*, int);
 int rect_vh_end(RectViewsHost*);
 template <typename T>
 int launch_rectify_map(cc_ctx*, const ChainD&, double, const int64_t[2], T*, T*, int, int, size_t, cudaStream_t);
-int launch_reproj_jtj(cc_ctx*, const cc_intr*, double, const cc_view*, int, const double*,
-                      const double*, int, double*, double*, cudaStream_t);
-int launch_calc_errors(cc_ctx*, const cc_intr*, const cc_view*, int, const double*, const double*,
-                       int, int, const double*, const double*, int, double*, cudaStream_t);
-int launch_lm_schur(cc_ctx*, const double*, int, double, double*, double*, cudaStream_t);
-int lm_fit_host(cc_ctx*, cc_intr*, double, unsigned, cc_view*, int, const double*, const double*, int, int, double,
-                double*, int*);
-int launch_lm_update(cc_ctx*, const double*, const double*, double, unsigned, const double*, const cc_view*,
-                     int, cc_view*, double*, cudaStream_t);
-int lm_fit_device(cc_ctx*, cc_intr*, double, unsigned, cc_view*, int, const double*, const double*, int, int, double,
-                  double*, int*, cudaStream_t);
-int launch_initial_guess(cc_ctx*, const double*, const double*, int, int, int, int, double, cc_intr*, cc_view*,
-                         cudaStream_t);
 
 static int check_params(const cc_ctx* ctx, const cc_intr* intr, const cc_view* view) {
     CC_REQUIRE(ctx != nullptr, "ctx is NULL");
@@ -527,6 +514,111 @@ static int rectify_map(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, do
     return launch_rectify_map<T>(ctx, ch, ratio, axs_min, map_row, map_col, sz1, sz2, pitch, (cudaStream_t)stream);
 }
 
+// ---- fit: residual / J'J, calculate_errors, Levenberg-Marquardt ------------------
+// Each check runs every rule of its entry points before the device is touched, anything is uploaded or launched.
+// A pointer is required only when the call reads it.  img is read as 16-byte (row, col) pairs: the device forms
+// check its alignment; a staged host call is aligned by construction.
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+static int check_reproj_jtj(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                            const double* obj, const double* img, int ncorners, const double* per_view,
+                            const double* shared, bool host) {
+    CC_REQUIRE(ctx && intr, "NULL argument");
+    CC_REQUIRE(nviews >= 0 && ncorners > 0, "bad sizes");
+    CC_REQUIRE(shared != nullptr, "shared is NULL");
+    CC_REQUIRE(nviews == 0 || (views && obj && img && per_view), host ? "NULL host pointer" : "NULL device pointer");
+    CC_REQUIRE(intr->checker_size != 0.0, "checker_size must be non-zero");
+    CC_REQUIRE(host || aligned16(img), "img must be 16-byte aligned");
+    return CC_OK;
+}
+
+static int check_calculate_errors(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                                  const double* obj, const double* img, int n1, int n2, const double* inv_rows,
+                                  const double* inv_cols, int inverse_samples, const double* sums, bool host) {
+    CC_REQUIRE(ctx && intr && sums, "NULL argument");
+    CC_REQUIRE(nviews >= 0 && n1 >= 1 && n2 >= 1 && inverse_samples >= 0, "bad sizes");
+    CC_REQUIRE(nviews == 0 || (views && obj && img), host ? "NULL host pointer" : "NULL device pointer");
+    CC_REQUIRE(inverse_samples == 0 || nviews == 0 || (inv_rows && inv_cols), "NULL sample pointer");
+    CC_REQUIRE(intr->checker_size != 0.0 && intr->frow != 0.0 && intr->fcol != 0.0, "bad intrinsics");
+    CC_REQUIRE(host || aligned16(img), "img must be 16-byte aligned");
+    CC_REQUIRE(calc_errors_smem(n1, n2) <= kCalcErrorsSmemMax, "too many corners per view for the fused kernel");
+    return CC_OK;
+}
+
+// The host form fits at least one view; the device form may hold no views on a rank of a sharded fit.
+static int check_lm_fit(const cc_ctx* ctx, const cc_intr* intr, double aspect, unsigned free_mask,
+                        const cc_view* views, int nviews, const double* obj, const double* img, int ncorners,
+                        int max_iter, double eps, bool host) {
+    CC_REQUIRE(ctx && intr && obj, "NULL argument");
+    CC_REQUIRE(nviews >= (host ? 1 : 0) && ncorners > 0, "bad sizes");
+    CC_REQUIRE(nviews == 0 || (views && img), "NULL view / image-point array");
+    CC_REQUIRE(free_mask != 0u && free_mask < 16u, "free_mask selects among the 4 shared parameters");
+    CC_REQUIRE(max_iter >= 0 && eps >= 0.0, "bad stopping rule");
+    CC_REQUIRE(aspect > 0.0 && intr->fcol != 0.0 && intr->checker_size != 0.0, "bad starting intrinsics");
+    CC_REQUIRE(host || aligned16(img), "img must be 16-byte aligned");
+    return CC_OK;
+}
+
+static int check_lm_schur(const cc_ctx* ctx, const double* per_view, int nviews, double lambda, const double* yz,
+                          const double* schur) {
+    CC_REQUIRE(ctx && schur, "NULL argument");
+    CC_REQUIRE(nviews >= 0, "bad sizes");
+    CC_REQUIRE(nviews == 0 || (per_view && yz), "NULL device pointer");
+    CC_REQUIRE(lambda >= 0.0 && lambda == lambda, "lambda must be non-negative");
+    return CC_OK;
+}
+
+static int check_lm_update(const cc_ctx* ctx, const double* shared, const double* schur, double lambda,
+                           unsigned free_mask, const double* yz, const cc_view* views_in, int nviews,
+                           const cc_view* views_out, const double* delta) {
+    CC_REQUIRE(ctx && shared && schur && delta, "NULL argument");
+    CC_REQUIRE(nviews >= 0, "bad sizes");
+    CC_REQUIRE(nviews == 0 || (yz && views_in && views_out), "NULL device pointer");
+    CC_REQUIRE(lambda >= 0.0 && lambda == lambda, "lambda must be non-negative");
+    CC_REQUIRE(free_mask != 0u && free_mask < 16u, "free_mask selects among the 4 shared parameters");
+    return CC_OK;
+}
+
+static int check_initial_guess(const cc_ctx* ctx, const double* obj, const double* img, int nviews, int ncorners,
+                               int sz1, int sz2, const cc_intr* intr, const cc_view* views) {
+    CC_REQUIRE(ctx && intr && obj, "NULL argument");
+    CC_REQUIRE(nviews >= 0 && ncorners >= 4 && sz1 > 0 && sz2 > 0, "bad sizes (a homography needs >= 4 corners)");
+    CC_REQUIRE(nviews == 0 || (views && img), "NULL view / image-point array");
+    return CC_OK;
+}
+
+// One host array of a staged call: `up` (if not NULL) is uploaded before the body runs, `down` (if not NULL)
+// receives the array after it.  A span may be both.
+struct HostSpan {
+    const void* up;
+    void* down;
+    size_t bytes;
+};
+
+// The host form of a fit entry point: the spans go to slot 0 at 256-byte offsets, up on the slot's stream; body runs
+// the device form's launcher on the slot's device copies (d[i] for span i) and that stream; then the downloads, and
+// one synchronisation.  The caller has checked the arguments and entered the context's device.
+template <size_t N, typename Body>
+static int stage_host(cc_ctx* ctx, const HostSpan (&spans)[N], Body body) {
+    size_t off[N + 1] = {0};
+    for (size_t i = 0; i < N; ++i) off[i + 1] = off[i] + round_up(spans[i].bytes, 256);
+    int rc = ensure_slot(ctx, 0, off[N], 0);
+    if (rc) return rc;
+    cudaStream_t st = ctx->pipe_stream[0];
+    void* d[N];
+    for (size_t i = 0; i < N; ++i) {
+        d[i] = static_cast<uint8_t*>(ctx->pipe_in[0]) + off[i];
+        if (spans[i].up && spans[i].bytes)
+            CC_CUDA(cudaMemcpyAsync(d[i], spans[i].up, spans[i].bytes, cudaMemcpyHostToDevice, st));
+    }
+    if ((rc = body(d, st))) return rc;
+    for (size_t i = 0; i < N; ++i)
+        if (spans[i].down && spans[i].bytes)
+            CC_CUDA(cudaMemcpyAsync(spans[i].down, d[i], spans[i].bytes, cudaMemcpyDeviceToHost, st));
+    CC_CUDA(cudaStreamSynchronize(st));
+    return CC_OK;
+}
+
 }  // namespace cc
 
 using namespace cc;
@@ -867,18 +959,13 @@ int cc_get_axes(double ratio, double checker_size, int n1, int n2, int sz1, int 
     return CC_OK;
 }
 
-// ---- residual / Jacobian ---------------------------------------------------------
+// ---- residual / Jacobian, calculate_errors ---------------------------------------
 int cc_reproj_jtj_f64(cc_ctx* ctx, const cc_intr* intr, double aspect, const cc_view* views,
                       int nviews, const double* obj, const double* img, int ncorners,
                       double* per_view, double* shared, void* stream) {
-    CC_REQUIRE(ctx && intr, "NULL argument");
-    CC_REQUIRE(nviews >= 0 && ncorners > 0, "bad sizes");
-    CC_REQUIRE(shared != nullptr, "shared is NULL");
-    CC_REQUIRE(nviews == 0 || (views && obj && img && per_view), "NULL device pointer");
-    CC_REQUIRE(intr->checker_size != 0.0, "checker_size must be non-zero");
+    int rc = check_reproj_jtj(ctx, intr, views, nviews, obj, img, ncorners, per_view, shared, false);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
+    if (rc || (rc = enter(ctx))) return rc;
     return launch_reproj_jtj(ctx, intr, aspect, views, nviews, obj, img, ncorners, per_view, shared,
                              (cudaStream_t)stream);
 }
@@ -886,54 +973,29 @@ int cc_reproj_jtj_f64(cc_ctx* ctx, const cc_intr* intr, double aspect, const cc_
 int cc_reproj_jtj_f64_host(cc_ctx* ctx, const cc_intr* intr, double aspect, const cc_view* views,
                            int nviews, const double* obj, const double* img, int ncorners,
                            double* per_view, double* shared) {
-    CC_REQUIRE(ctx && intr, "NULL argument");
-    CC_REQUIRE(nviews >= 0 && ncorners > 0, "bad sizes");
-    CC_REQUIRE(shared != nullptr, "shared is NULL");
-    CC_REQUIRE(nviews == 0 || (views && obj && img && per_view), "NULL host pointer");
-    CC_REQUIRE(intr->checker_size != 0.0, "checker_size must be non-zero");
+    int rc = check_reproj_jtj(ctx, intr, views, nviews, obj, img, ncorners, per_view, shared, true);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
-    const size_t nv = (size_t)(nviews > 0 ? nviews : 1);
-    const size_t b_views = round_up(nv * sizeof(cc_view), 256);
-    const size_t b_obj = round_up((size_t)ncorners * 3 * sizeof(double), 256);
-    const size_t b_img = round_up(nv * ncorners * 2 * sizeof(double), 256);
-    const size_t b_pv = round_up(nv * CC_PER_VIEW * sizeof(double), 256);
-    if ((rc = ensure_slot(ctx, 0, b_views + b_obj + b_img, b_pv + 256))) return rc;
-    cudaStream_t st = ctx->pipe_stream[0];
-    uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[0]);
-    uint8_t* dout = static_cast<uint8_t*>(ctx->pipe_out[0]);
-    cc_view* d_views = reinterpret_cast<cc_view*>(din);
-    double* d_obj = reinterpret_cast<double*>(din + b_views);
-    double* d_img = reinterpret_cast<double*>(din + b_views + b_obj);
-    double* d_pv = reinterpret_cast<double*>(dout);
-    double* d_sh = reinterpret_cast<double*>(dout + b_pv);
-    if (nviews > 0) {
-        CC_CUDA(cudaMemcpyAsync(d_views, views, (size_t)nviews * sizeof(cc_view), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(d_obj, obj, (size_t)ncorners * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(d_img, img, (size_t)nviews * ncorners * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-    }
-    if ((rc = launch_reproj_jtj(ctx, intr, aspect, d_views, nviews, d_obj, d_img, ncorners, d_pv, d_sh, st)))
-        return rc;
-    if (nviews > 0)
-        CC_CUDA(cudaMemcpyAsync(per_view, d_pv, (size_t)nviews * CC_PER_VIEW * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CC_CUDA(cudaMemcpyAsync(shared, d_sh, CC_SHARED * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CC_CUDA(cudaStreamSynchronize(st));
-    return CC_OK;
+    if (rc || (rc = enter(ctx))) return rc;
+    const size_t nv = (size_t)nviews, nc = nviews > 0 ? (size_t)ncorners : 0;
+    const HostSpan spans[] = {{views, nullptr, nv * sizeof(cc_view)},
+                              {obj, nullptr, nc * 3 * sizeof(double)},
+                              {img, nullptr, nv * nc * 2 * sizeof(double)},
+                              {nullptr, per_view, nv * CC_PER_VIEW * sizeof(double)},
+                              {nullptr, shared, CC_SHARED * sizeof(double)}};
+    return stage_host(ctx, spans, [&](void* const* d, cudaStream_t st) {
+        return launch_reproj_jtj(ctx, intr, aspect, (const cc_view*)d[0], nviews, (const double*)d[1],
+                                 (const double*)d[2], ncorners, (double*)d[3], (double*)d[4], st);
+    });
 }
 
 int cc_calculate_errors_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                             const double* obj, const double* img, int n1, int n2,
                             const double* inv_rows, const double* inv_cols, int inverse_samples,
                             double* sums, void* stream) {
-    CC_REQUIRE(ctx && intr && sums, "NULL argument");
-    CC_REQUIRE(nviews >= 0 && n1 >= 1 && n2 >= 1 && inverse_samples >= 0, "bad sizes");
-    CC_REQUIRE(nviews == 0 || (views && obj && img), "NULL device pointer");
-    CC_REQUIRE(inverse_samples == 0 || (inv_rows && inv_cols), "NULL sample pointer");
-    CC_REQUIRE(intr->checker_size != 0.0 && intr->frow != 0.0 && intr->fcol != 0.0, "bad intrinsics");
+    int rc = check_calculate_errors(ctx, intr, views, nviews, obj, img, n1, n2, inv_rows, inv_cols,
+                                    inverse_samples, sums, false);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
+    if (rc || (rc = enter(ctx))) return rc;
     return launch_calc_errors(ctx, intr, views, nviews, obj, img, n1, n2, inv_rows, inv_cols,
                               inverse_samples, sums, (cudaStream_t)stream);
 }
@@ -943,68 +1005,38 @@ int cc_calculate_errors_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* vie
 int cc_calculate_errors_f64_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                                  const double* obj, const double* img, int n1, int n2, const double* inv_rows,
                                  const double* inv_cols, int inverse_samples, double* sums) {
-    CC_REQUIRE(ctx && intr && sums, "NULL argument");
-    CC_REQUIRE(nviews >= 0 && n1 >= 1 && n2 >= 1 && inverse_samples >= 0, "bad sizes");
-    CC_REQUIRE(nviews == 0 || (views && obj && img), "NULL host pointer");
-    CC_REQUIRE(inverse_samples == 0 || nviews == 0 || (inv_rows && inv_cols), "NULL sample pointer");
-    CC_REQUIRE(intr->checker_size != 0.0 && intr->frow != 0.0 && intr->fcol != 0.0, "bad intrinsics");
+    int rc = check_calculate_errors(ctx, intr, views, nviews, obj, img, n1, n2, inv_rows, inv_cols,
+                                    inverse_samples, sums, true);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
-    const size_t nv = (size_t)(nviews > 0 ? nviews : 1), nc = (size_t)n1 * n2;
-    const size_t b_views = round_up(nv * sizeof(cc_view), 256);
-    const size_t b_obj = round_up(nc * 3 * sizeof(double), 256);
-    const size_t b_img = round_up(nv * nc * 2 * sizeof(double), 256);
-    const size_t b_inv = round_up(nv * (size_t)std::max(inverse_samples, 1) * sizeof(double), 256);
-    if ((rc = ensure_slot(ctx, 0, b_views + b_obj + b_img + 2 * b_inv, 256))) return rc;
-    cudaStream_t st = ctx->pipe_stream[0];
-    uint8_t* din = static_cast<uint8_t*>(ctx->pipe_in[0]);
-    cc_view* d_views = reinterpret_cast<cc_view*>(din);
-    double* d_obj = reinterpret_cast<double*>(din + b_views);
-    double* d_img = reinterpret_cast<double*>(din + b_views + b_obj);
-    double* d_ir = reinterpret_cast<double*>(din + b_views + b_obj + b_img);
-    double* d_ic = reinterpret_cast<double*>(din + b_views + b_obj + b_img + b_inv);
-    double* d_sums = static_cast<double*>(ctx->pipe_out[0]);
-    if (nviews > 0) {
-        CC_CUDA(cudaMemcpyAsync(d_views, views, (size_t)nviews * sizeof(cc_view), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(d_obj, obj, nc * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-        CC_CUDA(cudaMemcpyAsync(d_img, img, (size_t)nviews * nc * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-        if (inverse_samples > 0) {
-            CC_CUDA(cudaMemcpyAsync(d_ir, inv_rows, (size_t)nviews * inverse_samples * sizeof(double), cudaMemcpyHostToDevice, st));
-            CC_CUDA(cudaMemcpyAsync(d_ic, inv_cols, (size_t)nviews * inverse_samples * sizeof(double), cudaMemcpyHostToDevice, st));
-        }
-    }
-    if ((rc = launch_calc_errors(ctx, intr, d_views, nviews, d_obj, d_img, n1, n2, d_ir, d_ic, inverse_samples, d_sums, st)))
-        return rc;
-    CC_CUDA(cudaMemcpyAsync(sums, d_sums, 4 * sizeof(double), cudaMemcpyDeviceToHost, st));
-    CC_CUDA(cudaStreamSynchronize(st));
-    return CC_OK;
+    if (rc || (rc = enter(ctx))) return rc;
+    const size_t nv = (size_t)nviews, nc = nviews > 0 ? (size_t)n1 * n2 : 0, ns = nv * inverse_samples;
+    const HostSpan spans[] = {{views, nullptr, nv * sizeof(cc_view)},
+                              {obj, nullptr, nc * 3 * sizeof(double)},
+                              {img, nullptr, nv * nc * 2 * sizeof(double)},
+                              {inv_rows, nullptr, ns * sizeof(double)},
+                              {inv_cols, nullptr, ns * sizeof(double)},
+                              {nullptr, sums, 4 * sizeof(double)}};
+    return stage_host(ctx, spans, [&](void* const* d, cudaStream_t st) {
+        return launch_calc_errors(ctx, intr, (const cc_view*)d[0], nviews, (const double*)d[1], (const double*)d[2],
+                                  n1, n2, (const double*)d[3], (const double*)d[4], inverse_samples, (double*)d[5], st);
+    });
 }
 
-// ---- Levenberg-Marquardt step -----------------------------------------------------
+// ---- Levenberg-Marquardt -----------------------------------------------------------
 int cc_lm_schur_f64(cc_ctx* ctx, const double* per_view, int nviews, double lambda, double* yz,
                     double* schur, void* stream) {
-    CC_REQUIRE(ctx && schur, "NULL argument");
-    CC_REQUIRE(nviews >= 0, "bad sizes");
-    CC_REQUIRE(nviews == 0 || (per_view && yz), "NULL device pointer");
-    CC_REQUIRE(lambda >= 0.0 && lambda == lambda, "lambda must be non-negative");
+    int rc = check_lm_schur(ctx, per_view, nviews, lambda, yz, schur);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
+    if (rc || (rc = enter(ctx))) return rc;
     return launch_lm_schur(ctx, per_view, nviews, lambda, yz, schur, (cudaStream_t)stream);
 }
 
 int cc_lm_update_f64(cc_ctx* ctx, const double* shared, const double* schur, double lambda,
                      unsigned free_mask, const double* yz, const cc_view* views_in, int nviews,
                      cc_view* views_out, double* delta, void* stream) {
-    CC_REQUIRE(ctx && shared && schur && delta, "NULL argument");
-    CC_REQUIRE(nviews >= 0, "bad sizes");
-    CC_REQUIRE(nviews == 0 || (yz && views_in && views_out), "NULL device pointer");
-    CC_REQUIRE(lambda >= 0.0 && lambda == lambda, "lambda must be non-negative");
-    CC_REQUIRE(free_mask != 0u && free_mask < 16u, "free_mask selects among the 4 shared parameters");
+    int rc = check_lm_update(ctx, shared, schur, lambda, free_mask, yz, views_in, nviews, views_out, delta);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
+    if (rc || (rc = enter(ctx))) return rc;
     return launch_lm_update(ctx, shared, schur, lambda, free_mask, yz, views_in, nviews, views_out, delta,
                             (cudaStream_t)stream);
 }
@@ -1012,42 +1044,34 @@ int cc_lm_update_f64(cc_ctx* ctx, const double* shared, const double* schur, dou
 int cc_lm_fit_f64_host(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask, cc_view* views,
                        int nviews, const double* obj, const double* img, int ncorners, int max_iter,
                        double eps, double* rms, int* iterations) {
-    CC_REQUIRE(ctx && intr && views && obj && img, "NULL argument");
-    CC_REQUIRE(nviews > 0 && ncorners > 0, "bad sizes");
-    CC_REQUIRE(free_mask != 0u && free_mask < 16u, "free_mask selects among the 4 shared parameters");
-    CC_REQUIRE(max_iter >= 0 && eps >= 0.0, "bad stopping rule");
-    CC_REQUIRE(aspect > 0.0 && intr->fcol != 0.0 && intr->checker_size != 0.0, "bad starting intrinsics");
+    int rc = check_lm_fit(ctx, intr, aspect, free_mask, views, nviews, obj, img, ncorners, max_iter, eps, true);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
-    return lm_fit_host(ctx, intr, aspect, free_mask, views, nviews, obj, img, ncorners, max_iter, eps, rms,
-                       iterations);
+    if (rc || (rc = enter(ctx))) return rc;
+    const size_t nv = (size_t)nviews, nc = (size_t)ncorners;
+    const HostSpan spans[] = {{views, views, nv * sizeof(cc_view)},
+                              {obj, nullptr, nc * 3 * sizeof(double)},
+                              {img, nullptr, nv * nc * 2 * sizeof(double)}};
+    return stage_host(ctx, spans, [&](void* const* d, cudaStream_t st) {
+        return lm_fit_device(ctx, intr, aspect, free_mask, (cc_view*)d[0], nviews, (const double*)d[1],
+                             (const double*)d[2], ncorners, max_iter, eps, rms, iterations, st);
+    });
 }
 
 int cc_lm_fit_f64(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask, cc_view* views, int nviews,
                   const double* obj, const double* img, int ncorners, int max_iter, double eps, double* rms,
                   int* iterations, void* stream) {
-    CC_REQUIRE(ctx && intr && obj, "NULL argument");
-    CC_REQUIRE(nviews >= 0 && ncorners > 0, "bad sizes");
-    CC_REQUIRE(nviews == 0 || (views && img), "NULL view / image-point array");
-    CC_REQUIRE(free_mask != 0u && free_mask < 16u, "free_mask selects among the 4 shared parameters");
-    CC_REQUIRE(max_iter >= 0 && eps >= 0.0, "bad stopping rule");
-    CC_REQUIRE(aspect > 0.0 && intr->fcol != 0.0 && intr->checker_size != 0.0, "bad starting intrinsics");
+    int rc = check_lm_fit(ctx, intr, aspect, free_mask, views, nviews, obj, img, ncorners, max_iter, eps, false);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
+    if (rc || (rc = enter(ctx))) return rc;
     return lm_fit_device(ctx, intr, aspect, free_mask, views, nviews, obj, img, ncorners, max_iter, eps, rms,
                          iterations, (cudaStream_t)stream);
 }
 
 int cc_lm_initial_guess_f64(cc_ctx* ctx, const double* obj, const double* img, int nviews, int ncorners, int sz1,
                             int sz2, double aspect, cc_intr* intr, cc_view* views, void* stream) {
-    CC_REQUIRE(ctx && intr && obj, "NULL argument");
-    CC_REQUIRE(nviews >= 0 && ncorners >= 4 && sz1 > 0 && sz2 > 0, "bad sizes (a homography needs >= 4 corners)");
-    CC_REQUIRE(nviews == 0 || (views && img), "NULL view / image-point array");
+    int rc = check_initial_guess(ctx, obj, img, nviews, ncorners, sz1, sz2, intr, views);
     CC_GUARD;
-    int rc = enter(ctx);
-    if (rc) return rc;
+    if (rc || (rc = enter(ctx))) return rc;
     return launch_initial_guess(ctx, obj, img, nviews, ncorners, sz1, sz2, aspect, intr, views, (cudaStream_t)stream);
 }
 

@@ -11,6 +11,32 @@
 
 namespace cc {
 
+// Rodrigues on the device (sincos: not bit-identical to rodrigues_host, so no point map or rectification uses it);
+// returns theta^2
+__device__ __forceinline__ double rodrigues(const double r[3], double R[9]) {
+    const double th2 = fma(r[2], r[2], fma(r[1], r[1], r[0] * r[0]));
+    const double th = sqrt(th2);
+    if (th < 2.220446049250313e-16) {
+#pragma unroll
+        for (int i = 0; i < 9; ++i) R[i] = (i % 4 == 0) ? 1.0 : 0.0;
+        return th2;
+    }
+    double s, c;
+    sincos(th, &s, &c);
+    const double c1 = 1.0 - c, it = 1.0 / th;
+    const double nx = r[0] * it, ny = r[1] * it, nz = r[2] * it;
+    R[0] = fma(c1 * nx, nx, c);
+    R[1] = fma(c1 * nx, ny, -(s * nz));
+    R[2] = fma(c1 * nx, nz, s * ny);
+    R[3] = fma(c1 * ny, nx, s * nz);
+    R[4] = fma(c1 * ny, ny, c);
+    R[5] = fma(c1 * ny, nz, -(s * nx));
+    R[6] = fma(c1 * nz, nx, -(s * ny));
+    R[7] = fma(c1 * nz, ny, s * nx);
+    R[8] = fma(c1 * nz, nz, c);
+    return th2;
+}
+
 // ---- world -> pixel: src/meta.jl:29  intrinsic o distort o Perspective o extrinsic o scale
 __device__ __forceinline__ void world2img(const ChainD& ch, double x, double y, double z,
                                           double& row, double& col) {

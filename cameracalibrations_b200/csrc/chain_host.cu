@@ -39,21 +39,7 @@ void rodrigues_host(const double r[3], double R[9]) {
 void build_chain(const cc_intr* in, const cc_view* vw, ChainD* ch) {
     rodrigues_host(vw->rvec, ch->R);
     for (int i = 0; i < 3; ++i) ch->t[i] = vw->tvec[i];
-    for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 3; ++j) ch->Rinv[3 * i + j] = ch->R[3 * j + i];
-    for (int i = 0; i < 3; ++i) {
-        const double* m = ch->Rinv + 3 * i;
-        ch->tinv[i] = std::fma(m[2], -ch->t[2], std::fma(m[1], -ch->t[1], m[0] * -ch->t[0]));
-    }
-    ch->frow = in->frow; ch->fcol = in->fcol;
-    ch->crow = in->crow; ch->ccol = in->ccol;
-    ch->k = in->k;
-    ch->a_row = 1.0 / in->frow;
-    ch->a_col = 1.0 / in->fcol;
-    ch->b_row = ch->a_row * (-in->crow);
-    ch->b_col = ch->a_col * (-in->ccol);
-    ch->inv_cs = 1.0 / in->checker_size;
-    ch->cs_back = 1.0 / ch->inv_cs;
+    complete_chain(*in, *ch);
 }
 
 void narrow_chain(const ChainD& d, ChainF* f) {

@@ -22,6 +22,27 @@ struct Chain {
 using ChainD = Chain<double>;
 using ChainF = Chain<float>;
 
+// The rest of a chain from its R and t and the intrinsics: inv(extrinsic), inv(intrinsic), scale and its inverse.
+// Fused only where the source says fma(), so the host build (-ffp-contract=off) and the device build (-fmad=false)
+// give the same bits.
+__host__ __device__ inline void complete_chain(const cc_intr& in, ChainD& ch) {
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) ch.Rinv[3 * i + j] = ch.R[3 * j + i];
+    for (int i = 0; i < 3; ++i) {
+        const double* m = ch.Rinv + 3 * i;
+        ch.tinv[i] = fma(m[2], -ch.t[2], fma(m[1], -ch.t[1], m[0] * -ch.t[0]));
+    }
+    ch.frow = in.frow; ch.fcol = in.fcol;
+    ch.crow = in.crow; ch.ccol = in.ccol;
+    ch.k = in.k;
+    ch.a_row = 1.0 / in.frow;
+    ch.a_col = 1.0 / in.fcol;
+    ch.b_row = ch.a_row * (-in.crow);
+    ch.b_col = ch.a_col * (-in.ccol);
+    ch.inv_cs = 1.0 / in.checker_size;
+    ch.cs_back = 1.0 / ch.inv_cs;
+}
+
 // host: rotation vector -> matrix and derived maps (chain_host.cu)
 void rodrigues_host(const double r[3], double R[9]);
 void build_chain(const cc_intr* in, const cc_view* vw, ChainD* out);
@@ -29,8 +50,6 @@ void narrow_chain(const ChainD& d, ChainF* f);
 void rectify_free_plans(struct ::cc_ctx* ctx);
 void rectify_free_sched(struct ::cc_ctx* ctx);
 void ingest_free(struct ::cc_ctx* ctx);
-int scratch_acquire(struct ::cc_ctx* ctx, size_t elems, cudaStream_t st);
-int scratch_release(struct ::cc_ctx* ctx, cudaStream_t st);
 int jpeg_info(const uint8_t* data, size_t length, int* sz1, int* sz2, int* channels);
 int jpeg_decode_u8c3(struct ::cc_ctx* ctx, const uint8_t* const* jpegs, const size_t* lengths, int n, uint8_t* dst,
                      int sz1, int sz2, size_t pitch, size_t frame_stride, cudaStream_t st);
@@ -102,7 +121,7 @@ struct cc_ctx {
     double* jtj_scratch;
     size_t jtj_scratch_elems;
     // the scratch is shared by reproj_jtj / calc_errors / lm_*: calls on DIFFERENT streams are ordered
-    // through an event recorded on the previous user's stream (scratch_acquire)
+    // through an event recorded on the previous user's stream (lm_state.cuh: ScratchHold)
     cudaStream_t scratch_stream;
     cudaEvent_t scratch_event;
     int scratch_used;
@@ -193,6 +212,12 @@ __device__ __forceinline__ void stg_stream(float4* p, float4 v) {
 __device__ __forceinline__ void stg_stream(uint4* p, uint4 v) {
     asm volatile("st.global.cs.v4.u32 [%0], {%1,%2,%3,%4};"
                  :: "l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
+}
+
+__device__ __forceinline__ double warp_sum(double v) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
 }
 
 // 2^-23-accurate reciprocal seed on the SFU (MUFU.RCP64H)

@@ -21,23 +21,17 @@ namespace cc {
 
 constexpr int kInitWarps = 4;
 
-__device__ __forceinline__ double wsum(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
 // mean and isotropic scale (mean distance sqrt(2)) of n 2-D points with stride `stride` doubles
 __device__ __forceinline__ void hartley(const double* p, int n, int stride, int lane, double& mx, double& my, double& s) {
     double sx = 0.0, sy = 0.0;
     for (int i = lane; i < n; i += 32) { sx += p[(size_t)i * stride]; sy += p[(size_t)i * stride + 1]; }
-    mx = wsum(sx) / n; my = wsum(sy) / n;
+    mx = warp_sum(sx) / n; my = warp_sum(sy) / n;
     double sd = 0.0;
     for (int i = lane; i < n; i += 32) {
         const double dx = p[(size_t)i * stride] - mx, dy = p[(size_t)i * stride + 1] - my;
         sd += sqrt(dx * dx + dy * dy);
     }
-    sd = wsum(sd) / n;
+    sd = warp_sum(sd) / n;
     s = 1.4142135623730951 / fmax(sd, 1e-300);
 }
 
@@ -121,7 +115,7 @@ init_homography_kernel(const double* __restrict__ obj, const double* __restrict_
         for (int i = 0; i < 9; ++i)
 #pragma unroll
             for (int j = i; j < 9; ++j) {
-                const double v = wsum(acc[k]);
+                const double v = warp_sum(acc[k]);
                 if (lane == 0) { smA[warp][9 * i + j] = v; smA[warp][9 * j + i] = v; }
                 ++k;
             }
@@ -171,21 +165,6 @@ init_homography_kernel(const double* __restrict__ obj, const double* __restrict_
         scratch[(size_t)3 * nviews + view] = A0[0] * b0 + A1[0] * b1;
         scratch[(size_t)4 * nviews + view] = A0[1] * b0 + A1[1] * b1;
     }
-}
-
-__global__ void __launch_bounds__(256)
-init_reduce_kernel(const double* __restrict__ scratch, int nviews, double* __restrict__ out) {
-    __shared__ double sm[256];
-    const double* col = scratch + (size_t)blockIdx.x * nviews;
-    double s = 0.0;
-    for (int v = threadIdx.x; v < nviews; v += 256) s += col[v];
-    sm[threadIdx.x] = s;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) sm[threadIdx.x] += sm[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
 }
 
 // pose of every view from its homography and the intrinsics (frow, fcol, c0, c1)
@@ -275,11 +254,8 @@ int launch_initial_guess(cc_ctx* ctx, const double* obj, const double* img, int 
             obj, img, nviews, ncorners, c0, c1, static_cast<double*>(hs.p), static_cast<double*>(scr.p));
         ctx->launches++;
     }
-    init_reduce_kernel<<<5, 256, 0, st>>>(static_cast<double*>(scr.p), nviews, static_cast<double*>(red.p));
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    int rc = comm_allreduce_sum(ctx, static_cast<double*>(red.p), 5, st);
-    if (rc) return rc;
+    int rc = launch_reduce(ctx, nullptr, static_cast<double*>(scr.p), 5, nviews, static_cast<double*>(red.p), st);
+    if (rc || (rc = comm_allreduce_sum(ctx, static_cast<double*>(red.p), 5, st))) return rc;
     double n[5];
     CC_CUDA(cudaMemcpyAsync(n, red.p, sizeof(n), cudaMemcpyDeviceToHost, st));
     CC_CUDA(cudaStreamSynchronize(st));

@@ -122,39 +122,6 @@ lm_schur_state_kernel(const LmState* __restrict__ st, const LmBufs b, int nviews
     lm_schur_view(b.pv[st->cur], nviews, st->lambda, yz, scratch);
 }
 
-// out[c] = sum_v scratch[c][v] in a fixed order (same scheme as residual.cu)
-__global__ void __launch_bounds__(256)
-lm_reduce_kernel(const double* __restrict__ scratch, int nviews, double* __restrict__ out) {
-    __shared__ double sm[256];
-    const double* col = scratch + (size_t)blockIdx.x * nviews;
-    double s = 0.0;
-    for (int v = threadIdx.x; v < nviews; v += 256) s += col[v];
-    sm[threadIdx.x] = s;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) sm[threadIdx.x] += sm[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
-}
-
-__global__ void __launch_bounds__(256)
-lm_reduce_state_kernel(const LmState* __restrict__ st, const double* __restrict__ scratch, int nviews,
-                       double* __restrict__ out) {
-    if (st->done) return;
-    __shared__ double sm[256];
-    const double* col = scratch + (size_t)blockIdx.x * nviews;
-    double s = 0.0;
-    for (int v = threadIdx.x; v < nviews; v += 256) s += col[v];
-    sm[threadIdx.x] = s;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) sm[threadIdx.x] += sm[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
-}
-
 // delta layout: [0,4) di | [4] sum |de|^2 | [5] sum |pe|^2 | [6] 1 if the 4x4 solve succeeded | [7] spare
 __device__ __forceinline__ void
 lm_update_view(const double* __restrict__ shared, const double* __restrict__ schur, double lambda,
@@ -297,7 +264,8 @@ __global__ void lm_decide_kernel(LmState* __restrict__ st, const double* __restr
 int launch_lm_schur(cc_ctx* ctx, const double* per_view, int nviews, double lambda, double* yz,
                     double* schur, cudaStream_t st) {
     const int nv = nviews > 0 ? nviews : 1;
-    int rc = scratch_acquire(ctx, (size_t)kSchurComponents * nv, st);
+    ScratchHold hold(ctx, st);
+    int rc = hold.acquire((size_t)kSchurComponents * nv);
     if (rc) return rc;
     if (nviews > 0) {
         lm_schur_kernel<<<(nviews * kSchurLanes + kLmThreads - 1) / kLmThreads, kLmThreads, 0, st>>>(per_view, nviews, lambda, yz,
@@ -305,18 +273,16 @@ int launch_lm_schur(cc_ctx* ctx, const double* per_view, int nviews, double lamb
         ctx->launches++;
         CC_CUDA(cudaGetLastError());
     }
-    lm_reduce_kernel<<<kSchurComponents, 256, 0, st>>>(ctx->jtj_scratch, nviews, schur);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    if ((rc = scratch_release(ctx, st))) return rc;
-    return CC_OK;
+    if ((rc = launch_reduce(ctx, nullptr, ctx->jtj_scratch, kSchurComponents, nviews, schur, st))) return rc;
+    return hold.release();
 }
 
 int launch_lm_update(cc_ctx* ctx, const double* shared, const double* schur, double lambda,
                      unsigned free_mask, const double* yz, const cc_view* views_in, int nviews,
                      cc_view* views_out, double* delta, cudaStream_t st) {
     const int nv = nviews > 0 ? nviews : 1;
-    int rc = scratch_acquire(ctx, (size_t)kSchurComponents * nv, st);
+    ScratchHold hold(ctx, st);
+    int rc = hold.acquire((size_t)kSchurComponents * nv);
     if (rc) return rc;
     // at least one block: block 0 publishes the shared-parameter step even without local views
     const int blocks = std::max(1, (nviews + kLmThreads - 1) / kLmThreads);
@@ -324,16 +290,9 @@ int launch_lm_update(cc_ctx* ctx, const double* shared, const double* schur, dou
                                                     views_out, delta, ctx->jtj_scratch);
     ctx->launches++;
     CC_CUDA(cudaGetLastError());
-    lm_reduce_kernel<<<2, 256, 0, st>>>(ctx->jtj_scratch, nviews, delta + 4);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    if ((rc = scratch_release(ctx, st))) return rc;
-    return CC_OK;
+    if ((rc = launch_reduce(ctx, nullptr, ctx->jtj_scratch, 2, nviews, delta + 4, st))) return rc;
+    return hold.release();
 }
-
-// launchers of residual.cu
-int launch_reproj_jtj(cc_ctx*, const cc_intr*, double, const cc_view*, int, const double*, const double*, int,
-                      double*, double*, cudaStream_t);
 
 // ---------------------------------------------------------------------------------------------
 // The fit as one device-resident loop (cc_lm_fit_f64): replaces the OpenCV.calibrateCamera call of
@@ -399,10 +358,6 @@ static int lm_workspace(cc_ctx* ctx, int nviews, LmWorkspace** out) {
     return CC_OK;
 }
 
-// launchers of residual.cu
-int launch_reproj_jtj(cc_ctx*, const cc_intr*, double, const cc_view*, int, const double*, const double*, int,
-                      double*, double*, cudaStream_t);
-
 int lm_fit_device(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask, cc_view* views, int nviews,
                   const double* obj, const double* img, int ncorners, int max_iter, double eps, double* rms,
                   int* iterations, cudaStream_t st) {
@@ -410,7 +365,8 @@ int lm_fit_device(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask,
     int rc = lm_workspace(ctx, nviews, &w);
     if (rc) return rc;
     const int nv1 = nviews > 0 ? nviews : 1;
-    if ((rc = scratch_acquire(ctx, (size_t)kSchurComponents * nv1, st))) return rc;
+    ScratchHold hold(ctx, st);                       // the whole loop; the launchers below take it again
+    if ((rc = hold.acquire((size_t)kSchurComponents * nv1))) return rc;
     double* schur = w->small;
     double* red = w->small + 24;
     double* sh_cur = w->small + 48;
@@ -444,15 +400,15 @@ int lm_fit_device(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask,
             lm_schur_state_kernel<<<(nviews * kSchurLanes + kLmThreads - 1) / kLmThreads, kLmThreads, 0, st>>>(w->state, b, nviews, w->yz, ctx->jtj_scratch);
             ctx->launches++;
         }
-        lm_reduce_state_kernel<<<kSchurComponents, 256, 0, st>>>(w->state, ctx->jtj_scratch, nviews, schur);
-        ctx->launches++;
+        if ((rc = launch_reduce(ctx, w->state, ctx->jtj_scratch, kSchurComponents, nviews, schur, st))) return rc;
         if ((rc = comm_allreduce_sum(ctx, schur, CC_LM_SCHUR, st))) return rc;
         // phase 2: shared step, candidate views, step norms
         lm_update_state_kernel<<<blocks_v, kLmThreads, 0, st>>>(w->state, sh_cur, schur, free_mask, w->yz, b, nviews,
                                                                delta, ctx->jtj_scratch);
-        lm_reduce_state_kernel<<<2, 256, 0, st>>>(w->state, ctx->jtj_scratch, nviews, red + 21);
+        ctx->launches++;
+        if ((rc = launch_reduce(ctx, w->state, ctx->jtj_scratch, 2, nviews, red + 21, st))) return rc;
         lm_candidate_kernel<<<1, 1, 0, st>>>(w->state, delta);
-        ctx->launches += 3;
+        ctx->launches++;
         // candidate's residual and blocks
         if ((rc = launch_reproj_jtj_state(ctx, w->state, 1, b, aspect, intr->checker_size, nviews, obj, img,
                                           ncorners, red, st))) return rc;
@@ -464,7 +420,7 @@ int lm_fit_device(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask,
         CC_CUDA(cudaMemcpyAsync(&w->host_state[slot], w->state, sizeof(LmState), cudaMemcpyDeviceToHost, st));
         CC_CUDA(cudaEventRecord(w->ev[slot], st));
     }
-    if ((rc = scratch_release(ctx, st))) return rc;
+    if ((rc = hold.release())) return rc;
     // the one wait of the call: the caller gets the intrinsics back on the host
     LmState fin;
     CC_CUDA(cudaMemcpyAsync(&w->host_state[0], w->state, sizeof(LmState), cudaMemcpyDeviceToHost, st));
@@ -478,36 +434,6 @@ int lm_fit_device(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask,
     intr->k = fin.par[3];
     if (rms) *rms = std::sqrt(fin.sse / std::max(1.0, fin.npoints));
     if (iterations) *iterations = fin.iterations;
-    return CC_OK;
-}
-
-// The same fit with HOST arrays (single call of a binding): copies in, runs the device loop, copies out.
-struct DevBuf {
-    void* p = nullptr;
-    ~DevBuf() { if (p) cudaFree(p); }
-    cudaError_t alloc(size_t bytes) { return cudaMalloc(&p, bytes ? bytes : 8); }
-    template <typename T> T* as() { return static_cast<T*>(p); }
-};
-
-int lm_fit_host(cc_ctx* ctx, cc_intr* intr, double aspect, unsigned free_mask, cc_view* views, int nviews,
-                const double* obj, const double* img, int ncorners, int max_iter, double eps, double* rms,
-                int* iterations) {
-    cudaStream_t st = nullptr;
-    CC_CUDA(cudaStreamCreateWithFlags(&st, cudaStreamNonBlocking));
-    struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamDestroy(s); } } guard{st};
-    const size_t nv = (size_t)nviews;
-    DevBuf d_views, d_obj, d_img;
-    CC_CUDA(d_views.alloc(nv * sizeof(cc_view)));
-    CC_CUDA(d_obj.alloc((size_t)ncorners * 3 * sizeof(double)));
-    CC_CUDA(d_img.alloc(nv * ncorners * 2 * sizeof(double)));
-    CC_CUDA(cudaMemcpyAsync(d_views.p, views, nv * sizeof(cc_view), cudaMemcpyHostToDevice, st));
-    CC_CUDA(cudaMemcpyAsync(d_obj.p, obj, (size_t)ncorners * 3 * sizeof(double), cudaMemcpyHostToDevice, st));
-    CC_CUDA(cudaMemcpyAsync(d_img.p, img, nv * ncorners * 2 * sizeof(double), cudaMemcpyHostToDevice, st));
-    int rc = lm_fit_device(ctx, intr, aspect, free_mask, d_views.as<cc_view>(), nviews, d_obj.as<double>(),
-                           d_img.as<double>(), ncorners, max_iter, eps, rms, iterations, st);
-    if (rc) return rc;
-    CC_CUDA(cudaMemcpyAsync(views, d_views.p, nv * sizeof(cc_view), cudaMemcpyDeviceToHost, st));
-    CC_CUDA(cudaStreamSynchronize(st));
     return CC_OK;
 }
 

@@ -35,26 +35,7 @@ __device__ __forceinline__ void skew(const double v[3], double S[9]) {
 // Rodrigues and its derivative:
 //   dR/dr_i = ( r_i [r]x + [ r x ((I - R) e_i) ]x ) R / theta^2 ,  -> [e_i]x as theta -> 0
 __device__ void view_geom(const double r[3], ViewGeom& g) {
-    const double th2 = fma(r[2], r[2], fma(r[1], r[1], r[0] * r[0]));
-    const double th = sqrt(th2);
-    if (th < 2.220446049250313e-16) {
-#pragma unroll
-        for (int i = 0; i < 9; ++i) g.R[i] = (i % 4 == 0) ? 1.0 : 0.0;
-    } else {
-        double s, c;
-        sincos(th, &s, &c);
-        const double c1 = 1.0 - c, it = 1.0 / th;
-        const double nx = r[0] * it, ny = r[1] * it, nz = r[2] * it;
-        g.R[0] = fma(c1 * nx, nx, c);
-        g.R[1] = fma(c1 * nx, ny, -(s * nz));
-        g.R[2] = fma(c1 * nx, nz, s * ny);
-        g.R[3] = fma(c1 * ny, nx, s * nz);
-        g.R[4] = fma(c1 * ny, ny, c);
-        g.R[5] = fma(c1 * ny, nz, -(s * nx));
-        g.R[6] = fma(c1 * nz, nx, -(s * ny));
-        g.R[7] = fma(c1 * nz, ny, s * nx);
-        g.R[8] = fma(c1 * nz, nz, c);
-    }
+    const double th2 = rodrigues(r, g.R);
     if (th2 < 1e-24) {
 #pragma unroll
         for (int i = 0; i < 3; ++i) {
@@ -128,12 +109,6 @@ __device__ __forceinline__ void corner_jac(const ViewGeom& g, const double t[3],
     J[0][7] = 1.0;            J[1][7] = 0.0;
     J[0][8] = 0.0;            J[1][8] = 1.0;
     J[0][9] = in.frow * u * r2; J[1][9] = in.fcol * v * r2;
-}
-
-__device__ __forceinline__ double warp_sum(double v) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
 }
 
 // Sum 64 per-lane partials over the warp with a HALVING butterfly: at the step with partner mask m a
@@ -268,32 +243,14 @@ reproj_jtj_state_kernel(const LmState* __restrict__ st, int which, const LmBufs 
     reproj_jtj_view(in, b.views[slot], nviews, obj, img, ncorners, b.pv[slot], scratch);
 }
 
-__device__ __forceinline__ void reduce_components(const double* __restrict__ scratch, int nviews,
-                                                  double* __restrict__ out) {
-    __shared__ double sm[256];
-    const double* col = scratch + (size_t)blockIdx.x * nviews;
-    double s = 0.0;
-    for (int v = threadIdx.x; v < nviews; v += 256) s += col[v];
-    sm[threadIdx.x] = s;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-        if (threadIdx.x < o) sm[threadIdx.x] += sm[threadIdx.x + o];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
-}
+// out[c] = sum_v parts[c][v] (blockIdx.x = c) in a fixed order: strided serial partials, then a tree.  Inside the
+// device-resident LM loop the kernel returns at once when gate->done; gate == nullptr: it always runs.
 __global__ void __launch_bounds__(256)
-reduce_components_state_kernel(const LmState* __restrict__ st, const double* __restrict__ scratch, int nviews,
-                               double* __restrict__ out) {
-    if (st->done) return;
-    reduce_components(scratch, nviews, out);
-}
-
-// out[c] = sum_v scratch[c][v] in a fixed order: strided serial partials, then a tree
-__global__ void __launch_bounds__(256)
-reduce_components_kernel(const double* __restrict__ scratch, int nviews, double* __restrict__ out) {
+reduce_components_kernel(const LmState* __restrict__ gate, const double* __restrict__ parts, int nviews,
+                         double* __restrict__ out) {
+    if (gate && gate->done) return;
     __shared__ double sm[256];
-    const double* col = scratch + (size_t)blockIdx.x * nviews;
+    const double* col = parts + (size_t)blockIdx.x * nviews;
     double s = 0.0;
     for (int v = threadIdx.x; v < nviews; v += 256) s += col[v];
     sm[threadIdx.x] = s;
@@ -325,40 +282,11 @@ calc_errors_kernel(const cc_intr intr, const cc_view* __restrict__ views, int nv
 
     // expand the chain on the device (views live in device memory here)
     ChainD ch;
-    {
-        double r[3];
+    double r[3];
 #pragma unroll
-        for (int i = 0; i < 3; ++i) { r[i] = views[view].rvec[i]; ch.t[i] = views[view].tvec[i]; }
-        const double th2 = fma(r[2], r[2], fma(r[1], r[1], r[0] * r[0]));
-        const double th = sqrt(th2);
-        if (th < 2.220446049250313e-16) {
-#pragma unroll
-            for (int i = 0; i < 9; ++i) ch.R[i] = (i % 4 == 0) ? 1.0 : 0.0;
-        } else {
-            double s, c;
-            sincos(th, &s, &c);
-            const double c1 = 1.0 - c, it = 1.0 / th;
-            const double nx = r[0] * it, ny = r[1] * it, nz = r[2] * it;
-            ch.R[0] = fma(c1 * nx, nx, c);        ch.R[1] = fma(c1 * nx, ny, -(s * nz));
-            ch.R[2] = fma(c1 * nx, nz, s * ny);   ch.R[3] = fma(c1 * ny, nx, s * nz);
-            ch.R[4] = fma(c1 * ny, ny, c);        ch.R[5] = fma(c1 * ny, nz, -(s * nx));
-            ch.R[6] = fma(c1 * nz, nx, -(s * ny)); ch.R[7] = fma(c1 * nz, ny, s * nx);
-            ch.R[8] = fma(c1 * nz, nz, c);
-        }
-#pragma unroll
-        for (int i = 0; i < 3; ++i)
-#pragma unroll
-            for (int j = 0; j < 3; ++j) ch.Rinv[3 * i + j] = ch.R[3 * j + i];
-#pragma unroll
-        for (int i = 0; i < 3; ++i)
-            ch.tinv[i] = fma(ch.Rinv[3 * i + 2], -ch.t[2],
-                             fma(ch.Rinv[3 * i + 1], -ch.t[1], ch.Rinv[3 * i] * -ch.t[0]));
-        ch.frow = intr.frow; ch.fcol = intr.fcol; ch.crow = intr.crow; ch.ccol = intr.ccol;
-        ch.k = intr.k;
-        ch.a_row = 1.0 / intr.frow; ch.a_col = 1.0 / intr.fcol;
-        ch.b_row = ch.a_row * (-intr.crow); ch.b_col = ch.a_col * (-intr.ccol);
-        ch.inv_cs = 1.0 / intr.checker_size; ch.cs_back = 1.0 / ch.inv_cs;
-    }
+    for (int i = 0; i < 3; ++i) { r[i] = views[view].rvec[i]; ch.t[i] = views[view].tvec[i]; }
+    rodrigues(r, ch.R);
+    complete_chain(intr, ch);
 
     double s_rep = 0.0, s_pro = 0.0, s_dis = 0.0, s_inv = 0.0;
     const double2* im = reinterpret_cast<const double2*>(img) + (size_t)view * nc;
@@ -410,33 +338,43 @@ calc_errors_kernel(const cc_intr intr, const cc_view* __restrict__ views, int nv
     }
 }
 
-// The per-context scratch ([components][views] partials) is shared by reproj_jtj, calc_errors and the
-// LM kernels.  Every launcher brackets its use: scratch_acquire grows the buffer and, when the call
-// comes on a stream other than the previous user's, makes it wait for the event that user recorded
-// in scratch_release -- two streams of one context can never race on the buffer.
-int scratch_acquire(cc_ctx* ctx, size_t elems, cudaStream_t st) {
-    if (ctx->scratch_used && ctx->scratch_stream != st && ctx->scratch_event)
-        CC_CUDA(cudaStreamWaitEvent(st, ctx->scratch_event, 0));
-    if (ctx->jtj_scratch_elems >= elems) return CC_OK;
-    if (ctx->jtj_scratch) { CC_CUDA(cudaFree(ctx->jtj_scratch)); ctx->jtj_scratch = nullptr; }
-    ctx->jtj_scratch_elems = 0;
-    CC_CUDA(cudaMalloc(&ctx->jtj_scratch, elems * sizeof(double)));
-    ctx->jtj_scratch_elems = elems;
+cudaError_t ScratchHold::record() {
+    cudaError_t e = ctx_->scratch_event ? cudaSuccess : cudaEventCreateWithFlags(&ctx_->scratch_event,
+                                                                                  cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventRecord(ctx_->scratch_event, st_);
+    if (e == cudaSuccess) { ctx_->scratch_stream = st_; ctx_->scratch_used = 1; }
+    return e;
+}
+int ScratchHold::acquire(size_t elems) {
+    if (ctx_->scratch_used && ctx_->scratch_stream != st_ && ctx_->scratch_event)
+        CC_CUDA(cudaStreamWaitEvent(st_, ctx_->scratch_event, 0));
+    held_ = true;
+    if (ctx_->jtj_scratch_elems >= elems) return CC_OK;
+    if (ctx_->jtj_scratch) { CC_CUDA(cudaFree(ctx_->jtj_scratch)); ctx_->jtj_scratch = nullptr; }
+    ctx_->jtj_scratch_elems = 0;
+    CC_CUDA(cudaMalloc(&ctx_->jtj_scratch, elems * sizeof(double)));
+    ctx_->jtj_scratch_elems = elems;
     return CC_OK;
 }
-int scratch_release(cc_ctx* ctx, cudaStream_t st) {
-    if (!ctx->scratch_event) CC_CUDA(cudaEventCreateWithFlags(&ctx->scratch_event, cudaEventDisableTiming));
-    CC_CUDA(cudaEventRecord(ctx->scratch_event, st));
-    ctx->scratch_stream = st;
-    ctx->scratch_used = 1;
+int ScratchHold::release() {
+    held_ = false;
+    const cudaError_t e = record();
+    return e == cudaSuccess ? CC_OK : cuda_fail(e, "scratch event");
+}
+
+int launch_reduce(cc_ctx* ctx, const LmState* gate, const double* parts, int ncomp, int nviews, double* out,
+                  cudaStream_t st) {
+    reduce_components_kernel<<<ncomp, 256, 0, st>>>(gate, parts, nviews, out);
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
     return CC_OK;
 }
 
 int launch_reproj_jtj(cc_ctx* ctx, const cc_intr* intr, double aspect, const cc_view* views,
                       int nviews, const double* obj, const double* img, int ncorners,
                       double* per_view, double* shared, cudaStream_t st) {
-    CC_REQUIRE((reinterpret_cast<uintptr_t>(img) & 15u) == 0, "img must be 16-byte aligned");
-    int rc = scratch_acquire(ctx, (size_t)CC_SHARED * (size_t)(nviews > 0 ? nviews : 1), st);
+    ScratchHold hold(ctx, st);
+    int rc = hold.acquire((size_t)CC_SHARED * (size_t)(nviews > 0 ? nviews : 1));
     if (rc) return rc;
     if (nviews > 0) {
         SharedIntr in{intr->frow, intr->fcol, intr->crow, intr->ccol, intr->k, aspect,
@@ -446,17 +384,15 @@ int launch_reproj_jtj(cc_ctx* ctx, const cc_intr* intr, double aspect, const cc_
         ctx->launches++;
         CC_CUDA(cudaGetLastError());
     }
-    reduce_components_kernel<<<CC_SHARED, 256, 0, st>>>(ctx->jtj_scratch, nviews, shared);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    if ((rc = scratch_release(ctx, st))) return rc;
-    return CC_OK;
+    if ((rc = launch_reduce(ctx, nullptr, ctx->jtj_scratch, CC_SHARED, nviews, shared, st))) return rc;
+    return hold.release();
 }
 
 int launch_reproj_jtj_state(cc_ctx* ctx, const LmState* st, int which, const LmBufs& b, double aspect,
                             double checker_size, int nviews, const double* obj, const double* img,
                             int ncorners, double* shared_out, cudaStream_t stream) {
-    int rc = scratch_acquire(ctx, (size_t)CC_SHARED * (size_t)(nviews > 0 ? nviews : 1), stream);
+    ScratchHold hold(ctx, stream);
+    int rc = hold.acquire((size_t)CC_SHARED * (size_t)(nviews > 0 ? nviews : 1));
     if (rc) return rc;
     if (nviews > 0) {
         reproj_jtj_state_kernel<<<(nviews + kResWarps - 1) / kResWarps, kResThreads, 0, stream>>>(
@@ -464,20 +400,18 @@ int launch_reproj_jtj_state(cc_ctx* ctx, const LmState* st, int which, const LmB
         ctx->launches++;
         CC_CUDA(cudaGetLastError());
     }
-    reduce_components_state_kernel<<<CC_SHARED, 256, 0, stream>>>(st, ctx->jtj_scratch, nviews, shared_out);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    if ((rc = scratch_release(ctx, stream))) return rc;
-    return CC_OK;
+    if ((rc = launch_reduce(ctx, st, ctx->jtj_scratch, CC_SHARED, nviews, shared_out, stream))) return rc;
+    return hold.release();
 }
+
+size_t calc_errors_smem(int n1, int n2) { return (size_t)kResWarps * n1 * n2 * 3 * sizeof(double); }
 
 int launch_calc_errors(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
                        const double* obj, const double* img, int n1, int n2, const double* inv_rows,
                        const double* inv_cols, int inverse_samples, double* sums, cudaStream_t st) {
-    CC_REQUIRE((reinterpret_cast<uintptr_t>(img) & 15u) == 0, "img must be 16-byte aligned");
-    const size_t smem = (size_t)kResWarps * n1 * n2 * 3 * sizeof(double);
-    CC_REQUIRE(smem <= 200 * 1024, "too many corners per view for the fused kernel");
-    int rc = scratch_acquire(ctx, (size_t)CC_SHARED * (size_t)(nviews > 0 ? nviews : 1), st);
+    const size_t smem = calc_errors_smem(n1, n2);
+    ScratchHold hold(ctx, st);
+    int rc = hold.acquire((size_t)CC_SHARED * (size_t)(nviews > 0 ? nviews : 1));
     if (rc) return rc;
     if (nviews > 0) {
         if (smem > 48 * 1024)
@@ -489,11 +423,8 @@ int launch_calc_errors(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, i
         ctx->launches++;
         CC_CUDA(cudaGetLastError());
     }
-    reduce_components_kernel<<<4, 256, 0, st>>>(ctx->jtj_scratch, nviews, sums);
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    if ((rc = scratch_release(ctx, st))) return rc;
-    return CC_OK;
+    if ((rc = launch_reduce(ctx, nullptr, ctx->jtj_scratch, 4, nviews, sums, st))) return rc;
+    return hold.release();
 }
 
 }  // namespace cc
