@@ -11,7 +11,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# CAMCAL_B200_LIB: load another build of the same ABI (tuning variants under profiles/variants/)
+# CAMCAL_B200_LIB: load another build of the same ABI (the bounds-checked build, or another commit's for an A/B)
 LIB_PATH = os.environ.get("CAMCAL_B200_LIB") or os.path.join(_HERE, "libcamcal_b200.so")
 
 CC_OK = 0

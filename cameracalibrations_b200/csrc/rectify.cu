@@ -34,72 +34,20 @@ namespace cc {
 
 constexpr int kT = 32;                 // strip width along the first axis = lanes of a warp
 constexpr int kWarps = 4;              // consumer warps per CTA
-#ifndef CAMCAL_TL_F32
-#define CAMCAL_TL_F32 32
-#endif
-constexpr int kTLf = CAMCAL_TL_F32;    // f32c1: lines per tile (a warp owns kTLf / kWarps of them)
+constexpr int kTLf = 32;               // f32c1: lines per tile (a warp owns kTLf / kWarps of them)
+constexpr int kTLu = 32;               // u8c3: lines per tile
 constexpr int kTLmax = 32;             // most lines of a tile (sizes the per-stage q2 slots)
 // most frames one unit rectifies with one map (measured, profiles/r1_rectify.md: the costlier the
 // map, the larger the group; the cheaper, the finer the units for the tail of the ticket queue)
-#ifndef CAMCAL_FG_F32_EXACT
-#define CAMCAL_FG_F32_EXACT 12
-#endif
-#ifndef CAMCAL_FG_F32_FAST
-#define CAMCAL_FG_F32_FAST 4
-#endif
-#ifndef CAMCAL_FG_U8_EXACT
-#define CAMCAL_FG_U8_EXACT 16
-#endif
-#ifndef CAMCAL_FG_U8_FAST
-#define CAMCAL_FG_U8_FAST 16
-#endif
-constexpr int kFGf32Exact = CAMCAL_FG_F32_EXACT, kFGf32Fast = CAMCAL_FG_F32_FAST, kFGu8Exact = CAMCAL_FG_U8_EXACT, kFGu8Fast = CAMCAL_FG_U8_FAST;
-#ifndef CAMCAL_TL_U8
-#define CAMCAL_TL_U8 32
-#endif
-constexpr int kTLu = CAMCAL_TL_U8;     // u8c3: lines per tile
-// floor of the exact path, per axis: 0 = FRND.F64.FLOOR (XU pipe), 1 = DADD.RM (FP64 pipe)
-#ifndef CAMCAL_FLOOR1
-#define CAMCAL_FLOOR1 0
-#endif
-#ifndef CAMCAL_FLOOR2
-#define CAMCAL_FLOOR2 1
-#endif
-constexpr int kFloorMode1 = CAMCAL_FLOOR1, kFloorMode2 = CAMCAL_FLOOR2;
-#ifndef CAMCAL_MAX_STAGES
-#define CAMCAL_MAX_STAGES 8
-#endif
-constexpr int kMaxStages = CAMCAL_MAX_STAGES;
+constexpr int kFGf32Exact = 12, kFGf32Fast = 4, kFGu8Exact = 16, kFGu8Fast = 16;
+constexpr int kMaxStages = 8;
 // dynamic shared memory one CTA may spend on its ring (4 resident CTAs of 48 KB + static slots fit in 227 KB)
-#ifndef CAMCAL_RING_BYTES
-#define CAMCAL_RING_BYTES (48 * 1024)
-#endif
-// staged line pitch granularity in bytes, per pixel format (16: dense boxes; 128: all 32 banks, see plan_boxes)
-#ifndef CAMCAL_PITCH_ALIGN_U8
-#define CAMCAL_PITCH_ALIGN_U8 0        // 0: the bank-disjoint pitch of plan_boxes; else round the line up to this many bytes
-#endif
-#ifndef CAMCAL_PITCH_ALIGN_F32
-#define CAMCAL_PITCH_ALIGN_F32 16
-#endif
-#ifndef CAMCAL_PRODUCER_SLEEP
-#define CAMCAL_PRODUCER_SLEEP 256
-#endif
-constexpr int kProducerSleep = CAMCAL_PRODUCER_SLEEP;   // ns between the producer's probes of a full ring
-#ifndef CAMCAL_MINB
-#define CAMCAL_MINB 1
-#endif
-#ifndef CAMCAL_MINB_EXACT
-#define CAMCAL_MINB_EXACT 4
-#endif
-// __launch_bounds__ min CTAs/SM of the staged f32c1 kernels (fast / exact coordinates)
-constexpr int kMinBlocks = CAMCAL_MINB, kMinBlocksExact = CAMCAL_MINB_EXACT;
-#ifndef CAMCAL_MINB_U8
-#define CAMCAL_MINB_U8 1
-#endif
-#ifndef CAMCAL_MINB_U8_EXACT
-#define CAMCAL_MINB_U8_EXACT 3
-#endif
-constexpr int kMinBlocksU8 = CAMCAL_MINB_U8, kMinBlocksU8Exact = CAMCAL_MINB_U8_EXACT;
+constexpr int kRingBytes = 48 * 1024;
+// f32c1 staged line pitch granularity in bytes (dense boxes; u8c3 lines take the bank-disjoint pitch of box_dims)
+constexpr int kPitchAlignF32 = 16;
+// __launch_bounds__ min CTAs/SM of the staged kernels (fast / exact coordinates)
+constexpr int kMinBlocks = 1, kMinBlocksExact = 4;
+constexpr int kMinBlocksU8 = 1, kMinBlocksU8Exact = 3;
 constexpr int kConsumerThreads = 32 * kWarps;
 
 struct TileCfg {
@@ -112,8 +60,7 @@ struct TileCfg {
     int strips;            // tiles along the first axis
     uint32_t units;        // strips * ntiles2 * frame groups
     int fg;                // frames per group: the tile's map is built once per group and reused
-    uint32_t widen_mul;    // f32c1 exact: 2^29, the multiplier of the integer float->double widening (a kernel
-                           // parameter so that ptxas keeps ONE IMAD.WIDE instead of two shifts, rectify_f32c1.cuh)
+    uint32_t reserved;     // unused: keeps the offsets of the fields below, and with them the kernels' SASS
     // *_views_kernel only (frames with different views in ONE launch): units are (strip x, tile y, group) with
     // group = view * gpv + frame group of the view; the tile headers / q2 terms of view v start at v * tiles / v * sz2
     int fpv;               // frames per view
@@ -423,22 +370,17 @@ static BoxDims box_dims(int need1, int need2, int tilt, int pxb) {
     if (pxb == 4) {
         const int unit = 4;
         d.box1 = (need1 + unit - 1 + unit - 1) / unit * unit;          // + unit - 1: the origin is rounded down
-        const int align = CAMCAL_PITCH_ALIGN_F32;
-        d.pitch_b = (d.box1 * pxb + align - 1) / align * align;
+        d.pitch_b = (d.box1 * pxb + kPitchAlignF32 - 1) / kPitchAlignF32 * kPitchAlignF32;
         d.box1 = d.pitch_b / pxb;                                      // usable pixels per line
     } else {
         const int need_b = need1 * 3 + 15;                             // + 15: the byte origin is rounded down
         int pitch = (need_b + 15) / 16 * 16;
-#if CAMCAL_PITCH_ALIGN_U8 == 0
         const int want = tilt >= 0 ? 4 : 28;                           // pitch in words, mod 32
         const int dense = pitch;
         while ((pitch / 4) % 32 != want) pitch += 16;
         // a TMA box line holds at most 256 elements (bytes here): a footprint whose bank-disjoint pitch does
         // not fit keeps the dense pitch (some bank conflicts) rather than losing the staged path altogether
         if (pitch > 256 && dense <= 256) pitch = dense;
-#else
-        pitch = (pitch + CAMCAL_PITCH_ALIGN_U8 - 1) / CAMCAL_PITCH_ALIGN_U8 * CAMCAL_PITCH_ALIGN_U8;
-#endif
         d.pitch_b = pitch;
         d.box1 = pitch / 3;
     }
@@ -592,8 +534,7 @@ static EncodeTiledFn encoder(cc_ctx* ctx) {
 // stages.  The ring hides the TMA round trip: per SM, (stages - 1) x resident CTAs x the USEFUL bytes of a box must
 // cover bandwidth x latency (~30 KB of reads at the HBM roofline, profiles/r2_rectify.md)
 static int ring_stages(int box_bytes) {
-    int stages = std::min(kMaxStages, std::max(2, CAMCAL_RING_BYTES / box_bytes));
-    if (const char* e = getenv("CAMCAL_STAGES")) stages = std::min(kMaxStages, std::max(1, atoi(e)));   // tuning knob
+    int stages = std::min(kMaxStages, std::max(2, kRingBytes / box_bytes));
     while (stages > 2 && stages * box_bytes > 56 * 1024) --stages;
     return stages;
 }
@@ -614,15 +555,9 @@ static bool stage_box(cc_ctx* ctx, const void* src, int pxb, int sz1, int sz2, s
     cuuint64_t strides[2] = {(cuuint64_t)pitch_b, (cuuint64_t)(nframes > 1 ? frame_stride * pxb : pitch_b * sz2)};
     cuuint32_t box[3] = {(cuuint32_t)(pxb == 4 ? d.pitch_b / 4 : d.pitch_b), (cuuint32_t)d.box2, 1};
     cuuint32_t estr[3] = {1, 1, 1};
-    CUtensorMapL2promotion l2promo = CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    if (const char* e = getenv("CAMCAL_L2PROMO")) {     // tuning knob: 0 none, 64, 128, 256
-        const int v = atoi(e);
-        l2promo = v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                : v == 256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B;
-    }
     memset(tmap, 0, sizeof(*tmap));
     if (enc(tmap, pxb == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(src),
-            dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, l2promo,
+            dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
         return false;
     cfg->box1 = d.box1; cfg->box2 = d.box2; cfg->pitch_b = d.pitch_b; cfg->box_bytes = d.box_bytes;
@@ -704,7 +639,6 @@ static int persistent_grid(cc_ctx* ctx, int kslot, K kernel, size_t smem, const 
         plan->per_sm[exact] = per_sm;
         plan->per_sm_smem[exact] = smem;
     }
-    if (const char* e = getenv("CAMCAL_CTAS_PER_SM")) per_sm = std::min(per_sm, std::max(1, atoi(e)));   // tuning knob
     *gsz = std::min<uint32_t>(cfg.units, (uint32_t)ctx->sm_count * (uint32_t)std::max(per_sm, 1));
     if (getenv("CAMCAL_DEBUG"))
         fprintf(stderr, "[camcal] staged: box %dx%d pitch %d (%d B) stages %d units %u (fg %d) grid %u (%d/SM) smem %zu\n",
@@ -761,7 +695,7 @@ template <> struct RectFmt<float> {
     // least two frames (single frames, e.g. the per-view launches of cc_rectify_*_views, keep one); the views kernel
     // holds one frame per stage
     static size_t ring(TileCfg& cfg, bool views, int* nf) {
-        *nf = (!views && kF32FramesPerStage == 2 && cfg.stages >= 4 && cfg.fg >= 2) ? 2 : 1;
+        *nf = (!views && cfg.stages >= 4 && cfg.fg >= 2) ? 2 : 1;
         cfg.stages /= *nf;
         return (size_t)cfg.stages * *nf * cfg.box_bytes;
     }
@@ -778,12 +712,10 @@ template <> struct RectFmt<uint8_t> {
     static int staged_slot(int) { return 2; }
     static auto views(bool e) { return e ? rectify_u8c3_views_kernel<true> : rectify_u8c3_views_kernel<false>; }
     static auto direct(bool e) { return e ? rectify_u8c3_direct_kernel<true> : rectify_u8c3_direct_kernel<false>; }
-    // a stage holds kU8FramesPerStage boxes; + 16: the word-granular gather may read the aligned words that hold the
-    // last tap bytes
+    // one frame per stage; + 16: the word-granular gather may read the aligned words that hold the last tap bytes
     static size_t ring(TileCfg& cfg, bool, int* nf) {
-        *nf = kU8FramesPerStage;
-        cfg.stages = std::max(2, cfg.stages / kU8FramesPerStage);
-        return (size_t)cfg.stages * kU8FramesPerStage * cfg.box_bytes + 16;
+        *nf = 1;
+        return (size_t)cfg.stages * cfg.box_bytes + 16;
     }
     // the staged kernel writes whole 32-bit words: 4-byte aligned output lines
     static bool dst_ok(const uint8_t* dst, const RectFrames& fr, int nframes) {
@@ -821,7 +753,6 @@ int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const
     int rc = CC_OK;
     if (tma) {
         if ((rc = unit_cfg(ctx, &cfg, c.fr.sz1, c.fr.sz2, nframes, kT, F::tl, exact ? F::fg_exact : F::fg_fast))) return rc;
-        cfg.widen_mul = 0x20000000u;
         int nf = 1;
         const size_t smem = F::ring(cfg, false, &nf);
         const auto k = F::staged(exact, nf);
@@ -1056,7 +987,6 @@ static int views_window(cc_ctx* ctx, MultiPlan* mp, const RectCall<PX>& c, int v
     cfg.g0 = g0;
     CC_REQUIRE(units < (1ll << 31), "too many tiles in one call: split the batch");
     cfg.units = (uint32_t)units;
-    cfg.widen_mul = 0x20000000u;
     for (int v = 0; v < nv; ++v) {
         const RectGeom gv = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, wn);
         L->vt.v[v].pe = make_exact(c.views.chs[v0 + v], c.views.ratios[v0 + v]);

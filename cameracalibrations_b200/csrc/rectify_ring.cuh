@@ -27,31 +27,12 @@ __device__ __forceinline__ void ring_init(SmemRing* ring, int stages) {
     __syncthreads();
 }
 
-// CAMCAL_PRODUCER_PARK > 0: wait with the barrier's own suspend-time hint (the polling loop of
+// the producer waits for a free stage parked on the barrier's own suspend-time hint (a polling loop of
 // try_wait + nanosleep was 8 % of all executed warp instructions of the u8 kernel, ncu round 2)
-#ifndef CAMCAL_PRODUCER_PARK
-#define CAMCAL_PRODUCER_PARK 2000
-#endif
 __device__ __forceinline__ void producer_wait(uint64_t* bar, uint32_t parity) {
-    if (CAMCAL_PRODUCER_PARK > 0) mbar_wait_parked<CAMCAL_PRODUCER_PARK>(bar, parity);
-    else mbar_wait<kProducerSleep>(bar, parity);
+    mbar_wait_parked<2000>(bar, parity);
 }
 
-// consumers: CAMCAL_POS_TRACK 1 counts the frames of a unit in registers instead of reading the
-// slot per frame (measured 1 % SLOWER on c2 exact: 0.2123 vs 0.2100 ms -- two more live registers
-// in a 96-register kernel; kept as a knob); CAMCAL_ELECT: the arriving lane chosen with ELECT
-// instead of a lane-id compare (no S2R per frame; neutral)
-#ifndef CAMCAL_POS_TRACK
-#define CAMCAL_POS_TRACK 1
-#endif
-#ifndef CAMCAL_ELECT
-#define CAMCAL_ELECT 1
-#endif
-constexpr bool kPosTrack = CAMCAL_POS_TRACK != 0, kElectArrive = CAMCAL_ELECT != 0;
-// L2 eviction hint of the staged boxes (tma.cuh): 0 none, 1 evict_last, 2 evict_first, 3 evict_normal
-#ifndef CAMCAL_TMA_L2
-#define CAMCAL_TMA_L2 1
-#endif
 __device__ __forceinline__ uint32_t take_ticket(RectSched* sched, int lane_id) {
     uint32_t u = 0;
     if (lane_id == 0) u = atomicAdd(&sched->next, 1u);
@@ -61,7 +42,7 @@ __device__ __forceinline__ uint32_t take_ticket(RectSched* sched, int lane_id) {
 // PXB: multiplier from TileHdr.x0 to the tensor-map coordinate (1: f32c1 texels, and u8c3 whose x0 already is a byte offset).
 // A unit is (strip x, tile y, frame group): the producer publishes one slot per FRAME of the
 // group -- pos = (x, y, frame, number of frames of the unit on its first frame, else 0) -- the
-// consumers read the slot on a unit's first frame only (CAMCAL_POS_TRACK) and count the frames down.
+// consumers read the slot on a unit's first frame only and count the frames down.
 // NF: frames per ring stage (2: a stage holds the boxes of two consecutive frames of the unit -- one at
 // the odd end of a unit -- so the consumers pay one hand-over per pair)
 // VIEWS: frames with different views in one launch -- the third unit coordinate counts (view, frame group of
@@ -74,8 +55,7 @@ __device__ __forceinline__ void producer_loop(const CUtensorMap* tmap, const Rec
                                               const double* __restrict__ q2tab, RectSched* sched,
                                               SmemRing* ring, uint8_t* stage_mem, int lane_id) {
     if (lane_id == 0) tma_prefetch_desc(tmap);
-    [[maybe_unused]] uint64_t policy = 0;
-    if (CAMCAL_TMA_L2 != 0) policy = l2_policy<CAMCAL_TMA_L2>();
+    const uint64_t policy = l2_evict_last();
     int s = 0;
     uint32_t phase = 1;                            // a fresh barrier passes a parity-1 wait
     uint32_t u_next = take_ticket(sched, lane_id);
@@ -131,8 +111,7 @@ __device__ __forceinline__ void producer_loop(const CUtensorMap* tmap, const Rec
                 for (int j = 0; j < NF; ++j) {
                     if (j >= nload) break;
                     uint8_t* box = stage_mem + ((size_t)s * NF + j) * cfg.box_bytes;
-                    if (CAMCAL_TMA_L2 != 0) tma_load_3d_hint(box, tmap, &ring->full[s], x0 * PXB, y0, f + j, policy);
-                    else tma_load_3d(box, tmap, &ring->full[s], x0 * PXB, y0, f + j);
+                    tma_load_3d_hint(box, tmap, &ring->full[s], x0 * PXB, y0, f + j, policy);
                 }
             }
             if (++s == cfg.stages) { s = 0; phase ^= 1; }

@@ -89,49 +89,9 @@ __device__ __forceinline__ uint32_t blend_rgb(const Taps6& t0, const Taps6& t1, 
     return __byte_perm(__byte_perm(r, g, 0x0040), b, 0x0410);
 }
 
-// Two pixels at once (FMUL2/FFMA2).  A byte's bit pattern IS a float already -- the denormal
-// b * 2^-149 -- so one packed FMUL2 by 2^100 per pair of bytes makes it the normal float b * 2^-49
-// (exact); the blend runs in that scaled domain (all normal numbers, full relative precision) and
-// the final FFMA2 by 2^49 onto the rounding magic undoes the scale.
-constexpr float kTwo100 = 1.2676506002282294e30f;      // 2^100
 constexpr float kTwo49 = 562949953421312.0f;           // 2^49
-__device__ __forceinline__ float2 byte_f2(uint32_t wp, uint32_t wq, int k) {
-    return mul2(make_float2(__uint_as_float(__byte_perm(wp, 0u, 0x4440u + (unsigned)k)),
-                            __uint_as_float(__byte_perm(wq, 0u, 0x4440u + (unsigned)k))), bc2(kTwo100));
-}
-
 // distance of a blended value from the integer it rounds to, against the certification bound
 constexpr float kCertThr = 0.5f - 6.5e-5f;
-
-// scaled blended values -> packed 0x00BBGGRR per pixel (+ certification of the roundings)
-template <bool CERT>
-__device__ __forceinline__ void round_pack2(float2 vr, float2 vg, float2 vb, uint32_t& rgb_p, uint32_t& rgb_q,
-                                            bool& amb_p, bool& amb_q) {
-    const float2 m = bc2(12582912.0f), up = bc2(kTwo49);
-    const float2 fr = fma2(vr, up, m), fg = fma2(vg, up, m), fb = fma2(vb, up, m);     // rint(v) in the low byte
-    rgb_p = __byte_perm(__byte_perm(__float_as_uint(fr.x), __float_as_uint(fg.x), 0x0040), __float_as_uint(fb.x), 0x0410);
-    rgb_q = __byte_perm(__byte_perm(__float_as_uint(fr.y), __float_as_uint(fg.y), 0x0040), __float_as_uint(fb.y), 0x0410);
-    if (CERT) {
-        // v - rint(v): the scaling by 2^49 is exact, the FMA rounds once (|e| <= 0.5, far above ulp)
-        const float2 er = fma2(vr, up, sub2(m, fr)), eg = fma2(vg, up, sub2(m, fg)), eb = fma2(vb, up, sub2(m, fb));
-        amb_p = (fabsf(er.x) > kCertThr) | (fabsf(eg.x) > kCertThr) | (fabsf(eb.x) > kCertThr);
-        amb_q = (fabsf(er.y) > kCertThr) | (fabsf(eg.y) > kCertThr) | (fabsf(eb.y) > kCertThr);
-    }
-}
-
-// CERT: also report (per pixel) whether any channel is too close to a rounding boundary
-template <bool CERT>
-__device__ __forceinline__ void blend_rgb2(const Taps6& p0, const Taps6& p1, const Taps6& q0,
-                                           const Taps6& q1, float2 d1, float2 d2, uint32_t& rgb_p,
-                                           uint32_t& rgb_q, bool& amb_p, bool& amb_q) {
-    const float2 vr = bilerp_fast2(byte_f2(p0.lo, q0.lo, 0), byte_f2(p0.lo, q0.lo, 3),
-                                   byte_f2(p1.lo, q1.lo, 0), byte_f2(p1.lo, q1.lo, 3), d1, d2);
-    const float2 vg = bilerp_fast2(byte_f2(p0.lo, q0.lo, 1), byte_f2(p0.hi, q0.hi, 0),
-                                   byte_f2(p1.lo, q1.lo, 1), byte_f2(p1.hi, q1.hi, 0), d1, d2);
-    const float2 vb = bilerp_fast2(byte_f2(p0.lo, q0.lo, 2), byte_f2(p0.hi, q0.hi, 1),
-                                   byte_f2(p1.lo, q1.lo, 2), byte_f2(p1.hi, q1.hi, 1), d1, d2);
-    round_pack2<CERT>(vr, vg, vb, rgb_p, rgb_q, amb_p, amb_q);
-}
 
 __device__ __forceinline__ void store_rgb(uint8_t* q, uint32_t rgb) {
     q[0] = (uint8_t)rgb; q[1] = (uint8_t)(rgb >> 8); q[2] = (uint8_t)(rgb >> 16);
@@ -231,32 +191,14 @@ rectify_u8c3_direct_kernel(const __grid_constant__ RectExact pe, const __grid_co
 // re-blended in FP64 in the oracle's operation order and patched with byte stores.  The output is
 // bit-identical to the FP64 blend.
 //
-// Tap bytes: CAMCAL_U8_LOAD 1 reads every tap byte with LDS.U8 (no ALU work; the load unit
-// isolates the byte), 0 reads three aligned words per source line and isolates bytes with PRMT.
+// Tap bytes (exact variant): source line i2 is three aligned words + PRMT (ALU pipe), line i2+1 six
+// LDS.U8 (the load unit isolates the bytes).
+//
+// One frame per ring stage: two (as in rectify_f32c1.cuh) cost registers here and were measured
+// slower (profiles/r2_rectify.md).
 //
 // Stores: the 32 pixels of a warp's line are 96 contiguous bytes = 24 words.  Lane L (L % 4 != 3)
 // builds word L - L/4 from its own packed pixel and lane L+1's (one shuffle, one PRMT).
-#ifndef CAMCAL_U8_LOAD
-#define CAMCAL_U8_LOAD 3
-#endif
-#ifndef CAMCAL_U8_DEBUG
-#define CAMCAL_U8_DEBUG 0
-#endif
-// CAMCAL_U8_PAIR 1: two frames per ring stage (one hand-over per pair of frames, as in rectify_f32c1.cuh).
-// Measured SLOWER here (c3 fast 0.199 vs 0.195 ms, exact 0.354 vs 0.304): the loop over the stage's
-// frames costs registers (fast 96 -> 128, exact spills or 136 = two CTAs per SM); kept as a knob.
-#ifndef CAMCAL_U8_PAIR
-#define CAMCAL_U8_PAIR 0
-#endif
-constexpr int kU8FramesPerStage = CAMCAL_U8_PAIR != 0 ? 2 : 1;
-static_assert(kU8FramesPerStage == 1 || kPosTrack, "pairs of frames need the frame counters (CAMCAL_POS_TRACK)");
-#ifndef CAMCAL_U8_BORDER
-#define CAMCAL_U8_BORDER 1
-#endif
-constexpr bool kBorderUnrolledU8 = CAMCAL_U8_BORDER != 0;
-constexpr int kU8Load = CAMCAL_U8_LOAD;
-constexpr bool kU8Bytes = CAMCAL_U8_LOAD == 1;      // rel[] is a byte address (no word alignment / selector)
-constexpr bool kU8Mixed = CAMCAL_U8_LOAD >= 3;   // words for line i2, bytes for (part of) line i2+1
 constexpr float kMagic23 = 8388608.0f;                 // 2^23: rint(v) in the low mantissa byte, low 24 bits of the pattern zero
 
 template <int OFF>
@@ -272,59 +214,22 @@ __device__ __forceinline__ void stcs_if(bool p, uint32_t* q, uint32_t v) {
 // the 12 tap bytes of one pixel as denormal-float bit patterns: [c] a00, [3+c] a10, [6+c] a01, [9+c] a11
 struct TapF { uint32_t m[12]; };
 
-// A0: shared address of tap (0,0) of source line i2 (byte address when kU8Load, else rounded down
-// to a word with `sel` funnelling the bytes); A1: the same on line i2+1
-__device__ __forceinline__ TapF load_taps(uint32_t A0, uint32_t A1, unsigned sel, uint32_t A1b = 0) {
+// A0: shared address of tap (0,0) of source line i2 rounded down to a word, `sel` funnelling its bytes;
+// A1b: byte address of tap (0,0) of line i2+1
+__device__ __forceinline__ TapF load_taps(uint32_t A0, unsigned sel, uint32_t A1b) {
     TapF t;
-    if (kU8Load == 1) {
-        t.m[0] = lds_u8_off<0>(A0); t.m[1] = lds_u8_off<1>(A0); t.m[2] = lds_u8_off<2>(A0);
-        t.m[3] = lds_u8_off<3>(A0); t.m[4] = lds_u8_off<4>(A0); t.m[5] = lds_u8_off<5>(A0);
-        t.m[6] = lds_u8_off<0>(A1); t.m[7] = lds_u8_off<1>(A1); t.m[8] = lds_u8_off<2>(A1);
-        t.m[9] = lds_u8_off<3>(A1); t.m[10] = lds_u8_off<4>(A1); t.m[11] = lds_u8_off<5>(A1);
-    } else if (kU8Load == 3) {
-        // source line i2: three aligned words + PRMT (ALU pipe); line i2+1: six LDS.U8 (load unit)
-        const Taps6 r0 = lds6w(A0, sel);
-        t.m[0] = __byte_perm(r0.lo, 0u, 0x4440); t.m[1] = __byte_perm(r0.lo, 0u, 0x4441); t.m[2] = __byte_perm(r0.lo, 0u, 0x4442);
-        t.m[3] = __byte_perm(r0.lo, 0u, 0x4443); t.m[4] = __byte_perm(r0.hi, 0u, 0x4440); t.m[5] = __byte_perm(r0.hi, 0u, 0x4441);
-        t.m[6] = lds_u8_off<0>(A1b); t.m[7] = lds_u8_off<1>(A1b); t.m[8] = lds_u8_off<2>(A1b);
-        t.m[9] = lds_u8_off<3>(A1b); t.m[10] = lds_u8_off<4>(A1b); t.m[11] = lds_u8_off<5>(A1b);
-    } else if (kU8Load == 5) {
-        // as 3, with half of line i2's bytes isolated on the FMA pipe (IDP.4A with a one-hot vector)
-        const Taps6 r0 = lds6w(A0, sel);
-        t.m[0] = __dp4a(r0.lo, 0x00000001u, 0u); t.m[1] = __byte_perm(r0.lo, 0u, 0x4441); t.m[2] = __dp4a(r0.lo, 0x00010000u, 0u);
-        t.m[3] = __byte_perm(r0.lo, 0u, 0x4443); t.m[4] = __dp4a(r0.hi, 0x00000001u, 0u); t.m[5] = __byte_perm(r0.hi, 0u, 0x4441);
-        t.m[6] = lds_u8_off<0>(A1b); t.m[7] = lds_u8_off<1>(A1b); t.m[8] = lds_u8_off<2>(A1b);
-        t.m[9] = lds_u8_off<3>(A1b); t.m[10] = lds_u8_off<4>(A1b); t.m[11] = lds_u8_off<5>(A1b);
-    } else if (kU8Load == 4) {
-        // as 3, but only tap a11 (three bytes) through LDS.U8; a01 from two aligned words
-        const Taps6 r0 = lds6w(A0, sel);
-        const uint32_t r1lo = prmt(lds_u32(A1), lds_u32_off<4>(A1), sel);
-        t.m[0] = __byte_perm(r0.lo, 0u, 0x4440); t.m[1] = __byte_perm(r0.lo, 0u, 0x4441); t.m[2] = __byte_perm(r0.lo, 0u, 0x4442);
-        t.m[3] = __byte_perm(r0.lo, 0u, 0x4443); t.m[4] = __byte_perm(r0.hi, 0u, 0x4440); t.m[5] = __byte_perm(r0.hi, 0u, 0x4441);
-        t.m[6] = __byte_perm(r1lo, 0u, 0x4440); t.m[7] = __byte_perm(r1lo, 0u, 0x4441); t.m[8] = __byte_perm(r1lo, 0u, 0x4442);
-        t.m[9] = lds_u8_off<3>(A1b); t.m[10] = lds_u8_off<4>(A1b); t.m[11] = lds_u8_off<5>(A1b);
-    } else if (kU8Load == 2) {
-        // half of the bytes isolated on the FMA pipe (IDP.4A with a one-hot byte vector), half with PRMT (ALU pipe)
-        const Taps6 r0 = lds6w(A0, sel), r1 = lds6w(A1, sel);
-        t.m[0] = __dp4a(r0.lo, 0x00000001u, 0u); t.m[1] = __byte_perm(r0.lo, 0u, 0x4441); t.m[2] = __dp4a(r0.lo, 0x00010000u, 0u);
-        t.m[3] = __byte_perm(r0.lo, 0u, 0x4443); t.m[4] = __dp4a(r0.hi, 0x00000001u, 0u); t.m[5] = __byte_perm(r0.hi, 0u, 0x4441);
-        t.m[6] = __dp4a(r1.lo, 0x00000001u, 0u); t.m[7] = __byte_perm(r1.lo, 0u, 0x4441); t.m[8] = __dp4a(r1.lo, 0x00010000u, 0u);
-        t.m[9] = __byte_perm(r1.lo, 0u, 0x4443); t.m[10] = __dp4a(r1.hi, 0x00000001u, 0u); t.m[11] = __byte_perm(r1.hi, 0u, 0x4441);
-    } else {
-        const Taps6 r0 = lds6w(A0, sel), r1 = lds6w(A1, sel);
-        t.m[0] = __byte_perm(r0.lo, 0u, 0x4440); t.m[1] = __byte_perm(r0.lo, 0u, 0x4441); t.m[2] = __byte_perm(r0.lo, 0u, 0x4442);
-        t.m[3] = __byte_perm(r0.lo, 0u, 0x4443); t.m[4] = __byte_perm(r0.hi, 0u, 0x4440); t.m[5] = __byte_perm(r0.hi, 0u, 0x4441);
-        t.m[6] = __byte_perm(r1.lo, 0u, 0x4440); t.m[7] = __byte_perm(r1.lo, 0u, 0x4441); t.m[8] = __byte_perm(r1.lo, 0u, 0x4442);
-        t.m[9] = __byte_perm(r1.lo, 0u, 0x4443); t.m[10] = __byte_perm(r1.hi, 0u, 0x4440); t.m[11] = __byte_perm(r1.hi, 0u, 0x4441);
-    }
+    const Taps6 r0 = lds6w(A0, sel);
+    t.m[0] = __byte_perm(r0.lo, 0u, 0x4440); t.m[1] = __byte_perm(r0.lo, 0u, 0x4441); t.m[2] = __byte_perm(r0.lo, 0u, 0x4442);
+    t.m[3] = __byte_perm(r0.lo, 0u, 0x4443); t.m[4] = __byte_perm(r0.hi, 0u, 0x4440); t.m[5] = __byte_perm(r0.hi, 0u, 0x4441);
+    t.m[6] = lds_u8_off<0>(A1b); t.m[7] = lds_u8_off<1>(A1b); t.m[8] = lds_u8_off<2>(A1b);
+    t.m[9] = lds_u8_off<3>(A1b); t.m[10] = lds_u8_off<4>(A1b); t.m[11] = lds_u8_off<5>(A1b);
     return t;
 }
 __device__ __forceinline__ float2 tap2(const TapF& p, const TapF& q, int k) {
     return make_float2(__uint_as_float(p.m[k]), __uint_as_float(q.m[k]));
 }
 
-// one channel of two pixels: scaled blend, rounding, and (CERT) the distance from the rounded value
-template <bool CERT>
+// one channel of two pixels: scaled blend, rounding, and the distance from the rounded value
 __device__ __forceinline__ float2 blend_ch2(const TapF& p, const TapF& q, int c, float2 w00, float2 w10,
                                             float2 w01, float2 w11, float2& dist) {
     float2 acc = mul2(w00, tap2(p, q, c));
@@ -332,7 +237,7 @@ __device__ __forceinline__ float2 blend_ch2(const TapF& p, const TapF& q, int c,
     acc = fma2(w01, tap2(p, q, 6 + c), acc);
     acc = fma2(w11, tap2(p, q, 9 + c), acc);
     const float2 f = fma2(acc, bc2(kTwo49), bc2(kMagic23));
-    if (CERT) dist = fma2(acc, bc2(-kTwo49), add2(f, bc2(-kMagic23)));       // rint(v) - v, exact
+    dist = fma2(acc, bc2(-kTwo49), add2(f, bc2(-kMagic23)));       // rint(v) - v, exact
     return f;
 }
 __device__ __forceinline__ uint32_t pack_rgb(float fr, float fg, float fb) {
@@ -341,17 +246,16 @@ __device__ __forceinline__ uint32_t pack_rgb(float fr, float fg, float fb) {
 }
 __device__ __forceinline__ float max_abs3(float a, float b, float c) { return fmaxf(fmaxf(fabsf(a), fabsf(b)), fabsf(c)); }
 
-// two pixels (lines e, e+1 of a lane): packed 0x..BBGGRR each; CERT: max |v - rint(v)| per pixel
-template <bool CERT>
+// two pixels (lines e, e+1 of a lane): packed 0x..BBGGRR each, and max |v - rint(v)| per pixel
 __device__ __forceinline__ void blend_px2(const TapF& p, const TapF& q, float2 w00, float2 w10, float2 w01,
                                           float2 w11, uint32_t& rgb_p, uint32_t& rgb_q, float2& dmax) {
     float2 dr, dg, db;
-    const float2 fr = blend_ch2<CERT>(p, q, 0, w00, w10, w01, w11, dr);
-    const float2 fg = blend_ch2<CERT>(p, q, 1, w00, w10, w01, w11, dg);
-    const float2 fb = blend_ch2<CERT>(p, q, 2, w00, w10, w01, w11, db);
+    const float2 fr = blend_ch2(p, q, 0, w00, w10, w01, w11, dr);
+    const float2 fg = blend_ch2(p, q, 1, w00, w10, w01, w11, dg);
+    const float2 fb = blend_ch2(p, q, 2, w00, w10, w01, w11, db);
     rgb_p = pack_rgb(fr.x, fg.x, fb.x);
     rgb_q = pack_rgb(fr.y, fg.y, fb.y);
-    if (CERT) dmax = make_float2(max_abs3(dr.x, dg.x, db.x), max_abs3(dr.y, dg.y, db.y));
+    dmax = make_float2(max_abs3(dr.x, dg.x, db.x), max_abs3(dr.y, dg.y, db.y));
 }
 
 // ---- FP32-coordinate (fast) variant: integer blend on the raw tap bytes -----------------------
@@ -364,10 +268,6 @@ __device__ __forceinline__ void blend_px2(const TapF& p, const TapF& q, float2 w
 // is two IDP.2A -- no byte is ever isolated.  Per pixel: 6 LDS + 7 PRMT + 6 IDP.2A + 2 PRMT (pack)
 // = 21 instructions against 28.5 of the FP32 formulation (9 loads, 8 PRMT, 7.5 FFMA2/FMUL2, 4 pack).
 // Weight quantisation: 4 * 255 * 2^-17 = 0.008 LSB (the fast variant's contract is +-1 LSB).
-#ifndef CAMCAL_U8_FAST_IDP
-#define CAMCAL_U8_FAST_IDP 1
-#endif
-constexpr bool kU8FastIdp = CAMCAL_U8_FAST_IDP != 0;
 
 __device__ __forceinline__ uint32_t blend_px_idp(const Taps6& u, const Taps6& v, uint32_t W0, uint32_t W1) {
     const uint32_t X0 = __byte_perm(u.lo, v.lo, 0x5140), X1 = __byte_perm(u.lo, v.lo, 0x7362);
@@ -411,10 +311,6 @@ __device__ __noinline__ uint32_t reblend_exact_u8(const RectExact* pe, const Rec
     return out;
 }
 
-// CAMCAL_U8_MAXNREG_FAST > 0: cap the FP32-coordinate variant with __maxnreg__ instead of a min-blocks bound
-#ifndef CAMCAL_U8_MAXNREG_FAST
-#define CAMCAL_U8_MAXNREG_FAST 0
-#endif
 // the kernel body (the __global__ wrappers are below).  VIEWS: frames with different views in one launch
 // (cc_rectify_u8c3_views) -- coordinate parameters and axes of the unit's view come from the view table in the
 // kernel's parameter space (vt; index = TileHdr.view)
@@ -427,8 +323,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
     constexpr int TL = kTLu;                      // lines per tile
     constexpr int LPW = TL / kWarps;              // lines per warp per tile = pixels per lane
     constexpr int NP = LPW / 2;                   // pairs of lines
-    constexpr int NF = kU8FramesPerStage;         // frames per ring stage
-    constexpr bool IDP = !EXACT && kU8FastIdp && !kU8Bytes;   // fast variant: integer blend on vertical byte pairs
+    constexpr bool IDP = !EXACT;                  // fast variant: integer blend on vertical byte pairs
     static_assert(LPW % 2 == 0 && LPW <= 16, "pairs of lines; masks are 16 bits");
     extern __shared__ __align__(128) uint8_t stage_mem[];
     __shared__ SmemRing ring;
@@ -437,7 +332,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
     ring_init(&ring, cfg.stages);
 
     if (warp == kWarps) {                              // ---- producer warp
-        producer_loop<EXACT, TL, 1, kU8FramesPerStage, VIEWS>(&tmap, g, cfg, plan, q2tab, sched, &ring, stage_mem, lane_id);
+        producer_loop<EXACT, TL, 1, 1, VIEWS>(&tmap, g, cfg, plan, q2tab, sched, &ring, stage_mem, lane_id);
         return;
     }
 
@@ -452,9 +347,9 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
     const int widx = lane_id - (lane_id >> 2);
 
     // the map of the current unit
-    uint32_t rel[LPW];                                 // tap (0,0) offset inside a stage (bytes; word-aligned when !kU8Load)
-    [[maybe_unused]] uint32_t selv[LPW];               // !kU8Load: PRMT selector that funnels the 6 tap bytes out of 3 words
-    [[maybe_unused]] uint32_t relb[LPW];               // kU8Mixed: the unrounded byte offset
+    uint32_t rel[LPW];                                 // tap (0,0) offset inside a stage, rounded down to a word
+    uint32_t selv[LPW];                                // PRMT selector that funnels the 6 tap bytes out of 3 words
+    uint32_t relb[LPW];                                // the unrounded byte offset
     float2 w00[NP], w10[NP], w01[NP], w11[NP];         // weights * 2^100, pairs of lines
     uint32_t m_staged = 0, m_fill = 0, m_skip = 0;
     bool all_staged = false;
@@ -468,18 +363,14 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
     [[maybe_unused]] uint32_t view = 0;
     for (;;) {
         mbar_wait(&ring.full[s], phase);
-        // CAMCAL_POS_TRACK: the slot is read on a unit's first frame only; frame index and frames left
-        // are carried in warp-uniform registers (declared uniform through a shuffle) -- no LDS + two
-        // dependent branches in front of every frame
-        if (!kPosTrack || frames_left == 0) {
+        // the slot is read on a unit's first frame only; frame index and frames left are carried in
+        // warp-uniform registers (declared uniform through a shuffle) -- no LDS + two dependent branches
+        // in front of every frame
+        if (frames_left == 0) {
             pos = ring.pos[s];
             if (pos.z < 0) break;
-            if (kPosTrack) {
-                frame_z = __shfl_sync(0xffffffffu, pos.z, 0);
-                frames_left = __shfl_sync(0xffffffffu, pos.w, 0);
-            } else {
-                frame_z = pos.z;
-            }
+            frame_z = __shfl_sync(0xffffffffu, pos.z, 0);
+            frames_left = __shfl_sync(0xffffffffu, pos.w, 0);
         } else {
             pos.w = 0;
         }
@@ -512,12 +403,12 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                     double row, col, d1, d2;
                     rect_coord_nobranch(pe, rtd, q2p[e], row, col);
                     uint32_t t1, t2, h1, h2;
-                    floor_index<kFloorMode1>(row, Mk1, t1, h1, d1);
-                    floor_index<kFloorMode2>(col, Mk2, t2, h2, d2);
+                    floor_index<kFloorFrnd>(row, Mk1, t1, h1, d1);
+                    floor_index<kFloorDaddRm>(col, Mk2, t2, h2, d2);
                     const bool st = (((h1 ^ 0x43300000u) | (h2 ^ 0x43300000u)) == 0u) & (t1 < R1) & (t2 < R2);
                     rel[e] = rel0 + t2 * box_pitch_b + t1 * 3u;
-                    if (kU8Mixed) relb[e] = rel[e];
-                    if (!kU8Bytes) { selv[e] = sel6(rel[e]); rel[e] &= ~3u; }   // stages are 128-byte aligned: (address & 3) == (rel & 3)
+                    relb[e] = rel[e];
+                    selv[e] = sel6(rel[e]); rel[e] &= ~3u;   // stages are 128-byte aligned: (address & 3) == (rel & 3)
                     const double e1 = 1.0 - d1, e2 = 1.0 - d2;
                     const float v00 = (float)((e1 * e2) * up), v10 = (float)((d1 * e2) * up);
                     const float v01 = (float)((e1 * d2) * up), v11 = (float)((d1 * d2) * up);
@@ -540,18 +431,11 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                     uint32_t t1[2], t2[2];
                     floor_bits_fast2(row, mk1, t1[0], t1[1], d1);
                     floor_bits_fast2(col, mk2, t2[0], t2[1], d2);
-                    if (kU8FastIdp) {                  // W0 / W1 of the two pixels live in w00 / w10 (bit patterns)
-                        uint32_t a0, a1, c0, c1;
-                        idp_weights(d1.x, d2.x, a0, a1);
-                        idp_weights(d1.y, d2.y, c0, c1);
-                        w00[hh] = make_float2(__uint_as_float(a0), __uint_as_float(c0));
-                        w10[hh] = make_float2(__uint_as_float(a1), __uint_as_float(c1));
-                    } else {
-                        const float2 e1 = sub2(bc2(1.0f), d1), e2 = mul2(sub2(bc2(1.0f), d2), bc2(kTwo100));
-                        const float2 d2s = mul2(d2, bc2(kTwo100));
-                        w00[hh] = mul2(e1, e2); w10[hh] = mul2(d1, e2);
-                        w01[hh] = mul2(e1, d2s); w11[hh] = mul2(d1, d2s);
-                    }
+                    uint32_t a0, a1, c0, c1;           // W0 / W1 of the two pixels live in w00 / w10 (bit patterns)
+                    idp_weights(d1.x, d2.x, a0, a1);
+                    idp_weights(d1.y, d2.y, c0, c1);
+                    w00[hh] = make_float2(__uint_as_float(a0), __uint_as_float(c0));
+                    w10[hh] = make_float2(__uint_as_float(a1), __uint_as_float(c1));
                     const float rr[2] = {row.x, row.y}, cc_[2] = {col.x, col.y};
 #pragma unroll
                     for (int j = 0; j < 2; ++j) {
@@ -559,8 +443,8 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                         const uint32_t l1 = t1[j] - (uint32_t)kMagicBits, l2 = t2[j] - (uint32_t)kMagicBits;
                         const bool st = (l1 < R1) & (l2 < R2);
                         rel[e] = rel0 + l2 * box_pitch_b + l1 * 3u;
-                        if (kU8Mixed) relb[e] = rel[e];
-                        if (!kU8Bytes) { selv[e] = sel6(rel[e]); rel[e] &= ~3u; }
+                        relb[e] = rel[e];
+                        selv[e] = sel6(rel[e]); rel[e] &= ~3u;
                         if (st) m_staged |= 1u << e;
                         if (!VIEWS) {
                             // (unconditional: four FSETPs cost less than a divergent branch here; measured)
@@ -590,16 +474,11 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
         }
 
         // ---- every frame of the unit: gather, blend, store
-        // NF == 2: the stage holds frames frame_z and frame_z + 1 (only one at the odd end of a unit); the
-        // frames of a stage go through the same code one after the other (rolled: the hot block is long)
-        const int nf_here = (NF == 2 && frames_left > 1) ? 2 : 1;
-#pragma unroll 1
-        for (int hf = 0; hf < nf_here; ++hf) {
-        const uint8_t* sframe = src + (long long)(frame_z + hf) * g.frame_stride * 3;
+        const uint8_t* sframe = src + (long long)frame_z * g.frame_stride * 3;
         // (a running output pointer, as in the f32c1 kernel, costs this one registers: ptxas goes from
         // 96 to 104 and the fast variant from 4 to 3 CTAs per SM -- measured 0.204 vs 0.194 ms on c3)
-        uint8_t* oline = dst + (long long)(frame_z + hf) * g.frame_stride * 3 + off0;
-        const uint32_t sbase = stage0 + (uint32_t)(s * NF + hf) * (uint32_t)cfg.box_bytes;
+        uint8_t* oline = dst + (long long)frame_z * g.frame_stride * 3 + off0;
+        const uint32_t sbase = stage0 + (uint32_t)s * (uint32_t)cfg.box_bytes;
         const uint32_t sbase1 = sbase + box_pitch_b;
         if (all_staged) {
             uint32_t* ow = reinterpret_cast<uint32_t*>(oline) + widx;
@@ -607,10 +486,10 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
 #pragma unroll
             for (int hh = 0; hh < NP; ++hh) {
                 const int e = 2 * hh;
-#ifdef CAMCAL_CHECK_BOUNDS      // debug builds: every tap byte of both lines inside the stage
+#ifdef CAMCAL_CHECK_BOUNDS      // the chk build (Makefile): every tap byte of both lines inside the stage
                 for (int j = 0; j < 2; ++j) {
                     const uint32_t o = sbase + rel[e + j];
-                    if (o < sbase || o + box_pitch_b + (kU8Bytes ? 6u : 12u) > sbase + (uint32_t)cfg.box_bytes + 4u || (!kU8Bytes && (o & 3u))) __trap();
+                    if (o < sbase || o + box_pitch_b + 12u > sbase + (uint32_t)cfg.box_bytes + 4u || (o & 3u)) __trap();
                 }
 #endif
                 uint32_t rgb_p, rgb_q;
@@ -620,22 +499,13 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                     rgb_p = blend_px_idp(pu, pv, __float_as_uint(w00[hh].x), __float_as_uint(w10[hh].x));
                     rgb_q = blend_px_idp(qu, qv, __float_as_uint(w00[hh].y), __float_as_uint(w10[hh].y));
                 } else {
-                const TapF tp = load_taps(sbase + rel[e], sbase1 + rel[e], kU8Bytes ? 0u : selv[e], kU8Mixed ? sbase1 + relb[e] : 0u);
-                const TapF tq = load_taps(sbase + rel[e + 1], sbase1 + rel[e + 1], kU8Bytes ? 0u : selv[e + 1], kU8Mixed ? sbase1 + relb[e + 1] : 0u);
-#if CAMCAL_U8_DEBUG == 1        // tuning only: no unpack / blend (pipeline + store floor)
-                rgb_p = tp.m[0] ^ tp.m[7]; rgb_q = tq.m[0] ^ tq.m[7];
-                if (EXACT) dm[hh] = make_float2(0.f, 0.f);
-#else
-                blend_px2<EXACT>(tp, tq, w00[hh], w10[hh], w01[hh], w11[hh], rgb_p, rgb_q, dm[hh]);
-#endif
+                    const TapF tp = load_taps(sbase + rel[e], selv[e], sbase1 + relb[e]);
+                    const TapF tq = load_taps(sbase + rel[e + 1], selv[e + 1], sbase1 + relb[e + 1]);
+                    blend_px2(tp, tq, w00[hh], w10[hh], w01[hh], w11[hh], rgb_p, rgb_q, dm[hh]);
                 }
                 const uint32_t np_ = __shfl_down_sync(0xffffffffu, rgb_p, 1);
                 const uint32_t nq_ = __shfl_down_sync(0xffffffffu, rgb_q, 1);
-#if CAMCAL_U8_DEBUG == 2        // tuning only: compute everything, (almost) never store
-                const bool st_ok = (lq != 3) & (rgb_p == 0x12345678u);
-#else
                 const bool st_ok = lq != 3;
-#endif
                 stcs_if(st_ok, ow, __byte_perm(rgb_p, np_, wsel));
                 stcs_if(st_ok, reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(ow) + pitch3), __byte_perm(rgb_q, nq_, wsel));
                 ow = reinterpret_cast<uint32_t*>(reinterpret_cast<uint8_t*>(ow) + 2 * pitch3);
@@ -652,7 +522,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                         for (int j = 0; j < 2; ++j) {
                             const int e = 2 * hh + j;
                             if ((j ? dm[hh].y : dm[hh].x) > kCertThr) {
-                                const uint32_t bo = rel[e] + (kU8Bytes ? 0u : (selv[e] & 3u));
+                                const uint32_t bo = rel[e] + (selv[e] & 3u);
                                 store_rgb(oline + (long long)e * pitch3 + lane_id * 3,
                                           reblend_exact_u8(&pe, &gv, a, b0 + e, sbase + bo, sbase1 + bo));
                             }
@@ -660,31 +530,31 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                     }
                 }
             }
-        } else if (kBorderUnrolledU8) {
+        } else {
             // border tiles: staged and fill pixels unrolled over the map (static indices), byte stores;
-            // then one rolled pass for the generic remainder (it needs no map entry).  The rolled
-            // compare-chain loop below cost ~100 instructions per pixel.
+            // then one rolled pass for the generic remainder (it needs no map entry).  A rolled loop that
+            // selects the map entry through a compare chain costs ~100 instructions per pixel.
             uint8_t* o = oline + lane_id * 3;
 #pragma unroll
             for (int e = 0; e < LPW; ++e, o += pitch3) {
                 const uint32_t bit = 1u << e;
                 if (m_skip & bit) continue;
                 if (m_staged & bit) {
-                    const uint32_t sel = kU8Bytes ? 0u : selv[e];
+                    const uint32_t sel = selv[e];
                     if (IDP) {
                         store_rgb(o, blend_px_idp(lds6w(sbase + rel[e], sel), lds6w(sbase1 + rel[e], sel),
                                                   __float_as_uint((e & 1) ? w00[e / 2].y : w00[e / 2].x),
                                                   __float_as_uint((e & 1) ? w10[e / 2].y : w10[e / 2].x)));
                         continue;
                     }
-                    const TapF t = load_taps(sbase + rel[e], sbase1 + rel[e], sel, kU8Mixed ? sbase1 + relb[e] : 0u);
+                    const TapF t = load_taps(sbase + rel[e], sel, sbase1 + relb[e]);
                     const float f00 = (e & 1) ? w00[e / 2].y : w00[e / 2].x, f10 = (e & 1) ? w10[e / 2].y : w10[e / 2].x;
                     const float f01 = (e & 1) ? w01[e / 2].y : w01[e / 2].x, f11 = (e & 1) ? w11[e / 2].y : w11[e / 2].x;
                     uint32_t v, vq;
                     float2 dm1;
-                    blend_px2<EXACT>(t, t, bc2(f00), bc2(f10), bc2(f01), bc2(f11), v, vq, dm1);
+                    blend_px2(t, t, bc2(f00), bc2(f10), bc2(f01), bc2(f11), v, vq, dm1);
                     if (EXACT && dm1.x > kCertThr) {
-                        const uint32_t bo = rel[e] + (kU8Bytes ? 0u : (sel & 3u));
+                        const uint32_t bo = rel[e] + (sel & 3u);
                         v = reblend_exact_u8(&pe, &gv, a, b0 + e, sbase + bo, sbase1 + bo);
                     }
                     store_rgb(o, v);
@@ -703,63 +573,16 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                     if ((m_gen >> e) & 1u)
                         store_rgb(og, sample_direct_u8<EXACT>(pe, pf, rtd, rtf, gv, sframe, pitch3, frame_bytes, b0 + e, fill));
             }
-        } else {
-            // border tiles: per-pixel class, byte stores
-            uint8_t* o = oline + lane_id * 3;
-#pragma unroll 1
-            for (int e = 0; e < LPW; ++e, o += pitch3) {
-                if ((m_skip >> e) & 1u) continue;
-                uint32_t v;
-                if ((m_staged >> e) & 1u) {
-                    uint32_t r = 0, sel = 0;
-                    float f00 = 0, f10 = 0, f01 = 0, f11 = 0;
-#pragma unroll
-                    for (int j = 0; j < LPW; ++j)
-                        if (j == e) {
-                            r = rel[j];
-                            if (!kU8Bytes) sel = selv[j];
-                            f00 = (j & 1) ? w00[j / 2].y : w00[j / 2].x; f10 = (j & 1) ? w10[j / 2].y : w10[j / 2].x;
-                            f01 = (j & 1) ? w01[j / 2].y : w01[j / 2].x; f11 = (j & 1) ? w11[j / 2].y : w11[j / 2].x;
-                        }
-                    if (IDP) {
-                        v = blend_px_idp(lds6w(sbase + r, sel), lds6w(sbase1 + r, sel), __float_as_uint(f00), __float_as_uint(f10));
-                        store_rgb(o, v);
-                        continue;
-                    }
-                    const TapF t = load_taps(sbase + r, sbase1 + r, sel, sbase1 + r + (sel & 3u));
-                    uint32_t vq;
-                    float2 dm1;
-                    blend_px2<EXACT>(t, t, bc2(f00), bc2(f10), bc2(f01), bc2(f11), v, vq, dm1);
-                    if (EXACT && dm1.x > kCertThr) {
-                        const uint32_t bo = r + (kU8Bytes ? 0u : (sel & 3u));
-                        v = reblend_exact_u8(&pe, &gv, a, b0 + e, sbase + bo, sbase1 + bo);
-                    }
-                } else if ((m_fill >> e) & 1u) {
-                    v = fill;
-                } else {
-                    RowTermD rtd;
-                    RowTermF rtf;
-                    if (EXACT) rtd = rect_row_term(pe, gv.axs0 + a); else rtf = rect_row_term(pf, gv.axs0 + a);
-                    v = sample_direct_u8<EXACT>(pe, pf, rtd, rtf, gv, sframe, pitch3, frame_bytes, b0 + e, fill);
-                }
-                store_rgb(o, v);
-            }
         }
-        }   // frames of the stage
         __syncwarp();
-        if (kElectArrive ? elect_one() : lane_id == 0) mbar_arrive(&ring.empty[s]);
-        if (kPosTrack) { frames_left = max(frames_left - NF, 0); frame_z += NF; }
+        if (elect_one()) mbar_arrive(&ring.empty[s]);
+        frames_left = max(frames_left - 1, 0); ++frame_z;
         if (++s == cfg.stages) { s = 0; phase ^= 1; }
     }
 }
 
-#if CAMCAL_U8_MAXNREG_FAST > 0
-#define CAMCAL_U8_KERNEL_ATTR(EXACT) __launch_bounds__(kConsumerThreads + 32) __maxnreg__(EXACT ? 65536 / ((kConsumerThreads + 32) * kMinBlocksU8Exact) / 8 * 8 : CAMCAL_U8_MAXNREG_FAST)
-#else
-#define CAMCAL_U8_KERNEL_ATTR(EXACT) __launch_bounds__(kConsumerThreads + 32, EXACT ? kMinBlocksU8Exact : kMinBlocksU8)
-#endif
 template <bool EXACT>
-__global__ void CAMCAL_U8_KERNEL_ATTR(EXACT)
+__global__ void __launch_bounds__(kConsumerThreads + 32, EXACT ? kMinBlocksU8Exact : kMinBlocksU8)
 rectify_u8c3_kernel(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ RectExact pe,
                     const __grid_constant__ RectFast pf, const __grid_constant__ RectGeom g,
                     const __grid_constant__ TileCfg cfg, const TileHdr* __restrict__ plan,

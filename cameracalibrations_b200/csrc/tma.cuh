@@ -62,37 +62,19 @@ __device__ __forceinline__ void mbar_wait_parked(uint64_t* bar, uint32_t parity)
     while (!mbar_try_wait_hint(bar, parity, HINT_NS)) {}
 }
 // Polling costs issue slots that other CTAs on the SM could use: back off between probes.
-#ifndef CAMCAL_WAIT_SLEEP
-#define CAMCAL_WAIT_SLEEP 256
-#endif
-template <int SLEEP_NS = CAMCAL_WAIT_SLEEP>
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     if (mbar_try_wait(bar, parity)) return;
-    while (!mbar_try_wait(bar, parity)) {
-        if (SLEEP_NS > 0) __nanosleep(SLEEP_NS);
-    }
+    while (!mbar_try_wait(bar, parity)) __nanosleep(256);
 }
 
-// 3-D tiled tensor load global -> shared, completion signalled on an mbarrier
-__device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* map, uint64_t* bar,
-                                            int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes"
-        " [%0], [%1, {%3, %4, %5}], [%2];"
-        :: "r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)),
-           "r"(c0), "r"(c1), "r"(c2)
-        : "memory");
-}
-// the same with an L2 eviction-priority hint (createpolicy): the source lines of a staged box are
+// L2 eviction-priority policy for the staged boxes (createpolicy): the source lines of a box are
 // wanted again by the neighbouring tiles (halo) within microseconds, the output never is
-template <int POLICY>   // 1: evict_last, 2: evict_first, 3: evict_normal via an explicit policy
-__device__ __forceinline__ uint64_t l2_policy() {
+__device__ __forceinline__ uint64_t l2_evict_last() {
     uint64_t pol;
-    if (POLICY == 1) asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-    else if (POLICY == 2) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-    else asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol));
+    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
     return pol;
 }
+// 3-D tiled tensor load global -> shared with an L2 cache policy, completion signalled on an mbarrier
 __device__ __forceinline__ void tma_load_3d_hint(void* smem_dst, const CUtensorMap* map, uint64_t* bar,
                                                  int c0, int c1, int c2, uint64_t policy) {
     asm volatile(

@@ -1,6 +1,6 @@
 """Device-resident kernel timing of the rectification workloads (tuning loop; bench.py is the
 judged measurement).   python profiles/ktime.py [c2|c3] [f64|f32] [auto|tma|direct] [steps]
-Honors CAMCAL_B200_LIB (variant builds), CAMCAL_TPS, CAMCAL_STAGES."""
+Honors CAMCAL_B200_LIB (another build of the library, e.g. the parent commit's for an A/B)."""
 import os, sys
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import torch

@@ -1,6 +1,6 @@
 """Where the time of cc_rectify_f32c1_views goes: 64 x 1080p frames, 64 different views, one call.
-Per setting: host enqueue time (wall clock of the call, no synchronisation) against the device time
-(CUDA events), for the CTAs-per-SM cap of each launch (CAMCAL_CTAS_PER_SM, read per call)."""
+Per coordinate type: host enqueue time (wall clock of the call, no synchronisation) against the device
+time (CUDA events)."""
 import os, sys, time
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
 import numpy as np
@@ -50,15 +50,9 @@ torch.cuda.synchronize()
 print(f"cold call, 64 new views x 1080p: {(time.perf_counter() - t0) * 1e3:.2f} ms", flush=True)
 SHORT = len(sys.argv) > 1 and sys.argv[1] == "short"
 for coord in ("f32", "f64"):
-    for cap in (("",) if SHORT else ("", "1", "2")):
-        if cap:
-            os.environ["CAMCAL_CTAS_PER_SM"] = cap
-        else:
-            os.environ.pop("CAMCAL_CTAS_PER_SM", None)
-        ms, host_ms = run(coord)
-        print(f"views 64x1080p {coord} ctas/SM cap {cap or 'none':4s}: device {ms:.4f} ms  host enqueue {host_ms:.4f} ms  "
-              f"frac {8 * npx / (ms * 1e-3) / 1e9 / peak:.3f}", flush=True)
-os.environ.pop("CAMCAL_CTAS_PER_SM", None)
+    ms, host_ms = run(coord)
+    print(f"views 64x1080p {coord}: device {ms:.4f} ms  host enqueue {host_ms:.4f} ms  "
+          f"frac {8 * npx / (ms * 1e-3) / 1e9 / peak:.3f}", flush=True)
 if SHORT:
     sys.exit(0)
 # the same 64 frames with ONE view (map shared by the frames of a unit) and as 64 single-frame calls of one view

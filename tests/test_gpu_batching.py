@@ -30,7 +30,7 @@ pytestmark = pytest.mark.gpu
 
 F_FILL, F_SENT, F_SENT_ALONE = -3.0, -777.0, -555.0
 U_FILL, U_SENT, U_SENT_ALONE = (9, 8, 7), (201, 202, 203), (101, 102, 103)
-# most frames per group, rectify.cu (CAMCAL_FG_*): (pixel format, coordinates) -> fg_max
+# most frames per group, rectify.cu (kFGf32Exact, kFGf32Fast, kFGu8Exact, kFGu8Fast): (pixel format, coordinates) -> fg_max
 FG_MAX = {("f32", "f64"): 12, ("f32", "f32"): 4, ("u8", "f64"): 16, ("u8", "f32"): 16}
 TILE = 32                     # output tile: 32 x 32 pixels, both pixel formats
 
