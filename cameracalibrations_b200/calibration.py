@@ -15,6 +15,7 @@ Every numeric result comes from the CUDA kernels; there is no Python/numpy fallb
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import json
 import math
 import re
@@ -45,6 +46,37 @@ def _np_ptr(a: np.ndarray):
 
 def _t_ptr(t):
     return C.c_void_p(t.data_ptr())
+
+
+def _device(t) -> int:
+    """The device of a CUDA tensor."""
+    return t.device.index if t.device.index is not None else torch.cuda.current_device()
+
+
+def _where(x):
+    """(context, pointer of an array, entry point suffix, stream argument) of a call on x: a CUDA tensor runs on
+    its own device, on torch's current stream there; a numpy array takes the `_host` entry point on the default
+    device."""
+    if _is_torch(x):
+        dev = _device(x)
+        return _lib.context(dev), _t_ptr, "", (_stream_ptr(dev),)
+    return _lib.context(_default_device()), _np_ptr, "_host", ()
+
+
+def _check_points(t) -> None:
+    if not t.is_cuda:
+        raise TypeError("torch inputs must be CUDA tensors (numpy arrays take the host path)")
+    if t.dtype not in (torch.float32, torch.float64):
+        raise TypeError("float32 or float64 points only")
+
+
+def _points(pts):
+    """Interleaved points as the point maps take them: a tensor as it is, anything else as a numpy array that
+    stays float32 or becomes float64."""
+    if _is_torch(pts):
+        return pts
+    pts = np.asarray(pts)
+    return pts if pts.dtype in (np.float32, np.float64) else pts.astype(np.float64)
 
 
 class Calibration:
@@ -90,13 +122,13 @@ class Calibration:
         """(c::Calibration)(i::RowCol, idx), src/meta.jl:82; want_z=False is
         rectification(c, idx), src/meta.jl:99."""
         vi = self._index(extrinsic)
-        return _point_call("img2world", self, vi, (row, col), 3 if want_z else 2, want_z)
+        return _point_call("img2world", self, vi, (row, col), 3 if want_z else 2)
 
     def world2img(self, x, y, z=None, extrinsic=None):
         """(c::Calibration)(xyz::XYZ, idx), src/meta.jl:88; z=None means z = 0."""
         vi = self._index(extrinsic)
         ins = (x, y) if z is None else (x, y, z)
-        return _point_call("world2img", self, vi, ins, 2, z is not None)
+        return _point_call("world2img", self, vi, ins, 2)
 
     # -- points of many views in one call: c.(pts_v, v) over views v ----------------
     def img2world_views(self, row, col, extrinsics, counts, want_z: bool = True):
@@ -104,13 +136,12 @@ class Calibration:
         [sum(counts[:s]), sum(counts[:s+1])) use extrinsics[s] (view indices or file names, as
         warp_views takes them).  One call (one launch for CUDA tensors); every point's result is
         bit-identical to img2world with its segment's view."""
-        return _point_call("img2world", self, self._segments(extrinsics, counts), (row, col),
-                           3 if want_z else 2, want_z)
+        return _point_call("img2world", self, self._segments(extrinsics, counts), (row, col), 3 if want_z else 2)
 
     def world2img_views(self, x, y, z, extrinsics, counts):
         """World -> pixel over segments of views, as img2world_views; z=None means z = 0."""
         ins = (x, y) if z is None else (x, y, z)
-        return _point_call("world2img", self, self._segments(extrinsics, counts), ins, 2, z is not None)
+        return _point_call("world2img", self, self._segments(extrinsics, counts), ins, 2)
 
     def _segments(self, extrinsics, counts):
         """(views, nviews, offsets) of cc_*_views as numpy arrays: cc_view rows [rvec | tvec] and size_t
@@ -134,10 +165,7 @@ class Calibration:
     def __call__(self, pts, extrinsic=None):
         if isinstance(extrinsic, (list, tuple)):
             return self._call_views(pts, extrinsic)
-        if not _is_torch(pts):
-            pts = np.asarray(pts)
-            if pts.dtype not in (np.float32, np.float64):
-                pts = pts.astype(np.float64)
+        pts = _points(pts)
         if pts.shape[-1] == 2:
             return _aos_call("img2world", self, self._index(extrinsic), pts, 3)
         if pts.shape[-1] == 3:
@@ -173,10 +201,7 @@ def rectification(c: Calibration, extrinsic=None):
     vi = c._index(extrinsic)
 
     def f(rc):
-        if not _is_torch(rc):
-            rc = np.asarray(rc)
-            if rc.dtype != np.float32:
-                rc = rc.astype(np.float64, copy=False)
+        rc = _points(rc)
         if rc.shape[-1] != 2:                  # (row, col) are the first two coordinates
             rc = rc[..., :2]
             if rc.shape[-1] != 2:
@@ -194,80 +219,49 @@ def _aos_call(kind, c: Calibration, vi, pts, out_dim: int):
     views = (_np_ptr(vi[0]), vi[1], _np_ptr(vi[2])) if segs else (C.byref(c._views[vi]), 1, None)
     lead, in_dim = tuple(pts.shape[:-1]), int(pts.shape[-1])
     if _is_torch(pts):
-        if not pts.is_cuda:
-            raise TypeError("torch inputs must be CUDA tensors (numpy arrays take the host path)")
-        if pts.dtype not in (torch.float32, torch.float64):
-            raise TypeError("float32 or float64 points only")
+        _check_points(pts)
         pts = pts.contiguous()
         out = torch.empty(lead + (out_dim,), dtype=pts.dtype, device=pts.device)
-        dev = pts.device.index if pts.device.index is not None else torch.cuda.current_device()
-        ctx, ptr, host, tail = _lib.context(dev), _t_ptr, "", (_stream_ptr(dev),)
-        sfx = "f64" if pts.dtype == torch.float64 else "f32"
     else:
         pts = np.ascontiguousarray(pts, dtype=np.float32 if pts.dtype == np.float32 else np.float64)
         out = np.empty(lead + (out_dim,), dtype=pts.dtype)
-        ctx, ptr, host, tail = _lib.context(_default_device()), _np_ptr, "_host", ()
-        sfx = "f64" if pts.dtype == np.float64 else "f32"
+    ctx, ptr, host, tail = _where(pts)
     n = math.prod(lead)
     _check_total(vi, n, segs)
-    fn = getattr(lib, f"cc_{kind}_{sfx}_aos{host}")
+    fn = getattr(lib, f"cc_{kind}_{'f32' if pts.itemsize == 4 else 'f64'}_aos{host}")
     io = (ptr(pts), ptr(out), out_dim) if kind == "img2world" else (ptr(pts), in_dim, ptr(out))
     check(fn(ctx.handle, C.byref(c._intr), *views, *io, C.c_size_t(n), *tail))
     return out
 
 
-def _point_call(kind, c: Calibration, vi, ins, nout: int, flag: bool):
+def _point_call(kind, c: Calibration, vi, ins, nout: int):
     """kind: img2world (ins=row,col; outs x,y[,z]) or world2img (ins=x,y[,z]; outs row,col).
     vi: a view index, or the (views, nviews, offsets) of Calibration._segments for cc_*_views."""
-    first = ins[0]
     segs = isinstance(vi, tuple)     # the views form takes its point count from the offsets
-    head = (C.byref(c._intr),) + ((_np_ptr(vi[0]), vi[1], _np_ptr(vi[2])) if segs else (C.byref(c._views[vi]),))
-    sfx_v = "_views" if segs else ""
+    views = (_np_ptr(vi[0]), vi[1], _np_ptr(vi[2])) if segs else (C.byref(c._views[vi]),)
+    first = ins[0]
     if _is_torch(first):
-        if not first.is_cuda:
-            raise TypeError("torch inputs must be CUDA tensors (numpy arrays take the host path)")
-        dt = first.dtype
-        if dt not in (torch.float32, torch.float64):
-            raise TypeError("float32 or float64 points only")
+        _check_points(first)
         ins = [t.contiguous() for t in ins]
         n = ins[0].numel()
-        for t in ins:
-            if t.dtype != dt or t.numel() != n or t.device != first.device:
-                raise ValueError("coordinate arrays must share dtype, length and device")
-        outs = [torch.empty(n, dtype=dt, device=first.device) for _ in range(nout)]
-        dev = first.device.index if first.device.index is not None else torch.cuda.current_device()
-        ctx = _lib.context(dev)
-        sfx = "f64" if dt == torch.float64 else "f32"
-        fn = getattr(lib, f"cc_{kind}_{sfx}{sfx_v}")
-        if kind == "img2world":
-            args = [_t_ptr(ins[0]), _t_ptr(ins[1]), _t_ptr(outs[0]), _t_ptr(outs[1]),
-                    _t_ptr(outs[2]) if flag else None]
-        else:
-            args = [_t_ptr(ins[0]), _t_ptr(ins[1]), _t_ptr(ins[2]) if flag else None,
-                    _t_ptr(outs[0]), _t_ptr(outs[1])]
-        _check_total(vi, n, segs)
-        check(fn(ctx.handle, *head, *args, *(() if segs else (C.c_size_t(n),)), _stream_ptr(dev)))
-        return tuple(outs)
-    # host path
-    arrs = [np.asarray(a) for a in ins]
-    dt = np.float32 if arrs[0].dtype == np.float32 else np.float64
-    arrs = [np.ascontiguousarray(a, dtype=dt).reshape(-1) for a in arrs]
-    n = arrs[0].size
-    for a in arrs:
-        if a.size != n:
-            raise ValueError("coordinate arrays must have the same length")
-    outs = [np.empty(n, dtype=dt) for _ in range(nout)]
-    ctx = _lib.context(_default_device())
-    sfx = "f64" if dt == np.float64 else "f32"
-    fn = getattr(lib, f"cc_{kind}_{sfx}{sfx_v}_host")
-    if kind == "img2world":
-        args = [_np_ptr(arrs[0]), _np_ptr(arrs[1]), _np_ptr(outs[0]), _np_ptr(outs[1]),
-                _np_ptr(outs[2]) if flag else None]
+        if any(t.dtype != first.dtype or t.numel() != n or t.device != first.device for t in ins):
+            raise ValueError("coordinate arrays must share dtype, length and device")
+        outs = [torch.empty(n, dtype=first.dtype, device=first.device) for _ in range(nout)]
     else:
-        args = [_np_ptr(arrs[0]), _np_ptr(arrs[1]), _np_ptr(arrs[2]) if flag else None,
-                _np_ptr(outs[0]), _np_ptr(outs[1])]
+        dt = np.float32 if np.asarray(first).dtype == np.float32 else np.float64
+        ins = [np.ascontiguousarray(a, dtype=dt).reshape(-1) for a in ins]
+        n = ins[0].size
+        if any(a.size != n for a in ins):
+            raise ValueError("coordinate arrays must have the same length")
+        outs = [np.empty(n, dtype=dt) for _ in range(nout)]
+    ctx, ptr, host, tail = _where(ins[0])
     _check_total(vi, n, segs)
-    check(fn(ctx.handle, *head, *args, *(() if segs else (C.c_size_t(n),))))
+    fn = getattr(lib, f"cc_{kind}_{'f32' if ins[0].itemsize == 4 else 'f64'}{'_views' if segs else ''}{host}")
+
+    def slots(arrs, k):              # a missing z is a NULL pointer
+        return [ptr(a) for a in arrs] + [None] * (k - len(arrs))
+    io = slots(ins, 2) + slots(outs, 3) if kind == "img2world" else slots(ins, 3) + slots(outs, 2)
+    check(fn(ctx.handle, C.byref(c._intr), *views, *io, *(() if segs else (C.c_size_t(n),)), *tail))
     return tuple(outs)
 
 
@@ -322,6 +316,34 @@ def image_transformations(c: Calibration, extrinsic_index, imgpointss, checker_s
     return ratio, get_axes(ratio, checker_size, n_corners, sz)
 
 
+def _frames(frames, fill, coord: str, gather: str, out, single: bool):
+    """What warp and warp_views share: the frames as the library reads them, C-contiguous (a numpy array that is
+    not uint8 becomes float32), whether they are uint8 RGB, the output buffer, the fill value and the flags.
+    single: a frame without the leading axis is a batch of one, and the last value returned says so."""
+    flags = {"f64": _lib.COORD_F64, "f32": _lib.COORD_F32}[coord] | {
+        "auto": _lib.GATHER_AUTO, "direct": _lib.GATHER_DIRECT, "tma": _lib.GATHER_TMA}[gather]
+    if _is_torch(frames):
+        if not frames.is_cuda:
+            raise TypeError("torch frames must be CUDA tensors (numpy arrays take the host path)")
+        u8 = frames.dtype == torch.uint8
+        frames = frames.contiguous()
+    else:
+        u8 = np.asarray(frames).dtype == np.uint8
+        frames = np.ascontiguousarray(frames, dtype=np.uint8 if u8 else np.float32)
+    one = single and frames.ndim == (3 if u8 else 2)
+    if one:
+        frames = frames.reshape((1,) + tuple(frames.shape))
+    if frames.ndim != (4 if u8 else 3) or (u8 and frames.shape[-1] != 3):
+        raise ValueError("frames must be (nframes, sz2, sz1) float32 or (nframes, sz2, sz1, 3) uint8")
+    if out is None:
+        out = torch.empty_like(frames) if _is_torch(frames) else np.empty_like(frames)
+    if u8:
+        fv = (C.c_uint8 * 3)(*([0, 0, 0] if fill is None else [int(v) for v in fill]))
+    else:
+        fv = C.c_float(float("nan") if fill is None else float(fill))
+    return frames, u8, out, fv, flags, one
+
+
 def warp(c: Calibration, extrinsic, frames, ratio: float, axs_min, fill=None, coord: str = "f64",
          gather: str = "auto", out=None):
     """warp(img, tform, axs), src/plot_calibration.jl:40, for a batch of frames of one view.
@@ -333,42 +355,14 @@ def warp(c: Calibration, extrinsic, frames, ratio: float, axs_min, fill=None, co
     coord: "f64" (reference precision, bit-exact index/weight selection) | "f32" (fast path).
     """
     vi = c._index(extrinsic)
-    flags = {"f64": _lib.COORD_F64, "f32": _lib.COORD_F32}[coord] | {
-        "auto": _lib.GATHER_AUTO, "direct": _lib.GATHER_DIRECT, "tma": _lib.GATHER_TMA}[gather]
-    is_t = _is_torch(frames)
-    u8 = (frames.dtype == torch.uint8) if is_t else (np.asarray(frames).dtype == np.uint8)
-    base_nd = 3 if u8 else 2
-    if not is_t:
-        frames = np.ascontiguousarray(frames, dtype=np.uint8 if u8 else np.float32)
-    elif not frames.is_contiguous():
-        frames = frames.contiguous()
-    squeeze = frames.ndim == base_nd
-    f4 = frames.reshape((1,) + tuple(frames.shape)) if squeeze else frames
-    if f4.ndim != base_nd + 1 or (u8 and f4.shape[-1] != 3):
-        raise ValueError("frames must be (nframes, sz2, sz1) float32 or (nframes, sz2, sz1, 3) uint8")
-    nframes, sz2, sz1 = int(f4.shape[0]), int(f4.shape[1]), int(f4.shape[2])
+    frames, u8, out, fv, flags, one = _frames(frames, fill, coord, gather, out, single=True)
+    nframes, sz2, sz1 = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
     axs = (C.c_int64 * 2)(int(axs_min[0]), int(axs_min[1]))
-    intr, view = C.byref(c._intr), C.byref(c._views[vi])
-    if out is None:
-        out = torch.empty_like(f4) if is_t else np.empty_like(f4)
-    geom = (sz1, sz2, C.c_size_t(sz1), C.c_size_t(sz1 * sz2), nframes)
-    if u8:
-        fv = (C.c_uint8 * 3)(*([0, 0, 0] if fill is None else [int(v) for v in fill]))
-    else:
-        fv = C.c_float(float("nan") if fill is None else float(fill))
-    if is_t:
-        if not f4.is_cuda:
-            raise TypeError("torch frames must be CUDA tensors (numpy arrays take the host path)")
-        dev = f4.device.index if f4.device.index is not None else torch.cuda.current_device()
-        ctx = _lib.context(dev)
-        fn = lib.cc_rectify_u8c3 if u8 else lib.cc_rectify_f32c1
-        check(fn(ctx.handle, intr, view, float(ratio), axs, _t_ptr(f4), _t_ptr(out), *geom, fv, flags,
-                 _stream_ptr(dev)))
-    else:
-        ctx = _lib.context(_default_device())
-        fn = lib.cc_rectify_u8c3_host if u8 else lib.cc_rectify_f32c1_host
-        check(fn(ctx.handle, intr, view, float(ratio), axs, _np_ptr(f4), _np_ptr(out), *geom, fv, flags))
-    return out[0] if squeeze else out
+    ctx, ptr, host, tail = _where(frames)
+    fn = getattr(lib, f"cc_rectify_{'u8c3' if u8 else 'f32c1'}{host}")
+    check(fn(ctx.handle, C.byref(c._intr), C.byref(c._views[vi]), float(ratio), axs, ptr(frames), ptr(out),
+             sz1, sz2, C.c_size_t(sz1), C.c_size_t(sz1 * sz2), nframes, fv, flags, *tail))
+    return out[0] if one else out
 
 
 def warp_views(c: Calibration, extrinsics, frames, ratios, axs_mins, fill=None, coord: str = "f64",
@@ -382,39 +376,18 @@ def warp_views(c: Calibration, extrinsics, frames, ratios, axs_mins, fill=None, 
     array takes the host pipeline over all views in one call (cc_rectify_views_*_host) and returns numpy."""
     vis = [c._index(e) for e in extrinsics]
     nv = len(vis)
-    flags = {"f64": _lib.COORD_F64, "f32": _lib.COORD_F32}[coord] | {
-        "auto": _lib.GATHER_AUTO, "direct": _lib.GATHER_DIRECT, "tma": _lib.GATHER_TMA}[gather]
-    is_t = _is_torch(frames)
-    if is_t and not frames.is_cuda:
-        raise TypeError("warp_views takes CUDA tensors or numpy arrays")
-    if is_t:
-        u8 = frames.dtype == torch.uint8
-        frames = frames.contiguous()
-    else:
-        u8 = np.asarray(frames).dtype == np.uint8
-        frames = np.ascontiguousarray(frames, dtype=np.uint8 if u8 else np.float32)
-    if frames.ndim != (4 if u8 else 3) or (u8 and frames.shape[-1] != 3) or nv == 0 or frames.shape[0] % nv:
+    frames, u8, out, fv, flags, _ = _frames(frames, fill, coord, gather, out, single=False)
+    if nv == 0 or frames.shape[0] % nv:
         raise ValueError("frames must be (nviews * k, sz2, sz1) float32 or (nviews * k, sz2, sz1, 3) uint8")
     k, sz2, sz1 = int(frames.shape[0]) // nv, int(frames.shape[1]), int(frames.shape[2])
     views = (_lib.View * nv)(*[c._views[i] for i in vis])
     rat = (C.c_double * nv)(*[float(r) for r in ratios])
     axs = (C.c_int64 * (2 * nv))(*[int(a) for am in axs_mins for a in am])
-    if out is None:
-        out = torch.empty_like(frames) if is_t else np.empty_like(frames)
-    if u8:
-        fv = (C.c_uint8 * 3)(*([0, 0, 0] if fill is None else [int(v) for v in fill]))
-    else:
-        fv = C.c_float(float("nan") if fill is None else float(fill))
-    geom = (sz1, sz2, C.c_size_t(sz1), C.c_size_t(sz1 * sz2), k, fv, flags)
-    if is_t:
-        dev = frames.device.index if frames.device.index is not None else torch.cuda.current_device()
-        fn = lib.cc_rectify_u8c3_views if u8 else lib.cc_rectify_f32c1_views
-        check(fn(_lib.context(dev).handle, C.byref(c._intr), views, nv, rat, axs, _t_ptr(frames), _t_ptr(out), *geom,
-                 _stream_ptr(dev)))
-    else:
-        fn = lib.cc_rectify_views_u8c3_host if u8 else lib.cc_rectify_views_f32c1_host
-        check(fn(_lib.context(_default_device()).handle, C.byref(c._intr), views, nv, rat, axs, _np_ptr(frames),
-                 _np_ptr(out), *geom))
+    ctx, ptr, host, tail = _where(frames)
+    kern = "u8c3" if u8 else "f32c1"
+    fn = getattr(lib, f"cc_rectify_views_{kern}_host" if host else f"cc_rectify_{kern}_views")
+    check(fn(ctx.handle, C.byref(c._intr), views, nv, rat, axs, ptr(frames), ptr(out), sz1, sz2, C.c_size_t(sz1),
+             C.c_size_t(sz1 * sz2), k, fv, flags, *tail))
     return out
 
 
@@ -471,14 +444,6 @@ def rectify_map(c: Calibration, extrinsic, ratio: float, axs_min, sz, device=Non
 # ---------------------------------------------------------------------------------
 # residual / Jacobian / errors: src/buildcalibrations.jl:28-67
 # ---------------------------------------------------------------------------------
-def _views_array(extrinsics):
-    arr = (_lib.View * max(1, len(extrinsics)))()
-    for i, (r, t) in enumerate(extrinsics):
-        arr[i].rvec[:] = [float(v) for v in r]
-        arr[i].tvec[:] = [float(v) for v in t]
-    return arr
-
-
 def views_tensor(extrinsics, device):
     """(nviews, 6) float64 CUDA tensor with the cc_view layout [rvec | tvec]."""
     a = np.asarray([list(r) + list(t) for r, t in extrinsics], dtype=np.float64).reshape(-1, 6)
@@ -495,8 +460,7 @@ def allreduce_shared(t, group=None):
     through cc_allreduce_shared (raw NCCL inside libcamcal_b200, csrc/comm.cu).  torch.distributed
     is only the bootstrap that carries the NCCL unique id to the other ranks, once per context."""
     if _dist_world(group) > 1:
-        dev = t.device.index if t.device.index is not None else torch.cuda.current_device()
-        ctx = _lib.context(dev)
+        ctx = _lib.context(_device(t))
         ctx.comm_init_from_torch(group)
         ctx.allreduce(t)
     return t
@@ -512,28 +476,21 @@ def reproj_jtj(intr, aspect, views, obj, img, group=None):
     (NCCL sum through cc_allreduce_shared) so every rank holds the global J'J_ii, J'r_i and sum r^2.
     """
     ci = _lib.make_intr(*[float(v) for v in intr])
-    if _is_torch(img):
-        dev = img.device.index if img.device.index is not None else torch.cuda.current_device()
-        views = views.contiguous().to(torch.float64)
-        obj = obj.contiguous().to(torch.float64)
-        img = img.contiguous().to(torch.float64)
-        nv, nc = int(img.shape[0]), int(img.shape[1])
-        pv = torch.empty((nv, _lib.PER_VIEW), dtype=torch.float64, device=img.device)
-        sh = torch.empty(_lib.SHARED, dtype=torch.float64, device=img.device)
-        check(lib.cc_reproj_jtj_f64(_lib.context(dev).handle, C.byref(ci), float(aspect), _t_ptr(views),
-                                    nv, _t_ptr(obj), _t_ptr(img), nc, _t_ptr(pv), _t_ptr(sh),
-                                    _stream_ptr(dev)))
-        allreduce_shared(sh, group)
-        return pv, sh
-    views = np.ascontiguousarray(views, dtype=np.float64).reshape(-1, 6)
-    obj = np.ascontiguousarray(obj, dtype=np.float64)
-    img = np.ascontiguousarray(img, dtype=np.float64)
+    on_device = _is_torch(img)
+    if on_device:
+        views, obj, img = (t.contiguous().to(torch.float64) for t in (views, obj, img))
+        new = functools.partial(torch.empty, dtype=torch.float64, device=img.device)
+    else:
+        views = np.ascontiguousarray(views, dtype=np.float64).reshape(-1, 6)
+        obj, img = (np.ascontiguousarray(a, dtype=np.float64) for a in (obj, img))
+        new = np.empty
     nv, nc = int(img.shape[0]), int(img.shape[1])
-    pv = np.empty((nv, _lib.PER_VIEW))
-    sh = np.empty(_lib.SHARED)
-    check(lib.cc_reproj_jtj_f64_host(_lib.context(_default_device()).handle, C.byref(ci), float(aspect),
-                                     _np_ptr(views), nv, _np_ptr(obj), _np_ptr(img), nc, _np_ptr(pv),
-                                     _np_ptr(sh)))
+    pv, sh = new((nv, _lib.PER_VIEW)), new(_lib.SHARED)
+    ctx, ptr, host, tail = _where(img)
+    fn = getattr(lib, f"cc_reproj_jtj_f64{host}")
+    check(fn(ctx.handle, C.byref(ci), float(aspect), ptr(views), nv, ptr(obj), ptr(img), nc, ptr(pv), ptr(sh), *tail))
+    if on_device:
+        allreduce_shared(sh, group)
     return pv, sh
 
 

@@ -24,7 +24,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import check, lib
-from .calibration import _t_ptr, _stream_ptr, reproj_jtj, allreduce_shared, torch
+from .calibration import _device, _t_ptr, _stream_ptr, reproj_jtj, allreduce_shared, torch
 
 FREE_ALL = 0b1111
 FREE_NO_K = 0b0111          # CALIB_FIX_K1
@@ -114,7 +114,7 @@ def initial_guess(obj, imgs, sz, aspect=1.0):
 # ------------------------------------------------------------------ device steps
 def lm_schur(per_view, lam):
     """phase 1 on this rank's views: returns (yz (nv, 30), schur (21,)) device tensors"""
-    dev = per_view.device.index
+    dev = _device(per_view)
     nv = int(per_view.shape[0])
     yz = torch.empty((max(nv, 1), _lib.LM_YZ), dtype=torch.float64, device=per_view.device)
     schur = torch.empty(_lib.LM_SCHUR, dtype=torch.float64, device=per_view.device)
@@ -125,7 +125,7 @@ def lm_schur(per_view, lam):
 
 def lm_update(shared, schur, lam, free_mask, yz, views):
     """phase 2: returns (candidate views (nv, 6), delta (8,)) device tensors"""
-    dev = views.device.index
+    dev = _device(views)
     nv = int(views.shape[0])
     out = torch.empty_like(views)
     delta = torch.empty(_lib.LM_DELTA, dtype=torch.float64, device=views.device)
@@ -206,32 +206,48 @@ def lm_fit(intr0, views0, obj, imgs, checker_size=1.0, aspect=1.0, with_distorti
                 iterations=it, accepted=accepted, lam=lam, sse=sse)
 
 
+def _f64(a, dev):
+    """a as a C-contiguous float64 tensor on dev; a tensor already so is returned as it is."""
+    if torch.is_tensor(a):
+        return a.to(dtype=torch.float64, device=dev).contiguous()
+    return torch.as_tensor(np.asarray(a, float), dtype=torch.float64, device=dev).contiguous()
+
+
+def _fit_intr(intr0, aspect, with_distortion, checker_size):
+    """The starting cc_intr of a whole fit: frow = aspect * fcol, and k = 0 without distortion."""
+    return _lib.make_intr(aspect * intr0[1], intr0[1], intr0[2], intr0[3], intr0[4] if with_distortion else 0.0,
+                          checker_size)
+
+
+def _fit_result(ci, views, rms, its, **device):
+    """The result dict of a whole fit from the cc_intr, rms and iteration count the library wrote."""
+    return dict(intr=(ci.frow, ci.fcol, ci.crow, ci.ccol, ci.k), views=views, **device, rms=rms.value,
+                iterations=its.value)
+
+
 def lm_fit_device(intr0, views0, obj, imgs, checker_size=1.0, aspect=1.0, with_distortion=True, max_iter=30,
                   eps=1e-3, device=None, group=None):
     """cc_lm_fit_f64: the whole fit as ONE device-resident loop (csrc/lm.cu) over THIS rank's
     views; damping, accept/reject and the stopping rule live in device memory, an iteration costs
     two small NCCL all-reduces and no host synchronisation.  Same arguments and result as lm_fit;
-    device tensors may be passed for views0 / obj / imgs (views0 is then updated in place too)."""
+    device tensors may be passed for views0 / obj / imgs.  views0 itself is never written: the fit
+    runs on a copy, returned as views_device."""
     assert torch is not None and torch.cuda.is_available(), "lm_fit_device runs on the GPU: no CPU fallback"
     dev = torch.device("cuda", torch.cuda.current_device() if device is None else device)
-    f64 = dict(dtype=torch.float64, device=dev)
-    as_t = lambda a: a.to(**f64).contiguous() if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, float), **f64).contiguous()
-    views = as_t(views0).reshape(-1, 6)
+    views = _f64(views0, dev).reshape(-1, 6)
     if views.data_ptr() == (views0.data_ptr() if torch.is_tensor(views0) else 0):
         views = views.clone()
-    obj_t, img_t = as_t(obj), as_t(imgs)
+    obj_t, img_t = _f64(obj, dev), _f64(imgs, dev)
     nv, nc = int(views.shape[0]), int(obj_t.shape[0])
     ctx = _lib.context(dev.index)
     if _dist_on(group):
         ctx.comm_init_from_torch(group)
-    ci = _lib.make_intr(aspect * intr0[1], intr0[1], intr0[2], intr0[3], intr0[4] if with_distortion else 0.0,
-                        checker_size)
+    ci = _fit_intr(intr0, aspect, with_distortion, checker_size)
     rms, its = C.c_double(), C.c_int()
     check(lib.cc_lm_fit_f64(ctx.handle, C.byref(ci), float(aspect), FREE_ALL if with_distortion else FREE_NO_K,
                             _t_ptr(views), nv, _t_ptr(obj_t), _t_ptr(img_t), nc, int(max_iter), float(eps),
                             C.byref(rms), C.byref(its), _stream_ptr(dev.index)))
-    return dict(intr=(ci.frow, ci.fcol, ci.crow, ci.ccol, ci.k), views=views.cpu().numpy(), views_device=views,
-                rms=rms.value, iterations=its.value)
+    return _fit_result(ci, views.cpu().numpy(), rms, its, views_device=views)
 
 
 def initial_guess_device(obj, imgs, sz, aspect=1.0, device=None, group=None):
@@ -239,13 +255,11 @@ def initial_guess_device(obj, imgs, sz, aspect=1.0, device=None, group=None):
     rank's views (batched DLT + pose kernels, csrc/init.cu).  Returns (intr 5-tuple, views (nv, 6)
     CUDA tensor)."""
     dev = torch.device("cuda", torch.cuda.current_device() if device is None else device)
-    f64 = dict(dtype=torch.float64, device=dev)
-    as_t = lambda a: a.to(**f64).contiguous() if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, float), **f64).contiguous()
-    obj_t, img_t = as_t(obj), as_t(imgs)
+    obj_t, img_t = _f64(obj, dev), _f64(imgs, dev)
     nc = int(obj_t.shape[0])
     img_t = img_t.reshape(-1, nc, 2)
     nv = int(img_t.shape[0])
-    views = torch.empty((nv, 6), **f64)
+    views = torch.empty((nv, 6), dtype=torch.float64, device=dev)
     ctx = _lib.context(dev.index)
     if _dist_on(group):
         ctx.comm_init_from_torch(group)
@@ -263,12 +277,10 @@ def lm_fit_host(intr0, views0, obj, imgs, checker_size=1.0, aspect=1.0, with_dis
     obj = np.ascontiguousarray(obj, dtype=np.float64)
     imgs = np.ascontiguousarray(imgs, dtype=np.float64)
     nv, nc = int(imgs.shape[0]), int(obj.shape[0])
-    ci = _lib.make_intr(aspect * intr0[1], intr0[1], intr0[2], intr0[3], intr0[4] if with_distortion else 0.0,
-                        checker_size)
+    ci = _fit_intr(intr0, aspect, with_distortion, checker_size)
     rms, its = C.c_double(), C.c_int()
     vp = lambda a: a.ctypes.data_as(C.c_void_p)
     check(lib.cc_lm_fit_f64_host(_lib.context(device).handle, C.byref(ci), float(aspect),
                                  FREE_ALL if with_distortion else FREE_NO_K, vp(views), nv, vp(obj), vp(imgs), nc,
                                  int(max_iter), float(eps), C.byref(rms), C.byref(its)))
-    return dict(intr=(ci.frow, ci.fcol, ci.crow, ci.ccol, ci.k), views=views, rms=rms.value,
-                iterations=its.value)
+    return _fit_result(ci, views, rms, its)

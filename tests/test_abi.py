@@ -19,20 +19,66 @@ def cc():
     return m
 
 
-def _declared():
+def _header_params():
+    """{name: ["ptr" | "scalar" per parameter]} of every function include/camcal_b200.h declares"""
     hdr = open(os.path.join(ROOT, "include", "camcal_b200.h")).read()
     hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
-    return sorted(set(re.findall(r"\b(cc_[a-z0-9_]+)\s*\(", hdr)))
+    out = {}
+    for name, params in re.findall(r"\b(cc_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", hdr):
+        ps = [p.strip() for p in params.split(",") if p.strip() and p.strip() != "void"]
+        out[name] = ["ptr" if ("*" in p or "[" in p) else "scalar" for p in ps]
+    return out
+
+
+def _julia_ccalls():
+    """[(name, ["ptr" | "scalar" per argument])] of every ccall into libcamcal in the Julia shim"""
+    src = open(os.path.join(ROOT, "julia", "CameraCalibrationsB200.jl")).read()
+    calls = []
+    for m in re.finditer(r"ccall\(\(:(cc_[a-z0-9_]+),\s*libcamcal\),\s*\w+,\s*\(", src):
+        i, depth = m.end(), 1                   # the argument-type tuple: up to its matching ')'
+        j = i
+        while depth:
+            depth += {"(": 1, ")": -1}.get(src[j], 0)
+            j += 1
+        types, depth, cur = [], 0, ""
+        for ch in src[i:j - 1]:
+            if ch in "({":
+                depth += 1
+            elif ch in ")}":
+                depth -= 1
+            if ch == "," and depth == 0:
+                types.append(cur.strip())
+                cur = ""
+            else:
+                cur += ch
+        if cur.strip():
+            types.append(cur.strip())
+        calls.append((m.group(1), ["ptr" if re.match(r"(Ptr|Ref)\{", t) else "scalar" for t in types]))
+    return calls
 
 
 def test_library_exports_every_declared_symbol(cc):
     from cameracalibrations_b200 import _lib
-    names = _declared()
+    names = sorted(_header_params())
     assert len(names) >= 30
     for n in names:
         assert hasattr(_lib.lib, n), f"{n} declared in include/camcal_b200.h but not exported"
     assert set(names) == set(_lib.EXPORTS)          # the ctypes table binds all of them
     assert _lib.lib.cc_abi_version() == 1
+
+
+def test_bindings_pass_pointers_where_the_header_takes_them(cc):
+    """Every ctypes signature and every Julia ccall passes a pointer exactly where include/camcal_b200.h declares
+    one, and a scalar everywhere else."""
+    from cameracalibrations_b200 import _lib
+    hdr = _header_params()
+    for name, (_, args) in _lib._SIGS.items():
+        kinds = ["ptr" if a in (C.c_void_p, C.c_char_p) or issubclass(a, C._Pointer) else "scalar" for a in args]
+        assert kinds == hdr[name], (name, kinds, hdr[name])
+    calls = _julia_ccalls()
+    assert len(calls) >= 29
+    for name, kinds in calls:
+        assert name in hdr and kinds == hdr[name], (name, kinds, hdr.get(name))
 
 
 def test_no_cpu_fallback(cc):

@@ -5,13 +5,12 @@ oracle at the SoA tolerances.
 
 The CPU tests at the end need no device."""
 import ctypes as C
-import os
-import re
 
 import numpy as np
 import pytest
 
-from conftest import ROOT, C2_INTR, SYN_VIEW
+from conftest import C2_INTR, SYN_VIEW
+from test_abi import _header_params, _julia_ccalls
 
 torch = pytest.importorskip("torch")
 
@@ -382,18 +381,7 @@ def test_aos_entry_points_need_a_device():
         c(torch.zeros((4, 2), dtype=torch.float64), 0)   # CPU tensors do not take the host path
 
 
-def _header_params():
-    hdr = open(os.path.join(ROOT, "include", "camcal_b200.h")).read()
-    hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
-    out = {}
-    for name, params in re.findall(r"\bint\s+(cc_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", hdr):
-        ps = [p.strip() for p in params.split(",") if p.strip() and p.strip() != "void"]
-        out[name] = ["ptr" if ("*" in p or "[" in p) else "scalar" for p in ps]
-    return out
-
-
 def test_julia_aos_ccalls_match_the_header():
-    from test_gpu_point_views import _julia_ccalls
     hdr = _header_params()
     calls = [(n, k) for n, k in _julia_ccalls() if "_aos" in n]
     assert {n for n, _ in calls} == {"cc_img2world_f64_aos_host", "cc_world2img_f64_aos_host"}

@@ -4,13 +4,12 @@ entry point called with that segment's view; against the oracle at the single-vi
 
 The CPU tests at the end need no device."""
 import ctypes as C
-import os
-import re
 
 import numpy as np
 import pytest
 
-from conftest import ROOT, C2_INTR, SYN_VIEW
+from conftest import C2_INTR, SYN_VIEW
+from test_abi import _header_params, _julia_ccalls
 
 torch = pytest.importorskip("torch")
 
@@ -364,42 +363,6 @@ def test_views_entry_points_need_a_device(cc_cpu):
         with pytest.raises(cc_cpu.CamcalError) as e:
             call()
         assert e.value.status == -2                      # CC_ERR_NO_DEVICE
-
-
-def _header_params():
-    hdr = open(os.path.join(ROOT, "include", "camcal_b200.h")).read()
-    hdr = re.sub(r"/\*.*?\*/", "", hdr, flags=re.S)
-    out = {}
-    for name, params in re.findall(r"\bint\s+(cc_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", hdr):
-        ps = [p.strip() for p in params.split(",") if p.strip() and p.strip() != "void"]
-        out[name] = ["ptr" if ("*" in p or "[" in p) else "scalar" for p in ps]
-    return out
-
-
-def _julia_ccalls():
-    src = open(os.path.join(ROOT, "julia", "CameraCalibrationsB200.jl")).read()
-    calls = []
-    for m in re.finditer(r"ccall\(\(:(cc_[a-z0-9_]+),\s*libcamcal\),\s*Cint,\s*\(", src):
-        i, depth = m.end(), 1                   # the argument-type tuple: up to its matching ')'
-        j = i
-        while depth:
-            depth += {"(": 1, ")": -1}.get(src[j], 0)
-            j += 1
-        types, depth, cur = [], 0, ""
-        for ch in src[i:j - 1]:
-            if ch in "({":
-                depth += 1
-            elif ch in ")}":
-                depth -= 1
-            if ch == "," and depth == 0:
-                types.append(cur.strip())
-                cur = ""
-            else:
-                cur += ch
-        if cur.strip():
-            types.append(cur.strip())
-        calls.append((m.group(1), ["ptr" if re.match(r"(Ptr|Ref)\{", t) else "scalar" for t in types]))
-    return calls
 
 
 def test_julia_views_ccalls_match_the_header():

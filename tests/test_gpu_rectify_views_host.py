@@ -19,7 +19,7 @@ from conftest import camera_for
 from oracle import oracle_c as oc
 from test_gpu_batching import (F_FILL, F_SENT, U_FILL, U_SENT, _env, _frames_f32, _frames_u8, _staged_lines)
 from test_gpu_parity import _calib, _dev, _perturbed_views, _rect_case
-from test_gpu_point_views import _header_params, _julia_ccalls
+from test_abi import _header_params, _julia_ccalls
 
 GROUP = 64                    # views per staged launch (rectify.cu: kMaxViews)
 _FOOTPRINT = re.compile(r"\[camcal\] views: common footprint")
