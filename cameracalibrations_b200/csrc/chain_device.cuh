@@ -12,8 +12,8 @@
 namespace cc {
 
 // Rodrigues on the device (sincos: not bit-identical to rodrigues_host, so no point map or rectification uses it);
-// returns theta^2
-__device__ __forceinline__ double rodrigues(const double r[3], double R[9]) {
+// returns theta^2.  tsc (optional): receives (theta, sin theta, cos theta) when theta >= DBL_EPSILON.
+__device__ __forceinline__ double rodrigues(const double r[3], double R[9], double* tsc = nullptr) {
     const double th2 = fma(r[2], r[2], fma(r[1], r[1], r[0] * r[0]));
     const double th = sqrt(th2);
     if (th < 2.220446049250313e-16) {
@@ -23,6 +23,7 @@ __device__ __forceinline__ double rodrigues(const double r[3], double R[9]) {
     }
     double s, c;
     sincos(th, &s, &c);
+    if (tsc) { tsc[0] = th; tsc[1] = s; tsc[2] = c; }
     const double c1 = 1.0 - c, it = 1.0 / th;
     const double nx = r[0] * it, ny = r[1] * it, nz = r[2] * it;
     R[0] = fma(c1 * nx, nx, c);

@@ -33,10 +33,15 @@ __device__ __forceinline__ void skew(const double v[3], double S[9]) {
 }
 
 // Rodrigues and its derivative:
-//   dR/dr_i = ( r_i [r]x + [ r x ((I - R) e_i) ]x ) R / theta^2 ,  -> [e_i]x as theta -> 0
+//   dR/dr_i = ( r_i [r]x + [ r x w_i ]x ) R / theta^2 ,  = [e_i]x to rounding for theta < DBL_EPSILON
+//   w_i = (I - R) e_i = c1 (e_i - n n_i) - s (n x e_i),  n = r / theta,  s = sin theta,
+//   c1 = 1 - cos theta, formed as s^2 / (1 + cos theta) while cos theta > 0
+// Formed as e_i - R e_i instead, w_i loses its c1 part to rounding and the division by theta^2 magnifies the
+// loss (~2e-8 relative at theta = 1e-8); so does 1 - cos theta for small theta.  R is rodrigues() unchanged.
 __device__ void view_geom(const double r[3], ViewGeom& g) {
-    const double th2 = rodrigues(r, g.R);
-    if (th2 < 1e-24) {
+    double tsc[3];
+    const double th2 = rodrigues(r, g.R, tsc);
+    if (sqrt(th2) < 2.220446049250313e-16) {
 #pragma unroll
         for (int i = 0; i < 3; ++i) {
             double e[3] = {0.0, 0.0, 0.0};
@@ -45,13 +50,19 @@ __device__ void view_geom(const double r[3], ViewGeom& g) {
         }
         return;
     }
-    double S[9];
+    const double s = tsc[1], c = tsc[2], it = 1.0 / tsc[0];
+    const double c1 = c > 0.0 ? s * s / (1.0 + c) : 1.0 - c;
+    const double n[3] = {r[0] * it, r[1] * it, r[2] * it};
+    double S[9], Sn[9];
     skew(r, S);
+    skew(n, Sn);
     const double ith2 = 1.0 / th2;
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
-        double w[3] = {-g.R[i], -g.R[3 + i], -g.R[6 + i]};
-        w[i] += 1.0;
+        double w[3];                                   // n x e_i is column i of [n]x
+#pragma unroll
+        for (int j = 0; j < 3; ++j) w[j] = -(c1 * (n[j] * n[i])) - s * Sn[3 * j + i];
+        w[i] += c1;
         const double cr[3] = {r[1] * w[2] - r[2] * w[1], r[2] * w[0] - r[0] * w[2],
                               r[0] * w[1] - r[1] * w[0]};
         double C[9], M[9];

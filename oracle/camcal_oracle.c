@@ -355,8 +355,13 @@ void cco_rectify_u8c3(const cco_chain *ch, double inv_ratio,
 
 /* ------------------------------------------------------------------------- */
 /* Row a7: residual, Jacobian, normal-equation blocks.                         */
-/* dR/dr_i = ( r_i [r]x + [ r x ((I - R) e_i) ]x ) R / theta^2   (theta > 0)   */
-/*         = [e_i]x                                              (theta -> 0)  */
+/* dR/dr_i = ( r_i [r]x + [ r x w_i ]x ) R / theta^2          (theta > 0)      */
+/*         = [e_i]x                                (theta < DBL_EPSILON)      */
+/* w_i = (I - R) e_i = c1 (e_i - n n_i) - s (n x e_i),  n = r / theta,        */
+/* s = sin theta, c1 = 1 - cos theta formed as s^2 / (1 + cos theta) while    */
+/* cos theta > 0.  Formed as e_i - R e_i instead, w_i loses its c1 part to     */
+/* rounding and the division by theta^2 magnifies the loss: ~2e-8 relative at */
+/* theta = 1e-8; so does 1 - cos theta for small theta.                        */
 /* ------------------------------------------------------------------------- */
 static void skew(const double v[3], double S[9])
 {
@@ -375,8 +380,9 @@ static void matmul3(const double A[9], const double B[9], double C[9])
 
 static void rodrigues_jac(const double r[3], const double R[9], double dR[3][9])
 {
-    double th2 = r[0] * r[0] + r[1] * r[1] + r[2] * r[2];
-    if (th2 < 1e-24) {
+    double th2 = fma(r[2], r[2], fma(r[1], r[1], r[0] * r[0]));
+    double th = sqrt(th2);
+    if (th < DBL_EPSILON) {
         for (int i = 0; i < 3; ++i) {
             double e[3] = {0, 0, 0};
             e[i] = 1.0;
@@ -384,12 +390,17 @@ static void rodrigues_jac(const double r[3], const double R[9], double dR[3][9])
         }
         return;
     }
-    double S[9];
+    double s = sin(th), c = cos(th), it = 1.0 / th;
+    double c1 = c > 0.0 ? s * s / (1.0 + c) : 1.0 - c;
+    double n[3] = {r[0] * it, r[1] * it, r[2] * it};
+    double S[9], Sn[9];
     skew(r, S);
+    skew(n, Sn);
     for (int i = 0; i < 3; ++i) {
-        /* w = (I - R) e_i  = e_i - R[:,i] */
-        double w[3] = {-R[i], -R[3 + i], -R[6 + i]};
-        w[i] += 1.0;
+        /* w = c1 (e_i - n n_i) - s (n x e_i);  n x e_i is column i of [n]x */
+        double w[3];
+        for (int j = 0; j < 3; ++j) w[j] = -(c1 * (n[j] * n[i])) - s * Sn[3 * j + i];
+        w[i] += c1;
         double cr[3] = {r[1] * w[2] - r[2] * w[1], r[2] * w[0] - r[0] * w[2],
                         r[0] * w[1] - r[1] * w[0]};
         double C[9], M[9];
@@ -486,10 +497,10 @@ void cco_reproj_jtj(const cco_intr *in, double aspect, const cco_view *views,
 }
 
 /* src/buildcalibrations.jl:37-67 */
-void cco_calculate_errors(const cco_intr *in, const cco_view *views, int nviews,
-                          const double *obj, const double *img, int n1, int n2,
-                          const double *inv_rows, const double *inv_cols,
-                          int inverse_samples, double out[4])
+void cco_calculate_error_sums(const cco_intr *in, const cco_view *views, int nviews,
+                              const double *obj, const double *img, int n1, int n2,
+                              const double *inv_rows, const double *inv_cols,
+                              int inverse_samples, double sums[4])
 {
     int nc = n1 * n2;
     double reprojection = 0.0, projection = 0.0, distance = 0.0, inverse = 0.0;
@@ -542,9 +553,20 @@ void cco_calculate_errors(const cco_intr *in, const cco_view *views, int nviews,
         inverse += si;
     }
     free(px);
-    double n = (double)nc * nviews;                                /* :60-65 */
-    out[0] = sqrt(reprojection / n);
-    out[1] = sqrt(projection / n);
-    out[2] = sqrt(distance / (double)((n1 - 1) * (n2 - 1)) / nviews);
-    out[3] = sqrt(inverse / inverse_samples / nviews);
+    sums[0] = reprojection; sums[1] = projection; sums[2] = distance; sums[3] = inverse;
+}
+
+void cco_calculate_errors(const cco_intr *in, const cco_view *views, int nviews,
+                          const double *obj, const double *img, int n1, int n2,
+                          const double *inv_rows, const double *inv_cols,
+                          int inverse_samples, double out[4])
+{
+    double s[4];
+    cco_calculate_error_sums(in, views, nviews, obj, img, n1, n2, inv_rows, inv_cols,
+                             inverse_samples, s);
+    double n = (double)n1 * n2 * nviews;                           /* :60-65 */
+    out[0] = sqrt(s[0] / n);
+    out[1] = sqrt(s[1] / n);
+    out[2] = sqrt(s[2] / (double)((n1 - 1) * (n2 - 1)) / nviews);
+    out[3] = sqrt(s[3] / inverse_samples / nviews);
 }

@@ -138,6 +138,13 @@ void cco_calculate_errors(const cco_intr *in, const cco_view *views, int nviews,
                           const double *obj, const double *img, int n1, int n2,
                           const double *inv_rows, const double *inv_cols,
                           int inverse_samples, double out[4]);
+/* The four raw sums over all views that cco_calculate_errors normalises (what
+ * cc_calculate_errors_f64 returns): squared reprojection, projection, distance
+ * and inverse errors. */
+void cco_calculate_error_sums(const cco_intr *in, const cco_view *views, int nviews,
+                              const double *obj, const double *img, int n1, int n2,
+                              const double *inv_rows, const double *inv_cols,
+                              int inverse_samples, double sums[4]);
 
 #ifdef __cplusplus
 }

@@ -196,13 +196,15 @@ def reproj_jtj(intr, aspect, views, obj, img, want_jac=False, nthreads=0):
     return pv, sh, jac
 
 
-def calculate_errors(intr, views, obj, imgs, n_corners, inv_samples):
+def calculate_errors(intr, views, obj, imgs, n_corners, inv_samples, raw_sums=False):
+    """the reference's four errors; raw_sums: the four sums over all views they normalise"""
     obj, imgs, inv_samples = _f64(obj), _f64(imgs), _f64(inv_samples)
     nv, S = inv_samples.shape[0], inv_samples.shape[1]
     ir = np.ascontiguousarray(inv_samples[:, :, 0])
     ic = np.ascontiguousarray(inv_samples[:, :, 1])
     out = (C.c_double * 4)()
     i = make_intr(intr)
-    lib().cco_calculate_errors(C.byref(i), make_views(views), nv, _dp(obj), _dp(imgs),
-                               int(n_corners[0]), int(n_corners[1]), _dp(ir), _dp(ic), S, out)
+    fn = lib().cco_calculate_error_sums if raw_sums else lib().cco_calculate_errors
+    fn(C.byref(i), make_views(views), nv, _dp(obj), _dp(imgs), int(n_corners[0]), int(n_corners[1]),
+       _dp(ir), _dp(ic), S, out)
     return tuple(out)
