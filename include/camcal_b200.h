@@ -72,7 +72,7 @@ typedef struct cc_ctx cc_ctx; /* per-device scratch, staging buffers, streams */
 
 /* coordinate arithmetic of the rectification map */
 #define CC_COORD_F64 0u     /* reference precision: bit-exact index/weight selection  */
-#define CC_COORD_F32 1u     /* fast path: map within 1e-3 px of the FP64 map          */
+#define CC_COORD_F32 1u     /* fast path: map error bounded as for cc_rectify_map_f32  */
 /* how source texels are fetched */
 #define CC_GATHER_AUTO 0u   /* TMA-staged tiles when the frame layout allows, else direct */
 #define CC_GATHER_DIRECT 16u
@@ -267,8 +267,12 @@ int cc_rectify_map_f64(cc_ctx *ctx, const cc_intr *intr, const cc_view *view, do
                        const int64_t axs_min[2], double *map_row, double *map_col, int sz1,
                        int sz2, size_t pitch, void *stream);
 
-/* the map the CC_COORD_F32 fast path samples (same arithmetic as its kernels), FP32: stated to lie
- * within 1e-3 px of the FP64 map wherever that is inside the frame */
+/* the map the CC_COORD_F32 fast path samples (same arithmetic as its kernels), FP32: within 1e-3 px
+ * of the exact map wherever the FP64 map is inside the frame, the point is in front of the camera
+ * (P3 > 0) and the lens is monotone there (1 + 3k r^2 > 0); elsewhere within the conditioning bound of
+ * oracle/map_ref.py: |err| <= s u sum_z |d(row, col)/dz| |z| over the roundings z of the kernel's
+ * sequence, u = 2^-24, s = 1.0625 (past the fold of the lens: about 2e-2 px at in-frame pixels of a
+ * 4K camera with k = -0.12) */
 int cc_rectify_map_f32(cc_ctx *ctx, const cc_intr *intr, const cc_view *view, double ratio,
                        const int64_t axs_min[2], float *map_row, float *map_col, int sz1,
                        int sz2, size_t pitch, void *stream);
