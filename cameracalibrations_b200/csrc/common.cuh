@@ -134,19 +134,22 @@ struct cc_ctx {
     size_t pipe_out_bytes[NSLOT];
     // TMA descriptor encode entry point (driver API, resolved at ctx creation)
     void* encode_tiled;
-    // rectification tile plans (rectify.cu: RectPlan), most recent NPLAN parameter sets
+    // rectification footprints of single views (rectify.cu: RectPlan, host memory only), most recent NPLAN
+    // parameter sets
     static const int NPLAN = 64;
     void* rect_plans[NPLAN];
     int rect_plan_next;
-    // tile plans of groups of views rectified in one launch (rectify.cu: MultiPlan), most recent NMULTI groups
-    static const int NMULTI = 4;
-    void* multi_plans[NMULTI];
-    int multi_plan_next;
-    // cc_rectify_views_*_host: group plans go up on rect_upload; a plan's fence joins the slot streams on
-    // rect_join (rect_join_event: one per slot); multi_retired: evicted plans whose buffers did not fit a new one
+    // the device tables every staged rectification launch reads (rectify.cu: GroupPlan): plans of one view in
+    // the first NPLAN slots, plans of more views in the last NGROUP, each part evicting round-robin
+    // (group_plan_next[0] / [1]).  Tables go up on rect_upload; an evicted plan's buffers are overwritten after
+    // its readers, or the plan is retired (plans_retired) and freed once they have finished.
+    // cc_rectify_views_*_host joins its slot streams on rect_join (rect_join_event: one per slot).
+    static const int NGROUP = 4;
+    void* group_plans[NPLAN + NGROUP];
+    int group_plan_next[2];
     cudaStream_t rect_upload, rect_join;
     cudaEvent_t rect_join_event[NSLOT];
-    void* multi_retired;
+    void* plans_retired;
     // ticket counters of the persistent rectification kernels (rectify.cu: RectSched)
     static const int NSCHED = 16;
     void* sched_pool;

@@ -22,6 +22,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <mutex>
 #include <new>
 #include <thread>
@@ -209,50 +210,21 @@ static void host_coord(const ChainD& ch, double inv_ratio, long long I1, long lo
 // depends on the calibration, ratio/axes, frame size and tile shape only -- not on the pixels --
 // so it is built once on the host, uploaded once and reused by every later call with the same
 // parameters (a video stream): the kernels' producer warp then only issues TMA loads.
+//
+// Two objects hold it.  RectPlan: the footprints of one view, host memory only, cached per view
+// (ctx->rect_plans).  GroupPlan (below): the device tables (tile headers, q2 terms) of a group of
+// 1..64 views for one common staged box; every staged launch reads one.
 struct PlanKey { ChainD ch; double ratio; RectGeom g; int tw, tl, pxb; };
 
 struct RectPlan {
     PlanKey key;
     int n1, n2;                    // tiles along the first / second axis
     int need1, need2;              // largest footprint (pixels), incl. taps and slack
-    int box1, box2, box_bytes;     // staged box (pixels) and its size; box_bytes == 0: not stageable
-    int pitch_b;                   // bytes per staged line
     int tilt;                      // sign of d(source line)/d(first output index): which way a warp's taps change lines
     std::vector<int> origin;       // per tile: floor(min row), floor(min col) of the perimeter samples
     std::vector<unsigned char> p3_ok;
-    std::vector<TileHdr> hdr;      // tile headers
     std::vector<double> q2;        // exact path: second-axis world term of every output line
-    TileHdr* d_hdr;
-    double* d_q2;
-    int per_sm[2];                 // resident CTAs per SM of the staged kernel, [exact], cached (0: not queried yet)
-    size_t per_sm_smem[2];
 };
-
-static void plan_free(RectPlan* p) {
-    if (!p) return;
-    if (p->d_hdr) cudaFree(p->d_hdr);
-    if (p->d_q2) cudaFree(p->d_q2);
-    delete p;
-}
-
-static void multi_free(void* mp);
-static void multi_free_retired(cc_ctx* ctx);
-
-void rectify_free_plans(cc_ctx* ctx) {
-    for (int i = 0; i < cc_ctx::NPLAN; ++i) {
-        plan_free(static_cast<RectPlan*>(ctx->rect_plans[i]));
-        ctx->rect_plans[i] = nullptr;
-    }
-    for (int i = 0; i < cc_ctx::NMULTI; ++i) {
-        multi_free(ctx->multi_plans[i]);
-        ctx->multi_plans[i] = nullptr;
-    }
-    multi_free_retired(ctx);
-    if (ctx->rect_upload) { cudaStreamSynchronize(ctx->rect_upload); cudaStreamDestroy(ctx->rect_upload); ctx->rect_upload = nullptr; }
-    if (ctx->rect_join) { cudaStreamSynchronize(ctx->rect_join); cudaStreamDestroy(ctx->rect_join); ctx->rect_join = nullptr; }
-    for (int k = 0; k < cc_ctx::NSLOT; ++k)
-        if (ctx->rect_join_event[k]) { cudaEventDestroy(ctx->rect_join_event[k]); ctx->rect_join_event[k] = nullptr; }
-}
 
 static void plan_footprints(RectPlan* p, bool threads) {
     const ChainD& ch = p->key.ch;
@@ -430,38 +402,6 @@ static void fill_headers(const RectPlan* p, const BoxDims& d, TileHdr* hdr) {
     }
 }
 
-static void plan_boxes(RectPlan* p) {
-    const RectGeom& g = p->key.g;
-    const BoxDims d = box_dims(p->need1, p->need2, p->tilt, p->key.pxb);
-    p->box1 = d.box1; p->box2 = d.box2; p->pitch_b = d.pitch_b; p->box_bytes = d.box_bytes;
-    // the second-axis world terms do not depend on the box (the views call needs them for unstageable plans too)
-    p->q2.resize((size_t)g.sz2);
-    const double inv_ratio = 1.0 / p->key.ratio;
-    for (int b = 0; b < g.sz2; ++b)       // rect_q2() of rectify_device.cuh, same two products
-        p->q2[b] = ((double)((long long)g.axs1 + b) * inv_ratio) * p->key.ch.inv_cs;
-    if (!p->box_bytes) return;
-    p->hdr.resize((size_t)p->n1 * p->n2);
-    fill_headers(p, d, p->hdr.data());
-}
-
-// tile headers and q2 terms of a plan to the device (once); false: out of device memory
-static bool plan_upload(RectPlan* p, cudaStream_t st) {
-    if (p->d_hdr || p->hdr.empty()) return true;
-    const size_t hb = p->hdr.size() * sizeof(TileHdr), qb = p->q2.size() * sizeof(double);
-    if (cudaMalloc(&p->d_hdr, hb) != cudaSuccess || cudaMalloc(&p->d_q2, qb) != cudaSuccess ||
-        cudaMemcpyAsync(p->d_hdr, p->hdr.data(), hb, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(p->d_q2, p->q2.data(), qb, cudaMemcpyHostToDevice, st) != cudaSuccess) {
-        cudaGetLastError();
-        if (p->d_hdr) cudaFree(p->d_hdr);
-        if (p->d_q2) cudaFree(p->d_q2);
-        p->d_hdr = nullptr; p->d_q2 = nullptr;
-        return false;
-    }
-    // later calls may come on other streams: make the tables visible to all of them
-    cudaStreamSynchronize(st);
-    return true;
-}
-
 static RectPlan* plan_find(cc_ctx* ctx, const PlanKey& key) {
     for (int i = 0; i < cc_ctx::NPLAN; ++i) {
         RectPlan* p = static_cast<RectPlan*>(ctx->rect_plans[i]);
@@ -470,24 +410,25 @@ static RectPlan* plan_find(cc_ctx* ctx, const PlanKey& key) {
     return nullptr;
 }
 
-// footprints, box and headers of one parameter set: host arithmetic only (safe to run on several threads;
+// footprints and q2 terms of one parameter set: host arithmetic only (safe to run on several threads;
 // threads: split a large plan over host threads itself -- off when the caller already runs one plan per thread)
 static RectPlan* plan_build(const PlanKey& key, bool threads) {
     RectPlan* p = new (std::nothrow) RectPlan();
     if (!p) return nullptr;
-    p->key = key; p->d_hdr = nullptr; p->d_q2 = nullptr;
-    p->per_sm[0] = p->per_sm[1] = 0; p->per_sm_smem[0] = p->per_sm_smem[1] = 0;
+    p->key = key;
     plan_footprints(p, threads);
-    plan_boxes(p);
+    const RectGeom& g = key.g;
+    p->q2.resize((size_t)g.sz2);
+    const double inv_ratio = 1.0 / key.ratio;
+    for (int b = 0; b < g.sz2; ++b)       // rect_q2() of rectify_device.cuh, same two products
+        p->q2[b] = ((double)((long long)g.axs1 + b) * inv_ratio) * key.ch.inv_cs;
     return p;
 }
 
+// footprints are host memory only: evicting one frees it at once
 static void plan_insert(cc_ctx* ctx, RectPlan* p) {
     const int slot = ctx->rect_plan_next++ % cc_ctx::NPLAN;
-    if (ctx->rect_plans[slot]) {
-        cudaDeviceSynchronize();       // an evicted plan may still be read by a running kernel
-        plan_free(static_cast<RectPlan*>(ctx->rect_plans[slot]));
-    }
+    delete static_cast<RectPlan*>(ctx->rect_plans[slot]);
     ctx->rect_plans[slot] = p;
 }
 
@@ -497,21 +438,6 @@ static PlanKey plan_key(const ChainD& ch, double ratio, const RectGeom& g, int t
     key.ch = ch; key.ratio = ratio; key.g = g; key.g.nframes = 0; key.g.frame_stride = 0;
     key.tw = tw; key.tl = tl; key.pxb = pxb;
     return key;
-}
-
-// find or build the plan of this (calibration, geometry, tile shape); its tables go to the device on first use
-static RectPlan* plan_get(cc_ctx* ctx, const ChainD& ch, double ratio, const RectGeom& g, int tw, int tl,
-                          int pxb, cudaStream_t st) {
-    const PlanKey key = plan_key(ch, ratio, g, tw, tl, pxb);
-    if (RectPlan* p = plan_find(ctx, key)) return plan_upload(p, st) ? p : nullptr;
-    RectPlan* p = plan_build(key, true);
-    if (!p) return nullptr;
-    if (!plan_upload(p, st)) {
-        plan_free(p);
-        return nullptr;
-    }
-    plan_insert(ctx, p);
-    return p;
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -565,35 +491,14 @@ static bool stage_box(cc_ctx* ctx, const void* src, int pxb, int sz1, int sz2, s
     return true;
 }
 
-// Decide whether the TMA-staged variant applies and build its tensor map + tile config.
-static bool plan_tma(cc_ctx* ctx, const ChainD& ch, double ratio, const RectGeom& g, const void* src, int pxb, int tl,
-                     cudaStream_t st, CUtensorMap* tmap, TileCfg* cfg, RectPlan** plan_out) {
-    if (!tma_aligned(src, pxb, g.pitch, g.frame_stride, g.nframes) || !encoder(ctx)) return false;
-    RectPlan* plan = plan_get(ctx, ch, ratio, g, kT, tl, pxb, st);
-    if (!plan || !plan->box_bytes) return false;
-    const BoxDims d = {plan->box1, plan->box2, plan->pitch_b, plan->box_bytes};
-    if (!stage_box(ctx, src, pxb, g.sz1, g.sz2, g.pitch, g.frame_stride, g.nframes, d, tmap, cfg)) return false;
-    *plan_out = plan;
-    return true;
-}
-
-// cudaFuncAttributeMaxDynamicSharedMemorySize belongs to the KERNEL (per device), not to a plan:
-// the library remembers the largest value it has set per staged kernel and device and only ever
-// raises it (a smaller plan must not lower the limit under a cached larger one, whichever context
-// of the process made either call).
-static std::mutex g_smem_mu;
+// cudaFuncAttributeMaxDynamicSharedMemorySize and the occupancy belong to the KERNEL (per device), not
+// to a plan.  Per staged kernel (slot) and device the library remembers the largest attribute it has
+// set and only ever raises it (a smaller ring must not lower the limit under a larger one, whichever
+// context of the process made either call), and the resident CTAs per SM of every dynamic
+// shared-memory size it has queried (the query costs microseconds per call).
+static std::mutex g_kernel_mu;
 static size_t g_smem_attr[64][12];
-template <typename K>
-static int set_smem(cc_ctx* ctx, int kslot, K kernel, size_t bytes) {
-    if (bytes <= 32 * 1024) return CC_OK;     // static smem (barriers + headers) counts against the 48 KB default too
-    std::lock_guard<std::mutex> lk(g_smem_mu);
-    size_t& cur = g_smem_attr[ctx->device & 63][kslot];
-    if (bytes > cur) {
-        CC_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-        cur = bytes;
-    }
-    return CC_OK;
-}
+static std::map<size_t, int> g_per_sm[64][12];
 
 // Ticket counters: a small ring of self-resetting counters per context.  Launches on different
 // streams may overlap, so consecutive launches take different counters, and a counter is only
@@ -627,17 +532,24 @@ void rectify_free_sched(cc_ctx* ctx) {
 }
 
 // persistent grid of a staged kernel: every CTA slot of the device (tickets do the balancing)
-template <typename K, typename PL>
-static int persistent_grid(cc_ctx* ctx, int kslot, K kernel, size_t smem, const TileCfg& cfg, PL* plan, bool exact,
-                           uint32_t* gsz) {
-    // the occupancy query and the shared-memory attribute cost microseconds per call: once per plan
-    int rc = set_smem(ctx, kslot, kernel, smem);
-    if (rc) return rc;
-    int per_sm = plan->per_sm_smem[exact] == smem ? plan->per_sm[exact] : 0;
-    if (per_sm == 0) {
-        CC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kConsumerThreads + 32, smem));
-        plan->per_sm[exact] = per_sm;
-        plan->per_sm_smem[exact] = smem;
+template <typename K>
+static int persistent_grid(cc_ctx* ctx, int kslot, K kernel, size_t smem, const TileCfg& cfg, uint32_t* gsz) {
+    int per_sm = 0;
+    {
+        std::lock_guard<std::mutex> lk(g_kernel_mu);
+        size_t& cur = g_smem_attr[ctx->device & 63][kslot];
+        if (smem > 32 * 1024 && smem > cur) {     // static smem (barriers + headers) counts against the 48 KB default too
+            CC_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            cur = smem;
+        }
+        std::map<size_t, int>& occ = g_per_sm[ctx->device & 63][kslot];
+        const auto it = occ.find(smem);
+        if (it != occ.end()) {
+            per_sm = it->second;
+        } else {
+            CC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kConsumerThreads + 32, smem));
+            occ[smem] = per_sm;
+        }
     }
     *gsz = std::min<uint32_t>(cfg.units, (uint32_t)ctx->sm_count * (uint32_t)std::max(per_sm, 1));
     if (getenv("CAMCAL_DEBUG"))
@@ -731,78 +643,38 @@ template <> struct RectFmt<uint8_t> {
     }
 };
 
-// One launch of the single-view kernels: frames [0, nframes) of view v at src / dst (the call's layout), on st.
-template <typename PX>
-int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const PX* src, PX* dst, cudaStream_t st) {
-    using F = RectFmt<PX>;
-    if (nframes == 0) return CC_OK;
-    const ChainD& ch = c.views.chs[v];
-    const double ratio = c.views.ratios[v];
-    const RectGeom g = make_geom(c.views.axs_mins + 2 * v, c.fr.sz1, c.fr.sz2, c.fr.pitch, c.fr.frame_stride, nframes);
-    const RectExact pe = make_exact(ch, ratio);
-    const RectFast pf = make_fast(ch, ratio, g);
-    const bool exact = !(c.flags & CC_COORD_F32);
-    CUtensorMap tmap;
-    TileCfg cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    RectPlan* plan = nullptr;
-    const bool tma = !(c.flags & CC_GATHER_DIRECT) && F::dst_ok(dst, c.fr, nframes) &&
-                     plan_tma(ctx, ch, ratio, g, src, F::pxb, F::tl, st, &tmap, &cfg, &plan);
-    if ((c.flags & CC_GATHER_TMA) && !tma)
-        return set_error(CC_ERR_INVALID_ARG, "TMA gather not available for this layout / footprint");
-    int rc = CC_OK;
-    if (tma) {
-        if ((rc = unit_cfg(ctx, &cfg, c.fr.sz1, c.fr.sz2, nframes, kT, F::tl, exact ? F::fg_exact : F::fg_fast))) return rc;
-        int nf = 1;
-        const size_t smem = F::ring(cfg, false, &nf);
-        const auto k = F::staged(exact, nf);
-        uint32_t gsz = 0;
-        if ((rc = persistent_grid(ctx, F::staged_slot(nf) + !exact, k, smem, cfg, plan, exact, &gsz))) return rc;
-        RectSched* sched = nullptr;
-        if ((rc = sched_acquire(ctx, st, &sched))) return rc;
-        F::launch(k, gsz, kConsumerThreads + 32, smem, st, c, tmap, pe, pf, g, cfg, plan->d_hdr, plan->d_q2, sched, src, dst);
-        sched_release(ctx, st);
-    } else {
-        int lines = 0;
-        const dim3 grid = direct_grid(ctx, c.fr.sz1, c.fr.sz2, nframes, &lines);
-        F::launch(F::direct(exact), grid, kConsumerThreads, 0, st, c, pe, pf, g, lines, src, dst);
-    }
-    ctx->launches++;
-    CC_CUDA(cudaGetLastError());
-    return CC_OK;
-}
-
 // --------------------------------------------------------------------------------------
-// Frames with different views in ONE launch (cc_rectify_*_views; the reference's plot loop,
-// src/plot_calibration.jl:36-42).  The views of a group share the frame layout, so they share the tensor map
-// and -- with the largest footprint of the group as the common staged box -- the ring; what differs per view
-// (coordinate parameters, axes, tile headers, q2 terms) is indexed by the unit's view.  One launch per view
-// (round 2's first version) spent more time in 64 ramp-ups, tails and host launches than in the work.
+// Group plans: the device tables of every staged launch.  The tile headers and q2 terms of 1..64 views for their
+// common staged box (the largest footprint of the group: any box at least as large as a view's footprint gives the
+// same pixels), concatenated per view; a single-view launch reads the plan of its one view.  Plans of one view take
+// the first NPLAN slots of ctx->group_plans, plans of more views the last NGROUP; each part evicts round-robin.
+// One lifecycle, whichever call installs the plan:
+//   - its tables go up on ctx->rect_upload, and every launch that reads them waits for `ready` (plan_read_begin);
+//   - `fence` follows the last launch that read them (plan_read_end); a launch on another stream waits for it
+//     first, so it covers every reader;
+//   - an evicted plan's buffers are overwritten after its fence (the upload stream waits for it) or, when too
+//     small, the plan is retired and freed once its fence has passed;
+//   - its host tables go once `ready` has passed: a device call waits for its own upload at once, a host call
+//     (RectViewsHost) at its end, or when it evicts the plan earlier.
+// Nothing here synchronises the device.
 // --------------------------------------------------------------------------------------
-struct MultiPlan {
+struct GroupPlan {
     std::vector<PlanKey> keys;     // the views of the group, in order
     BoxDims d;                     // the common staged box
     int n1, n2;
     TileHdr* d_hdr;                // [view][tile]
     double* d_q2;                  // [view][sz2]
     size_t hdr_cap, q2_cap;        // bytes allocated at d_hdr / d_q2
-    int per_sm[2];
-    size_t per_sm_smem[2];
     std::vector<TileHdr> h_hdr;    // the tables on the host, until their upload has completed
     std::vector<double> h_q2;
-    // The host form (cc_rectify_views_*_host) uploads on its own stream: `ready` follows the upload, and the slot
-    // streams wait for it.  `fence` follows the last launches that read the tables, on `fence_stream` (a device
-    // call on another stream waits for it first, so it covers every reader): the host form reuses or frees the
-    // buffers of an evicted plan after it, without synchronising the device.
-    cudaEvent_t ready;
-    cudaEvent_t fence;
+    cudaEvent_t ready;             // follows the upload; nullptr once it has completed
+    cudaEvent_t fence;             // follows the last launch that read the tables, on fence_stream
     cudaStream_t fence_stream;
-    bool fenced;
-    MultiPlan* next_retired;       // cc_ctx::multi_retired: evicted, freed once its fence has passed
+    int pins;                      // groups of a host call whose chunks are still being enqueued: never evicted
+    GroupPlan* next_retired;       // cc_ctx::plans_retired
 };
 
-static void multi_free(void* p) {
-    MultiPlan* mp = static_cast<MultiPlan*>(p);
+static void group_free(GroupPlan* mp) {
     if (!mp) return;
     if (mp->d_hdr) cudaFree(mp->d_hdr);
     if (mp->d_q2) cudaFree(mp->d_q2);
@@ -811,23 +683,53 @@ static void multi_free(void* p) {
     delete mp;
 }
 
-// plans retired by the host form: their readers are fenced, so this waits for those only
-static void multi_free_retired(cc_ctx* ctx) {
-    MultiPlan* mp = static_cast<MultiPlan*>(ctx->multi_retired);
-    ctx->multi_retired = nullptr;
+// retired plans: this waits for their readers only
+static void retired_free(cc_ctx* ctx) {
+    GroupPlan* mp = static_cast<GroupPlan*>(ctx->plans_retired);
+    ctx->plans_retired = nullptr;
     while (mp) {
-        MultiPlan* next = mp->next_retired;
-        if (mp->fenced) cudaEventSynchronize(mp->fence);
-        multi_free(mp);
+        GroupPlan* next = mp->next_retired;
+        cudaEventSynchronize(mp->fence);
+        group_free(mp);
         mp = next;
     }
 }
 
-static MultiPlan* multi_find(cc_ctx* ctx, const std::vector<PlanKey>& keys) {
-    for (int i = 0; i < cc_ctx::NMULTI; ++i) {
-        MultiPlan* mp = static_cast<MultiPlan*>(ctx->multi_plans[i]);
-        if (mp && mp->keys.size() == keys.size() && memcmp(mp->keys.data(), keys.data(), keys.size() * sizeof(PlanKey)) == 0)
-            return mp;
+// the host tables of a plan, once its upload has completed
+static cudaError_t group_release_host(GroupPlan* mp) {
+    cudaError_t e = cudaSuccess;
+    if (mp->ready) {
+        e = cudaEventSynchronize(mp->ready);
+        cudaEventDestroy(mp->ready);
+        mp->ready = nullptr;
+    }
+    std::vector<TileHdr>().swap(mp->h_hdr);
+    std::vector<double>().swap(mp->h_q2);
+    return e;
+}
+
+void rectify_free_plans(cc_ctx* ctx) {
+    for (void*& p : ctx->rect_plans) { delete static_cast<RectPlan*>(p); p = nullptr; }
+    for (void*& p : ctx->group_plans) { group_free(static_cast<GroupPlan*>(p)); p = nullptr; }
+    retired_free(ctx);
+    if (ctx->rect_upload) { cudaStreamSynchronize(ctx->rect_upload); cudaStreamDestroy(ctx->rect_upload); ctx->rect_upload = nullptr; }
+    if (ctx->rect_join) { cudaStreamSynchronize(ctx->rect_join); cudaStreamDestroy(ctx->rect_join); ctx->rect_join = nullptr; }
+    for (int k = 0; k < cc_ctx::NSLOT; ++k)
+        if (ctx->rect_join_event[k]) { cudaEventDestroy(ctx->rect_join_event[k]); ctx->rect_join_event[k] = nullptr; }
+}
+
+// the slots of plans of `nviews` views: their part of ctx->group_plans and its round-robin counter
+struct PlanSlots { void** at; int n; int* next; };
+static PlanSlots plan_slots(cc_ctx* ctx, size_t nviews) {
+    const int part = nviews == 1 ? 0 : 1;
+    return {ctx->group_plans + (part ? cc_ctx::NPLAN : 0), part ? cc_ctx::NGROUP : cc_ctx::NPLAN, &ctx->group_plan_next[part]};
+}
+
+static GroupPlan* group_find(cc_ctx* ctx, const PlanKey* keys, size_t nviews) {
+    const PlanSlots s = plan_slots(ctx, nviews);
+    for (int i = 0; i < s.n; ++i) {
+        GroupPlan* mp = static_cast<GroupPlan*>(s.at[i]);
+        if (mp && mp->keys.size() == nviews && memcmp(mp->keys.data(), keys, nviews * sizeof(PlanKey)) == 0) return mp;
     }
     return nullptr;
 }
@@ -865,7 +767,7 @@ static std::vector<int> plans_missing(const std::vector<PlanKey>& keys, const st
 
 // the common box and the host tables of a group from its views' footprints (host arithmetic only);
 // nullptr: a view has no plan (out of memory) or the group cannot be staged
-static MultiPlan* multi_assemble(const std::vector<PlanKey>& keys, const std::vector<RectPlan*>& pl, int pxb) {
+static GroupPlan* group_assemble(const std::vector<PlanKey>& keys, const std::vector<RectPlan*>& pl, int pxb) {
     const int nviews = (int)keys.size();
     int need1 = 0, need2 = 0;
     long long tilt = 0;
@@ -874,7 +776,7 @@ static MultiPlan* multi_assemble(const std::vector<PlanKey>& keys, const std::ve
         need1 = std::max(need1, pl[v]->need1); need2 = std::max(need2, pl[v]->need2);
         tilt += pl[v]->tilt;
     }
-    MultiPlan* mp = new (std::nothrow) MultiPlan();
+    GroupPlan* mp = new (std::nothrow) GroupPlan();
     if (!mp) return nullptr;
     mp->keys = keys;
     mp->d = box_dims(need1, need2, tilt >= 0 ? 1 : -1, pxb);
@@ -893,61 +795,145 @@ static MultiPlan* multi_assemble(const std::vector<PlanKey>& keys, const std::ve
     return mp;
 }
 
-// find or build the plan of a group of views; nullptr: not stageable (or out of memory) -- the caller falls
-// back to one launch per view
-static MultiPlan* multi_get(cc_ctx* ctx, const ChainD* chs, const double* ratios, const RectGeom* gs, int nviews,
-                            int tw, int tl, int pxb, cudaStream_t st) {
-    std::vector<PlanKey> keys((size_t)nviews);
-    for (int v = 0; v < nviews; ++v) keys[v] = plan_key(chs[v], ratios[v], gs[v], tw, tl, pxb);
-    if (MultiPlan* mp = multi_find(ctx, keys)) return mp;
-    // footprints per view: the cached RectPlans, the missing ones built on host threads and cached without their
-    // device tables (the group uploads its own).  Assembled before inserting: inserting may evict an earlier plan.
-    std::vector<RectPlan*> pl((size_t)nviews, nullptr);
-    for (int v = 0; v < nviews; ++v) pl[v] = plan_find(ctx, keys[v]);
-    const std::vector<int> missing = plans_missing(keys, pl);
-    plans_build(keys, pl, missing);
-    MultiPlan* mp = multi_assemble(keys, pl, pxb);
+// Installs mp (host tables assembled) in a slot of its part and enqueues the upload of its tables.  The slot's
+// plan is evicted (a host call pins at most two plans, and a part has four slots or more).  Takes mp: freed on
+// failure.
+static cudaError_t group_install(cc_ctx* ctx, GroupPlan* mp) {
+    const PlanSlots s = plan_slots(ctx, mp->keys.size());
+    int slot = -1;
+    for (int i = 0; i < s.n && slot < 0; ++i) {
+        const int k = (*s.next + i) % s.n;
+        if (!s.at[k] || !static_cast<GroupPlan*>(s.at[k])->pins) slot = k;
+    }
+    *s.next = slot + 1;
+    const size_t hb = mp->h_hdr.size() * sizeof(TileHdr), qb = mp->h_q2.size() * sizeof(double);
+    cudaError_t e = ctx->rect_upload ? cudaSuccess : cudaStreamCreateWithFlags(&ctx->rect_upload, cudaStreamNonBlocking);
+    if (GroupPlan* old = static_cast<GroupPlan*>(s.at[slot])) {
+        s.at[slot] = nullptr;
+        group_release_host(old);                            // an upload of this host call may still read them
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->rect_upload, old->fence, 0);
+        if (e == cudaSuccess && old->hdr_cap >= hb && old->q2_cap >= qb) {   // overwritten after its readers
+            mp->d_hdr = old->d_hdr; mp->d_q2 = old->d_q2; mp->hdr_cap = old->hdr_cap; mp->q2_cap = old->q2_cap;
+            old->d_hdr = nullptr; old->d_q2 = nullptr;
+            group_free(old);
+        } else {
+            old->next_retired = static_cast<GroupPlan*>(ctx->plans_retired);
+            ctx->plans_retired = old;
+        }
+    }
+    if (e == cudaSuccess && !mp->d_hdr) {                   // room for the most views of its part: later plans reuse it
+        const size_t most = mp->keys.size() == 1 ? 1 : kMaxViews;
+        const size_t hcap = std::max(hb, (size_t)mp->n1 * mp->n2 * most * sizeof(TileHdr));
+        const size_t qcap = std::max(qb, (size_t)mp->keys[0].g.sz2 * most * sizeof(double));
+        if ((e = cudaMalloc(&mp->d_hdr, hcap)) == cudaSuccess) e = cudaMalloc(&mp->d_q2, qcap);
+        mp->hdr_cap = hcap; mp->q2_cap = qcap;
+    }
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&mp->ready, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&mp->fence, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(mp->d_hdr, mp->h_hdr.data(), hb, cudaMemcpyHostToDevice, ctx->rect_upload);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(mp->d_q2, mp->h_q2.data(), qb, cudaMemcpyHostToDevice, ctx->rect_upload);
+    if (e == cudaSuccess) e = cudaEventRecord(mp->ready, ctx->rect_upload);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        if (ctx->rect_upload) cudaStreamSynchronize(ctx->rect_upload);   // no copy out of mp left in flight
+        group_free(mp);
+        return e;
+    }
+    s.at[slot] = mp;
+    return cudaSuccess;
+}
+
+// The plan of views keys[0, n) for a device call: cached, or built from the views' footprints (the cached ones; the
+// missing ones built on host threads and cached as well) and installed.  The call waits for its own upload only,
+// then the host tables go.  nullptr: the views cannot be staged together (or out of memory): the caller falls back.
+static GroupPlan* plan_get(cc_ctx* ctx, const PlanKey* keys, int n, int pxb) {
+    if (GroupPlan* mp = group_find(ctx, keys, (size_t)n)) return mp;
+    const std::vector<PlanKey> kv(keys, keys + n);
+    std::vector<RectPlan*> pl((size_t)n, nullptr);
+    for (int v = 0; v < n; ++v) pl[v] = plan_find(ctx, keys[v]);
+    const std::vector<int> missing = plans_missing(kv, pl);
+    plans_build(kv, pl, missing);
+    GroupPlan* mp = group_assemble(kv, pl, pxb);           // before inserting: inserting may evict a footprint it reads
     for (int v : missing) if (pl[v]) plan_insert(ctx, pl[v]);
     if (!mp) return nullptr;
-    const size_t hb = mp->h_hdr.size() * sizeof(TileHdr), qb = mp->h_q2.size() * sizeof(double);
-    if (cudaMalloc(&mp->d_hdr, hb) != cudaSuccess || cudaMalloc(&mp->d_q2, qb) != cudaSuccess ||
-        cudaMemcpyAsync(mp->d_hdr, mp->h_hdr.data(), hb, cudaMemcpyHostToDevice, st) != cudaSuccess ||
-        cudaMemcpyAsync(mp->d_q2, mp->h_q2.data(), qb, cudaMemcpyHostToDevice, st) != cudaSuccess) {
-        cudaGetLastError();
-        multi_free(mp);
-        return nullptr;
-    }
-    mp->hdr_cap = hb; mp->q2_cap = qb;
-    cudaStreamSynchronize(st);         // the host vectors go away; later calls may come on other streams
-    std::vector<TileHdr>().swap(mp->h_hdr);
-    std::vector<double>().swap(mp->h_q2);
-    const int slot = ctx->multi_plan_next++ % cc_ctx::NMULTI;
-    if (ctx->multi_plans[slot]) {
-        cudaDeviceSynchronize();       // an evicted plan may still be read by a running kernel
-        multi_free(ctx->multi_plans[slot]);
-    }
-    ctx->multi_plans[slot] = mp;
+    retired_free(ctx);
+    if (group_install(ctx, mp) != cudaSuccess) return nullptr;
+    group_release_host(mp);
     return mp;
 }
 
-// a launch on `st` reads mp's tables: readers on another stream come first (the fence then covers them all)
-static void multi_read_begin(MultiPlan* mp, cudaStream_t st) {
+// a launch on `st` reads mp's tables: after their upload, and after the readers on another stream (the fence then
+// covers them all)
+static void plan_read_begin(GroupPlan* mp, cudaStream_t st) {
     if (mp->ready) cudaStreamWaitEvent(st, mp->ready, 0);
-    if (mp->fenced && mp->fence_stream != st) cudaStreamWaitEvent(st, mp->fence, 0);
+    if (mp->fence_stream != st) cudaStreamWaitEvent(st, mp->fence, 0);
 }
-static void multi_read_end(MultiPlan* mp, cudaStream_t st) {
-    if (!mp->fence && cudaEventCreateWithFlags(&mp->fence, cudaEventDisableTiming) != cudaSuccess) { mp->fence = nullptr; return; }
+static void plan_read_end(GroupPlan* mp, cudaStream_t st) {
     cudaEventRecord(mp->fence, st);
-    mp->fenced = true;
     mp->fence_stream = st;
 }
 
+// One launch of the single-view kernels: frames [0, nframes) of view v at src / dst (the call's layout), on st.
+template <typename PX>
+int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const PX* src, PX* dst, cudaStream_t st) {
+    using F = RectFmt<PX>;
+    if (nframes == 0) return CC_OK;
+    const ChainD& ch = c.views.chs[v];
+    const double ratio = c.views.ratios[v];
+    const RectGeom g = make_geom(c.views.axs_mins + 2 * v, c.fr.sz1, c.fr.sz2, c.fr.pitch, c.fr.frame_stride, nframes);
+    const RectExact pe = make_exact(ch, ratio);
+    const RectFast pf = make_fast(ch, ratio, g);
+    const bool exact = !(c.flags & CC_COORD_F32);
+    CUtensorMap tmap;
+    TileCfg cfg;
+    memset(&cfg, 0, sizeof(cfg));
+    // the staged kernel applies when TMA can address the frames and the view's footprint can be staged
+    GroupPlan* mp = nullptr;
+    if (!(c.flags & CC_GATHER_DIRECT) && F::dst_ok(dst, c.fr, nframes) && tma_aligned(src, F::pxb, g.pitch, g.frame_stride, nframes) &&
+        encoder(ctx)) {
+        const PlanKey key = plan_key(ch, ratio, g, kT, F::tl, F::pxb);
+        mp = plan_get(ctx, &key, 1, F::pxb);
+        if (mp && !stage_box(ctx, src, F::pxb, g.sz1, g.sz2, g.pitch, g.frame_stride, nframes, mp->d, &tmap, &cfg)) mp = nullptr;
+    }
+    if ((c.flags & CC_GATHER_TMA) && !mp)
+        return set_error(CC_ERR_INVALID_ARG, "TMA gather not available for this layout / footprint");
+    int rc = CC_OK;
+    if (mp) {
+        if ((rc = unit_cfg(ctx, &cfg, c.fr.sz1, c.fr.sz2, nframes, kT, F::tl, exact ? F::fg_exact : F::fg_fast))) return rc;
+        int nf = 1;
+        const size_t smem = F::ring(cfg, false, &nf);
+        const auto k = F::staged(exact, nf);
+        uint32_t gsz = 0;
+        if ((rc = persistent_grid(ctx, F::staged_slot(nf) + !exact, k, smem, cfg, &gsz))) return rc;
+        RectSched* sched = nullptr;
+        if ((rc = sched_acquire(ctx, st, &sched))) return rc;
+        plan_read_begin(mp, st);
+        F::launch(k, gsz, kConsumerThreads + 32, smem, st, c, tmap, pe, pf, g, cfg, mp->d_hdr, mp->d_q2, sched, src, dst);
+        plan_read_end(mp, st);
+        sched_release(ctx, st);
+    } else {
+        int lines = 0;
+        const dim3 grid = direct_grid(ctx, c.fr.sz1, c.fr.sz2, nframes, &lines);
+        F::launch(F::direct(exact), grid, kConsumerThreads, 0, st, c, pe, pf, g, lines, src, dst);
+    }
+    ctx->launches++;
+    CC_CUDA(cudaGetLastError());
+    return CC_OK;
+}
+
+// --------------------------------------------------------------------------------------
+// Frames with different views in ONE launch (cc_rectify_*_views; the reference's plot loop,
+// src/plot_calibration.jl:36-42).  The views of a group share the frame layout, so they share the tensor map
+// and -- with the largest footprint of the group as the common staged box -- the ring; what differs per view
+// (coordinate parameters, axes, tile headers, q2 terms) is indexed by the unit's view.  One launch per view
+// (round 2's first version) spent more time in 64 ramp-ups, tails and host launches than in the work.
+// --------------------------------------------------------------------------------------
 struct ViewsLaunch {
     CUtensorMap tmap;
     TileCfg cfg;
     ViewTable vt;
     RectGeom g;
-    MultiPlan* mp;
+    GroupPlan* mp;
 };
 
 // frame groups of fg frames (inside views of fpv frames) that meet frames [w0, w0 + wn) of a group; *g0: the first
@@ -963,7 +949,7 @@ static long long window_groups(int fpv, int fg, int w0, int wn, uint32_t* g0) {
 // tensor map, unit configuration and view table of one launch of a group's plan (views [v0, v0 + nv) of the call)
 // over frames [w0, w0 + wn) of the group; src: the window's first frame.  *ok = false: the launch does not apply
 template <typename PX>
-static int views_window(cc_ctx* ctx, MultiPlan* mp, const RectCall<PX>& c, int v0, int nv, const PX* src, int w0,
+static int views_window(cc_ctx* ctx, GroupPlan* mp, const RectCall<PX>& c, int v0, int nv, const PX* src, int w0,
                         int wn, ViewsLaunch* L, bool* ok) {
     using F = RectFmt<PX>;
     const RectFrames& fr = c.fr;
@@ -1009,14 +995,14 @@ static int views_run(cc_ctx* ctx, ViewsLaunch* L, const RectCall<PX>& c, const P
     const size_t smem = F::ring(L->cfg, true, &nf);
     const auto k = F::views(exact);
     uint32_t gsz = 0;
-    int rc = persistent_grid(ctx, F::views_slot + !exact, k, smem, L->cfg, L->mp, exact, &gsz);
+    int rc = persistent_grid(ctx, F::views_slot + !exact, k, smem, L->cfg, &gsz);
     RectSched* sched = nullptr;
     if (!rc) rc = sched_acquire(ctx, st, &sched);
     if (rc) return rc;
-    multi_read_begin(L->mp, st);
+    plan_read_begin(L->mp, st);
     F::launch(k, gsz, kConsumerThreads + 32, smem, st, c, L->tmap, L->vt, L->g, L->cfg, L->mp->d_hdr, L->mp->d_q2, sched,
               src, dst);
-    multi_read_end(L->mp, st);
+    plan_read_end(L->mp, st);
     sched_release(ctx, st);
     ctx->launches++;
     CC_CUDA(cudaGetLastError());
@@ -1035,10 +1021,12 @@ int launch_rectify_group(cc_ctx* ctx, const RectCall<PX>& c, int v0, int nv, con
     if ((c.flags & CC_GATHER_DIRECT) || !F::dst_ok(dst, fr, nframes) || nv < 1 || nv > kMaxViews || fr.fpv < 1 ||
         !tma_aligned(src, F::pxb, fr.pitch, fr.frame_stride, nframes) || !encoder(ctx))
         return CC_OK;
-    std::vector<RectGeom> gs((size_t)nv);
-    for (int v = 0; v < nv; ++v)
-        gs[v] = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, nframes);
-    MultiPlan* mp = multi_get(ctx, c.views.chs + v0, c.views.ratios + v0, gs.data(), nv, kT, F::tl, F::pxb, st);
+    std::vector<PlanKey> keys((size_t)nv);
+    for (int v = 0; v < nv; ++v) {
+        const RectGeom g = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, nframes);
+        keys[v] = plan_key(c.views.chs[v0 + v], c.views.ratios[v0 + v], g, kT, F::tl, F::pxb);
+    }
+    GroupPlan* mp = plan_get(ctx, keys.data(), nv, F::pxb);
     if (!mp) {
         if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %d not stageable (pxb %d)\n", nv, F::pxb);
         return CC_OK;
@@ -1052,9 +1040,9 @@ int launch_rectify_group(cc_ctx* ctx, const RectCall<PX>& c, int v0, int nv, con
 // --------------------------------------------------------------------------------------
 // Frames of many views from host memory (cc_rectify_views_*_host): the chunk pipeline of abi.cu moves the
 // frames; this session owns the group plans of the call.  Each group of up to 64 views gets its plan once per
-// call.  A missing plan is built on host threads while the device streams the previous group's chunks, goes up
-// on the context's upload stream, and the slot streams wait for its `ready` event.  Nothing here synchronises
-// the device: an evicted plan's buffers are reused (or retired) after its fence.
+// call.  A missing plan is built on host threads while the device streams the previous group's chunks, then
+// installed like any other (group_install).  The plan of a group is pinned from the moment the call takes it
+// until the group's last chunk is enqueued, so no install of the call evicts it.
 // --------------------------------------------------------------------------------------
 struct RectViewsHost {
     cc_ctx* ctx;
@@ -1062,7 +1050,7 @@ struct RectViewsHost {
     RectFrames fr;                         // the layout of the slot buffers: frames pitch * sz2 apart
     int ngroups, pxb, tl;
     bool stage;                            // the layout can be staged at all
-    std::vector<MultiPlan*> mp;            // per group: its plan (nullptr: per-view launches)
+    std::vector<GroupPlan*> mp;            // per group: its plan, pinned until retired (nullptr: per-view launches)
     std::vector<char> state;               // per group: 0 nothing yet, 1 being built, 2 ready
     std::vector<char> used;                // per group: a launch read its plan since the last fence
     // the group being built off this thread: keys, copies of the cached footprints, result
@@ -1070,10 +1058,7 @@ struct RectViewsHost {
     std::thread job;
     std::vector<PlanKey> job_keys;
     std::vector<RectPlan> job_found;
-    MultiPlan* job_out;
-    std::vector<MultiPlan*> installed;     // plans this call uploaded (their host tables go at the end)
-    std::vector<std::vector<TileHdr>> held_hdr;   // host tables of plans evicted during the call (uploads in flight)
-    std::vector<std::vector<double>> held_q2;
+    GroupPlan* job_out;
 };
 
 static std::vector<PlanKey> group_keys(const RectViewsHost* h, int gi) {
@@ -1090,7 +1075,12 @@ static std::vector<PlanKey> group_keys(const RectViewsHost* h, int gi) {
 static void vh_start(RectViewsHost* h, int gi) {
     if (gi >= h->ngroups || h->state[gi] || !h->stage) return;
     std::vector<PlanKey> keys = group_keys(h, gi);
-    if (MultiPlan* mp = multi_find(h->ctx, keys)) { h->mp[gi] = mp; h->state[gi] = 2; return; }
+    if (GroupPlan* mp = group_find(h->ctx, keys.data(), keys.size())) {
+        h->mp[gi] = mp;
+        ++mp->pins;
+        h->state[gi] = 2;
+        return;
+    }
     // copies of the cached footprints: the context's plan cache may change while the job runs
     h->job_found.clear();
     h->job_found.reserve(keys.size());
@@ -1107,71 +1097,28 @@ static void vh_start(RectViewsHost* h, int gi) {
         for (size_t v = 0; v < keys.size(); ++v) if (found_at[v] >= 0) pl[v] = &h->job_found[found_at[v]];
         const std::vector<int> missing = plans_missing(keys, pl);
         plans_build(keys, pl, missing);
-        h->job_out = multi_assemble(keys, pl, h->pxb);
-        for (int v : missing) plan_free(pl[v]);        // the footprints live on in the group plan only
+        h->job_out = group_assemble(keys, pl, h->pxb);
+        for (int v : missing) delete pl[v];            // the footprints live on in the group plan only
     };
     try { h->job = std::thread(work); }
     catch (...) { work(); }                             // no thread to be had: built here
 }
 
-// wait for the job of group gi; the tables go up on the upload stream into a free or evicted slot (never the
-// plan of group gi - 1, whose chunks may still be enqueued)
+// wait for the job of group gi and install its plan
 static int vh_install(RectViewsHost* h, int gi) {
-    cc_ctx* ctx = h->ctx;
     if (h->job.joinable()) h->job.join();
     h->job_found.clear();
-    MultiPlan* mp = h->job_out;
+    GroupPlan* mp = h->job_out;
     h->job_out = nullptr;
     h->state[gi] = 2;
     if (!mp) {
         if (getenv("CAMCAL_DEBUG")) fprintf(stderr, "[camcal] views: group of %zu not stageable (pxb %d)\n", h->job_keys.size(), h->pxb);
         return CC_OK;
     }
-    const MultiPlan* keep = gi > 0 ? h->mp[gi - 1] : nullptr;
-    int slot = -1;
-    for (int i = 0; i < cc_ctx::NMULTI && slot < 0; ++i) {
-        const int s = (ctx->multi_plan_next + i) % cc_ctx::NMULTI;
-        if (!ctx->multi_plans[s] || ctx->multi_plans[s] != keep) slot = s;
-    }
-    ctx->multi_plan_next = slot + 1;
-    const size_t hb = mp->h_hdr.size() * sizeof(TileHdr), qb = mp->h_q2.size() * sizeof(double);
-    if (MultiPlan* old = static_cast<MultiPlan*>(ctx->multi_plans[slot])) {
-        ctx->multi_plans[slot] = nullptr;
-        h->installed.erase(std::remove(h->installed.begin(), h->installed.end(), old), h->installed.end());
-        h->held_hdr.emplace_back(); h->held_hdr.back().swap(old->h_hdr);
-        h->held_q2.emplace_back(); h->held_q2.back().swap(old->h_q2);
-        if (old->fenced) CC_CUDA(cudaStreamWaitEvent(ctx->rect_upload, old->fence, 0));
-        if (old->hdr_cap >= hb && old->q2_cap >= qb) {  // same frame size: the upload overwrites it after its readers
-            mp->d_hdr = old->d_hdr; mp->d_q2 = old->d_q2; mp->hdr_cap = old->hdr_cap; mp->q2_cap = old->q2_cap;
-            old->d_hdr = nullptr; old->d_q2 = nullptr;
-            multi_free(old);
-        } else {                                        // freed at the start of the next host call
-            old->next_retired = static_cast<MultiPlan*>(ctx->multi_retired);
-            ctx->multi_retired = old;
-        }
-    }
-    if (!mp->d_hdr) {                                   // room for a full group: later groups of this size reuse it
-        const size_t hcap = std::max(hb, (size_t)mp->n1 * mp->n2 * kMaxViews * sizeof(TileHdr));
-        const size_t qcap = std::max(qb, (size_t)h->fr.sz2 * kMaxViews * sizeof(double));
-        if (cudaMalloc(&mp->d_hdr, hcap) != cudaSuccess || cudaMalloc(&mp->d_q2, qcap) != cudaSuccess) {
-            cudaGetLastError();
-            multi_free(mp);
-            return set_error(CC_ERR_CUDA, "out of device memory for the tile plans of a group of views");
-        }
-        mp->hdr_cap = hcap; mp->q2_cap = qcap;
-    }
-    if (cudaEventCreateWithFlags(&mp->ready, cudaEventDisableTiming) != cudaSuccess) {
-        mp->ready = nullptr;
-        multi_free(mp);
-        cudaGetLastError();
-        return set_error(CC_ERR_CUDA, "cannot create the upload event of a group plan");
-    }
-    ctx->multi_plans[slot] = mp;
-    h->installed.push_back(mp);
+    const cudaError_t e = group_install(h->ctx, mp);
+    if (e != cudaSuccess) return cuda_fail(e, "tile plans of a group of views");
     h->mp[gi] = mp;
-    CC_CUDA(cudaMemcpyAsync(mp->d_hdr, mp->h_hdr.data(), hb, cudaMemcpyHostToDevice, ctx->rect_upload));
-    CC_CUDA(cudaMemcpyAsync(mp->d_q2, mp->h_q2.data(), qb, cudaMemcpyHostToDevice, ctx->rect_upload));
-    CC_CUDA(cudaEventRecord(mp->ready, ctx->rect_upload));
+    ++mp->pins;
     return CC_OK;
 }
 
@@ -1180,8 +1127,7 @@ template <typename PX>
 int rect_vh_begin(cc_ctx* ctx, const RectCall<PX>& dc, RectViewsHost** out) {
     using F = RectFmt<PX>;
     *out = nullptr;
-    multi_free_retired(ctx);
-    if (!ctx->rect_upload) CC_CUDA(cudaStreamCreateWithFlags(&ctx->rect_upload, cudaStreamNonBlocking));
+    retired_free(ctx);
     if (!ctx->rect_join) CC_CUDA(cudaStreamCreateWithFlags(&ctx->rect_join, cudaStreamNonBlocking));
     for (int k = 0; k < cc_ctx::NSLOT; ++k)
         if (!ctx->rect_join_event[k]) CC_CUDA(cudaEventCreateWithFlags(&ctx->rect_join_event[k], cudaEventDisableTiming));
@@ -1227,32 +1173,35 @@ int rect_vh_launch(RectViewsHost* h, const RectCall<PX>& dc, int gi, int w0, int
     return views_run(h->ctx, &L, dc, src, dst, st);
 }
 
-// no chunk of this call reads group gi's plan after the ones enqueued so far: its fence joins the slot streams
+// no chunk of this call reads group gi's plan after the ones enqueued so far: its fence joins the slot streams, and
+// the plan is unpinned
 void rect_vh_retire(RectViewsHost* h, int gi) {
     cc_ctx* ctx = h->ctx;
-    MultiPlan* mp = gi < h->ngroups ? h->mp[gi] : nullptr;
-    if (!mp || !h->used[gi]) return;
+    GroupPlan* mp = gi < h->ngroups ? h->mp[gi] : nullptr;
+    if (!mp) return;
+    h->mp[gi] = nullptr;
+    --mp->pins;
+    if (!h->used[gi]) return;
     h->used[gi] = 0;
     for (int k = 0; k < cc_ctx::NSLOT; ++k) {
         if (!ctx->pipe_stream[k]) continue;
         cudaEventRecord(ctx->rect_join_event[k], ctx->pipe_stream[k]);
         cudaStreamWaitEvent(ctx->rect_join, ctx->rect_join_event[k], 0);
     }
-    multi_read_end(mp, ctx->rect_join);
+    plan_read_end(mp, ctx->rect_join);
 }
 
-// after the last chunk (or an error): every plan fenced, the uploads complete, the host tables released
+// after the last chunk (or an error): every plan fenced and unpinned, the uploads complete, the host tables released
 int rect_vh_end(RectViewsHost* h) {
     if (!h) return CC_OK;
     cc_ctx* ctx = h->ctx;
     if (h->job.joinable()) h->job.join();
-    if (h->job_out) multi_free(h->job_out);
+    group_free(h->job_out);
     for (int gi = 0; gi < h->ngroups; ++gi) rect_vh_retire(h, gi);
-    const cudaError_t e = cudaStreamSynchronize(ctx->rect_upload);
-    for (MultiPlan* mp : h->installed) {
-        std::vector<TileHdr>().swap(mp->h_hdr);
-        std::vector<double>().swap(mp->h_q2);
-        if (mp->ready) { cudaEventDestroy(mp->ready); mp->ready = nullptr; }
+    cudaError_t e = cudaSuccess;
+    for (void* p : ctx->group_plans) {
+        const cudaError_t r = p ? group_release_host(static_cast<GroupPlan*>(p)) : cudaSuccess;
+        if (e == cudaSuccess) e = r;
     }
     delete h;
     return e == cudaSuccess ? CC_OK : cuda_fail(e, "plan upload");

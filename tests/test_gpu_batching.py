@@ -59,11 +59,11 @@ def _env(**kv):
 
 
 _STAGED = re.compile(r"\[camcal\] staged: box \d+x\d+ pitch \d+ \((\d+) B\) stages (\d+) units (\d+) "
-                     r"\(fg (\d+)\) grid \d+ \(\d+/SM\) smem (\d+)")
+                     r"\(fg (\d+)\) grid \d+ \((\d+)/SM\) smem (\d+)")
 
 
 def _staged_lines(err):
-    return [dict(zip(("box_bytes", "stages", "units", "fg", "smem"), map(int, m))) for m in _STAGED.findall(err)]
+    return [dict(zip(("box_bytes", "stages", "units", "fg", "per_sm", "smem"), map(int, m))) for m in _STAGED.findall(err)]
 
 
 def _one_staged(err):
@@ -87,7 +87,7 @@ def _mirror_fg(units_per_group, fg_max, n):
 
 
 def _check_ring(d, fmt, fg):
-    """Stages and shared memory of the launch the debug line reports (rectify.cu, plan_tma and the launchers):
+    """Stages and shared memory of the launch the debug line reports (rectify.cu, stage_box and the launchers):
     a 48 KB ring of 2..8 boxes, at most 56 KB; f32 puts two frames in a stage when the ring holds >= 4 boxes and
     the units have >= 2 frames (rectify_f32c1_kernel, NF == 2).  Returns True when the pair kernel ran."""
     bb = d["box_bytes"]
@@ -281,6 +281,33 @@ def test_staged_frame_groups_small_frame(cc, capfd, small, fmt, coord, fg):
 def test_staged_frame_groups_large_box(cc, capfd, large_box, coord, fg):
     """A ring of fewer than 4 boxes keeps one frame per stage whatever the group size."""
     _sweep(cc, capfd, large_box, "f32", coord, fg, lambda fg_eff: False)
+
+
+def test_occupancy_belongs_to_the_kernel(cc, capfd):
+    """The resident CTAs per SM of a staged kernel depend on the kernel, not on which kernel ran first on a plan.
+    With fast coordinates the fp32 pair kernel and the single-frame kernel have different register counts (84 and
+    75), and on a ring of an even number of stages they ask for the same shared memory (a 3.5 KB box: 8 stages of
+    one frame or 4 of two).  1, 64, 1 frames on one plan and 64, 1, 64 on a second plan with the same box: each
+    kernel reports the same CTAs per SM in both orders, and one frame alone equals the first frame of the 64."""
+    case = _Case(cc, (1024, 768), 64, seed=1600, ratio_scale=1.5, ramps=())
+    fd = case.dev("f32")
+    per_sm, box = {False: set(), True: set()}, set()
+    for ratio, order in ((case.ratio, (1, 64, 1)), (case.ratio * (1 + 1e-9), (64, 1, 64))):
+        outs = {}
+        for n in order:
+            out = _prefilled(fd[:n], "f32", F_SENT)
+            capfd.readouterr()
+            with _env(CAMCAL_DEBUG="1"):
+                cc.warp(case.c, 0, fd[:n], ratio, case.axs, fill=F_FILL, coord="f32", out=out)
+            d = _one_staged(capfd.readouterr().err)
+            pair = _check_ring(d, "f32", d["fg"])
+            assert pair == (n == 64) and d["stages"] * (2 if pair else 1) == 8, (ratio, n, d)
+            per_sm[pair].add(d["per_sm"])
+            box.add((d["box_bytes"], d["smem"]))
+            outs[n] = out
+        assert torch.equal(outs[1][0].view(torch.int32), outs[64][0].view(torch.int32)), ratio
+    assert len(box) == 1, box                            # one box and one shared-memory size for both kernels
+    assert len(per_sm[False]) == 1 and len(per_sm[True]) == 1, per_sm
 
 
 def _u8_stageable(sz):

@@ -520,23 +520,29 @@ def test_rectify_u8c3_exact_ties_take_the_fp64_blend(cc):
         assert (ref != np.array([9, 8, 7], dtype=np.uint8)).any()
 
 
-def test_rectify_plan_cache_many_parameter_sets(cc):
-    """More parameter sets than the context caches tile plans for (64), revisited in a different
-    order and on two streams: every call must match the oracle (plans are keyed by calibration,
-    ratio, axes and frame geometry; an evicted plan is rebuilt)."""
+def _plan_cache_cases(cc):
+    """67 parameter sets of one 128 x 96 camera, more than the context caches one-view plans for (64): the
+    calibration, (view, chain, ratio, axes) per set, two frames on the device and the oracle's results"""
     sz = (128, 96)
     intr = camera_for(sz)
     rng = np.random.default_rng(3)
     frames = rng.random((2, sz[1], sz[0]), dtype=np.float32)
-    fd = _dev(frames)
     cases = []
-    N = 67
-    for i in range(N):
+    for i in range(67):
         view = ((0.05 + 0.004 * i, -0.04, 0.02 * (i % 3)), (-9.3 + 0.05 * i, -6.4, 30.0 + 0.3 * i))
         ch, ip, ratio, axs = _rect_case(intr, sz, view=view)
         cases.append((view, ch, ratio, axs))
     c = _calib(cc, intr, [v for v, _, _, _ in cases])
     refs = [oc.rectify_f32c1(ch, 1.0 / ratio, axs, frames, fill=-3.0) for _, ch, ratio, axs in cases]
+    return c, cases, _dev(frames), refs
+
+
+def test_rectify_plan_cache_many_parameter_sets(cc):
+    """More parameter sets than the context caches tile plans for (64), revisited in a different
+    order and on two streams: every call must match the oracle (plans are keyed by calibration,
+    ratio, axes and frame geometry; an evicted plan is rebuilt)."""
+    c, cases, fd, refs = _plan_cache_cases(cc)
+    N = len(cases)
     side = torch.cuda.Stream()
     side.wait_stream(torch.cuda.current_stream())
     for order in (range(N), reversed(range(N)), (0, 5, 0, N - 1, 5, 0)):
@@ -548,6 +554,25 @@ def test_rectify_plan_cache_many_parameter_sets(cc):
                 got2 = cc.warp(c, i, fd, ratio, axs, fill=-3.0, coord="f64")
             side.synchronize()
             assert np.array_equal(got2.cpu().numpy(), refs[i]), i
+
+
+def test_rectify_plan_cache_unsynchronised_streams(cc):
+    """The same 67 parameter sets in the same three orders, the calls alternating between two streams with no
+    synchronisation until the end: plans are evicted and rebuilt while launches on the other stream may still
+    read them.  Every output must match the oracle."""
+    c, cases, fd, refs = _plan_cache_cases(cc)
+    N = len(cases)
+    streams = (torch.cuda.current_stream(), torch.cuda.Stream())
+    streams[1].wait_stream(streams[0])
+    outs = []
+    for order in (range(N), reversed(range(N)), (0, 5, 0, N - 1, 5, 0)):
+        for j, i in enumerate(order):
+            _, ch, ratio, axs = cases[i]
+            with torch.cuda.stream(streams[j % 2]):
+                outs.append((i, cc.warp(c, i, fd, ratio, axs, fill=-3.0)))
+    torch.cuda.synchronize()
+    for i, out in outs:
+        assert np.array_equal(out.cpu().numpy(), refs[i]), i
 
 
 def test_rectify_alternating_large_and_small_boxes(cc):

@@ -329,24 +329,42 @@ def test_gather_direct_and_repeated_views(cc, capfd, fmt):
 @pytest.mark.parametrize("fmt", ["f32", "u8"])
 def test_host_call_between_device_calls(cc, fmt, coord):
     """device _views (caller's stream, not synchronised) -> host form with the same groups -> device _views
-    again: all three agree bit for bit."""
-    sz = (256, 192)
-    vs = _Views(cc, 70, sz, scale=0.015)
-    frames = vs.frames(fmt, 140, 1500)
+    again: all three agree bit for bit.  65 views: a group of 64 and a group of one, whose plan is a one-view
+    plan.  Before and after the host call, single-view warp calls of views 0..63 run on a side stream that is
+    never synchronised until the end: their one-view plans push the last group's plan out of the cache, so the
+    host call installs it again over a plan that a side-stream launch may still read.  Each single-view result
+    equals its view's frames of the device call."""
+    sz, nv = (256, 192), 65
+    vs = _Views(cc, nv, sz, scale=0.015)
+    frames = vs.frames(fmt, 2 * nv, 1500)
     fd = _dev(frames)
     outs = []
     for _ in range(2):
         o = torch.empty_like(fd)
         o[...] = torch.tensor(_sent(fmt), dtype=o.dtype, device=o.device)
         outs.append(o)
-    cc.warp_views(vs.c, list(range(70)), fd, vs.ratios, vs.axss, fill=_fill(fmt), coord=coord, out=outs[0])
+    side = torch.cuda.Stream()
+    side.wait_stream(torch.cuda.current_stream())
+
+    def singles():
+        with torch.cuda.stream(side):
+            return [cc.warp(vs.c, v, fd[2 * v:2 * v + 2], vs.ratios[v], vs.axss[v], fill=_fill(fmt), coord=coord)
+                    for v in range(GROUP)]
+
+    cc.warp_views(vs.c, list(range(nv)), fd, vs.ratios, vs.axss, fill=_fill(fmt), coord=coord, out=outs[0])
+    before = singles()
     host = _out_like(frames, fmt)
     with _env(CAMCAL_CHUNK_MB="1"):
         assert vs.host(fmt, frames, host, coord=coord) == 0
-    cc.warp_views(vs.c, list(range(70)), fd, vs.ratios, vs.axss, fill=_fill(fmt), coord=coord, out=outs[1])
+    after = singles()
+    cc.warp_views(vs.c, list(range(nv)), fd, vs.ratios, vs.axss, fill=_fill(fmt), coord=coord, out=outs[1])
+    torch.cuda.synchronize()
     a, b = outs[0].cpu().numpy(), outs[1].cpu().numpy()
     _assert_equal(host, a, "host vs device before")
     _assert_equal(b, a, "device after vs before")
+    for v in range(GROUP):
+        _assert_equal(before[v].cpu().numpy(), a[2 * v:2 * v + 2], ("single before", v))
+        _assert_equal(after[v].cpu().numpy(), a[2 * v:2 * v + 2], ("single after", v))
     if coord == "f64":
         _assert_equal(host, vs.oracle(fmt, frames, 2), "oracle")
 
