@@ -106,6 +106,10 @@ _SIGS = {
     "cc_rectify_u8c3_views": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _sz, _sz, _i, _u8p, _u, _vp]),
     "cc_rectify_views_f32c1_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _sz, _sz, _i, _f, _u]),
     "cc_rectify_views_u8c3_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _vp, _vp, _i, _i, _sz, _sz, _i, _u8p, _u]),
+    "cc_rectify_axes_f32c1": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _i, _vp, _i, _i, _sz, _sz, _vp, _sz, _sz, _i, _f, _u, _vp]),
+    "cc_rectify_axes_u8c3": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _i, _vp, _i, _i, _sz, _sz, _vp, _sz, _sz, _i, _u8p, _u, _vp]),
+    "cc_rectify_axes_f32c1_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _i, _vp, _i, _i, _sz, _sz, _vp, _sz, _sz, _i, _f, _u]),
+    "cc_rectify_axes_u8c3_host": (_i, [_vp, _pI, _vp, _i, _vp, _vp, _i, _i, _vp, _i, _i, _sz, _sz, _vp, _sz, _sz, _i, _u8p, _u]),
     "cc_rectify_map_f64": (_i, [_vp, _pI, _pV, _d, _i64p, _vp, _vp, _i, _i, _sz, _vp]),
     "cc_rectify_map_f32": (_i, [_vp, _pI, _pV, _d, _i64p, _vp, _vp, _i, _i, _sz, _vp]),
     "cc_jpeg_info": (_i, [_vp, _sz, C.POINTER(_i), C.POINTER(_i), C.POINTER(_i)]),

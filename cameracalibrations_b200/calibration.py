@@ -316,10 +316,13 @@ def image_transformations(c: Calibration, extrinsic_index, imgpointss, checker_s
     return ratio, get_axes(ratio, checker_size, n_corners, sz)
 
 
-def _frames(frames, fill, coord: str, gather: str, out, single: bool):
+def _frames(frames, fill, coord: str, gather: str, out, single: bool, out_size=None):
     """What warp and warp_views share: the frames as the library reads them, C-contiguous (a numpy array that is
     not uint8 becomes float32), whether they are uint8 RGB, the output buffer, the fill value and the flags.
-    single: a frame without the leading axis is a batch of one, and the last value returned says so."""
+    single: a frame without the leading axis is a batch of one, and the last value returned says so.
+    out_size = (out_sz1, out_sz2): output frames of that size, (nframes, out_sz2, out_sz1[, 3]); `out` must have
+    that shape (a single frame: without the leading axis) and the frames' dtype and be C-contiguous on the frames'
+    device."""
     flags = {"f64": _lib.COORD_F64, "f32": _lib.COORD_F32}[coord] | {
         "auto": _lib.GATHER_AUTO, "direct": _lib.GATHER_DIRECT, "tma": _lib.GATHER_TMA}[gather]
     if _is_torch(frames):
@@ -335,8 +338,22 @@ def _frames(frames, fill, coord: str, gather: str, out, single: bool):
         frames = frames.reshape((1,) + tuple(frames.shape))
     if frames.ndim != (4 if u8 else 3) or (u8 and frames.shape[-1] != 3):
         raise ValueError("frames must be (nframes, sz2, sz1) float32 or (nframes, sz2, sz1, 3) uint8")
-    if out is None:
-        out = torch.empty_like(frames) if _is_torch(frames) else np.empty_like(frames)
+    if out_size is None:
+        if out is None:
+            out = torch.empty_like(frames) if _is_torch(frames) else np.empty_like(frames)
+    else:
+        o1, o2 = int(out_size[0]), int(out_size[1])
+        shape = (int(frames.shape[0]), o2, o1) + ((3,) if u8 else ())
+        if out is None:
+            out = (torch.empty(shape, dtype=frames.dtype, device=frames.device) if _is_torch(frames)
+                   else np.empty(shape, dtype=frames.dtype))
+        else:
+            want = shape[1:] if one else shape        # a single frame without the leading axis: out without it too
+            if (tuple(out.shape) != want or out.dtype != frames.dtype or _is_torch(out) != _is_torch(frames)
+                    or (_is_torch(out) and out.device != frames.device)
+                    or not (out.is_contiguous() if _is_torch(out) else out.flags.c_contiguous)):
+                raise ValueError(f"out must be a C-contiguous {want} array of the frames' dtype and device")
+            out = out.reshape(shape)
     if u8:
         fv = (C.c_uint8 * 3)(*([0, 0, 0] if fill is None else [int(v) for v in fill]))
     else:
@@ -345,7 +362,7 @@ def _frames(frames, fill, coord: str, gather: str, out, single: bool):
 
 
 def warp(c: Calibration, extrinsic, frames, ratio: float, axs_min, fill=None, coord: str = "f64",
-         gather: str = "auto", out=None):
+         gather: str = "auto", out=None, out_size=None):
     """warp(img, tform, axs), src/plot_calibration.jl:40, for a batch of frames of one view.
 
     frames: float32 (nframes, sz2, sz1) or uint8 (nframes, sz2, sz1, 3), C-contiguous -- i.e.
@@ -353,12 +370,21 @@ def warp(c: Calibration, extrinsic, frames, ratio: float, axs_min, fill=None, co
     frame may omit the leading axis.  numpy -> host pipeline; CUDA torch tensor -> device.
     fill defaults to the reference's: NaN for float frames, black for RGB{N0f8}.
     coord: "f64" (reference precision, bit-exact index/weight selection) | "f32" (fast path).
+    out_size = (out_sz1, out_sz2): output axes axs_min .+ (0:out_sz1-1, 0:out_sz2-1) of any size (downscale, crop,
+    upscale), result (nframes, out_sz2, out_sz1[, 3]) (cc_rectify_axes_*); None: the input's size.
     """
     vi = c._index(extrinsic)
-    frames, u8, out, fv, flags, one = _frames(frames, fill, coord, gather, out, single=True)
+    frames, u8, out, fv, flags, one = _frames(frames, fill, coord, gather, out, single=True, out_size=out_size)
     nframes, sz2, sz1 = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
     axs = (C.c_int64 * 2)(int(axs_min[0]), int(axs_min[1]))
     ctx, ptr, host, tail = _where(frames)
+    if out_size is not None:
+        o1, o2 = int(out_size[0]), int(out_size[1])
+        fn = getattr(lib, f"cc_rectify_axes_{'u8c3' if u8 else 'f32c1'}{host}")
+        check(fn(ctx.handle, C.byref(c._intr), (_lib.View * 1)(c._views[vi]), 1, (C.c_double * 1)(float(ratio)), axs,
+                 o1, o2, ptr(frames), sz1, sz2, C.c_size_t(sz1), C.c_size_t(sz1 * sz2), ptr(out), C.c_size_t(o1),
+                 C.c_size_t(o1 * o2), nframes, fv, flags, *tail))
+        return out[0] if one else out
     fn = getattr(lib, f"cc_rectify_{'u8c3' if u8 else 'f32c1'}{host}")
     check(fn(ctx.handle, C.byref(c._intr), C.byref(c._views[vi]), float(ratio), axs, ptr(frames), ptr(out),
              sz1, sz2, C.c_size_t(sz1), C.c_size_t(sz1 * sz2), nframes, fv, flags, *tail))
@@ -366,17 +392,18 @@ def warp(c: Calibration, extrinsic, frames, ratio: float, axs_min, fill=None, co
 
 
 def warp_views(c: Calibration, extrinsics, frames, ratios, axs_mins, fill=None, coord: str = "f64",
-               gather: str = "auto", out=None):
+               gather: str = "auto", out=None, out_size=None):
     """Rectify frames that belong to DIFFERENT views in one call -- the loop of the reference's plot
     (src/plot_calibration.jl:36-42: every calibration image with its own extrinsic, ratio, axes).
 
     extrinsics: view indices / file names, one per group; frames: (nviews * k, sz2, sz1) float32 or
     (nviews * k, sz2, sz1, 3) uint8 -- frames [v*k, (v+1)*k) belong to extrinsics[v]; ratios[v], axs_mins[v]
     as returned by image_transformations for that view.  A CUDA tensor is rectified on its stream; a numpy
-    array takes the host pipeline over all views in one call (cc_rectify_views_*_host) and returns numpy."""
+    array takes the host pipeline over all views in one call (cc_rectify_views_*_host) and returns numpy.
+    out_size = (out_sz1, out_sz2): every view's output axes have that size, as for warp (cc_rectify_axes_*)."""
     vis = [c._index(e) for e in extrinsics]
     nv = len(vis)
-    frames, u8, out, fv, flags, _ = _frames(frames, fill, coord, gather, out, single=False)
+    frames, u8, out, fv, flags, _ = _frames(frames, fill, coord, gather, out, single=False, out_size=out_size)
     if nv == 0 or frames.shape[0] % nv:
         raise ValueError("frames must be (nviews * k, sz2, sz1) float32 or (nviews * k, sz2, sz1, 3) uint8")
     k, sz2, sz1 = int(frames.shape[0]) // nv, int(frames.shape[1]), int(frames.shape[2])
@@ -385,6 +412,12 @@ def warp_views(c: Calibration, extrinsics, frames, ratios, axs_mins, fill=None, 
     axs = (C.c_int64 * (2 * nv))(*[int(a) for am in axs_mins for a in am])
     ctx, ptr, host, tail = _where(frames)
     kern = "u8c3" if u8 else "f32c1"
+    if out_size is not None:
+        o1, o2 = int(out_size[0]), int(out_size[1])
+        fn = getattr(lib, f"cc_rectify_axes_{kern}{host}")
+        check(fn(ctx.handle, C.byref(c._intr), views, nv, rat, axs, o1, o2, ptr(frames), sz1, sz2, C.c_size_t(sz1),
+                 C.c_size_t(sz1 * sz2), ptr(out), C.c_size_t(o1), C.c_size_t(o1 * o2), k, fv, flags, *tail))
+        return out
     fn = getattr(lib, f"cc_rectify_views_{kern}_host" if host else f"cc_rectify_{kern}_views")
     check(fn(ctx.handle, C.byref(c._intr), views, nv, rat, axs, ptr(frames), ptr(out), sz1, sz2, C.c_size_t(sz1),
              C.c_size_t(sz1 * sz2), k, fv, flags, *tail))

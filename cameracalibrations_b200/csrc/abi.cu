@@ -295,8 +295,9 @@ static std::vector<int> chunk_schedule(int nframes, size_t frame_bytes, int max_
 // Every rectification entry point calls rectify_device or rectify_host with its views and its frame layout: a
 // single-view call is one view whose frames per view are the call's nframes; `many` marks the `_views` calls.
 
-// Every rule of a rectification call, checked before anything is written, enqueued or the device is touched.  The
-// map entry points pass fr.fpv = 0: no frames.
+// Every rule of a rectification call, checked before anything is written, enqueued or the device is touched: the
+// source's, then the output's (the same as the source's unless the call is cc_rectify_axes_*).  The map entry points
+// pass fr.fpv = 0: no frames.
 static int check_rect(const cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
                       const int64_t* axs_mins, const RectFrames& fr, const void* src, const void* dst, bool fill_ok) {
     CC_REQUIRE(ctx != nullptr, "ctx is NULL");
@@ -313,6 +314,12 @@ static int check_rect(const cc_ctx* ctx, const cc_intr* intr, const cc_view* vie
         CC_REQUIRE(fr.pitch >= (size_t)fr.sz1, "pitch smaller than sz1");
         CC_REQUIRE(nframes <= 1 || fr.frame_stride >= fr.pitch * (size_t)(fr.sz2 - 1) + fr.sz1, "frames overlap");
         CC_REQUIRE(fr.pitch * (size_t)fr.sz2 < (size_t)1 << 30, "frame too large (pitch*sz2 must be < 2^30)");
+        CC_REQUIRE(fr.out_sz1 > 0 && fr.out_sz2 > 0, "output size must be positive");
+        CC_REQUIRE(fr.out_sz1 < (1 << 22) && fr.out_sz2 < (1 << 22), "output extent must be < 2^22");
+        CC_REQUIRE(fr.out_pitch >= (size_t)fr.out_sz1, "out_pitch smaller than out_sz1");
+        CC_REQUIRE(nframes <= 1 || fr.out_frame_stride >= fr.out_pitch * (size_t)(fr.out_sz2 - 1) + fr.out_sz1,
+                   "output frames overlap");
+        CC_REQUIRE(fr.out_pitch * (size_t)fr.out_sz2 < (size_t)1 << 30, "output frame too large (out_pitch*out_sz2 must be < 2^30)");
     }
     const int64_t lim = (int64_t)1 << 30;
     for (int v = 0; v < nviews; ++v) {
@@ -355,7 +362,8 @@ static int rectify_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views
     c.views.chs = chs.data();
     cudaStream_t stream_ = (cudaStream_t)stream;
     if (!many) return launch_rectify(ctx, c, 0, fr.fpv, src, dst, stream_);
-    const size_t view_elems = (size_t)fr.fpv * fr.frame_stride * RectPx<PX>::channels;
+    const size_t view_elems = (size_t)fr.fpv * fr.frame_stride * RectPx<PX>::channels;          // source
+    const size_t out_view_elems = (size_t)fr.fpv * fr.out_frame_stride * RectPx<PX>::channels;  // output
     std::vector<char> done((size_t)nviews, 0);
     bool single = true;
     if (const char* e = getenv("CAMCAL_VIEWS_SINGLE")) single = atoi(e) != 0;
@@ -364,7 +372,7 @@ static int rectify_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views
     for (int v0 = 0; single && v0 < nviews; v0 += per) {
         const int nv = std::min(per, nviews - v0);
         bool ok = false;
-        if ((rc = launch_rectify_group(ctx, c, v0, nv, src + v0 * view_elems, dst + v0 * view_elems, stream_, &ok)))
+        if ((rc = launch_rectify_group(ctx, c, v0, nv, src + v0 * view_elems, dst + v0 * out_view_elems, stream_, &ok)))
             return rc;
         if (ok) { for (int v = v0; v < v0 + nv; ++v) done[v] = 1; ndone += nv; }
     }
@@ -386,7 +394,7 @@ static int rectify_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views
     for (int v = 0; v < nviews; ++v) {
         if (done[v]) continue;
         cudaStream_t st = lanes > 1 ? ctx->pipe_stream[v % lanes] : stream_;
-        if ((rc = launch_rectify(ctx, c, v, fr.fpv, src + v * view_elems, dst + v * view_elems, st))) break;
+        if ((rc = launch_rectify(ctx, c, v, fr.fpv, src + v * view_elems, dst + v * out_view_elems, st))) break;
     }
     if (lanes > 1) {                                  // join even after an error: nothing stays forked
         for (int k = 0; k < lanes; ++k) {
@@ -401,18 +409,19 @@ static int rectify_device(cc_ctx* ctx, const cc_intr* intr, const cc_view* views
     return rc;
 }
 
-// m frames from `from` to `to` (kind: which way): one side is a slot, frames pitch * sz2 apart, the other the caller's
-// host frames, frame_stride apart.  One copy when the host frames are dense, else one 2-D copy per frame.
-static int copy_frames(const RectFrames& fr, size_t pxb, int m, const void* from, void* to, cudaMemcpyKind kind,
-                       cudaStream_t st) {
-    const size_t line = fr.pitch * pxb, slot_frame = line * fr.sz2, host_frame = fr.frame_stride * pxb;
-    const bool up = kind == cudaMemcpyHostToDevice, dense = host_frame == slot_frame && fr.pitch == (size_t)fr.sz1;
+// m frames of sz1 x sz2 pixels from `from` to `to` (kind: which way): one side is a slot, frames pitch * sz2 apart, the
+// other the caller's host frames, frame_stride apart (an upload moves source frames, a download output frames).  One
+// copy when the host frames are dense, else one 2-D copy per frame.
+static int copy_frames(int sz1, int sz2, size_t pitch, size_t frame_stride, size_t pxb, int m, const void* from, void* to,
+                       cudaMemcpyKind kind, cudaStream_t st) {
+    const size_t line = pitch * pxb, slot_frame = line * sz2, host_frame = frame_stride * pxb;
+    const bool up = kind == cudaMemcpyHostToDevice, dense = host_frame == slot_frame && pitch == (size_t)sz1;
     const size_t from_frame = up ? host_frame : slot_frame, to_frame = up ? slot_frame : host_frame;
     for (int f = 0; f < (dense ? 1 : m); ++f) {
         const uint8_t* s = static_cast<const uint8_t*>(from) + (size_t)f * from_frame;
         uint8_t* d = static_cast<uint8_t*>(to) + (size_t)f * to_frame;
         const cudaError_t e = dense ? cudaMemcpyAsync(d, s, (size_t)m * slot_frame, kind, st)
-                                    : cudaMemcpy2DAsync(d, line, s, line, (size_t)fr.sz1 * pxb, fr.sz2, kind, st);
+                                    : cudaMemcpy2DAsync(d, line, s, line, (size_t)sz1 * pxb, sz2, kind, st);
         if (e != cudaSuccess) return cuda_fail(e, "copy");
     }
     return CC_OK;
@@ -438,18 +447,24 @@ static int rectify_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, 
     std::vector<ChainD> chs((size_t)nviews);
     for (int v = 0; v < nviews; ++v) build_chain(intr, views + v, &chs[v]);
     c.views.chs = chs.data();
-    const size_t pxb = RectPx<PX>::bytes, frame_bytes = fr.pitch * (size_t)fr.sz2 * pxb;
+    const size_t pxb = RectPx<PX>::bytes, frame_bytes = fr.pitch * (size_t)fr.sz2 * pxb,
+                 out_frame_bytes = fr.out_pitch * (size_t)fr.out_sz2 * pxb;
     c.fr.frame_stride = fr.pitch * (size_t)fr.sz2;           // device frames are stored pitch*sz2
+    c.fr.out_frame_stride = fr.out_pitch * (size_t)fr.out_sz2;
     const int nframes = nviews * fr.fpv, gframes = many ? rectify_views_per_launch() * fr.fpv : nframes;
     int per = 0;
-    const std::vector<int> chunks = chunk_schedule(nframes, frame_bytes, gframes, &per);
+    // the chunk is sized by the larger side of a frame: neither slot buffer exceeds the chunk bytes
+    const std::vector<int> chunks = chunk_schedule(nframes, std::max(frame_bytes, out_frame_bytes), gframes, &per);
     const int nchunks = (int)chunks.size();
     std::vector<int> first((size_t)nchunks + 1, 0);
     for (int i = 0; i < nchunks; ++i) first[i + 1] = first[i] + chunks[i];
     const uint8_t* hsrc = reinterpret_cast<const uint8_t*>(src);
     uint8_t* hdst = reinterpret_cast<uint8_t*>(dst);
-    // frame f of a chunk in slot buffer p
-    auto at = [&](void* p, int f) { return reinterpret_cast<PX*>(static_cast<uint8_t*>(p) + (size_t)f * frame_bytes); };
+    // frame f of a chunk in slot k's input / output buffer
+    auto at = [&](int k, int f) { return reinterpret_cast<PX*>(static_cast<uint8_t*>(ctx->pipe_in[k]) + (size_t)f * frame_bytes); };
+    auto out_at = [&](int k, int f) {
+        return reinterpret_cast<PX*>(static_cast<uint8_t*>(ctx->pipe_out[k]) + (size_t)f * out_frame_bytes);
+    };
     RectViewsHost* vh = nullptr;
     if (many && (rc = rect_vh_begin(ctx, c, &vh))) return rc;
     std::vector<char> uploaded((size_t)nchunks, 0), prepared((size_t)((nframes + gframes - 1) / gframes), 0);
@@ -458,9 +473,10 @@ static int rectify_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, 
     auto upload = [&](int i) -> int {
         if (i >= nchunks || uploaded[i]) return CC_OK;
         const int k = i % cc_ctx::NSLOT;
-        int r = ensure_slot(ctx, k, per * frame_bytes + 64, per * frame_bytes + 64);
-        if (!r) r = copy_frames(fr, pxb, chunks[i], hsrc + (size_t)first[i] * fr.frame_stride * pxb, ctx->pipe_in[k],
-                                cudaMemcpyHostToDevice, ctx->pipe_stream[k]);
+        int r = ensure_slot(ctx, k, per * frame_bytes + 64, per * out_frame_bytes + 64);
+        if (!r) r = copy_frames(fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, pxb, chunks[i],
+                                hsrc + (size_t)first[i] * fr.frame_stride * pxb, ctx->pipe_in[k], cudaMemcpyHostToDevice,
+                                ctx->pipe_stream[k]);
         uploaded[i] = r == CC_OK;
         return r;
     };
@@ -477,20 +493,19 @@ static int rectify_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, 
         if (rc) break;
         const int k = i % cc_ctx::NSLOT;
         cudaStream_t st = ctx->pipe_stream[k];
-        if (!vh) rc = launch_rectify(ctx, c, 0, m, at(ctx->pipe_in[k], 0), at(ctx->pipe_out[k], 0), st);
+        if (!vh) rc = launch_rectify(ctx, c, 0, m, at(k, 0), out_at(k, 0), st);
         for (int gi = g_lo; vh && rc == CC_OK && gi <= g_hi; ++gi) {
             const int a = std::max(f0, gi * gframes), b = std::min(f0 + m, (gi + 1) * gframes);
             bool ok = false;
-            rc = rect_vh_launch(vh, c, gi, a - gi * gframes, b - a, at(ctx->pipe_in[k], a - f0),
-                                at(ctx->pipe_out[k], a - f0), st, &ok);
+            rc = rect_vh_launch(vh, c, gi, a - gi * gframes, b - a, at(k, a - f0), out_at(k, a - f0), st, &ok);
             for (int v = a / fr.fpv; rc == CC_OK && !ok && v <= (b - 1) / fr.fpv; ++v) {
                 const int fa = std::max(a, v * fr.fpv), fb = std::min(b, (v + 1) * fr.fpv);
-                rc = launch_rectify(ctx, c, v, fb - fa, at(ctx->pipe_in[k], fa - f0), at(ctx->pipe_out[k], fa - f0), st);
+                rc = launch_rectify(ctx, c, v, fb - fa, at(k, fa - f0), out_at(k, fa - f0), st);
             }
         }
         if (rc) break;
-        rc = copy_frames(fr, pxb, m, ctx->pipe_out[k], hdst + (size_t)f0 * fr.frame_stride * pxb, cudaMemcpyDeviceToHost,
-                         st);
+        rc = copy_frames(fr.out_sz1, fr.out_sz2, fr.out_pitch, fr.out_frame_stride, pxb, m, ctx->pipe_out[k],
+                         hdst + (size_t)f0 * fr.out_frame_stride * pxb, cudaMemcpyDeviceToHost, st);
         for (; vh && (retired < g_hi || (retired == g_hi && f0 + m == std::min(nframes, (g_hi + 1) * gframes))); ++retired)
             rect_vh_retire(vh, retired);
     }
@@ -503,7 +518,7 @@ static int rectify_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, 
 template <typename T>
 static int rectify_map(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio, const int64_t* axs_min,
                        T* map_row, T* map_col, int sz1, int sz2, size_t pitch, void* stream) {
-    int rc = check_rect(ctx, intr, view, 1, &ratio, axs_min, {sz1, sz2, pitch, pitch * (size_t)sz2, 0}, nullptr,
+    int rc = check_rect(ctx, intr, view, 1, &ratio, axs_min, rect_frames(sz1, sz2, pitch, pitch * (size_t)sz2, 0), nullptr,
                         nullptr, true);
     if (rc) return rc;
     CC_REQUIRE(map_row && map_col, "NULL map pointer");
@@ -832,7 +847,7 @@ int cc_rectify_f32c1(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, doub
                      const int64_t axs_min[2], const float* src, float* dst, int sz1, int sz2,
                      size_t pitch, size_t frame_stride, int nframes, float fill, unsigned flags,
                      void* stream) {
-    return rectify_device(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+    return rectify_device(ctx, intr, view, 1, &ratio, axs_min, src, dst, rect_frames(sz1, sz2, pitch, frame_stride, nframes), fill,
                           flags, stream, false);
 }
 
@@ -840,7 +855,7 @@ int cc_rectify_u8c3(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, doubl
                     const int64_t axs_min[2], const uint8_t* src, uint8_t* dst, int sz1, int sz2,
                     size_t pitch, size_t frame_stride, int nframes, const uint8_t fill[3],
                     unsigned flags, void* stream) {
-    return rectify_device(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+    return rectify_device(ctx, intr, view, 1, &ratio, axs_min, src, dst, rect_frames(sz1, sz2, pitch, frame_stride, nframes), fill,
                           flags, stream, false);
 }
 
@@ -848,7 +863,7 @@ int cc_rectify_f32c1_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* view
                            const int64_t* axs_mins, const float* src, float* dst, int sz1, int sz2, size_t pitch,
                            size_t frame_stride, int frames_per_view, float fill, unsigned flags, void* stream) {
     return rectify_device(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
-                          {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, stream, true);
+                          rect_frames(sz1, sz2, pitch, frame_stride, frames_per_view), fill, flags, stream, true);
 }
 
 int cc_rectify_u8c3_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
@@ -856,14 +871,14 @@ int cc_rectify_u8c3_views(cc_ctx* ctx, const cc_intr* intr, const cc_view* views
                           size_t frame_stride, int frames_per_view, const uint8_t fill[3], unsigned flags,
                           void* stream) {
     return rectify_device(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
-                          {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, stream, true);
+                          rect_frames(sz1, sz2, pitch, frame_stride, frames_per_view), fill, flags, stream, true);
 }
 
 int cc_rectify_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,
                           const int64_t axs_min[2], const float* src, float* dst, int sz1, int sz2,
                           size_t pitch, size_t frame_stride, int nframes, float fill,
                           unsigned flags) {
-    return rectify_host(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+    return rectify_host(ctx, intr, view, 1, &ratio, axs_min, src, dst, rect_frames(sz1, sz2, pitch, frame_stride, nframes), fill,
                         flags, false);
 }
 
@@ -871,7 +886,7 @@ int cc_rectify_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, 
                          const int64_t axs_min[2], const uint8_t* src, uint8_t* dst, int sz1,
                          int sz2, size_t pitch, size_t frame_stride, int nframes,
                          const uint8_t fill[3], unsigned flags) {
-    return rectify_host(ctx, intr, view, 1, &ratio, axs_min, src, dst, {sz1, sz2, pitch, frame_stride, nframes}, fill,
+    return rectify_host(ctx, intr, view, 1, &ratio, axs_min, src, dst, rect_frames(sz1, sz2, pitch, frame_stride, nframes), fill,
                         flags, false);
 }
 
@@ -881,7 +896,7 @@ int cc_rectify_views_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view*
                                 int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
                                 float fill, unsigned flags) {
     return rectify_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
-                        {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, true);
+                        rect_frames(sz1, sz2, pitch, frame_stride, frames_per_view), fill, flags, true);
 }
 
 int cc_rectify_views_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
@@ -889,7 +904,47 @@ int cc_rectify_views_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* 
                                int sz1, int sz2, size_t pitch, size_t frame_stride, int frames_per_view,
                                const uint8_t fill[3], unsigned flags) {
     return rectify_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
-                        {sz1, sz2, pitch, frame_stride, frames_per_view}, fill, flags, true);
+                        rect_frames(sz1, sz2, pitch, frame_stride, frames_per_view), fill, flags, true);
+}
+
+// any output extent: output frames out_sz1 x out_sz2, lines out_pitch and frames out_frame_stride apart; one view takes
+// the single-view path, more the `_views` path
+int cc_rectify_axes_f32c1(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                          const int64_t* axs_mins, int out_sz1, int out_sz2, const float* src, int sz1, int sz2,
+                          size_t pitch, size_t frame_stride, float* dst, size_t out_pitch, size_t out_frame_stride,
+                          int frames_per_view, float fill, unsigned flags, void* stream) {
+    return rectify_device(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                          {sz1, sz2, pitch, frame_stride, frames_per_view, out_sz1, out_sz2, out_pitch, out_frame_stride},
+                          fill, flags, stream, nviews > 1);
+}
+
+int cc_rectify_axes_u8c3(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews, const double* ratios,
+                         const int64_t* axs_mins, int out_sz1, int out_sz2, const uint8_t* src, int sz1, int sz2,
+                         size_t pitch, size_t frame_stride, uint8_t* dst, size_t out_pitch, size_t out_frame_stride,
+                         int frames_per_view, const uint8_t fill[3], unsigned flags, void* stream) {
+    return rectify_device(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                          {sz1, sz2, pitch, frame_stride, frames_per_view, out_sz1, out_sz2, out_pitch, out_frame_stride},
+                          fill, flags, stream, nviews > 1);
+}
+
+int cc_rectify_axes_f32c1_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                               const double* ratios, const int64_t* axs_mins, int out_sz1, int out_sz2,
+                               const float* src, int sz1, int sz2, size_t pitch, size_t frame_stride, float* dst,
+                               size_t out_pitch, size_t out_frame_stride, int frames_per_view, float fill,
+                               unsigned flags) {
+    return rectify_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                        {sz1, sz2, pitch, frame_stride, frames_per_view, out_sz1, out_sz2, out_pitch, out_frame_stride},
+                        fill, flags, nviews > 1);
+}
+
+int cc_rectify_axes_u8c3_host(cc_ctx* ctx, const cc_intr* intr, const cc_view* views, int nviews,
+                              const double* ratios, const int64_t* axs_mins, int out_sz1, int out_sz2,
+                              const uint8_t* src, int sz1, int sz2, size_t pitch, size_t frame_stride, uint8_t* dst,
+                              size_t out_pitch, size_t out_frame_stride, int frames_per_view, const uint8_t fill[3],
+                              unsigned flags) {
+    return rectify_host(ctx, intr, views, nviews, ratios, axs_mins, src, dst,
+                        {sz1, sz2, pitch, frame_stride, frames_per_view, out_sz1, out_sz2, out_pitch, out_frame_stride},
+                        fill, flags, nviews > 1);
 }
 
 int cc_rectify_map_f64(cc_ctx* ctx, const cc_intr* intr, const cc_view* view, double ratio,

@@ -85,14 +85,21 @@ struct PointSrc {
 template <typename PX> struct RectPx;
 template <> struct RectPx<float> { static constexpr int channels = 1, bytes = 4; using Fill = float; };
 template <> struct RectPx<uint8_t> { static constexpr int channels = 3, bytes = 3; using Fill = uchar3; };
-// A rectification call.  Frames are sz1 x sz2 pixels, lines `pitch` pixels and frames `frame_stride` pixels apart.
-// View v (chs[v], ratios[v], axs_mins[2v .. 2v+1]) rectifies frames [v * fpv, (v + 1) * fpv); a single-view call is
-// one view with all the frames.
+// A rectification call.  Source frames are sz1 x sz2 pixels, lines `pitch` pixels and frames `frame_stride` pixels
+// apart; output frames out_sz1 x out_sz2, lines out_pitch and frames out_frame_stride apart (the cc_rectify_* entry
+// points other than cc_rectify_axes_*: the source's own geometry, rect_frames).  View v (chs[v], ratios[v],
+// axs_mins[2v .. 2v+1]) rectifies frames [v * fpv, (v + 1) * fpv); a single-view call is one view with all the frames.
 struct RectFrames {
     int sz1, sz2;
     size_t pitch, frame_stride;
     int fpv;
+    int out_sz1, out_sz2;
+    size_t out_pitch, out_frame_stride;
 };
+// a call whose output has the source's geometry
+inline RectFrames rect_frames(int sz1, int sz2, size_t pitch, size_t frame_stride, int fpv) {
+    return {sz1, sz2, pitch, frame_stride, fpv, sz1, sz2, pitch, frame_stride};
+}
 struct RectViews {
     const ChainD* chs;
     const double* ratios;

@@ -79,6 +79,10 @@ struct TileCfg {
 constexpr int kMaxViews = 64;
 struct ViewParams { RectExact pe; RectFast pf; RectGeom g; };
 struct ViewTable { ViewParams v[kMaxViews]; };
+// the parameters of the views kernels (tensor map, view table, geometry, configuration, five pointers, fill and frame
+// bytes, with alignment padding) must fit the 32764 bytes of kernel parameter space
+static_assert(sizeof(CUtensorMap) + sizeof(ViewTable) + sizeof(RectGeom) + sizeof(TileCfg) + 5 * sizeof(void*) + 64 <= 32764,
+              "the view table does not fit the kernel parameter space");
 
 // f32c1: per-tile header precomputed on the host (RectPlan), read straight from global memory
 struct __align__(16) TileHdr {
@@ -155,13 +159,14 @@ rectify_map_f32_kernel(const RectFast p, const RectGeom g, float* __restrict__ m
 // --------------------------------------------------------------------------------------
 // host side
 // --------------------------------------------------------------------------------------
-static RectGeom make_geom(const int64_t axs_min[2], int sz1, int sz2, size_t pitch,
-                          size_t frame_stride, int nframes) {
+// the geometry of `nframes` frames of a call: the output and the source of fr
+static RectGeom make_geom(const int64_t axs_min[2], const RectFrames& fr, int nframes) {
     RectGeom g;
     memset(&g, 0, sizeof(g));
     g.axs0 = (int)axs_min[0]; g.axs1 = (int)axs_min[1];
-    g.sz1 = sz1; g.sz2 = sz2; g.pitch = (long long)pitch; g.frame_stride = (long long)frame_stride;
+    g.sz1 = fr.out_sz1; g.sz2 = fr.out_sz2; g.pitch = (long long)fr.out_pitch; g.frame_stride = (long long)fr.out_frame_stride;
     g.nframes = nframes;
+    g.src_sz1 = fr.sz1; g.src_sz2 = fr.sz2; g.src_pitch = (long long)fr.pitch; g.src_frame_stride = (long long)fr.frame_stride;
     return g;
 }
 
@@ -207,7 +212,7 @@ static void host_coord(const ChainD& ch, double inv_ratio, long long I1, long lo
 
 // Tile plan.  For every output tile: the bounding box of its source footprint (32 samples on the
 // tile perimeter, evaluated in double) and everything the kernels derive from it.  A plan
-// depends on the calibration, ratio/axes, frame size and tile shape only -- not on the pixels --
+// depends on the calibration, ratio/axes, output and source frame sizes and tile shape only -- not on the pixels --
 // so it is built once on the host, uploaded once and reused by every later call with the same
 // parameters (a video stream): the kernels' producer warp then only issues TMA loads.
 //
@@ -278,12 +283,12 @@ static void plan_footprints(RectPlan* p, bool threads) {
             if (!finite) continue;                  // origin stays at (-4, -4): the range tests fail
             tilt += (c_last > c_first) - (c_last < c_first);
             // clamp so that far-away footprints still give a legal (fully out-of-frame) box
-            const double rc = std::min(std::max(rmin, -4.0), (double)g.sz1 + 4.0);
-            const double cc_ = std::min(std::max(cmin, -4.0), (double)g.sz2 + 4.0);
+            const double rc = std::min(std::max(rmin, -4.0), (double)g.src_sz1 + 4.0);
+            const double cc_ = std::min(std::max(cmin, -4.0), (double)g.src_sz2 + 4.0);
             p->origin[2 * t] = (int)std::floor(rc);
             p->origin[2 * t + 1] = (int)std::floor(cc_);
             // tiles entirely outside the frame never gather
-            if (rmax < 1.0 || cmax < 1.0 || rmin > g.sz1 || cmin > g.sz2) continue;
+            if (rmax < 1.0 || cmax < 1.0 || rmin > g.src_sz1 || cmin > g.src_sz2) continue;
             m1 = std::max(m1, (int)(std::floor(rmax) - std::floor(rmin)));
             m2 = std::max(m2, (int)(std::floor(cmax) - std::floor(cmin)));
         }
@@ -380,16 +385,16 @@ static void fill_headers(const RectPlan* p, const BoxDims& d, TileHdr* hdr) {
             const int x0 = floor_to(p->origin[2 * t] - 2, 4);
             h.x0 = x0;
             g_lo = std::max(0, x0);
-            g_hi = std::min(x0 + d.box1 - 2, g.sz1 - 2);
+            g_hi = std::min(x0 + d.box1 - 2, g.src_sz1 - 2);
             h.base_off = (uint32_t)(g_lo - x0) * 4u;
         } else {
             const int xb0 = floor_to((p->origin[2 * t] - 2) * 3, 16);
             h.x0 = xb0;
             g_lo = std::max(0, xb0 >= 0 ? (xb0 + 2) / 3 : 0);                       // 3 g1 >= xb0
-            g_hi = std::min((xb0 + d.pitch_b - 6) >= 0 ? (xb0 + d.pitch_b - 6) / 3 : -1, g.sz1 - 2);   // 3 g1 + 6 <= xb0 + pitch
+            g_hi = std::min((xb0 + d.pitch_b - 6) >= 0 ? (xb0 + d.pitch_b - 6) / 3 : -1, g.src_sz1 - 2);   // 3 g1 + 6 <= xb0 + pitch
             h.base_off = (uint32_t)(3 * g_lo - xb0);
         }
-        const int lo2 = std::max(0, -y0), hi2 = std::min(d.box2 - 2, g.sz2 - 2 - y0);
+        const int lo2 = std::max(0, -y0), hi2 = std::min(d.box2 - 2, g.src_sz2 - 2 - y0);
         h.y0 = y0;
         h.R1 = p->p3_ok[t] ? (uint32_t)std::max(0, g_hi - g_lo + 1) : 0u;
         h.R2 = (uint32_t)std::max(0, hi2 - lo2 + 1);
@@ -435,7 +440,7 @@ static void plan_insert(cc_ctx* ctx, RectPlan* p) {
 static PlanKey plan_key(const ChainD& ch, double ratio, const RectGeom& g, int tw, int tl, int pxb) {
     PlanKey key;
     memset(&key, 0, sizeof(key));
-    key.ch = ch; key.ratio = ratio; key.g = g; key.g.nframes = 0; key.g.frame_stride = 0;
+    key.ch = ch; key.ratio = ratio; key.g = g; key.g.nframes = 0; key.g.frame_stride = 0; key.g.src_frame_stride = 0;
     key.tw = tw; key.tl = tl; key.pxb = pxb;
     return key;
 }
@@ -631,10 +636,10 @@ template <> struct RectFmt<uint8_t> {
     }
     // the staged kernel writes whole 32-bit words: 4-byte aligned output lines
     static bool dst_ok(const uint8_t* dst, const RectFrames& fr, int nframes) {
-        return (reinterpret_cast<uintptr_t>(dst) & 3u) == 0 && ((fr.pitch * 3) & 3u) == 0 &&
-               (nframes <= 1 || ((fr.frame_stride * 3) & 3u) == 0);
+        return (reinterpret_cast<uintptr_t>(dst) & 3u) == 0 && ((fr.out_pitch * 3) & 3u) == 0 &&
+               (nframes <= 1 || ((fr.out_frame_stride * 3) & 3u) == 0);
     }
-    // frame_bytes: the bytes of one frame that belong to the caller (the last line is only sz1 pixels long)
+    // frame_bytes: the bytes of one source frame that belong to the caller (the last line is only sz1 pixels long)
     template <typename K, typename... A>
     static void launch(K k, dim3 grid, int threads, size_t smem, cudaStream_t st, const RectCall<uint8_t>& c,
                        const A&... a) {
@@ -880,7 +885,7 @@ int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const
     if (nframes == 0) return CC_OK;
     const ChainD& ch = c.views.chs[v];
     const double ratio = c.views.ratios[v];
-    const RectGeom g = make_geom(c.views.axs_mins + 2 * v, c.fr.sz1, c.fr.sz2, c.fr.pitch, c.fr.frame_stride, nframes);
+    const RectGeom g = make_geom(c.views.axs_mins + 2 * v, c.fr, nframes);
     const RectExact pe = make_exact(ch, ratio);
     const RectFast pf = make_fast(ch, ratio, g);
     const bool exact = !(c.flags & CC_COORD_F32);
@@ -889,17 +894,17 @@ int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const
     memset(&cfg, 0, sizeof(cfg));
     // the staged kernel applies when TMA can address the frames and the view's footprint can be staged
     GroupPlan* mp = nullptr;
-    if (!(c.flags & CC_GATHER_DIRECT) && F::dst_ok(dst, c.fr, nframes) && tma_aligned(src, F::pxb, g.pitch, g.frame_stride, nframes) &&
+    if (!(c.flags & CC_GATHER_DIRECT) && F::dst_ok(dst, c.fr, nframes) && tma_aligned(src, F::pxb, c.fr.pitch, c.fr.frame_stride, nframes) &&
         encoder(ctx)) {
         const PlanKey key = plan_key(ch, ratio, g, kT, F::tl, F::pxb);
         mp = plan_get(ctx, &key, 1, F::pxb);
-        if (mp && !stage_box(ctx, src, F::pxb, g.sz1, g.sz2, g.pitch, g.frame_stride, nframes, mp->d, &tmap, &cfg)) mp = nullptr;
+        if (mp && !stage_box(ctx, src, F::pxb, c.fr.sz1, c.fr.sz2, c.fr.pitch, c.fr.frame_stride, nframes, mp->d, &tmap, &cfg)) mp = nullptr;
     }
     if ((c.flags & CC_GATHER_TMA) && !mp)
         return set_error(CC_ERR_INVALID_ARG, "TMA gather not available for this layout / footprint");
     int rc = CC_OK;
     if (mp) {
-        if ((rc = unit_cfg(ctx, &cfg, c.fr.sz1, c.fr.sz2, nframes, kT, F::tl, exact ? F::fg_exact : F::fg_fast))) return rc;
+        if ((rc = unit_cfg(ctx, &cfg, c.fr.out_sz1, c.fr.out_sz2, nframes, kT, F::tl, exact ? F::fg_exact : F::fg_fast))) return rc;
         int nf = 1;
         const size_t smem = F::ring(cfg, false, &nf);
         const auto k = F::staged(exact, nf);
@@ -913,7 +918,7 @@ int launch_rectify(cc_ctx* ctx, const RectCall<PX>& c, int v, int nframes, const
         sched_release(ctx, st);
     } else {
         int lines = 0;
-        const dim3 grid = direct_grid(ctx, c.fr.sz1, c.fr.sz2, nframes, &lines);
+        const dim3 grid = direct_grid(ctx, c.fr.out_sz1, c.fr.out_sz2, nframes, &lines);
         F::launch(F::direct(exact), grid, kConsumerThreads, 0, st, c, pe, pf, g, lines, src, dst);
     }
     ctx->launches++;
@@ -957,8 +962,8 @@ static int views_window(cc_ctx* ctx, GroupPlan* mp, const RectCall<PX>& c, int v
     TileCfg& cfg = L->cfg;
     memset(&cfg, 0, sizeof(cfg));
     if (!stage_box(ctx, src, F::pxb, fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, wn, mp->d, &L->tmap, &cfg)) return CC_OK;
-    cfg.strips = (fr.sz1 + kT - 1) / kT;
-    cfg.ntiles2 = (fr.sz2 + F::tl - 1) / F::tl;
+    cfg.strips = (fr.out_sz1 + kT - 1) / kT;
+    cfg.ntiles2 = (fr.out_sz2 + F::tl - 1) / F::tl;
     cfg.tiles = cfg.strips * cfg.ntiles2;
     // frames per group: as unit_cfg (keep ~8 units per resident CTA slot), within a view
     const long long want = (long long)ctx->sm_count * 6 * 8;
@@ -974,7 +979,7 @@ static int views_window(cc_ctx* ctx, GroupPlan* mp, const RectCall<PX>& c, int v
     CC_REQUIRE(units < (1ll << 31), "too many tiles in one call: split the batch");
     cfg.units = (uint32_t)units;
     for (int v = 0; v < nv; ++v) {
-        const RectGeom gv = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, wn);
+        const RectGeom gv = make_geom(c.views.axs_mins + 2 * (v0 + v), fr, wn);
         L->vt.v[v].pe = make_exact(c.views.chs[v0 + v], c.views.ratios[v0 + v]);
         L->vt.v[v].pf = make_fast(c.views.chs[v0 + v], c.views.ratios[v0 + v], gv);
         L->vt.v[v].g = gv;
@@ -1023,7 +1028,7 @@ int launch_rectify_group(cc_ctx* ctx, const RectCall<PX>& c, int v0, int nv, con
         return CC_OK;
     std::vector<PlanKey> keys((size_t)nv);
     for (int v = 0; v < nv; ++v) {
-        const RectGeom g = make_geom(c.views.axs_mins + 2 * (v0 + v), fr.sz1, fr.sz2, fr.pitch, fr.frame_stride, nframes);
+        const RectGeom g = make_geom(c.views.axs_mins + 2 * (v0 + v), fr, nframes);
         keys[v] = plan_key(c.views.chs[v0 + v], c.views.ratios[v0 + v], g, kT, F::tl, F::pxb);
     }
     GroupPlan* mp = plan_get(ctx, keys.data(), nv, F::pxb);
@@ -1047,7 +1052,7 @@ int launch_rectify_group(cc_ctx* ctx, const RectCall<PX>& c, int v0, int nv, con
 struct RectViewsHost {
     cc_ctx* ctx;
     RectViews views;
-    RectFrames fr;                         // the layout of the slot buffers: frames pitch * sz2 apart
+    RectFrames fr;                         // the layout of the slot buffers: frames pitch * sz2 / out_pitch * out_sz2 apart
     int ngroups, pxb, tl;
     bool stage;                            // the layout can be staged at all
     std::vector<GroupPlan*> mp;            // per group: its plan, pinned until retired (nullptr: per-view launches)
@@ -1065,7 +1070,7 @@ static std::vector<PlanKey> group_keys(const RectViewsHost* h, int gi) {
     const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->views.n - v0);
     std::vector<PlanKey> keys((size_t)nv);
     for (int v = 0; v < nv; ++v) {
-        const RectGeom g = make_geom(h->views.axs_mins + 2 * (v0 + v), h->fr.sz1, h->fr.sz2, h->fr.pitch, 0, 0);
+        const RectGeom g = make_geom(h->views.axs_mins + 2 * (v0 + v), h->fr, 0);
         keys[v] = plan_key(h->views.chs[v0 + v], h->views.ratios[v0 + v], g, kT, h->tl, h->pxb);
     }
     return keys;
@@ -1122,7 +1127,7 @@ static int vh_install(RectViewsHost* h, int gi) {
     return CC_OK;
 }
 
-// dc: the call in the layout of the slot buffers (frames pitch * sz2 apart)
+// dc: the call in the layout of the slot buffers (frames pitch * sz2 / out_pitch * out_sz2 apart)
 template <typename PX>
 int rect_vh_begin(cc_ctx* ctx, const RectCall<PX>& dc, RectViewsHost** out) {
     using F = RectFmt<PX>;
@@ -1164,7 +1169,7 @@ template <typename PX>
 int rect_vh_launch(RectViewsHost* h, const RectCall<PX>& dc, int gi, int w0, int wn, const PX* src, PX* dst,
                    cudaStream_t st, bool* ok) {
     *ok = false;
-    if (!h->mp[gi]) return CC_OK;
+    if (!h->mp[gi] || !RectFmt<PX>::dst_ok(dst, dc.fr, wn)) return CC_OK;
     const int v0 = gi * kMaxViews, nv = std::min(kMaxViews, h->views.n - v0);
     ViewsLaunch L;
     int rc = views_window(h->ctx, h->mp[gi], dc, v0, nv, src, w0, wn, &L, ok);
@@ -1213,7 +1218,7 @@ int rectify_views_per_launch() { return kMaxViews; }
 template <typename T>
 int launch_rectify_map(cc_ctx* ctx, const ChainD& chd, double ratio, const int64_t axs_min[2], T* map_row, T* map_col,
                        int sz1, int sz2, size_t pitch, cudaStream_t st) {
-    const RectGeom g = make_geom(axs_min, sz1, sz2, pitch, pitch * (size_t)sz2, 1);
+    const RectGeom g = make_geom(axs_min, rect_frames(sz1, sz2, pitch, pitch * (size_t)sz2, 1), 1);
     const dim3 grid((sz1 + kT - 1) / kT, (sz2 + kT - 1) / kT);
     if constexpr (std::is_same_v<T, double>)
         rectify_map_kernel<<<grid, kConsumerThreads, 0, st>>>(make_exact(chd, ratio), g, map_row, map_col);

@@ -97,7 +97,7 @@ __device__ __forceinline__ void store_rgb(uint8_t* q, uint32_t rgb) {
     q[0] = (uint8_t)rgb; q[1] = (uint8_t)(rgb >> 8); q[2] = (uint8_t)(rgb >> 16);
 }
 
-// generic per-pixel path with every check and direct global taps
+// generic per-pixel path with every check and direct global taps (pitch3, frame_bytes: the source's)
 template <bool EXACT>
 __device__ __forceinline__ uint32_t sample_direct_u8(const RectExact& pe, const RectFast& pf,
                                                      const RowTermD& rtd, const RowTermF& rtf,
@@ -110,11 +110,11 @@ __device__ __forceinline__ uint32_t sample_direct_u8(const RectExact& pe, const 
     if (EXACT) {
         double row, col;
         rect_coord(pe, rtd, rect_q2(pe, g.axs1 + b), row, col);
-        if (!(lin_ok(row, g.sz1) & lin_ok(col, g.sz2))) return fill;
+        if (!(lin_ok(row, g.src_sz1) & lin_ok(col, g.src_sz2))) return fill;
         lin_floor(row, g1, d1d);
         lin_floor(col, g2, d2d);
-        lin_fix_edge(g.sz1, g1, d1d);
-        lin_fix_edge(g.sz2, g2, d2d);
+        lin_fix_edge(g.src_sz1, g1, d1d);
+        lin_fix_edge(g.src_sz2, g2, d2d);
         g1 -= 1; g2 -= 1;
     } else {
         float row, col;
@@ -123,7 +123,7 @@ __device__ __forceinline__ uint32_t sample_direct_u8(const RectExact& pe, const 
         lin_floor_fast(row, t1, d1f);
         lin_floor_fast(col, t2, d2f);
         g1 = t1 - (kMagicBits + 1); g2 = t2 - (kMagicBits + 1);
-        if (!(((unsigned)g1 <= (unsigned)(g.sz1 - 2)) & ((unsigned)g2 <= (unsigned)(g.sz2 - 2)))) return fill;
+        if (!(((unsigned)g1 <= (unsigned)(g.src_sz1 - 2)) & ((unsigned)g2 <= (unsigned)(g.src_sz2 - 2)))) return fill;
     }
     const unsigned off = (unsigned)g2 * pitch3 + (unsigned)g1 * 3u;
     Taps6 t0, t1;
@@ -157,8 +157,8 @@ rectify_u8c3_direct_kernel(const __grid_constant__ RectExact pe, const __grid_co
     const int a = blockIdx.x * kT + lane_id;
     if (a >= g.sz1) return;
     const int frame = blockIdx.z;
-    const uint8_t* sframe = src + (long long)frame * g.frame_stride * 3;
-    const unsigned pitch3 = (unsigned)g.pitch * 3u;
+    const uint8_t* sframe = src + (long long)frame * g.src_frame_stride * 3;
+    const unsigned spitch3 = (unsigned)g.src_pitch * 3u, pitch3 = (unsigned)g.pitch * 3u;
     const uint32_t fill = fill3.x | (fill3.y << 8) | (fill3.z << 16);
     RowTermD rtd;
     RowTermF rtf;
@@ -167,7 +167,7 @@ rectify_u8c3_direct_kernel(const __grid_constant__ RectExact pe, const __grid_co
     const int b_end = min(b_begin + lines_per_cta, g.sz2);
     uint8_t* o = dst + ((long long)frame * g.frame_stride + (long long)(b_begin + warp) * g.pitch + a) * 3;
     for (int b = b_begin + warp; b < b_end; b += kWarps, o += (long long)kWarps * pitch3)
-        store_rgb(o, sample_direct_u8<EXACT>(pe, pf, rtd, rtf, g, sframe, pitch3, frame_bytes, b, fill));
+        store_rgb(o, sample_direct_u8<EXACT>(pe, pf, rtd, rtf, g, sframe, spitch3, frame_bytes, b, fill));
 }
 
 // ---- staged kernel (persistent; scheduling and producer: rectify_ring.cuh) ------------------
@@ -336,7 +336,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
         return;
     }
 
-    // ---- consumer warps
+    // ---- consumer warps (pitch3: the output's; the taps of the hot path come from the box at its own pitch)
     const unsigned pitch3 = (unsigned)g.pitch * 3u;
     const uint32_t box_pitch_b = (uint32_t)cfg.pitch_b;       // bytes per box line (multiple of 128)
     const uint32_t stage0 = smem_u32(stage_mem);
@@ -415,7 +415,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                     if (e & 1) { w00[e / 2].y = v00; w10[e / 2].y = v10; w01[e / 2].y = v01; w11[e / 2].y = v11; }
                     else       { w00[e / 2].x = v00; w10[e / 2].x = v10; w01[e / 2].x = v01; w11[e / 2].x = v11; }
                     if (st) m_staged |= 1u << e;
-                    else if (!(lin_ok(row, g.sz1) & lin_ok(col, g.sz2))) m_fill |= 1u << e;   // rare: border tiles
+                    else if (!(lin_ok(row, g.src_sz1) & lin_ok(col, g.src_sz2))) m_fill |= 1u << e;   // rare: border tiles
                 }
             } else {
                 const RowTermF rtf = rect_row_term(pf, gv.axs0 + a_c);
@@ -448,7 +448,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                         if (st) m_staged |= 1u << e;
                         if (!VIEWS) {
                             // (unconditional: four FSETPs cost less than a divergent branch here; measured)
-                            const bool inframe = (rr[j] >= 1.0f) & (rr[j] < (float)g.sz1) & (cc_[j] >= 1.0f) & (cc_[j] < (float)g.sz2);
+                            const bool inframe = (rr[j] >= 1.0f) & (rr[j] < (float)g.src_sz1) & (cc_[j] >= 1.0f) & (cc_[j] < (float)g.src_sz2);
                             if (!inframe) m_fill |= 1u << e;
                         }
                     }
@@ -463,8 +463,8 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
                         float2 row, col;
                         rect_coord2(pf, rtf, ip, row, col);
                         ip = add2(ip, bc2(2.0f));
-                        if (!((row.x >= 1.0f) & (row.x < (float)g.sz1) & (col.x >= 1.0f) & (col.x < (float)g.sz2))) m_fill |= 1u << (2 * hh);
-                        if (!((row.y >= 1.0f) & (row.y < (float)g.sz1) & (col.y >= 1.0f) & (col.y < (float)g.sz2))) m_fill |= 1u << (2 * hh + 1);
+                        if (!((row.x >= 1.0f) & (row.x < (float)g.src_sz1) & (col.x >= 1.0f) & (col.x < (float)g.src_sz2))) m_fill |= 1u << (2 * hh);
+                        if (!((row.y >= 1.0f) & (row.y < (float)g.src_sz1) & (col.y >= 1.0f) & (col.y < (float)g.src_sz2))) m_fill |= 1u << (2 * hh + 1);
                     }
                 }
             }
@@ -474,7 +474,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
         }
 
         // ---- every frame of the unit: gather, blend, store
-        const uint8_t* sframe = src + (long long)frame_z * g.frame_stride * 3;
+        const uint8_t* sframe = src + (long long)frame_z * g.src_frame_stride * 3;
         // (a running output pointer, as in the f32c1 kernel, costs this one registers: ptxas goes from
         // 96 to 104 and the fast variant from 4 to 3 CTAs per SM -- measured 0.204 vs 0.194 ms on c3)
         uint8_t* oline = dst + (long long)frame_z * g.frame_stride * 3 + off0;
@@ -571,7 +571,7 @@ __device__ __forceinline__ void rectify_u8c3_body(const CUtensorMap& tmap, const
 #pragma unroll 1
                 for (int e = 0; e < LPW; ++e, og += pitch3)
                     if ((m_gen >> e) & 1u)
-                        store_rgb(og, sample_direct_u8<EXACT>(pe, pf, rtd, rtf, gv, sframe, pitch3, frame_bytes, b0 + e, fill));
+                        store_rgb(og, sample_direct_u8<EXACT>(pe, pf, rtd, rtf, gv, sframe, (unsigned)gv.src_pitch * 3u, frame_bytes, b0 + e, fill));
             }
         }
         __syncwarp();

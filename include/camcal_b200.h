@@ -203,7 +203,7 @@ int cc_world2img_f32_aos_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *v
 /* ---- full-frame rectification:  warp(img, tform, axs)  src/plot_calibration.jl:40
  *      with tform = real2image[i] o push(.,0) o inv(LinearMap(ratio*I)) (:17-18) and
  *      axs from get_axes (:1-6): output index (I1, I2) = axs_min + (a, b), same size
- *      as the input.  Bilinear, OnGrid, out-of-range -> fill.  `ratio` is pixels per
+ *      as the input (cc_rectify_axes_* below: any output size).  Bilinear, OnGrid, out-of-range -> fill.  `ratio` is pixels per
  *      world unit (get_ratio, :8-13).  flags = CC_COORD_* | CC_GATHER_*.
  *      All `nframes` frames share the view: the map is computed once per tile and group of
  *      frames, so batches rectify faster per frame than single-frame calls.  The first call
@@ -262,6 +262,52 @@ int cc_rectify_views_u8c3_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *
                                const double *ratios, const int64_t *axs_mins, const uint8_t *src,
                                uint8_t *dst, int sz1, int sz2, size_t pitch, size_t frame_stride,
                                int frames_per_view, const uint8_t fill[3], unsigned flags);
+/* Rectification into output axes of any size: warp(img, tform, axs) with axs any two index ranges
+ * (downscale, crop, upscale), one view or many.
+ *  - Output layout: pixel (a+1, b+1) of output frame f, 0 <= a < out_sz1, 0 <= b < out_sz2, is
+ *    stored at dst + f*out_frame_stride + b*out_pitch + a (u8c3: times 3 bytes).
+ *  - It holds warp(img_f, tform_v, (axs_mins[2v] .+ (0:out_sz1-1), axs_mins[2v+1] .+ (0:out_sz2-1)))
+ *    at that index: the world point ((axs_min[0]+a)/ratio, (axs_min[1]+b)/ratio, 0), the scale
+ *    convention of cc_rectify_*.
+ *  - Source frames: sz1 x sz2 pixels, lines `pitch` and frames `frame_stride` pixels apart, as for
+ *    cc_rectify_*.
+ *  - Views: frames [v*frames_per_view, (v+1)*frames_per_view) of src and of dst use views[v],
+ *    ratios[v] and axs_mins[2v .. 2v+1]; all views share the output extent.
+ *  - nviews == 1 takes the path of cc_rectify_f32c1 / _u8c3 (the _host forms: of their _host forms);
+ *    nviews > 1 the path of cc_rectify_*_views / cc_rectify_views_*_host: groups of up to 64 views per
+ *    staged launch, one launch per view where a group cannot be staged.  flags as for cc_rectify_*.
+ *  - When the output extent, pitch and frame stride equal the source's, the output is byte-identical
+ *    to that entry point's and the call makes the same number of launches.
+ *  - CC_COORD_F64: a pixel's value does not depend on the output window that contains it (a crop of a
+ *    larger call equals that call's window bit for bit).  CC_COORD_F32: the kernels sample the map
+ *    cc_rectify_map_f32 returns for the same (ratio, axs_min, out_sz1, out_sz2), with its accuracy.
+ *  - CC_ERR_INVALID_ARG, nothing written and nothing enqueued: out_sz1 or out_sz2 outside (0, 2^22),
+ *    out_pitch < out_sz1, overlapping output frames (more than one frame), out_pitch*out_sz2 >= 2^30,
+ *    and every rule of cc_rectify_* on the source, src != dst included.
+ *  - The _host forms take host memory and return when dst holds the result; host padding between
+ *    output lines and frames is never written. */
+int cc_rectify_axes_f32c1(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                          const double *ratios, const int64_t *axs_mins, int out_sz1, int out_sz2,
+                          const float *src, int sz1, int sz2, size_t pitch, size_t frame_stride,
+                          float *dst, size_t out_pitch, size_t out_frame_stride,
+                          int frames_per_view, float fill, unsigned flags, void *stream);
+int cc_rectify_axes_u8c3(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                         const double *ratios, const int64_t *axs_mins, int out_sz1, int out_sz2,
+                         const uint8_t *src, int sz1, int sz2, size_t pitch, size_t frame_stride,
+                         uint8_t *dst, size_t out_pitch, size_t out_frame_stride,
+                         int frames_per_view, const uint8_t fill[3], unsigned flags, void *stream);
+int cc_rectify_axes_f32c1_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                               const double *ratios, const int64_t *axs_mins, int out_sz1,
+                               int out_sz2, const float *src, int sz1, int sz2, size_t pitch,
+                               size_t frame_stride, float *dst, size_t out_pitch,
+                               size_t out_frame_stride, int frames_per_view, float fill,
+                               unsigned flags);
+int cc_rectify_axes_u8c3_host(cc_ctx *ctx, const cc_intr *intr, const cc_view *views, int nviews,
+                              const double *ratios, const int64_t *axs_mins, int out_sz1,
+                              int out_sz2, const uint8_t *src, int sz1, int sz2, size_t pitch,
+                              size_t frame_stride, uint8_t *dst, size_t out_pitch,
+                              size_t out_frame_stride, int frames_per_view,
+                              const uint8_t fill[3], unsigned flags);
 /* the map alone (source row/col sampled by each output pixel), FP64, frame layout */
 int cc_rectify_map_f64(cc_ctx *ctx, const cc_intr *intr, const cc_view *view, double ratio,
                        const int64_t axs_min[2], double *map_row, double *map_col, int sz1,

@@ -293,6 +293,77 @@ function warp_views(d::DeviceCalibration, imgs::Array{UInt8,4}, ratios::Vector{F
     out
 end
 
+# Output axes of any size, as warp(img, tform, axs) takes them: the result has size (length.(axs)..., n) and
+# element (a, b) holds output index (axs[1][a], axs[2][b]) -- a downscale, a crop or an upscale of the frames.
+# Axes of the input's own size (get_axes) give what the methods above give.  cc_rectify_axes_*_host.
+function warp_batch(c::Calibration, i::Int, imgs::Array{Float32,3}, ratio::Float64,
+                    axs::NTuple{2,UnitRange{Int}}; fill::Float32 = NaN32, fast::Bool = false)
+    sz1, sz2, nf = size(imgs)
+    o1, o2 = length.(axs)
+    out = Array{Float32,3}(undef, o1, o2, nf)
+    axs_min = Int64[first(axs[1]), first(axs[2])]
+    check(ccall((:cc_rectify_axes_f32c1_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ref{CcView}, Cint, Ref{Cdouble}, Ptr{Int64}, Cint, Cint, Ptr{Cfloat},
+                 Cint, Cint, Csize_t, Csize_t, Ptr{Cfloat}, Csize_t, Csize_t, Cint, Cfloat, Cuint),
+                context().handle, Ref(CcIntr(c)), Ref(CcView(c, i)), 1, Ref(ratio), axs_min, o1, o2, imgs,
+                sz1, sz2, sz1, sz1 * sz2, out, o1, o1 * o2, nf, fill, fast ? 1 : 0))
+    out
+end
+
+function warp_batch(c::Calibration, i::Int, imgs::Array{UInt8,4}, ratio::Float64,
+                    axs::NTuple{2,UnitRange{Int}}; fill::NTuple{3,UInt8} = (0x00, 0x00, 0x00),
+                    fast::Bool = false)
+    @assert size(imgs, 1) == 3
+    _, sz1, sz2, nf = size(imgs)
+    o1, o2 = length.(axs)
+    out = Array{UInt8,4}(undef, 3, o1, o2, nf)
+    axs_min = Int64[first(axs[1]), first(axs[2])]
+    check(ccall((:cc_rectify_axes_u8c3_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ref{CcView}, Cint, Ref{Cdouble}, Ptr{Int64}, Cint, Cint, Ptr{UInt8},
+                 Cint, Cint, Csize_t, Csize_t, Ptr{UInt8}, Csize_t, Csize_t, Cint, Ptr{UInt8}, Cuint),
+                context().handle, Ref(CcIntr(c)), Ref(CcView(c, i)), 1, Ref(ratio), axs_min, o1, o2, imgs,
+                sz1, sz2, sz1, sz1 * sz2, out, o1, o1 * o2, nf, UInt8[fill...], fast ? 1 : 0))
+    out
+end
+
+# The plot loop into output axes of any size: every view's axes have the same lengths, the result has size
+# (length.(axss[1])..., n).  cc_rectify_axes_*_host.
+function warp_views(d::DeviceCalibration, imgs::Array{Float32,3}, ratios::Vector{Float64},
+                    axss::Vector{NTuple{2,UnitRange{Int}}}; fill::Float32 = NaN32, fast::Bool = false)
+    sz1, sz2, nf = size(imgs)
+    nv = length(d.views)
+    @assert nv > 0 && nf % nv == 0 && nv == length(ratios) == length(axss)
+    o1, o2 = length.(axss[1])
+    @assert all(a -> length.(a) == (o1, o2), axss)
+    out = Array{Float32,3}(undef, o1, o2, nf)
+    axs_mins = Int64[first(a[j]) for a in axss for j in 1:2]
+    check(ccall((:cc_rectify_axes_f32c1_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Cdouble}, Ptr{Int64}, Cint, Cint, Ptr{Cfloat},
+                 Cint, Cint, Csize_t, Csize_t, Ptr{Cfloat}, Csize_t, Csize_t, Cint, Cfloat, Cuint),
+                context().handle, Ref(d.intr), d.views, nv, ratios, axs_mins, o1, o2, imgs,
+                sz1, sz2, sz1, sz1 * sz2, out, o1, o1 * o2, nf ÷ nv, fill, fast ? 1 : 0))
+    out
+end
+
+function warp_views(d::DeviceCalibration, imgs::Array{UInt8,4}, ratios::Vector{Float64},
+                    axss::Vector{NTuple{2,UnitRange{Int}}}; fill::NTuple{3,UInt8} = (0x00, 0x00, 0x00),
+                    fast::Bool = false)
+    @assert size(imgs, 1) == 3
+    _, sz1, sz2, nf = size(imgs)
+    nv = length(d.views)
+    @assert nv > 0 && nf % nv == 0 && nv == length(ratios) == length(axss)
+    o1, o2 = length.(axss[1])
+    @assert all(a -> length.(a) == (o1, o2), axss)
+    out = Array{UInt8,4}(undef, 3, o1, o2, nf)
+    axs_mins = Int64[first(a[j]) for a in axss for j in 1:2]
+    check(ccall((:cc_rectify_axes_u8c3_host, libcamcal), Cint,
+                (Ptr{Cvoid}, Ref{CcIntr}, Ptr{CcView}, Cint, Ptr{Cdouble}, Ptr{Int64}, Cint, Cint, Ptr{UInt8},
+                 Cint, Cint, Csize_t, Csize_t, Ptr{UInt8}, Csize_t, Csize_t, Cint, Ptr{UInt8}, Cuint),
+                context().handle, Ref(d.intr), d.views, nv, ratios, axs_mins, o1, o2, imgs,
+                sz1, sz2, sz1, sz1 * sz2, out, o1, o1 * o2, nf ÷ nv, UInt8[fill...], fast ? 1 : 0))
+    out
+end
+
 # ---- image ingest on the device: RGB.(FileIO.load(file)) for JPEG files, src/plot_calibration.jl:37 --
 # The compressed bytes go to the GPU (nvJPEG + a transposition kernel inside the library); the result is a
 # DEVICE pointer to (3, sz1, sz2, n) bytes -- the u8c3 layout cc_rectify_u8c3[_views] take -- so a plot loop
